@@ -7,9 +7,11 @@ per positive, loss 1 - sigmoid (reference BPRModel.py:144), exact Keras Adam(1e-
 A "step" is one batch: fused gather + loss + scatter-add kernel, then the fused Adam pass.
 Metric: training interactions (triplets) per second.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is produced.
+--dump-outputs DIR writes what the last timed step returned (its mean loss and the user / item tables it updated) as
+DIR/<name>.npy, float32; the inputs are seeded, so two builds run with the same arguments can be compared array by array.
 
 Beside the headline the line carries, each with its own `roofline` block:
   neumf            BASELINE.json configs[0] (NeuMF, ML-1M shape, batch 16 384): the reference class graph (numFactor 32,
@@ -316,6 +318,9 @@ def product_arm(args):
     step_ms = np.array([e[0].elapsed_time(e[2]) for e in evs])
     fb_ms = np.array([e[0].elapsed_time(e[1]) for e in evs])
     total_ms = float(step_ms.sum())
+    if args.dump_outputs and rank == 0:
+        # taken here: the legs below keep training the same tables
+        dump_outputs(args.dump_outputs, {"loss": loss_buf, "user_embedding": net.user.w, "item_embedding": net.item.w})
 
     # ---- (2) same steps back to back (tables stay in L2, as in the real training loop) -----------
     order = [(k * world + rank) % n_batches for k in range(K)]
@@ -519,6 +524,13 @@ def product_arm(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor as out_dir/<name>.npy in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def extras_cpu_baselines(budget_s=2.5):
@@ -1017,7 +1029,10 @@ def main():
     ap.add_argument("--impl", default="brk", choices=["brk", "reference", "cpu_legs"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "brk":
+        ap.error("--dump-outputs applies to --impl brk")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         reference_arm(args)

@@ -150,6 +150,34 @@ def test_bpr_twenty_bench_identical_steps_match_the_oracle(dev):
     np.testing.assert_allclose(net.item.w.cpu().numpy(), orc.item, rtol=1e-4, atol=2e-5)
 
 
+def test_bench_dump_outputs_hold_the_last_timed_step(dev, tmp_path):
+    """bench.py --steps K --warmup W --dump-outputs DIR: K timed steps, and the dumped loss and tables are those after the
+    W + K steps over batches 0 .. W + K - 1 of the bench frame, against oracle/bpr.py (tolerances of the test above)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from binrec_b200 import synth
+    from oracle import bpr as OB, philox as OP
+    W, K = 3, 2
+    bench = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    r = subprocess.run([sys.executable, bench, "--steps", str(K), "--warmup", str(W), "--no-extras", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == K
+    got = {n: np.load(tmp_path / f"{n}.npy") for n in ("loss", "user_embedding", "item_embedding")}
+    assert all(a.dtype == np.float32 for a in got.values())
+    users, items = synth.make_interactions()
+    U, I, d, B = synth.ML1M_USERS, synth.ML1M_ITEMS, 64, 16384
+    orc = OB.BPROracle(U, I, d, seed=42)
+    indptr, sitems = OP.build_csr(users, items, U)
+    neg = OP.bpr_negatives(users[:(W + K) * B], 7, 0, I, indptr, sitems)
+    ref = [orc.step(users[b * B:(b + 1) * B], items[b * B:(b + 1) * B], neg[b * B:(b + 1) * B]) for b in range(W + K)]
+    np.testing.assert_allclose(got["loss"], np.float32(ref[-1]).reshape(1), rtol=1e-5)
+    np.testing.assert_allclose(got["user_embedding"], orc.user, rtol=1e-4, atol=2e-5)
+    np.testing.assert_allclose(got["item_embedding"], orc.item, rtol=1e-4, atol=2e-5)
+
+
 def test_twotower_three_steps_at_baseline_shape_match_the_oracle(dev):
     """BASELINE.json configs[2] shape: 6040 x 3706, E = S = 128, in-batch softmax batch 1000, Adagrad 0.1 -- three fp32 steps."""
     from binrec_b200.twoTower import TwoTowerModel
