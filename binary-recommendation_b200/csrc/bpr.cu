@@ -257,10 +257,17 @@ struct BprCoopParams {
   int64_t arena_n4;
   int32_t rank, world;
   float inv_global;               // 1 / (world * batch): gradient scale of the global mean loss
-  unsigned long long* dbg;        // optional [n_steps][8] globaltimer stamps of block 0 (BRK_COOP_TRACE)
+  // optional [n_steps][8] globaltimer stamps of block 0 (BRK_COOP_TRACE).  world == 1: 0 step start, 2 phase 1 done,
+  // 1 gradient barrier passed, 3 Adam done, 6 trailing barrier passed (= 3 when skipped); step 0 also holds 7 kernel entry
+  // and, in word 4, 1 if the Adam ran from shared memory (0: global memory).  world > 1: see profiles/dp_trace.py.
+  unsigned long long* dbg;
   long long spin_budget;          // clock64 budget of one cross-GPU wait (default ~30 s; BRK_PEER_SPIN_MS)
   int32_t prefetch;               // bulk L2 prefetch of the table state at kernel entry (BRK_BPR_NO_PREFETCH=1 turns it off)
   unsigned int* bar;              // grid-barrier words {count, error, base} (null: cg::grid.sync, BRK_BPR_CG_SYNC=1)
+  // Adam operands in shared memory (world == 1): CTA b owns float4 [b * slice4[k], (b + 1) * slice4[k]) of table k's
+  // w / m / v / g; 0 = Adam straight from global memory (slices too large, or BRK_BPR_NO_SMEM_ADAM=1)
+  int32_t slice4[2];
+  int32_t last_sync;              // 1: grid barrier after the launch's last step too (only BRK_BPR_NO_SMEM_ADAM=1 keeps it)
 };
 
 __device__ __forceinline__ void coop_st_release_sys(uint32_t* p, uint32_t v) {
@@ -306,6 +313,13 @@ __device__ __forceinline__ void bpr_stage_step(const BprCoopParams& P, const Bpr
 }
 
 constexpr int kStageThreads = 64;   // threads per CTA that stage the next step during the Adam phase
+
+__device__ __forceinline__ bool coop_mbar_try_wait(uint32_t bar, uint32_t parity) {
+  uint32_t ok;
+  asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
+               : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
+  return ok != 0;
+}
 
 template <int LPR, int NCH>
 __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParams P) {
@@ -355,36 +369,66 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
   const int d4 = P.user.d >> 2;
   const int lane_in = threadIdx.x & (LPR - 1);
   const int sub = (threadIdx.x & 31) / LPR;
-  const int64_t group = (int64_t(blockIdx.x) * kThreads + threadIdx.x) / LPR;
-  const int64_t n_groups = int64_t(gridDim.x) * kThreads / LPR;
-  const int64_t warp_first = group - sub;
-  const int64_t tid = int64_t(blockIdx.x) * kThreads + threadIdx.x, nthr = int64_t(gridDim.x) * kThreads;
+  // 32-bit thread and group indices (a cooperative grid is a few hundred CTAs): the kernel runs at its 64-register bound
+  const int group = int(blockIdx.x * kThreads + threadIdx.x) / LPR;
+  const int n_groups = int(gridDim.x) * kThreads / LPR;
+  const int warp_first = group - sub;
+  const int tid = int(blockIdx.x * kThreads + threadIdx.x), nthr = int(gridDim.x) * kThreads;
   // no __restrict__/read-only path here: phase 2 of this same kernel rewrites the tables, so rows are
   // read with ld.global.cg (L2 only) -- another SM's L1 could otherwise hold a stale line across steps
   const float4* Wu4 = reinterpret_cast<const float4*>(P.user.w);
   const float4* Wi4 = reinterpret_cast<const float4*>(P.item.w);
   const double* pw = reinterpret_cast<const double*>(P.state);
-  double p1 = pw[1], p2 = pw[2];                       // running beta powers, advanced per step in registers
+  // Running beta powers, advanced once per step: step s reads pair s & 1 and thread 0 writes pair (s + 1) & 1, which no
+  // thread reads again before the next __syncthreads.  Shared rather than registers: the kernel runs at its register bound.
+  __shared__ double beta_pow[2][2];
+  if (threadIdx.x == 0) { beta_pow[0][0] = pw[1]; beta_pow[0][1] = pw[2]; }
   const brk_table tabs[2] = {P.user, P.item};
 
   // The whole optimizer state is asked into L2 up front with BULK prefetches (one instruction per CTA and array slice,
   // streamed by the copy engine of the SM): when other work has evicted the 10 MB since the last launch -- bench.py's
   // flushed-L2 measurement is exactly that -- phase 2 of the first step otherwise starts on cold m / v / g lines.
   // (Per-line prefetch.global.L2, 80 k requests, cost more than it hid: section 4.3 of DESIGN.md.)
-  if (P.prefetch && threadIdx.x == 0) {
+  // With the shared-memory Adam (P.slice4) the CTA's slices of w, m and v are instead bulk-copied into its shared memory
+  // (the same one instruction per array slice, completing on `adam_bar`): they stream in while phase 1 runs, phase 1 only
+  // reads w from global memory and never m or v, and the first Adam phase waits for them.  g keeps its L2 prefetch.
+  // Shared layout: [w | m | v], each nA float4 = this CTA's user slice followed by its item slice.
+  extern __shared__ float4 adam_smem[];
+  __shared__ __align__(8) uint64_t adam_bar;
+  const bool smem_adam = P.slice4[0] > 0;
+  coop_stamp(P, 0, 7);
+  if (P.dbg && P.world == 1 && blockIdx.x == 0 && threadIdx.x == 0) P.dbg[4] = smem_adam ? 1u : 0u;   // which Adam ran
+  if (threadIdx.x == 0) {
+    const uint32_t bar = uint32_t(__cvta_generic_to_shared(&adam_bar));
+    if (smem_adam) {
+      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar) : "memory");
+      asm volatile("fence.mbarrier_init.release.cluster;\n\tfence.proxy.async.shared::cta;" ::: "memory");
+    }
+    uint32_t nb[2], tx = 0;
+    int64_t offs[2];
+#pragma unroll
     for (int k = 0; k < 2; ++k) {
       const int64_t bytes = tabs[k].rows * tabs[k].d * 4;
-      int64_t per = (bytes + gridDim.x - 1) / gridDim.x;
+      int64_t per = smem_adam ? int64_t(P.slice4[k]) * 16 : (bytes + gridDim.x - 1) / gridDim.x;
       per = (per + 15) & ~int64_t(15);
-      const int64_t off = int64_t(blockIdx.x) * per;
-      if (off < bytes) {
-        const uint32_t n = uint32_t(((off + per <= bytes ? per : bytes - off)) & ~int64_t(15));
-        if (n) {
-          const float* arrs[4] = {tabs[k].w, tabs[k].g, P.world > 1 ? nullptr : tabs[k].m, P.world > 1 ? nullptr : tabs[k].v};
+      offs[k] = int64_t(blockIdx.x) * per;
+      nb[k] = offs[k] < bytes ? uint32_t((offs[k] + per <= bytes ? per : bytes - offs[k]) & ~int64_t(15)) : 0u;
+      tx += nb[k];
+    }
+    if (smem_adam) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(3 * tx) : "memory");
 #pragma unroll
-          for (int a = 0; a < 4; ++a)
-            if (arrs[a] != nullptr && brk_aligned16(arrs[a]))
-              asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char*>(arrs[a]) + off), "r"(n) : "memory");
+    for (int k = 0; k < 2; ++k) {
+      if (nb[k] == 0) continue;
+      const float* arrs[4] = {tabs[k].g, tabs[k].w, P.world > 1 ? nullptr : tabs[k].m, P.world > 1 ? nullptr : tabs[k].v};
+#pragma unroll
+      for (int a = 0; a < 4; ++a) {
+        const char* src = reinterpret_cast<const char*>(arrs[a]) + offs[k];
+        if (smem_adam && a > 0) {
+          const uint32_t dst = uint32_t(__cvta_generic_to_shared(adam_smem)) + (a - 1) * tx + (k ? nb[0] : 0u);
+          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                       ::"r"(dst), "l"(src), "r"(nb[k]), "r"(bar) : "memory");
+        } else if (P.prefetch && arrs[a] != nullptr && brk_aligned16(arrs[a])) {
+          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(nb[k]) : "memory");
         }
       }
     }
@@ -403,8 +447,8 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
     else { uid = P.u + sd.off; pid = P.p + sd.off; nid = P.n + sd.off; }
     // ---- phase 1: fused gather + loss + gradient REDs (same math as bpr_vec) ----
     float loss_local = 0.f;
-    for (int64_t wb = warp_first; wb < batch; wb += n_groups) {
-      const int64_t b = wb + sub;
+    for (int wb = warp_first; wb < batch; wb += n_groups) {
+      const int b = wb + sub;
       const bool valid = b < batch;
       int64_t ru = 0, rp = 0, rn = 0;
       if (valid) { ru = __ldcg(uid + b); rp = __ldcg(pid + b); rn = __ldcg(nid + b); }
@@ -444,21 +488,61 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
     }
     const double part = block_sum_double(double(loss_local), red);
     if (threadIdx.x == 0) atomicAdd(P.loss_acc + (s & 1), part);
-    if (P.world > 1) gcollect(); else gsync();
+    if (P.world > 1) {
+      gcollect();
+    } else {
+      coop_stamp(P, s, 2);                              // phase 1 done in block 0
+      gsync();
+    }
     coop_stamp(P, s, 1);
     // ---- phase 2: exact Keras Adam over every element of both tables; zero the accumulators.  In sampling
     //      mode the first two warps of each CTA stage step s+1 instead (ids + negatives) ----
-    p1 *= double(P.h.beta1); p2 *= double(P.h.beta2);
+    const double p1 = beta_pow[s & 1][0] * double(P.h.beta1), p2 = beta_pow[s & 1][1] * double(P.h.beta2);
+    if (threadIdx.x == 0) { beta_pow[(s + 1) & 1][0] = p1; beta_pow[(s + 1) & 1][1] = p2; }
     const float alpha = float(double(P.h.lr) * sqrt(1.0 - p2) / (1.0 - p1));
     const bool staging = sample && s + 1 < P.n_steps;
     const bool stager = staging && threadIdx.x < kStageThreads;
-    const int64_t atid = staging ? int64_t(blockIdx.x) * (kThreads - kStageThreads) + (threadIdx.x - kStageThreads) : tid;
-    const int64_t anthr = staging ? int64_t(gridDim.x) * (kThreads - kStageThreads) : nthr;
+    const int atid = staging ? int(blockIdx.x) * (kThreads - kStageThreads) + (int(threadIdx.x) - kStageThreads) : tid;
+    const int anthr = staging ? int(gridDim.x) * (kThreads - kStageThreads) : nthr;
     if (stager) {
       bpr_stage_step(P, P.use_inline ? P.inline_steps[s + 1] : P.steps[s + 1], (s + 1) & 1,
                      int64_t(blockIdx.x) * kStageThreads + threadIdx.x, int64_t(gridDim.x) * kStageThreads);
     }
-    if (P.world == 1) {
+    if (P.world == 1 && smem_adam) {
+      // This CTA's slices only: w, m, v from shared memory (the entry copies, then what the previous step left there),
+      // g from L2 where the REDs landed; the new w goes to global memory for the next step's gathers and to shared
+      // memory, m and v stay on chip until the end of the launch.
+      if (s == 0) {
+        const uint32_t bar = uint32_t(__cvta_generic_to_shared(&adam_bar));
+        while (!coop_mbar_try_wait(bar, 0)) {}
+      }
+      if (!stager) {
+        int64_t o4[2];
+        int n4[2];
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+          const int64_t tot = tabs[k].rows * tabs[k].d / 4;
+          o4[k] = int64_t(blockIdx.x) * P.slice4[k];
+          n4[k] = o4[k] < tot ? int(tot - o4[k] < P.slice4[k] ? tot - o4[k] : P.slice4[k]) : 0;
+        }
+        const int nA = n4[0] + n4[1];
+        float4* sw = adam_smem; float4* sm = sw + nA; float4* sv = sm + nA;
+        const int t0 = staging ? int(threadIdx.x) - kStageThreads : int(threadIdx.x);
+        const int T = staging ? kThreads - kStageThreads : kThreads;
+        // One element at a time.  Issuing a thread's two g loads before either update (a CTA owns 265 float4 for 256
+        // threads at the bench shape) fits the 64 registers only with per-step recomputation elsewhere, and measured
+        // slower: Adam phase 2.1 -> 2.8 us, 600-step hot launch 1.45 -> 1.38 G interactions/s (DESIGN.md 7.1).
+        for (int j = t0; j < nA; j += T) {
+          const bool u = j < n4[0];
+          float4* w4 = reinterpret_cast<float4*>(u ? P.user.w : P.item.w) + (u ? o4[0] + j : o4[1] + (j - n4[0]));
+          float4* g4 = reinterpret_cast<float4*>(u ? P.user.g : P.item.g) + (u ? o4[0] + j : o4[1] + (j - n4[0]));
+          float4 w = sw[j], m = sm[j], v = sv[j];
+          adam4(w, m, v, __ldcg(g4), alpha, P.h.beta1, P.h.beta2, P.h.eps);
+          sw[j] = w; sm[j] = m; sv[j] = v;
+          *w4 = w; *g4 = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+      }
+    } else if (P.world == 1) {
       if (!stager) {
 #pragma unroll
         for (int k = 0; k < 2; ++k) {
@@ -539,13 +623,42 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
       if (P.losses) P.losses[s] = float(P.loss_acc[s & 1] / double(batch));
       P.loss_acc[s & 1] = 0.0;
     }
-    gsync();
+    if (P.world == 1) coop_stamp(P, s, 3);              // Adam done in block 0
+    // The barrier orders this step's Adam stores before the next step's gathers.  After the last step kernel completion
+    // does that for whatever follows on the stream, so a single-GPU launch ends without it: the barrier counter then gets
+    // one arrival round fewer, and bar_target (written to bar[2] below) counts exactly the rounds that ran.
+    if (P.world > 1 || s + 1 < P.n_steps || P.last_sync) gsync();
     coop_stamp(P, s, 6);
     if (P.world > 1 && *reinterpret_cast<volatile uint32_t*>(P.dp_sync + 4) != 0u) break;   // aborted (uniform after the barrier)
   }
+  if (smem_adam) {                                      // m and v back to global memory, one bulk store per array slice
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // this thread's shared stores -> visible to the copies
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      uint32_t nb[2];
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        const int64_t bytes = tabs[k].rows * tabs[k].d * 4, off = int64_t(blockIdx.x) * P.slice4[k] * 16;
+        nb[k] = off < bytes ? uint32_t(bytes - off < int64_t(P.slice4[k]) * 16 ? bytes - off : int64_t(P.slice4[k]) * 16) : 0u;
+      }
+      const uint32_t base = uint32_t(__cvta_generic_to_shared(adam_smem)), tx = nb[0] + nb[1];
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        if (nb[k] == 0) continue;
+        const int64_t off = int64_t(blockIdx.x) * P.slice4[k] * 16;
+        float* dsts[2] = {tabs[k].m, tabs[k].v};
+#pragma unroll
+        for (int a = 0; a < 2; ++a)
+          asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
+                       ::"l"(reinterpret_cast<char*>(dsts[a]) + off), "r"(base + (a + 1) * tx + (k ? nb[0] : 0u)), "r"(nb[k])
+                       : "memory");
+      }
+      asm volatile("cp.async.bulk.commit_group;\n\tcp.async.bulk.wait_group 0;" ::: "memory");
+    }
+  }
   if (tid == 0 && !(P.world > 1 && *reinterpret_cast<volatile uint32_t*>(P.dp_sync + 4) != 0u)) {
     double* pwo = reinterpret_cast<double*>(P.state);
-    P.state[0] += P.n_steps; pwo[1] = p1; pwo[2] = p2;
+    P.state[0] += P.n_steps; pwo[1] = beta_pow[P.n_steps & 1][0]; pwo[2] = beta_pow[P.n_steps & 1][1];
     if (P.world > 1) P.dp_sync[3] += uint32_t(P.n_steps);
     if (P.bar) P.bar[2] = bar_target;
   }
@@ -702,18 +815,41 @@ static int launch_coop_steps(brk_ctx* ctx, const brk_table* user, const brk_tabl
     case 16: fn = (void*)bpr_steps_coop<16, 1>; slot = 4; break;
     default: fn = (void*)bpr_steps_coop<32, 1>; slot = 5; break;
   }
-  static int per_sm_cache[6] = {0, 0, 0, 0, 0, 0};      // occupancy is a property of the kernel: query once
+  // Occupancy is a property of the kernel: queried once per instance.  `per_sm` CTAs of it fit an SM without dynamic shared
+  // memory, and `smem_cap` is the dynamic shared memory a CTA may take while still `per_sm` of them fit: the shared-memory
+  // Adam is only used within that budget, so it never shrinks the grid.
+  static int per_sm_cache[6] = {0, 0, 0, 0, 0, 0};
+  static size_t smem_cap_cache[6] = {0, 0, 0, 0, 0, 0};
   int per_sm = per_sm_cache[slot];
   if (per_sm == 0) {
     BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kThreads, 0));
     BRK_REQUIRE(per_sm > 0, BRK_E_STATE, "brk_bpr_train_steps: cooperative kernel does not fit");
+    size_t cap_bytes = 0;
+    BRK_CUDA(cudaOccupancyAvailableDynamicSMemPerBlock(&cap_bytes, fn, per_sm, kThreads));
     per_sm_cache[slot] = per_sm;
+    smem_cap_cache[slot] = cap_bytes;
   }
   int64_t want = (max_count * lpr + kThreads - 1) / kThreads;
   const int64_t cap = int64_t(per_sm) * ctx->sm_count;
   const int grid = int(want < cap ? (want < 1 ? 1 : want) : cap);
+  // CTA slices of the tables (the same cut as the bulk L2 prefetch): w, m and v of both take 3 * (slice_u + slice_i) float4
+  size_t smem = 0;
+  const brk_table* tabs[2] = {user, item};
+  for (int k = 0; k < 2; ++k) {
+    const int64_t n4 = tabs[k]->rows * d / 4;
+    const int64_t s4 = (n4 + grid - 1) / grid;
+    P.slice4[k] = int32_t(s4 < (int64_t(1) << 20) ? s4 : 0);
+    smem += 3 * size_t(s4) * 16;
+  }
+  const bool smem_ok = P.world == 1 && !getenv("BRK_BPR_NO_SMEM_ADAM") && smem <= smem_cap_cache[slot] &&
+                       P.slice4[0] > 0 && P.slice4[1] > 0 && brk_aligned16(user->m) && brk_aligned16(user->v) &&
+                       brk_aligned16(item->m) && brk_aligned16(item->v);
+  if (!smem_ok) { P.slice4[0] = P.slice4[1] = 0; smem = 0; }
+  P.last_sync = getenv("BRK_BPR_NO_SMEM_ADAM") ? 1 : 0;
+  // above the default 48 KB a kernel needs the opt-in attribute, which is per device: set it for the current one
+  if (smem > 48 * 1024) BRK_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   void* args[] = {(void*)&P};
-  BRK_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, 0, st));
+  BRK_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, st));
   return 0;
 }
 
