@@ -5,7 +5,6 @@
 // Mapping: a group of LPR lanes owns a triplet, each lane holds NCH float4 chunks of u, p and n in
 // registers; the dot product is a group shuffle-reduction; gradients leave as 16-byte vector REDs.
 #include "neumf_common.cuh"      // TabRef / locate / mark_row: row-sharded table addressing
-#include <cooperative_groups.h>
 #include <stdlib.h>
 #include <vector>
 
@@ -218,7 +217,7 @@ bpr_scalar(const float* __restrict__ Wu, const float* __restrict__ Wi, float* __
 }
 
 // ---- whole training steps in ONE cooperative kernel ------------------------------------------------
-// K steps x (fused fwd/bwd -> grid.sync -> exact Keras Adam over both tables -> grid.sync): no kernel
+// K steps x (fused fwd/bwd -> grid barrier -> exact Keras Adam over both tables -> grid barrier): no kernel
 // launch and no host involvement between steps; both phases are single-wave and latency-bound, so the
 // launch gaps and cold starts between separate kernels were ~40 % of the step.
 // Sampling mode (P.n == nullptr): the kernel draws its own Philox negatives.  Two warps of every CTA
@@ -263,7 +262,7 @@ struct BprCoopParams {
   unsigned long long* dbg;
   long long spin_budget;          // clock64 budget of one cross-GPU wait (default ~30 s; BRK_PEER_SPIN_MS)
   int32_t prefetch;               // bulk L2 prefetch of the table state at kernel entry (BRK_BPR_NO_PREFETCH=1 turns it off)
-  unsigned int* bar;              // grid-barrier words {count, error, base} (null: cg::grid.sync, BRK_BPR_CG_SYNC=1)
+  unsigned int* bar;              // grid-barrier words {count, error, base} (common.cuh)
   // Adam operands in shared memory (world == 1): CTA b owns float4 [b * slice4[k], (b + 1) * slice4[k]) of table k's
   // w / m / v / g; 0 = Adam straight from global memory (slices too large, or BRK_BPR_NO_SMEM_ADAM=1)
   int32_t slice4[2];
@@ -323,46 +322,17 @@ __device__ __forceinline__ bool coop_mbar_try_wait(uint32_t bar, uint32_t parity
 
 template <int LPR, int NCH>
 __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParams P) {
-  namespace cg = cooperative_groups;
-  cg::grid_group grid = cg::this_grid();
-  // Grid barrier: one release-RED on a monotonically increasing counter + an acquire spin by thread 0 (the base of this
-  // launch lives in device memory: bar[2]); cg::grid.sync() measured 0.3-0.5 us more per barrier (neumf_fused.cu).
-  unsigned int bar_target = P.bar ? *reinterpret_cast<volatile unsigned int*>(P.bar + 2) : 0u;
-  auto gsync = [&]() {
-    if (P.bar == nullptr) { grid.sync(); return; }
-    __syncthreads();
-    bar_target += gridDim.x;
-    if (threadIdx.x == 0) {
-      asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(P.bar) : "memory");
-      const long long t0 = clock64();
-      unsigned int v;
-      do {
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(P.bar) : "memory");
-        if (clock64() - t0 > 8000000000LL) { atomicExch(P.bar + 1, 1u); __trap(); }
-      } while (int(v - bar_target) < 0);
-    }
-    __syncthreads();
-  };
+  unsigned int bar_target = *reinterpret_cast<volatile unsigned int*>(P.bar + 2);
   // Data parallel: in front of a cross-GPU flag exchange only block 0 has to know that every local block has arrived (it is
   // the one that tells the peers); the other blocks go straight on to poll the flags -- their own rank's flag among them,
   // which block 0 posts after this collection -- so the second half of a full barrier (everybody spinning on the counter)
   // is not paid twice per step.
   auto gcollect = [&]() {
-    if (P.bar == nullptr) { grid.sync(); return; }
-    __syncthreads();
-    bar_target += gridDim.x;
-    if (threadIdx.x == 0) {
-      asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(P.bar) : "memory");
-      if (blockIdx.x == 0) {
-        const long long t0 = clock64();
-        unsigned int v;
-        do {
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(P.bar) : "memory");
-          if (clock64() - t0 > 8000000000LL) { atomicExch(P.bar + 1, 1u); __trap(); }
-        } while (int(v - bar_target) < 0);
-      }
+    brk_grid_arrive(P.bar, bar_target);
+    if (blockIdx.x == 0) {
+      brk_grid_wait(P.bar, bar_target);
+      __syncthreads();
     }
-    if (blockIdx.x == 0) __syncthreads();
   };
   __shared__ double red[32];
   const bool sample = P.n == nullptr;
@@ -435,7 +405,7 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
   }
   if (sample) {                                         // step 0 is staged by everybody, up front
     bpr_stage_step(P, P.use_inline ? P.inline_steps[0] : P.steps[0], 0, tid, nthr);
-    gsync();
+    brk_grid_barrier(P.bar, bar_target);
   }
   for (int s = 0; s < P.n_steps; ++s) {
     const BprStep sd = P.use_inline ? P.inline_steps[s] : P.steps[s];
@@ -492,7 +462,7 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
       gcollect();
     } else {
       coop_stamp(P, s, 2);                              // phase 1 done in block 0
-      gsync();
+      brk_grid_barrier(P.bar, bar_target);
     }
     coop_stamp(P, s, 1);
     // ---- phase 2: exact Keras Adam over every element of both tables; zero the accumulators.  In sampling
@@ -627,7 +597,7 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
     // The barrier orders this step's Adam stores before the next step's gathers.  After the last step kernel completion
     // does that for whatever follows on the stream, so a single-GPU launch ends without it: the barrier counter then gets
     // one arrival round fewer, and bar_target (written to bar[2] below) counts exactly the rounds that ran.
-    if (P.world > 1 || s + 1 < P.n_steps || P.last_sync) gsync();
+    if (P.world > 1 || s + 1 < P.n_steps || P.last_sync) brk_grid_barrier(P.bar, bar_target);
     coop_stamp(P, s, 6);
     if (P.world > 1 && *reinterpret_cast<volatile uint32_t*>(P.dp_sync + 4) != 0u) break;   // aborted (uniform after the barrier)
   }
@@ -660,7 +630,7 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
     double* pwo = reinterpret_cast<double*>(P.state);
     P.state[0] += P.n_steps; pwo[1] = beta_pow[P.n_steps & 1][0]; pwo[2] = beta_pow[P.n_steps & 1][1];
     if (P.world > 1) P.dp_sync[3] += uint32_t(P.n_steps);
-    if (P.bar) P.bar[2] = bar_target;
+    P.bar[2] = bar_target;
   }
 }
 
@@ -798,7 +768,7 @@ static int launch_coop_steps(brk_ctx* ctx, const brk_table* user, const brk_tabl
   }
   P.dbg = (g_coop_trace && n_steps <= 4096) ? g_coop_trace : nullptr;
   P.prefetch = getenv("BRK_BPR_NO_PREFETCH") ? 0 : 1;
-  P.bar = getenv("BRK_BPR_CG_SYNC") ? nullptr : ctx->bpr_bar;
+  P.bar = ctx->bar[BRK_BAR_BPR];
   {
     const char* e = getenv("BRK_PEER_SPIN_MS");              // budget of one cross-GPU wait; default ~30 s at 2 GHz
     const long long ms = e ? atoll(e) : 0;

@@ -5,6 +5,10 @@
 #include <stdio.h>
 #include "../../include/brk_b200.h"
 
+// brk_ctx::bar: one block of grid-barrier words per cooperative kernel family
+enum { BRK_BAR_BPR, BRK_BAR_TT, BRK_BAR_NEUMF, BRK_BAR_FAMILIES };
+#define BRK_BAR_LINE_WORDS 32
+
 struct brk_ctx {
   int device;
   int sm_count;
@@ -24,11 +28,13 @@ struct brk_ctx {
   // one-launch NeuMF step (csrc/neumf_fused.cu): per-tile slots of partial sums, summed after a grid barrier
   float*        neumf_part;
   size_t        neumf_part_floats;
-  // one-launch two-tower step (csrc/twotower_fused.cu): per-tile softmax partials, grid-barrier words {count, error, base}
+  // one-launch two-tower step (csrc/twotower_fused.cu): per-tile softmax partials
   float*        tt_part;
   size_t        tt_part_floats;
-  unsigned int* tt_bar;
-  unsigned int* bpr_bar;      // bpr_steps_coop: grid-barrier words {count, error, base}
+  // grid-barrier words of the cooperative step kernels (layout at brk_grid_barrier): bar[BRK_BAR_*], each on its own
+  // 128-byte line of one allocation (bar[0]).  Launches of one family on one context are stream-ordered: a launch reads
+  // the base (and tag) that its predecessor wrote back.
+  unsigned int* bar[BRK_BAR_FAMILIES];
   // any-width NeuMF path (csrc/neumf_generic.cu): feature-major intermediates
   float*        neumf_gen;
   size_t        neumf_gen_floats;
@@ -149,6 +155,38 @@ __device__ __forceinline__ double block_sum_double(double x, double* smem) {
     for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
   }
   return x;
+}
+
+// Grid barrier of a cooperative launch: one release-RED per CTA on an arrival counter that only grows, then an acquire
+// spin by thread 0 (cg::grid.sync() costs two fences and an atomic with return: ~1 us more per barrier in nfz::fused_step,
+// 0.3-0.5 us in bpr_steps_coop).  Words of one kernel family (brk_ctx::bar):
+//   [0] count  arrivals since the context was created (wraps; compared as a signed difference)
+//   [1] error  set by a wait that timed out (and by nfz's tagged-slot waits)
+//   [2] base   count at which the next launch starts: read by every CTA at entry, written back by one thread after the
+//              launch's last barrier, so launches chain (and replay from a CUDA graph) with no host bookkeeping
+//   [3] tag    nfz only: tag of the last launch's self-validating slot words (a launch uses the next one, never 0)
+// `target` starts at the base and is the count at which every CTA of the current round has arrived.  The wait is bounded:
+// a lost CTA sets the error word and TRAPS (the launch fails at the next synchronisation) instead of hanging the GPU.
+constexpr long long kBrkBarrierSpin = 8000000000LL;   // clock64 cycles
+__device__ __forceinline__ void brk_grid_arrive(unsigned int* bar, unsigned int& target) {
+  __syncthreads();
+  target += gridDim.x;
+  if (threadIdx.x == 0) asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(bar) : "memory");
+}
+__device__ __forceinline__ void brk_grid_wait(unsigned int* bar, unsigned int target) {
+  if (threadIdx.x == 0) {
+    const long long t0 = clock64();
+    unsigned int v;
+    do {
+      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(bar) : "memory");
+      if (clock64() - t0 > kBrkBarrierSpin) { atomicExch(bar + 1, 1u); __trap(); }
+    } while (int(v - target) < 0);
+  }
+}
+__device__ __forceinline__ void brk_grid_barrier(unsigned int* bar, unsigned int& target) {
+  brk_grid_arrive(bar, target);
+  brk_grid_wait(bar, target);
+  __syncthreads();
 }
 
 // Philox4x32-10 (Random123).  Known answers in tests/test_philox.py.

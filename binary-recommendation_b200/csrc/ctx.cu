@@ -35,10 +35,10 @@ extern "C" int brk_create(brk_ctx** out, int device) {
   BRK_CUDA(cudaMemset(c->loss_acc, 0, BRK_LOSS_SLOTS * sizeof(double)));
   BRK_CUDA(cudaMalloc(&c->tickets, BRK_TICKETS * sizeof(unsigned int)));
   BRK_CUDA(cudaMemset(c->tickets, 0, BRK_TICKETS * sizeof(unsigned int)));
-  BRK_CUDA(cudaMalloc(&c->tt_bar, 4 * sizeof(unsigned int)));
-  BRK_CUDA(cudaMemset(c->tt_bar, 0, 4 * sizeof(unsigned int)));
-  BRK_CUDA(cudaMalloc(&c->bpr_bar, 4 * sizeof(unsigned int)));
-  BRK_CUDA(cudaMemset(c->bpr_bar, 0, 4 * sizeof(unsigned int)));
+  const size_t bar_bytes = BRK_BAR_FAMILIES * BRK_BAR_LINE_WORDS * sizeof(unsigned int);
+  BRK_CUDA(cudaMalloc(&c->bar[0], bar_bytes));
+  BRK_CUDA(cudaMemset(c->bar[0], 0, bar_bytes));
+  for (int k = 1; k < BRK_BAR_FAMILIES; ++k) c->bar[k] = c->bar[0] + k * BRK_BAR_LINE_WORDS;
   c->scratch = nullptr;
   c->scratch_bytes = 0;
   for (int j = 0; j < BRK_FORK_STREAMS; ++j) {
@@ -77,8 +77,7 @@ extern "C" int brk_destroy(brk_ctx* c) {
   if (c->neumf_part) cudaFree(c->neumf_part);
   if (c->neumf_gen) cudaFree(c->neumf_gen);
   if (c->tt_part) cudaFree(c->tt_part);
-  if (c->tt_bar) cudaFree(c->tt_bar);
-  if (c->bpr_bar) cudaFree(c->bpr_bar);
+  if (c->bar[0]) cudaFree(c->bar[0]);
   for (int j = 0; j < BRK_FORK_STREAMS; ++j)
     if (c->fork_stream[j]) { cudaStreamDestroy(c->fork_stream[j]); cudaEventDestroy(c->ev_fork[j]); cudaEventDestroy(c->ev_join[j]); }
   if (c->copy_ready) {

@@ -17,7 +17,6 @@
 // ld.acquire.sys; every spin has a clock64() deadline that raises an error flag instead of hanging.
 #include <stdlib.h>
 #include "common.cuh"
-#include <cooperative_groups.h>
 
 namespace {
 

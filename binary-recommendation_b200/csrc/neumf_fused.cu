@@ -12,7 +12,7 @@
 //   * the weight gradients dW1 / dW2 / dW3 are tensor-core products accumulated in TMEM; bias / head gradients are
 //     warp-butterfly reductions into shared-memory accumulators;
 //   * NO atomics on shared addresses: every CTA stores its tile's partial sums (BatchNorm statistics, the whole
-//     dense-gradient block, the loss) into its own slot of a small HBM/L2 scratch, and after a grid.sync() the
+//     dense-gradient block, the loss) into its own slot of a small HBM/L2 scratch, and after a grid barrier the
 //     slots are summed in a fixed order -- the BatchNorm totals by every CTA, the dense gradients by the CTA that
 //     owns that slice of the parameter block.  (First version: float atomics on the 2.7 k dense-gradient words
 //     from 128 CTAs took 17 us of a 49 us step, the double atomics of the statistics ~2 us per barrier.)  Results
@@ -23,14 +23,11 @@
 //
 // Thread roles (256 threads): warp w reads TMEM lane quadrant q = w & 3 (sample s = 32 q + lane) and column half
 // hf = w >> 2 of every accumulator; one elected thread issues the MMAs.
-#include <cooperative_groups.h>
 #include <stdlib.h>
 #include <string.h>
 #include "neumf_common.cuh"
 #include "tc.cuh"
 #include "tc_tiles.cuh"
-
-namespace cg = cooperative_groups;
 
 namespace nfz {
 
@@ -89,9 +86,7 @@ struct Extra {
   unsigned int* ticket;
   float* part;                 // [n_tiles][S::PT] per-tile partial sums (cooperative launches)
   int32_t coop;                // 1: cooperative launch (slots + grid barriers); 0: independent tiles (atomics + last-CTA ticket)
-  unsigned int* bar;           // [0] arrival counter of the grid barrier (never reset), [1] time-out flag
-  unsigned int bar_base;       // value of the counter when this launch starts (the host keeps the running total)
-  unsigned int tag;            // launch tag of the self-validating slot words (unique per launch on this context, never 0)
+  unsigned int* bar;           // grid-barrier words {count, error, base, tag} of the context (cooperative launches; common.cuh)
   // exact Keras Adam inside the same launch (after the last barrier): do_adam != 0
   int32_t do_adam;
   brk_adam_hyper hyp;
@@ -305,33 +300,16 @@ __device__ __forceinline__ void build_image(uint8_t* dst, F value) {
   }
 }
 
-// Grid-wide barrier of a cooperative launch: one release-RED on a monotonically increasing counter and an acquire
-// spin by thread 0 (cg::grid.sync() costs two fences and an atomic with return; measured ~1 us more per barrier).
-// `target` is the counter value at which every CTA has arrived.  A bounded spin: a lost CTA raises bar[1] and TRAPS (the
-// launch fails with a CUDA error at the next synchronisation) instead of hanging the GPU or returning a half-reduced step.
-__device__ __forceinline__ void grid_barrier(unsigned int* bar, unsigned int& target) {
-  __syncthreads();
-  target += gridDim.x;
-  if (threadIdx.x == 0) {
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(bar) : "memory");
-    const long long t0 = clock64();
-    unsigned int v;
-    do {
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(bar) : "memory");
-      if (clock64() - t0 > 4000000000LL) { atomicExch(bar + 1, 1u); __trap(); }
-    } while (int(v - target) < 0);
-  }
-  __syncthreads();
-}
-
 // ---- after the tiles: the dense gradients -- the slots of all tiles, summed in tile order by the CTA that owns the
 //      parameter slice (float4 granularity) -- and, with do_adam, the exact Keras Adam of optim.cu over the dense block and
 //      the four tables in the same pass.  Run by EVERY CTA of a cooperative launch: the tile CTAs and the helper CTAs that
 //      only exist so that a small batch does not leave this phase (20 MB of optimizer traffic) to a handful of SMs.
 template <class S>
-__device__ __forceinline__ void dense_reduce_and_adam(const Args& A, const Extra& X, unsigned int& bar_target, float4* f4red, float alpha) {
+__device__ __forceinline__ void dense_reduce_and_adam(const Args& A, const Extra& X, unsigned int bar_target, uint32_t tag,
+                                                      float4* f4red, float alpha) {
   const int t = threadIdx.x;
-  grid_barrier(X.bar, bar_target);
+  brk_grid_barrier(X.bar, bar_target);
+  if (blockIdx.x == 0 && t == 0) { X.bar[2] = bar_target; X.bar[3] = tag; }   // the next launch's barrier base and last tag
   const float b1c = X.hyp.beta1, b2c = X.hyp.beta2, ob1c = 1.0f - X.hyp.beta1, ob2c = 1.0f - X.hyp.beta2, epsc = X.hyp.eps;
   auto adam1 = [&](float& w, float& m, float& v, float g) {
     m = b1c * m + ob1c * g;
@@ -458,6 +436,7 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
   __shared__ double red[32];
   __shared__ bool last;
   __shared__ float alpha_s;
+  __shared__ uint32_t base_s, tag_s;
 
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31, q = warp & 3, hf = warp >> 2, s = q * 32 + lane;
   const int64_t b0 = int64_t(blockIdx.x) * TS;
@@ -468,7 +447,17 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
   const bool coop = X.coop != 0;
   float* slot = X.part + size_t(blockIdx.x) * S::PT;  // this tile's partial sums (cooperative launches)
   float* dp = slot + S::pDense;
-  unsigned int bar_target = X.bar_base;
+  // cooperative launches: the barrier base and the last launch's slot-word tag, loaded here and published to shared memory
+  // (registers are the kernel's limit) just before the first __syncthreads, so that the round trip overlaps the set-up
+  // loads; dense_reduce_and_adam writes both back after the barrier
+  unsigned int base = 0u, last_tag = 0u;
+  if (coop && t == 0) {
+    base = *reinterpret_cast<volatile unsigned int*>(X.bar + 2);
+    last_tag = *reinterpret_cast<volatile unsigned int*>(X.bar + 3);
+  }
+  auto publish_launch_words = [&]() {
+    if (coop && t == 0) { base_s = base; tag_s = last_tag + 1u != 0u ? last_tag + 1u : 1u; }   // zeroed slots carry tag 0
+  };
   const uint32_t bar_a = tc::smem_u32(&bar);
   uint32_t phase = 0;
   const int c1 = hf * HC1, c2 = hf * HC2;            // first column of this thread's half in layers 1 / 2
@@ -487,8 +476,9 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
       const double p1 = pw[1] * double(X.hyp.beta1), p2 = pw[2] * double(X.hyp.beta2);
       alpha_s = float(double(X.hyp.lr) * sqrt(1.0 - p2) / (1.0 - p1));
     }
+    publish_launch_words();
     __syncthreads();
-    dense_reduce_and_adam<S>(A, X, bar_target, reinterpret_cast<float4*>(Q), alpha_s);
+    dense_reduce_and_adam<S>(A, X, base_s, tag_s, reinterpret_cast<float4*>(Q), alpha_s);
     return;
   }
 
@@ -510,7 +500,8 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
     const double p1 = pw[1] * double(X.hyp.beta1), p2 = pw[2] * double(X.hyp.beta2);
     alpha_s = float(double(X.hyp.lr) * sqrt(1.0 - p2) / (1.0 - p1));
   }
-  __syncthreads();                                          // ids, Wd
+  publish_launch_words();
+  __syncthreads();                                          // ids, Wd, launch words
   // x0 rows: every load of the thread is issued here and lands while the images are being built
   constexpr int LPR = E / 4, RPP = NT / LPR, NP = TS / RPP;
   const int gc4 = t % LPR, grr = t / LPR;
@@ -605,8 +596,8 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
     float a[HC1], b[HC1];
 #pragma unroll
     for (int j = 0; j < HC1; ++j) { a[j] = h1[j]; b[j] = h1[j] * h1[j]; }
-    cta_feature_sums_tagged<HC1>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pS1), X.tag, nullptr, nullptr);
-    gather_tagged<2 * H1>(reinterpret_cast<const unsigned long long*>(X.part + S::pS1), S::PT / 2, X.n_tiles, X.tag, dred, tot, X.bar + 1);
+    cta_feature_sums_tagged<HC1>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pS1), tag_s, nullptr, nullptr);
+    gather_tagged<2 * H1>(reinterpret_cast<const unsigned long long*>(X.part + S::pS1), S::PT / 2, X.n_tiles, tag_s, dred, tot, X.bar + 1);
     for (int f = t; f < H1; f += NT) {
       const double m = tot[f] / double(A.B);
       const double var = fmax(tot[H1 + f] / double(A.B) - m * m, 0.0);
@@ -660,10 +651,10 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
 #pragma unroll
     for (int j = 0; j < HC2; ++j) { a[j] = h2[j]; b[j] = h2[j] * h2[j]; }
     stamp(X, 12);
-    cta_feature_sums_tagged<HC2>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pS2), X.tag, nullptr, nullptr);
+    cta_feature_sums_tagged<HC2>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pS2), tag_s, nullptr, nullptr);
     stamp(X, 13);
     stamp(X, 14);
-    gather_tagged<2 * H2>(reinterpret_cast<const unsigned long long*>(X.part + S::pS2), S::PT / 2, X.n_tiles, X.tag, dred, tot, X.bar + 1);
+    gather_tagged<2 * H2>(reinterpret_cast<const unsigned long long*>(X.part + S::pS2), S::PT / 2, X.n_tiles, tag_s, dred, tot, X.bar + 1);
     stamp(X, 15);
     for (int f = t; f < H2; f += NT) {
       const double m = tot[f] / double(A.B);
@@ -842,8 +833,8 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
 #pragma unroll
       for (int j = 0; j < HC2; ++j) { a[j] = dy2[j]; b[j] = dy2[j] * ((h2[j] - mean2[c2 + j]) * rstd2[c2 + j]); }
       // the tile's sums are also its share of the BatchNorm parameter gradients: d beta = sum dy, d gamma = sum dy xhat
-      cta_feature_sums_tagged<HC2>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pD2), X.tag, dp + S::obe2, dp + S::og2);
-      gather_tagged<2 * H2>(reinterpret_cast<const unsigned long long*>(X.part + S::pD2), S::PT / 2, X.n_tiles, X.tag, dred, tot, X.bar + 1);
+      cta_feature_sums_tagged<HC2>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pD2), tag_s, dp + S::obe2, dp + S::og2);
+      gather_tagged<2 * H2>(reinterpret_cast<const unsigned long long*>(X.part + S::pD2), S::PT / 2, X.n_tiles, tag_s, dred, tot, X.bar + 1);
       for (int f = t; f < H2; f += NT) { sdy2[f] = float(tot[f] / double(A.B)); sdyx2[f] = float(tot[H2 + f] / double(A.B)); }
       __syncthreads();
     }
@@ -899,8 +890,8 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
       float a[HC1], b[HC1];
 #pragma unroll
       for (int j = 0; j < HC1; ++j) { a[j] = dy1[j]; b[j] = dy1[j] * ((h1[j] - mean1[c1 + j]) * rstd1[c1 + j]); }
-      cta_feature_sums_tagged<HC1>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pD1), X.tag, dp + S::obe1, dp + S::og1);
-      gather_tagged<2 * H1>(reinterpret_cast<const unsigned long long*>(X.part + S::pD1), S::PT / 2, X.n_tiles, X.tag, dred, tot, X.bar + 1);
+      cta_feature_sums_tagged<HC1>(a, b, part, reinterpret_cast<unsigned long long*>(slot + S::pD1), tag_s, dp + S::obe1, dp + S::og1);
+      gather_tagged<2 * H1>(reinterpret_cast<const unsigned long long*>(X.part + S::pD1), S::PT / 2, X.n_tiles, tag_s, dred, tot, X.bar + 1);
       for (int f = t; f < H1; f += NT) { sdy1[f] = float(tot[f] / double(A.B)); sdyx1[f] = float(tot[H1 + f] / double(A.B)); }
       __syncthreads();
     }
@@ -1012,7 +1003,7 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
     }
     if (coop) {
       for (int f = S::ND + t; f < S::NDP; f += NT) dp[f] = 0.f;           // pad words of the block
-      dense_reduce_and_adam<S>(A, X, bar_target, reinterpret_cast<float4*>(Q), alpha_s);   // every tile buffer is dead by now
+      dense_reduce_and_adam<S>(A, X, base_s, tag_s, reinterpret_cast<float4*>(Q), alpha_s);   // every tile buffer is dead by now
       if (blockIdx.x == 0) {                                // BN moving statistics, loss
         if (BN) {
           for (int f = t; f < H1; f += NT) {
@@ -1054,8 +1045,6 @@ __global__ void __launch_bounds__(NT, (S::smem <= 110 * 1024) ? 2 : 1) fused_ste
   stamp(X, 11);
 }
 
-unsigned int g_launch_tag = 0;   // launch tags of the self-validating slot words: one sequence for every instance and context
-
 struct AdamReq {                 // optional: exact Keras Adam in the same launch (single process, mirrored tables)
   const brk_neumf_model* m;
   brk_adam_hyper h;
@@ -1064,20 +1053,17 @@ struct AdamReq {                 // optional: exact Keras Adam in the same launc
 
 template <class S>
 int run(brk_ctx* ctx, const Args& A, const AdamReq* adam, cudaStream_t st, int* handled) {
-  static int max_blocks = -1;
-  static unsigned int* bar = nullptr;                       // grid-barrier counter of this kernel instance
-  static unsigned int bar_count = 0;                        // host mirror of the counter (launches are stream-ordered)
   auto fn = fused_step<S>;
-  if (max_blocks < 0) {
-    BRK_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, int(S::smem > 120 * 1024 ? S::smem : 120 * 1024)));
-    int per_sm = 0;
-    BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, NT, S::smem));
+  // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of the kernel, queried once
+  BRK_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, int(S::smem > 120 * 1024 ? S::smem : 120 * 1024)));
+  static int per_sm = -1;
+  if (per_sm < 0) {
+    int occ = 0;
+    BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, NT, S::smem));
     const int by_tmem = 512 / S::TCOLS;                     // TMEM columns per SM
-    if (per_sm > by_tmem) per_sm = by_tmem;
-    BRK_CUDA(cudaMalloc(&bar, 2 * sizeof(unsigned int)));
-    BRK_CUDA(cudaMemset(bar, 0, 2 * sizeof(unsigned int)));
-    max_blocks = per_sm * ctx->sm_count;
+    per_sm = occ < by_tmem ? occ : by_tmem;
   }
+  const int max_blocks = per_sm * ctx->sm_count;
   const int64_t n_tiles = (A.B + TS - 1) / TS;
   Extra X;
   memset(&X, 0, sizeof(X));
@@ -1107,10 +1093,7 @@ int run(brk_ctx* ctx, const Args& A, const AdamReq* adam, cudaStream_t st, int* 
   X.part = ctx->neumf_part; X.coop = 1;
   // helper CTAs up to one per SM: the final reduction / Adam phase is spread over the whole GPU even for a small batch
   const unsigned grid = unsigned(n_tiles > ctx->sm_count ? n_tiles : (ctx->sm_count < max_blocks ? ctx->sm_count : max_blocks));
-  X.bar = bar; X.bar_base = bar_count;
-  bar_count += grid;                                         // ONE counter barrier per training launch (before the reduction / Adam)
-  X.tag = ++g_launch_tag;
-  if (X.tag == 0u) X.tag = ++g_launch_tag;
+  X.bar = ctx->bar[BRK_BAR_NEUMF];
   if (adam != nullptr) {
     const brk_table* tb[4] = {&adam->m->uMLP, &adam->m->iMLP, &adam->m->uMF, &adam->m->iMF};
     for (int k = 0; k < 4; ++k) {

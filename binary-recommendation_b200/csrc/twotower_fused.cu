@@ -23,8 +23,8 @@
 // TMEM) on 128 x 128 tiles staged by cp.async in the swizzle of the view that reads them (tc_tiles.cuh); no operand is
 // transposed in memory.  T = ceil(B / 128); the launch needs max(T^2, 4T) <= SM count co-resident CTAs (B <= 1536 on
 // a B200); larger batches, other modes (rdZero) and widths above 128 take the multi-kernel step.
-// The grid barrier is one red.release + an acquire spin on a counter whose base lives in device memory (bar[2]), so
-// the launch can be captured into a CUDA graph and replayed (TwoTowerModel.fit does).
+// The grid barrier (brk_grid_barrier, common.cuh) keeps its base in device memory (bar[2]), so the launch can be captured
+// into a CUDA graph and replayed (TwoTowerModel.fit does).
 #include "common.cuh"
 #include "tc.cuh"
 #include "tc_tiles.cuh"
@@ -54,7 +54,7 @@ struct Params {
   float* dz[2];                                                      // dq, dc [B][S]
   float2* part;                                                      // [T * 128][T]: (max, sum exp) of row x column tile
   double* acc; float* loss_out;
-  unsigned int* bar;                                                 // [0] counter, [1] error flag, [2] base of this launch
+  unsigned int* bar;                                                 // grid-barrier words {count, error, base} (common.cuh)
   unsigned long long* trace;                                         // BRK_TT_TRACE: %globaltimer stamps of block 0
   // Keras Adagrad in the same launch (brk_twotower_train_step): touched rows of the two tables + the two Dense blocks
   int do_opt; float lr, eps;
@@ -113,21 +113,6 @@ __device__ __forceinline__ void gather_tile(uint8_t* dst, const float* __restric
     const int nb = (w + 8 * k < valid) ? cb : 0;
     cp_async16(d + k * 1024, nb ? (const void*)(table + int64_t(ids_s[w + 8 * k]) * d_ + c4 * 4) : (const void*)table, nb);
   }
-}
-
-__device__ __forceinline__ void grid_barrier(unsigned int* bar, unsigned int& target) {
-  __syncthreads();
-  target += gridDim.x;
-  if (threadIdx.x == 0) {
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(bar) : "memory");
-    const long long t0 = clock64();
-    unsigned int v;
-    do {
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(bar) : "memory");
-      if (clock64() - t0 > 4000000000LL) { atomicExch(bar + 1, 1u); __trap(); }      // a lost CTA: flag it and fail the launch instead of hanging
-    } while (int(v - target) < 0);
-  }
-  __syncthreads();
 }
 
 // 64 accumulator columns [c0, c0 + 64) of this thread's TMEM lane
@@ -217,7 +202,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
     tc::fence_before_sync();
   }
   stamp(P, 1);
-  grid_barrier(P.bar, bar_target);
+  brk_grid_barrier(P.bar, bar_target);
   stamp(P, 2);
 
   // ---------------- phase S: one score tile per CTA ----------------
@@ -287,7 +272,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
     }
   }
   stamp(P, 3);
-  grid_barrier(P.bar, bar_target);
+  brk_grid_barrier(P.bar, bar_target);
   stamp(P, 4);
   if (tile_cta) {
     if (h == 0) {                                                       // log-sum-exp of the row over its T tiles (log2 domain)
@@ -376,7 +361,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
     cp_async_commit();
   }
   stamp(P, 5);
-  grid_barrier(P.bar, bar_target);
+  brk_grid_barrier(P.bar, bar_target);
   stamp(P, 6);
   if (b == 0 && t == 0) {                                               // every loss contribution was added before the barrier
     if (P.loss_out) P.loss_out[0] = float(*reinterpret_cast<volatile double*>(P.acc));
@@ -435,7 +420,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
   stamp(P, 7);
   // ---------------- phase O: Keras Adagrad (optim.cu AdagradOp) on what this step touched ----------------
   if (P.training && P.do_opt) {
-    grid_barrier(P.bar, bar_target);
+    brk_grid_barrier(P.bar, bar_target);
     if (b == 0 && t == 0) P.bar[2] = bar_target;
     // rows: every warp takes a run of `per` (tower, sample) pairs, one per lane: the ids are loaded and the touched bits
     // cleared in ONE round trip each (the lane whose atomicAnd saw the bit set owns the row -- ids repeat in a batch); then
@@ -517,16 +502,11 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
       return 0;
   if (!brk_aligned16(ws->q) || !brk_aligned16(ws->c) || (training && (!brk_aligned16(ws->dq) || !brk_aligned16(ws->dc)))) return 0;
   const size_t smem = 3 * size_t(TILE) + 1024;
-  static bool attr_done = false;
-  static int max_blocks = 0;
-  if (!attr_done) {
-    BRK_CUDA(cudaFuncSetAttribute(fused_step, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    int occ = 0;
-    BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fused_step, NT, smem));
-    max_blocks = occ * ctx->sm_count;
-    attr_done = true;
-  }
-  if (grid > max_blocks) return 0;
+  // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of the kernel, queried once
+  BRK_CUDA(cudaFuncSetAttribute(fused_step, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  static int per_sm = -1;
+  if (per_sm < 0) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fused_step, NT, smem));
+  if (grid > per_sm * ctx->sm_count) return 0;
   const size_t part_floats = size_t(T) * TS * T * 2;
   if (ctx->tt_part_floats < part_floats) {
     if (ctx->tt_part) BRK_CUDA(cudaFree(ctx->tt_part));
@@ -542,7 +522,7 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
   P.B = B; P.T = T; P.training = training;
   P.z[0] = ws->q; P.z[1] = ws->c; P.dz[0] = ws->dq; P.dz[1] = ws->dc;
   P.part = reinterpret_cast<float2*>(ctx->tt_part);
-  P.acc = ws->acc; P.loss_out = loss_out; P.bar = ctx->tt_bar;
+  P.acc = ws->acc; P.loss_out = loss_out; P.bar = ctx->bar[BRK_BAR_TT];
   const char* tr = getenv("BRK_TT_TRACE");
   P.trace = tr ? reinterpret_cast<unsigned long long*>(strtoull(tr, nullptr, 16)) : nullptr;
   if (do_opt && training) {                           // in-kernel Adagrad needs the touched bitmasks (row ownership) and float4 blocks
