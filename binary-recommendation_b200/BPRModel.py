@@ -541,19 +541,37 @@ class BPRModel(RModel):
         self.compileModel(None, meta["numUser"], meta["numItem"], meta["numFactor"])
         self.productIds = list(meta.get("productIds", []))
 
-    def predictForUsers(self, customerIds, numberOfItem=5):
+    def predictForUsers(self, customerIds, numberOfItem=5, excludeSeen=False):
         """Top products for a batch of users (not in the reference, whose BPRModel stops after training; the scores
         are bpr_predict's, src/models/bpr.py:122-133): one bf16 tcgen05 scoring GEMM with the fused top-K epilogue
-        over the whole catalog (hotpath.BruteForceIndex) -> [[(str(product), str(score)), ...] per user]."""
-        users = torch.as_tensor(np.asarray([int(c) for c in customerIds], dtype=np.int32)).to(self.model.device)
+        over the whole catalog (hotpath.BruteForceIndex) -> [[(str(product), str(score)), ...] per user].
+        excludeSeen=True leaves out each user's training pairs (trainDf), so a user with fewer unseen products than
+        numberOfItem gets a shorter list; it needs the training pairs (ValueError after a checkpoint restore alone)."""
+        if excludeSeen and self._trainDf is None:
+            raise ValueError("excludeSeen needs the training pairs (trainDf), which this model does not hold")
+        cu = np.asarray([int(c) for c in customerIds], dtype=np.int64)
+        users = torch.as_tensor(cu.astype(np.int32)).to(self.model.device)
         if users.numel() and (int(users.min()) < 0 or int(users.max()) >= self.model.user.rows):
             raise ValueError("unknown customer id")
         if users.numel() == 0:
             return []
         index = H.BruteForceIndex(k=numberOfItem).index(self.model.item.w)
-        v, ix = index(H.gather_rows(self.model.user.w, users))
+        q = H.gather_rows(self.model.user.w, users)
+        if excludeSeen:
+            # the requested users' rows of the per-user seen lists, in request order
+            trU, trI = self._trainDf
+            indptr, seen = synth.build_csr(trU, trI, self.model.user.rows)
+            starts, lens = indptr[cu], indptr[cu + 1] - indptr[cu]
+            ptr = np.zeros(len(cu) + 1, dtype=np.int64)
+            np.cumsum(lens, out=ptr[1:])
+            ids = seen[np.repeat(starts - ptr[:-1], lens) + np.arange(ptr[-1])]
+            dev = self.model.device
+            v, ix = index.query_with_exclusions(q, (torch.from_numpy(ptr).to(dev),
+                                                    torch.from_numpy(ids.astype(np.int32)).to(dev)))
+        else:
+            v, ix = index(q)
         v, ix = v.cpu().numpy(), ix.cpu().numpy()
-        return [[(str(int(j)), str(s)) for s, j in zip(v[r], ix[r])] for r in range(len(v))]
+        return [[(str(int(j)), str(s)) for s, j in zip(v[r], ix[r]) if j >= 0] for r in range(len(v))]
 
     def extractPositivesNegatives(self, customerId) -> list:
         """Exhaustive (positive, non-interacted) pairs of one customer -- BPRModel.py:111-119."""

@@ -328,9 +328,11 @@ class NeuMFNet:
     def predict(self, dataset):
         return torch.cat([self.predict_on_batch(u, i)[0] for u, i, _ in dataset.batches()]).unsqueeze(1)
 
-    def score_all(self, usersId, itemsId, k):
+    def score_all(self, usersId, itemsId, k, exclude=None):
         """Top-k over the whole catalog for each user (topKRatings' "NFC" path, topKmetrics.py:29-33):
-        NeuMF has no factorised scorer, so every (user, item) pair goes through the fused forward."""
+        NeuMF has no factorised scorer, so every (user, item) pair goes through the fused forward.  `exclude`: an
+        (indptr, ids) CSR over the rows of usersId listing positions in itemsId to leave out (hotpath.exclusion_csr);
+        they are masked in each chunk's scores before the selection, and short rows are padded with (-inf, -1)."""
         dev = self.device
         items = torch.as_tensor(np.asarray(itemsId, dtype=np.int32)).to(dev)
         I = items.numel()
@@ -341,7 +343,10 @@ class NeuMFNet:
         for s in range(0, len(users), chunk):
             uu = torch.as_tensor(users[s:s + chunk]).to(dev)
             out, _ = self.predict_on_batch(uu.repeat_interleave(I), items.repeat(uu.numel()))
-            v, ix = H.topk_rows(out.view(uu.numel(), I), k)
+            S = out.view(uu.numel(), I)
+            if exclude is not None:
+                H.mask_excluded(S, exclude[0][s:s + uu.numel() + 1], exclude[1], 0)
+            v, ix = H.topk_rows(S, k)
             vals.append(v); idxs.append(ix)
         return torch.cat(vals), torch.cat(idxs)
 

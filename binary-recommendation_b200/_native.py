@@ -131,6 +131,8 @@ SIGNATURES = {
     "brk_rows_to_bf16": (C.c_int, [_P, _P, _I64, _I32, _P, _I32, _P]),
     "brk_score_topk_workspace_bytes": (C.c_int64, [_P, _I64, _I64, _I32]),
     "brk_score_topk_bf16": (C.c_int, [_P, _P, _I64, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _I64, _P]),
+    "brk_score_topk_bf16_excl": (C.c_int, [_P, _P, _I64, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _P, _P, _I64, _P]),
+    "brk_mask_excluded": (C.c_int, [_P, _P, _I64, _I64, _I32, _P, _P, _P]),
     "brk_topk_metrics": (C.c_int, [_P, _P, _I64, _I32, _P, _P, _P, _I64, _P, _P, _P]),
     "brk_rank_eval_rows": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _P, _I32, _P, _P, _P, _P]),
     "brk_topk_rows": (C.c_int, [_P, _P, _I64, _I64, _I32, _P, _P, _P]),

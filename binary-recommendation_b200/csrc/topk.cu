@@ -24,6 +24,7 @@
 #include "common.cuh"
 #include "tc.cuh"
 #include <cuda_bf16.h>
+#include <limits.h>
 #include <math_constants.h>
 #include <stdlib.h>
 
@@ -50,7 +51,14 @@ struct TopkParams {
   int32_t probe;         // diagnostics: 1 = epilogue only drains TMEM (measures the TMEM-read ceiling)
   float* out_vals;       // [n_splits * kHalves, U, k]
   int32_t* out_ids;
+  const int64_t* excl_indptr;   // EXCL only: [U + 1] absolute offsets into excl_ids
+  const int32_t* excl_ids;      // EXCL only: excluded global ids, ascending within each row
 };
+
+// Exclusion cursor of one epilogue thread (EXCL instantiations): a pointer into its row's list, the entries left from
+// there and the id it points at.  Static shared memory, not registers -- the kernel sits at the 168-register cap of two
+// CTAs per SM -- touched only on the candidate path.  Budgeted as 4 KB (ptxas places 3 KB).
+constexpr size_t kExclCursorBytes = 4096;
 
 template <int K>
 __device__ __forceinline__ void topk_insert(float (&vals)[K], int32_t (&ids)[K], float v, int32_t id) {
@@ -65,7 +73,7 @@ __device__ __forceinline__ void topk_insert(float (&vals)[K], int32_t (&ids)[K],
   if (v > vals[0]) { vals[0] = v; ids[0] = id; }
 }
 
-template <int K_CAP>
+template <int K_CAP, bool EXCL>
 __global__ void __launch_bounds__(kThreadsTopk, 2)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_c,
                   const TopkParams P) {
@@ -73,6 +81,9 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
   // slow-path scratch of the epilogue threads: STATIC shared memory, so that the compiler emits STS / LDS for it (carved
   // out of the dynamic block through a generic pointer it was 32 generic ST.E per spilled chunk)
   __shared__ float scratch_s[kEpiWarps * 32 * 32];
+  __shared__ const int32_t* excl_cur_s[EXCL ? kEpiWarps * 32 : 1];
+  __shared__ int32_t excl_left_s[EXCL ? kEpiWarps * 32 : 1];
+  __shared__ int32_t excl_next_s[EXCL ? kEpiWarps * 32 : 1];
   // 1024-byte alignment for the 128-byte swizzle
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const uint32_t smem_a = tc::smem_u32(smem);
@@ -165,6 +176,47 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
     float* scratch = scratch_s + (threadIdx.x - 64);
     constexpr int kScratchStride = kEpiWarps * 32;
 
+    // Exclusions: the thread meets its row's candidates in ascending global id (tiles, flagged chunks and mask bits
+    // all ascend), so one monotone cursor into the row's ascending list answers every membership test.  It starts at
+    // the first listed id >= this split's first id; rows >= U (padding of the last m-tile) get an empty list.
+    if constexpr (EXCL) {
+      const int e = threadIdx.x - 64;
+      int64_t pos = 0, end = 0;
+      if (row < P.U) {
+        pos = P.excl_indptr[row];
+        end = P.excl_indptr[row + 1];
+        const int64_t first = int64_t(tile_begin) * kBN + P.id_offset;
+        int64_t hi = end;
+        while (pos < hi) {                                // lower bound of `first`
+          const int64_t mid = pos + ((hi - pos) >> 1);
+          if (P.excl_ids[mid] < first) pos = mid + 1; else hi = mid;
+        }
+      }
+      const int64_t left = end - pos;                     // a row lists at most I < 2^31 distinct ids
+      excl_cur_s[e] = P.excl_ids + pos;
+      excl_left_s[e] = int32_t(left < INT_MAX ? left : INT_MAX);
+      excl_next_s[e] = pos < end ? P.excl_ids[pos] : INT_MAX;
+    }
+    // Listed ids of the 32 columns starting at global id `lo`, as a bit mask (EXCL only).  Advances the cursor past
+    // lo + 31; chunks must be presented in ascending order.  Applied to a chunk's candidate mask before the insertion
+    // loop, so that loop carries no extra register (a per-candidate test there spilled the register list).
+    auto excluded_bits = [&](int32_t lo) -> uint32_t {
+      const int e = threadIdx.x - 64;
+      int32_t next = excl_next_s[e];
+      if (next >= lo + 32) return 0u;                    // the launcher keeps lo + 32 <= INT_MAX
+      const int32_t* cur = excl_cur_s[e];
+      int32_t left = excl_left_s[e];
+      uint32_t bits = 0u;
+      do {
+        if (next >= lo) bits |= 1u << (next - lo);
+        next = (--left > 0) ? *++cur : INT_MAX;
+      } while (next < lo + 32);
+      excl_cur_s[e] = cur;
+      excl_left_s[e] = left;
+      excl_next_s[e] = next;
+      return bits;
+    };
+
     auto process = [&](uint32_t (&r)[32], int64_t col0, bool ragged) {
       if (P.probe == 1) {                               // keep the loads alive, do nothing else
         uint32_t x = 0;
@@ -180,10 +232,15 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
       if (ragged) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) scratch[j * kScratchStride] = V(j);
+        uint32_t live = 0xffffffffu;                      // EXCL: columns not listed
+        if constexpr (EXCL) live = ~excluded_bits(int32_t(col0) + P.id_offset);
 #pragma unroll 1
         for (int j = 0; j < 32; ++j) {
           const float x = scratch[j * kScratchStride];
           if (col0 + j < P.I && x > thr) {
+            if constexpr (EXCL) {
+              if (!((live >> j) & 1u)) continue;
+            }
             topk_insert<K_CAP>(vals, ids, x, int32_t(col0 + j) + P.id_offset);
             thr = vals[K_CAP - 1];
           }
@@ -214,6 +271,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             }
           }
         }
+        if constexpr (EXCL) mask &= ~excluded_bits(int32_t(col0) + P.id_offset);
 #pragma unroll 1
         while (mask) {                                  // ascending column = ascending item id
           const int j = __ffs(mask) - 1;
@@ -394,11 +452,27 @@ topk_rows_kernel(const float* __restrict__ scores, int64_t R, int64_t I, int k, 
   }
 }
 
-template <int K_CAP>
+// Excluded items of materialised score rows: scores[r, id - col_offset] = -inf for every id of row r's list inside
+// [col_offset, col_offset + I).  One warp per row, lanes striding the list.  topk_rows_kernel never inserts -inf, so
+// masking followed by it selects among the remaining columns and pads with -1 like the fused path.
+__global__ void __launch_bounds__(256)
+mask_excluded_kernel(float* __restrict__ scores, int64_t R, int64_t I, int32_t col_offset,
+                     const int64_t* __restrict__ indptr, const int32_t* __restrict__ ids) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  if (row >= R) return;
+  const int64_t end = indptr[row + 1];
+  for (int64_t p = indptr[row] + lane; p < end; p += 32) {
+    const int64_t c = int64_t(__ldg(ids + p)) - col_offset;
+    if (c >= 0 && c < I) scores[row * I + c] = -CUDART_INF_F;
+  }
+}
+
+template <int K_CAP, bool EXCL>
 int launch_topk(const CUtensorMap& tq, const CUtensorMap& tcm, const TopkParams& P, dim3 grid, size_t smem,
                 cudaStream_t st) {
-  BRK_CUDA(cudaFuncSetAttribute(score_topk_kernel<K_CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  score_topk_kernel<K_CAP><<<grid, kThreadsTopk, smem, st>>>(tq, tcm, P);
+  BRK_CUDA(cudaFuncSetAttribute(score_topk_kernel<K_CAP, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  score_topk_kernel<K_CAP, EXCL><<<grid, kThreadsTopk, smem, st>>>(tq, tcm, P);
   BRK_LAUNCH_CHECK();
   return 0;
 }
@@ -444,10 +518,14 @@ extern "C" int64_t brk_score_topk_workspace_bytes(brk_ctx* ctx, int64_t U, int64
   return int64_t(S) * kHalves * U * k * 8;
 }
 
-extern "C" int brk_score_topk_bf16(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* c_bf16,
-                                   int64_t I, int32_t dpad, int32_t k, int32_t id_offset, float* out_vals,
-                                   int32_t* out_ids, void* workspace, int64_t workspace_bytes, void* stream) {
+namespace {
+
+// brk_score_topk_bf16 (excl_indptr == nullptr: the EXCL = false kernels) and brk_score_topk_bf16_excl
+int score_topk(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* c_bf16, int64_t I, int32_t dpad,
+               int32_t k, int32_t id_offset, const int64_t* excl_indptr, const int32_t* excl_ids, float* out_vals,
+               int32_t* out_ids, void* workspace, int64_t workspace_bytes, void* stream) {
   BRK_REQUIRE(ctx && q_bf16 && c_bf16 && out_vals && out_ids, BRK_E_ARG, "brk_score_topk_bf16: null argument");
+  const bool excl = excl_indptr != nullptr;
   BRK_REQUIRE(U > 0 && I > 0 && U < (int64_t(1) << 31) && I < (int64_t(1) << 31), BRK_E_ARG,
               "brk_score_topk_bf16: U=%lld I=%lld", (long long)U, (long long)I);
   BRK_REQUIRE(dpad > 0 && dpad % kKBlock == 0 && dpad / kKBlock <= kMaxKB, BRK_E_ARG,
@@ -458,6 +536,7 @@ extern "C" int brk_score_topk_bf16(brk_ctx* ctx, const uint16_t* q_bf16, int64_t
 
   TopkParams P;
   P.U = U; P.I = I; P.KB = dpad / kKBlock; P.k = k; P.id_offset = id_offset;
+  P.excl_indptr = excl_indptr; P.excl_ids = excl_ids;
   P.probe = getenv("BRK_TOPK_PROBE") ? atoi(getenv("BRK_TOPK_PROBE")) : 0;
   int S, tps;
   P.n_tiles = plan_splits(ctx->sm_count * (dpad <= 128 ? 2 : 1), U, I, &S, &tps);
@@ -467,11 +546,12 @@ extern "C" int brk_score_topk_bf16(brk_ctx* ctx, const uint16_t* q_bf16, int64_t
   // two CTAs per SM (each with its own pair of TMEM accumulators) when the query tile leaves room: while one CTA's epilogue
   // warps wait for their next accumulator the other's keep the SM busy
   const size_t budget = a_bytes <= 32 * 1024 ? size_t(113) * 1024 : size_t(227) * 1024;
-  int stages = int((budget - 1024 - 256 - kScratchBytes - a_bytes) / kBBytes);
+  int stages = int((budget - 1024 - 256 - kScratchBytes - (excl ? kExclCursorBytes : 0) - a_bytes) / kBBytes);
   if (stages > 6) stages = 6;
   BRK_REQUIRE(stages >= 2, BRK_E_ARG, "brk_score_topk_bf16: no room for a 2-stage pipeline at dpad=%d", dpad);
   P.stages = stages;
-  const size_t smem = 1024 + a_bytes + size_t(stages) * kBBytes + 256;   // + kScratchBytes of static shared memory
+  // + kScratchBytes (+ kExclCursorBytes) of static shared memory
+  const size_t smem = 1024 + a_bytes + size_t(stages) * kBBytes + 256;
 
   const int parts = S * kHalves;                       // partial lists per user row
   const int64_t need = int64_t(parts) * U * k * 8;
@@ -490,11 +570,44 @@ extern "C" int brk_score_topk_bf16(brk_ctx* ctx, const uint16_t* q_bf16, int64_t
 
   const dim3 grid(unsigned((U + kBM - 1) / kBM), unsigned(S));
   int rc;
-  if (k <= 10) rc = launch_topk<10>(tq, tcm, P, grid, smem, st);
-  else if (k <= 16) rc = launch_topk<16>(tq, tcm, P, grid, smem, st);
-  else rc = launch_topk<32>(tq, tcm, P, grid, smem, st);
+  if (k <= 10) rc = excl ? launch_topk<10, true>(tq, tcm, P, grid, smem, st) : launch_topk<10, false>(tq, tcm, P, grid, smem, st);
+  else if (k <= 16) rc = excl ? launch_topk<16, true>(tq, tcm, P, grid, smem, st) : launch_topk<16, false>(tq, tcm, P, grid, smem, st);
+  else rc = excl ? launch_topk<32, true>(tq, tcm, P, grid, smem, st) : launch_topk<32, false>(tq, tcm, P, grid, smem, st);
   if (rc) return rc;
   topk_merge_kernel<<<unsigned((U + 255) / 256), 256, 0, st>>>(pv, pi, parts, U, k, out_vals, out_ids);
+  BRK_LAUNCH_CHECK();
+  return 0;
+}
+
+}  // namespace
+
+extern "C" int brk_score_topk_bf16(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* c_bf16,
+                                   int64_t I, int32_t dpad, int32_t k, int32_t id_offset, float* out_vals,
+                                   int32_t* out_ids, void* workspace, int64_t workspace_bytes, void* stream) {
+  return score_topk(ctx, q_bf16, U, c_bf16, I, dpad, k, id_offset, nullptr, nullptr, out_vals, out_ids, workspace,
+                    workspace_bytes, stream);
+}
+
+extern "C" int brk_score_topk_bf16_excl(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* c_bf16,
+                                        int64_t I, int32_t dpad, int32_t k, int32_t id_offset,
+                                        const int64_t* excl_indptr, const int32_t* excl_ids, float* out_vals,
+                                        int32_t* out_ids, void* workspace, int64_t workspace_bytes, void* stream) {
+  BRK_REQUIRE(excl_indptr && excl_ids, BRK_E_ARG, "brk_score_topk_bf16_excl: null exclusion list");
+  // the kernel's exclusion cursor ends on INT_MAX and looks 32 ids past a chunk's first: every chunk of every item tile
+  // must stay below it
+  BRK_REQUIRE(int64_t(id_offset) + (I + kBN - 1) / kBN * kBN < int64_t(INT_MAX), BRK_E_ARG,
+              "brk_score_topk_bf16_excl: id_offset=%d + I=%lld reaches INT_MAX", id_offset, (long long)I);
+  return score_topk(ctx, q_bf16, U, c_bf16, I, dpad, k, id_offset, excl_indptr, excl_ids, out_vals, out_ids, workspace,
+                    workspace_bytes, stream);
+}
+
+extern "C" int brk_mask_excluded(brk_ctx* ctx, float* scores, int64_t R, int64_t I, int32_t col_offset,
+                                 const int64_t* excl_indptr, const int32_t* excl_ids, void* stream) {
+  BRK_REQUIRE(ctx && scores && excl_indptr && excl_ids, BRK_E_ARG, "brk_mask_excluded: null argument");
+  BRK_REQUIRE(R >= 0 && I > 0, BRK_E_ARG, "brk_mask_excluded: R=%lld I=%lld", (long long)R, (long long)I);
+  if (R == 0) return 0;
+  mask_excluded_kernel<<<unsigned((R * 32 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(scores, R, I, col_offset,
+                                                                                         excl_indptr, excl_ids);
   BRK_LAUNCH_CHECK();
   return 0;
 }

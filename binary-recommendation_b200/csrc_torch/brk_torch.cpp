@@ -140,6 +140,31 @@ std::tuple<at::Tensor, at::Tensor> score_topk(const at::Tensor& q_bf16, const at
                             ws.data_ptr(), wsb, stream_of(q_bf16)), "brk_score_topk_bf16");
   return {vals, ids};
 }
+// TFRS TopK.query_with_exclusions: the same selection with row r's listed global ids (CSR, ascending per row) left out
+std::tuple<at::Tensor, at::Tensor> score_topk_exclude(const at::Tensor& q_bf16, const at::Tensor& c_bf16, int64_t k, int64_t id_offset,
+                                                      const at::Tensor& excl_indptr, const at::Tensor& excl_ids) {
+  need(q_bf16, at::kBFloat16, "q_bf16"); need(c_bf16, at::kBFloat16, "c_bf16");
+  need(excl_indptr, at::kLong, "excl_indptr"); need(excl_ids, at::kInt, "excl_ids");
+  TORCH_CHECK(q_bf16.size(1) == c_bf16.size(1), "padded widths differ");
+  TORCH_CHECK(c_bf16.device() == q_bf16.device() && excl_indptr.device() == q_bf16.device() && excl_ids.device() == q_bf16.device(),
+              "score_topk_exclude: every tensor must be on the queries' device");
+  const int64_t U = q_bf16.size(0), I = c_bf16.size(0);
+  TORCH_CHECK(excl_indptr.dim() == 1 && excl_indptr.numel() >= U + 1, "excl_indptr: ", excl_indptr.numel(),
+              " entries, at least U + 1 = ", U + 1, " needed");
+  c10::cuda::CUDAGuard guard(q_bf16.device());
+  brk_ctx* ctx = ctx_for(q_bf16.get_device());
+  at::Tensor vals = at::empty({U, k}, q_bf16.options().dtype(at::kFloat)), ids = at::empty({U, k}, q_bf16.options().dtype(at::kInt));
+  if (U == 0) return {vals, ids};
+  // an empty list array still needs an address: the C ABI takes NULL for a missing argument
+  const at::Tensor xids = excl_ids.numel() ? excl_ids : at::zeros({1}, excl_ids.options());
+  const int64_t wsb = brk_score_topk_workspace_bytes(ctx, U, I, int32_t(k));
+  at::Tensor ws = at::empty({wsb > 16 ? wsb : 16}, q_bf16.options().dtype(at::kByte));
+  check(brk_score_topk_bf16_excl(ctx, reinterpret_cast<const uint16_t*>(q_bf16.data_ptr()), U, reinterpret_cast<const uint16_t*>(c_bf16.data_ptr()),
+                                 I, int32_t(q_bf16.size(1)), int32_t(k), int32_t(id_offset), excl_indptr.data_ptr<int64_t>(),
+                                 xids.data_ptr<int32_t>(), vals.data_ptr<float>(), ids.data_ptr<int32_t>(), ws.data_ptr(), wsb,
+                                 stream_of(q_bf16)), "brk_score_topk_bf16_excl");
+  return {vals, ids};
+}
 std::tuple<at::Tensor, at::Tensor> topk_merge(const at::Tensor& part_vals, const at::Tensor& part_ids) {
   need(part_vals, at::kFloat, "part_vals"); need(part_ids, at::kInt, "part_ids");
   TORCH_CHECK(part_vals.dim() == 3, "part_vals must be [S, U, k]");
@@ -193,6 +218,8 @@ TORCH_LIBRARY(brk, m) {
         "Tensor(e!) state, bool advance) -> ()", &adam_dense_keras);
   m.def("rows_to_bf16(Tensor x) -> Tensor", &rows_to_bf16);
   m.def("score_topk(Tensor q_bf16, Tensor c_bf16, int k, int id_offset) -> (Tensor, Tensor)", &score_topk);
+  m.def("score_topk_exclude(Tensor q_bf16, Tensor c_bf16, int k, int id_offset, Tensor excl_indptr, Tensor excl_ids) -> (Tensor, Tensor)",
+        &score_topk_exclude);
   m.def("topk_merge(Tensor part_vals, Tensor part_ids) -> (Tensor, Tensor)", &topk_merge);
   m.def("neumf_train_step(Tensor(a!)[] w, Tensor(b!)[] g, Tensor(c!)[] m, Tensor(d!)[] v, Tensor(e!) bn_moving, int[] spec, Tensor u, "
         "Tensor i, Tensor y, int first_index, int dropout_seed, int dropout_epoch, float lr, float beta1, float beta2, float eps, "

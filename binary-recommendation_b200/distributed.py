@@ -279,11 +279,16 @@ def gather_topk_parts(vals, ids):
     return torch.stack(pv), torch.stack(pi)
 
 
-def sharded_topk(queries, item_vectors_local, item_lo, k, merge=None, local_topk=None):
+def sharded_topk(queries, item_vectors_local, item_lo, k, merge=None, local_topk=None, exclude=None):
     """Top-k of `queries` against an item catalog range-sharded over the ranks: this rank holds rows
     [item_lo, item_lo + len(item_vectors_local)).  Result identical on every rank and identical to
-    the unsharded scan (same tie rule)."""
+    the unsharded scan (same tie rule).  `exclude`: one (indptr, ids) CSR of GLOBAL item ids per query row, the
+    same on every rank (each rank's scorer ignores ids outside its range); it applies to the default local scorer."""
     from . import hotpath as H
+    if exclude is not None and local_topk is not None:
+        raise ValueError("sharded_topk: exclude applies to the default local scorer, not to a custom local_topk")
+    if exclude is not None:
+        local_topk = lambda q, c, off: H.BruteForceIndex(k).index(c, id_offset=off).query_with_exclusions(q, exclude)
     local_topk = local_topk or (lambda q, c, off: H.BruteForceIndex(k).index(c, id_offset=off)(q))
     merge = merge or H.topk_merge
     v, i = local_topk(queries, item_vectors_local, item_lo)

@@ -9,6 +9,7 @@ import torch
 
 from . import _native as N
 from . import _torchext as T
+from . import synth
 
 
 def _i32(t, name):
@@ -290,6 +291,12 @@ class BruteForceIndex:
         self.id_offset = int(id_offset)
         return self
 
+    def _identify(self, ids):
+        """Global candidate ids -> identifiers (when index() was given some); -1 pads stay -1."""
+        if self._identifiers is None:
+            return ids
+        return self._identifiers[(ids - self.id_offset).clamp_min(0).long()].masked_fill(ids < 0, -1)
+
     def __call__(self, queries, k=None):
         if self._c is None:
             raise RuntimeError("BruteForceIndex: call index(candidates) first")
@@ -309,18 +316,70 @@ class BruteForceIndex:
         q = rows_to_bf16(queries)
         if T.ops() is not None:
             vals, ids = T.ops().score_topk(q, self._c, k, self.id_offset)
-            if self._identifiers is not None:
-                return vals, self._identifiers[(ids - self.id_offset).long()]
-            return vals, ids
+            return vals, self._identify(ids)
         lib, ctx = N.lib(), N.ctx(dev)
         ws_bytes = lib.brk_score_topk_workspace_bytes(ctx, U, self.num_candidates, k)
         ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         N.check(lib.brk_score_topk_bf16(ctx, N.ptr(q), U, N.ptr(self._c), self.num_candidates, q.shape[1], k,
                                         self.id_offset, N.ptr(vals), N.ptr(ids), N.ptr(ws), ws_bytes,
                                         N.stream_ptr()), "brk_score_topk_bf16")
-        if self._identifiers is not None:
-            return vals, self._identifiers[(ids - self.id_offset).long()]
-        return vals, ids
+        return vals, self._identify(ids)
+
+    def query_with_exclusions(self, queries, exclusions, k=None):
+        """TFRS TopK.query_with_exclusions: the call's (scores, identifiers) [U, k] with each query row's excluded
+        candidates left out.  `exclusions` is either a dense int tensor [U, n] of identifiers (candidate indices when
+        index() got no identifiers; entries not in the index, such as -1 padding, are ignored) or a CSR
+        (indptr int64 [>= U+1], ids int32) of global candidate ids (index + id_offset), ascending within each row --
+        see exclusion_csr.  Rows with fewer than k remaining candidates are padded with (-inf, -1)."""
+        if self._c is None:
+            raise RuntimeError("BruteForceIndex: call index(candidates) first")
+        if queries.shape[1] != self.dim:
+            raise ValueError(f"query dim {queries.shape[1]} != candidate dim {self.dim}")
+        k = min(int(k or self.k), self.num_candidates)
+        U, dev = queries.shape[0], queries.device
+        if isinstance(exclusions, torch.Tensor):
+            exclusions = self._dense_exclusions(exclusions, U)
+        indptr, xids = _check_csr(exclusions, U, dev)
+        if k > MAX_FUSED_K:
+            return self._call_materialised(queries, k, (indptr, xids))
+        vals = torch.empty((U, k), dtype=torch.float32, device=dev)
+        ids = torch.empty((U, k), dtype=torch.int32, device=dev)
+        if U == 0:
+            return vals, ids
+        q = rows_to_bf16(queries)
+        if T.ops() is not None:
+            vals, ids = T.ops().score_topk_exclude(q, self._c, k, self.id_offset, indptr, xids)
+            return vals, self._identify(ids)
+        lib, ctx = N.lib(), N.ctx(dev)
+        ws_bytes = lib.brk_score_topk_workspace_bytes(ctx, U, self.num_candidates, k)
+        ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
+        N.check(lib.brk_score_topk_bf16_excl(ctx, N.ptr(q), U, N.ptr(self._c), self.num_candidates, q.shape[1], k,
+                                             self.id_offset, N.ptr(indptr), N.ptr(xids), N.ptr(vals), N.ptr(ids),
+                                             N.ptr(ws), ws_bytes, N.stream_ptr()), "brk_score_topk_bf16_excl")
+        return vals, self._identify(ids)
+
+    def _dense_exclusions(self, E, U):
+        """Dense [U, n] identifiers -> CSR of global candidate ids (device plumbing: sort + searchsorted)."""
+        if E.dim() != 2 or E.shape[0] != U or E.dtype.is_floating_point or E.dtype == torch.bool:
+            raise TypeError(f"dense exclusions must be an integer tensor [{U}, n]")
+        E = E.to(self._c.device)
+        I = self.num_candidates
+        if self._identifiers is None:
+            hit = (E >= 0) & (E < I)
+            cand = E.long()
+        else:
+            ident = torch.as_tensor(self._identifiers, device=E.device)
+            sv, perm = torch.sort(ident)
+            pos = torch.searchsorted(sv, E.to(sv.dtype)).clamp_max(I - 1)
+            hit = sv[pos] == E.to(sv.dtype)
+            cand = perm[pos]
+        big = torch.iinfo(torch.int64).max
+        cand = torch.where(hit, cand + self.id_offset, big).sort(dim=1).values
+        n_row = hit.sum(dim=1)
+        indptr = torch.zeros(U + 1, dtype=torch.int64, device=E.device)
+        torch.cumsum(n_row, 0, out=indptr[1:])
+        ids = cand[torch.arange(cand.shape[1], device=E.device) < n_row[:, None]].to(torch.int32)
+        return indptr, ids
 
 
 def sgemm(a, b, trans_b=False):
@@ -336,9 +395,10 @@ def sgemm(a, b, trans_b=False):
     return out
 
 
-def _bruteforce_materialised(self, queries, k):
+def _bruteforce_materialised(self, queries, k, exclusions=None):
     """k > 32: bf16-rounded operands like the fused kernel (so shorter and longer lists agree on their common prefix up
-    to fp32 summation order), scores of <= 2^24 pairs at a time, multi-pass top-k."""
+    to fp32 summation order), scores of <= 2^24 pairs at a time, multi-pass top-k.  `exclusions`: a checked CSR of
+    global ids, masked out of each chunk's scores."""
     U, I = queries.shape[0], self.num_candidates
     dev = queries.device
     C = self._c[:, :self.dim].float().contiguous()
@@ -347,11 +407,12 @@ def _bruteforce_materialised(self, queries, k):
     chunk = max(1, (1 << 24) // max(I, 1))
     for s0 in range(0, U, chunk):
         q = _f32(queries[s0:s0 + chunk], "queries").to(torch.bfloat16).float().contiguous()
-        v, ix = topk_rows(sgemm(q, C, trans_b=True), k)
-        vals[s0:s0 + chunk] = v; ids[s0:s0 + chunk] = ix + self.id_offset
-    if self._identifiers is not None:
-        return vals, self._identifiers[(ids - self.id_offset).long()]
-    return vals, ids
+        S = sgemm(q, C, trans_b=True)
+        if exclusions is not None:
+            mask_excluded(S, exclusions[0][s0:s0 + S.shape[0] + 1], exclusions[1], self.id_offset)
+        v, ix = topk_rows(S, k)
+        vals[s0:s0 + chunk] = v; ids[s0:s0 + chunk] = torch.where(ix >= 0, ix + self.id_offset, ix)
+    return vals, self._identify(ids)
 
 
 BruteForceIndex._call_materialised = _bruteforce_materialised
@@ -371,10 +432,52 @@ def topk_merge(part_vals, part_ids):
     return vals, ids
 
 
-def topk_rows(scores, k):
-    """Top-k per row of a score matrix [R, I] (score desc, ties -> lower column)."""
+def exclusion_csr(rows, items, num_rows, device):
+    """Exclusion lists from (row, item) pairs: device (indptr int64 [num_rows + 1], ids int32), each row's items
+    distinct and ascending (synth.build_csr).  Pairs with a row outside [0, num_rows) or a negative item are dropped."""
+    rows = np.asarray(rows, dtype=np.int64); items = np.asarray(items, dtype=np.int64)
+    keep = (rows >= 0) & (rows < num_rows) & (items >= 0)
+    indptr, ids = synth.build_csr(rows[keep], items[keep], num_rows)
+    if len(ids) == 0:
+        ids = np.zeros(1, dtype=np.int32)          # the kernels take an address even for empty lists
+    return torch.from_numpy(indptr).to(device), torch.from_numpy(ids).to(device)
+
+
+def _check_csr(csr, rows, device):
+    """Validates an exclusion CSR for `rows` query rows before anything is launched: types, device, shapes.  The
+    offsets themselves stay on the device unread (no synchronisation); they must lie within ids."""
+    indptr, ids = csr
+    if not (isinstance(indptr, torch.Tensor) and isinstance(ids, torch.Tensor)):
+        raise TypeError("exclusions must be a tensor or an (indptr, ids) pair of tensors")
+    if indptr.dtype != torch.int64 or ids.dtype != torch.int32:
+        raise TypeError("exclusion indptr must be int64 and ids int32")
+    if indptr.device != torch.device(device) or ids.device != torch.device(device):
+        raise ValueError(f"exclusion CSR must be on {device}")
+    if indptr.dim() != 1 or indptr.numel() < rows + 1:
+        raise ValueError(f"exclusion indptr has {indptr.numel()} entries, {rows + 1} needed")
+    if ids.dim() != 1 or not indptr.is_contiguous() or not ids.is_contiguous():
+        raise ValueError("exclusion indptr and ids must be contiguous 1-D tensors")
+    if ids.numel() == 0:
+        ids = torch.zeros(1, dtype=torch.int32, device=device)
+    return indptr, ids
+
+
+def mask_excluded(scores, indptr, ids, col_offset=0):
+    """In place: scores[r, id - col_offset] = -inf for each listed id of row r inside the matrix (brk_mask_excluded)."""
+    R, I = scores.shape
+    indptr, ids = _check_csr((indptr, ids), R, scores.device)
+    N.check(N.lib().brk_mask_excluded(N.ctx(scores.device), N.ptr(scores), R, I, int(col_offset), N.ptr(indptr), N.ptr(ids),
+                                      N.stream_ptr()), "brk_mask_excluded")
+    return scores
+
+
+def topk_rows(scores, k, exclude=None):
+    """Top-k per row of a score matrix [R, I] (score desc, ties -> lower column).  `exclude`: an (indptr, ids) CSR
+    of columns to leave out per row (the input is not modified); rows left short are padded with (-inf, -1)."""
     scores = _f32(scores, "scores")
     R, I = scores.shape
+    if exclude is not None:
+        scores = mask_excluded(scores.clone(), exclude[0], exclude[1], 0)
     k = min(int(k), I)
     if k > MAX_FUSED_K:
         # the kernel selects at most 32 per pass: take 32, strike them out of a copy, repeat (the tie rule carries over:
@@ -384,7 +487,7 @@ def topk_rows(scores, k):
         for k0 in range(0, k, MAX_FUSED_K):
             v, j = topk_rows(work, min(MAX_FUSED_K, k - k0))
             vs.append(v); js.append(j)
-            work.scatter_(1, j.long(), float("-inf"))
+            work.scatter_(1, j.long().clamp_min(0), float("-inf"))      # a -1 pad: the row has nothing left above -inf
         return torch.cat(vs, 1), torch.cat(js, 1)
     vals = torch.empty((R, k), dtype=torch.float32, device=scores.device)
     ids = torch.empty((R, k), dtype=torch.int32, device=scores.device)

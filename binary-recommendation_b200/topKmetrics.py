@@ -25,17 +25,46 @@ def device_topk(user_vectors, item_vectors, k):
     return H.BruteForceIndex(k).index(item_vectors)(user_vectors)
 
 
-def topKRatings(k, model, usersId, itemsId, mtype=None):
+def exclusion_pairs_csr(pairs, usersId, itemsId, device):
+    """(user, item) pairs in the caller's id space -> exclusion CSR (hotpath.exclusion_csr) over the positions of
+    usersId (rows) and itemsId (columns).  Pairs whose user or item is not listed are ignored; an id listed twice
+    gets the pair at each of its positions."""
+    upos, ipos = {}, {}
+    for r, u in enumerate(usersId):
+        upos.setdefault(u, []).append(r)
+    for c, i in enumerate(itemsId):
+        ipos.setdefault(i, []).append(c)
+    rows, cols = [], []
+    for u, i in pairs:
+        ru, ci = upos.get(u), ipos.get(i)
+        if ru is not None and ci is not None:
+            for r in ru:
+                rows.extend([r] * len(ci)); cols.extend(ci)
+    return H.exclusion_csr(np.asarray(rows, dtype=np.int64), np.asarray(cols, dtype=np.int64), len(usersId), device)
+
+
+def topKRatings(k, model, usersId, itemsId, mtype=None, exclude=None):
     """Top-k (score, item) lists for every user in usersId over the catalog itemsId.
     `model` must offer score_vectors(usersId, itemsId) -> (user_vectors, item_vectors) for dot-product
     models (BPR, two-tower), or score_all(usersId, itemsId, k) for models with a non-factorised
-    scorer (mtype == "NFC": NeuMF, reference topKmetrics.py:29-33)."""
+    scorer (mtype == "NFC": NeuMF, reference topKmetrics.py:29-33).  `exclude`: (user, item) pairs to leave out of
+    that user's list, such as the training interactions; pairs outside usersId / itemsId are ignored.  A user with
+    fewer than k items left gets a shorter list."""
     usersId = list(usersId); itemsId = list(itemsId)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    csr = None if exclude is None else exclusion_pairs_csr(exclude, usersId, itemsId, getattr(model, "device", dev))
     if mtype == "NFC" or not hasattr(model, "score_vectors"):
-        vals, idx = model.score_all(usersId, itemsId, k)
+        if csr is None:
+            vals, idx = model.score_all(usersId, itemsId, k)
+        else:
+            vals, idx = model.score_all(usersId, itemsId, k, exclude=csr)
     else:
         uv, iv = model.score_vectors(usersId, itemsId)
-        vals, idx = device_topk(uv, iv, k)
+        if csr is None:
+            vals, idx = device_topk(uv, iv, k)
+        else:
+            csr = (csr[0].to(uv.device), csr[1].to(uv.device))
+            vals, idx = H.BruteForceIndex(k).index(iv).query_with_exclusions(uv, csr)
     vals = vals.cpu().numpy(); idx = idx.cpu().numpy()
     return [(u, [(vals[r, j], itemsId[idx[r, j]]) for j in range(idx.shape[1]) if idx[r, j] >= 0])
             for r, u in enumerate(usersId)]

@@ -22,7 +22,7 @@ import torch
 from . import _native as N
 from . import distributed as D
 from . import hotpath as H
-from .topKmetrics import topKMetrics
+from .topKmetrics import exclusion_pairs_csr, topKMetrics
 
 
 class StringLookup:
@@ -344,15 +344,23 @@ class TwoTowerModel:
 
     __call__ = call
 
-    def predict(self, usersId, batch_size=5000):
-        """(scores ndarray [U,k], identifiers list-of-lists [U][k]) like model.predict(usersId) at :230."""
+    def predict(self, usersId, batch_size=5000, exclude=None):
+        """(scores ndarray [U,k], identifiers list-of-lists [U][k]) like model.predict(usersId) at :230.  `exclude`:
+        (user, item) pairs in raw ids to leave out of that user's list (items are matched against setCandidates);
+        a user left with fewer than k candidates gets a shorter identifier list, its score row ends in -inf."""
         usersId = list(usersId)
+        csr = None if exclude is None else exclusion_pairs_csr(exclude, usersId, self._candidates, self.device)
         vs, ixs = [], []
         for s in range(0, len(usersId), batch_size):
-            v, ix = self.call(usersId[s:s + batch_size])
+            if csr is None:
+                v, ix = self.call(usersId[s:s + batch_size])
+            else:
+                info = usersId[s:s + batch_size]
+                q = self._tower_forward(self.userTower, torch.from_numpy(self.userTowerIn(info)).to(self.device))
+                v, ix = self.bruteForceLayer.query_with_exclusions(q, (csr[0][s:s + len(info) + 1], csr[1]))
             vs.append(v); ixs.append(ix)
         v = torch.cat(vs).cpu().numpy(); ix = torch.cat(ixs).cpu().numpy()
-        idents = [[self._candidates[j] for j in row] for row in ix]
+        idents = [[self._candidates[j] for j in row if j >= 0] for row in ix]
         return v, idents
 
     def score_vectors(self, usersId, itemsId):
@@ -380,11 +388,14 @@ def splitTrainTest(data, ratio, seed=0):
 
 def crossValidation(dataSets, k, learningRate, optimiser, loss, epoch, embNum, batchSize, randomZero=False,
                     rdZeroDataSets=None, testBatchSize=5000, semb=64, userKey="CUSTOMER_ID", itemKey="MATERIAL",
-                    resKey="RATING_TYPE", seed=42, verbose=0, rdZeroFilenames=None, bname=None):
+                    resKey="RATING_TYPE", seed=42, verbose=0, rdZeroFilenames=None, bname=None, excludeTrain=False):
     """k-fold cross-validation of twoTower.py:125-272 on in-memory folds (dicts of columns) or, like the reference,
     on a list of file names read through loadBinaryMovieLens.gfData: train on all folds but one,
     index the whole catalog, top-k for every user, topKMetrics against the held-out fold and against
-    the training folds ("full_" keys), averaged over folds."""
+    the training folds ("full_" keys), averaged over folds.
+    excludeTrain=True leaves each user's pairs of the training folds of dataSets out of their list (pairs added by
+    rdZeroDataSets are not excluded), the held-out protocol's usual form; the "full_" metrics then count no hits
+    by construction."""
     # keyword names of the reference's signature (twoTower.py:125): rdZeroFilenames = the folds with randomly added
     # zeros; bname = directory of its resource-usage logger (benchmarkLogger, out of scope here: accepted, unused)
     if rdZeroDataSets is None and rdZeroFilenames is not None:
@@ -411,11 +422,12 @@ def crossValidation(dataSets, k, learningRate, optimiser, loss, epoch, embNum, b
         model.compile(optimiser, learningRate=learningRate)
         model.fit(batch_dataset(train, batchSize, keys), epochs=epoch, verbose=verbose)
         model.setCandidates(matId, k)
-        scores, idents = model.predict(usersId, batch_size=testBatchSize)
+        others = [f for j, f in enumerate(folds) if j != it]
+        seen = [(u, m) for f in others for u, m in zip(f[userKey], f[itemKey])]
+        scores, idents = model.predict(usersId, batch_size=testBatchSize, exclude=seen if excludeTrain else None)
         topk = [(u, [(scores[r][j], idents[r][j]) for j in range(len(idents[r]))]) for r, u in enumerate(usersId)]
         res.append(topKMetrics(topk, list(zip(test[userKey], test[itemKey])), usersId, matId))
-        others = [f for j, f in enumerate(folds) if j != it]
-        fullRes.append(topKMetrics(topk, [(u, m) for f in others for u, m in zip(f[userKey], f[itemKey])], usersId, matId))
+        fullRes.append(topKMetrics(topk, seen, usersId, matId))
     averageMetrics = {}
     for m in res[0]:
         averageMetrics[m] = sum(r[m] for r in res) / len(folds)

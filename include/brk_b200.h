@@ -438,6 +438,26 @@ int64_t brk_score_topk_workspace_bytes(brk_ctx* ctx, int64_t U, int64_t I, int32
 int brk_score_topk_bf16(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* c_bf16,
                         int64_t I, int32_t dpad, int32_t k, int32_t id_offset, float* out_vals,
                         int32_t* out_ids, void* workspace, int64_t workspace_bytes, void* stream);
+/* Per-row exclusions (TFRS TopK.query_with_exclusions): the same top-k with row r's listed global ids left out.
+ * A global id is the local candidate index plus id_offset, the id space of the results, so one list serves every
+ * item-range shard.  Per row: the first k candidates that are not listed and score > -inf, by descending score, ties
+ * -> lower id; (-inf, -1) pads a row with fewer.  Listed ids outside [id_offset, id_offset + I) are ignored, and so
+ * are duplicates; with every list empty the result equals brk_score_topk_bf16's bit for bit.
+ *   excl_indptr  int64 [U+1], absolute offsets into excl_ids: row r lists excl_ids[excl_indptr[r] .. excl_indptr[r+1]).
+ *                It may be a view into a longer indptr (a chunk of rows passes indptr + s0, no rebasing).
+ *   excl_ids     int32, ascending within each row (a precondition the caller guarantees).
+ * Both are required (BRK_E_ARG if NULL); id_offset + I rounded up to 128 must stay below INT32_MAX.  The workspace
+ * size is brk_score_topk_workspace_bytes(...).  Listed ids are tested only for items that beat the row's running
+ * k-th best, so lists cost little unless they hold the row's best items. */
+int brk_score_topk_bf16_excl(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* c_bf16, int64_t I,
+                             int32_t dpad, int32_t k, int32_t id_offset, const int64_t* excl_indptr,
+                             const int32_t* excl_ids, float* out_vals, int32_t* out_ids, void* workspace,
+                             int64_t workspace_bytes, void* stream);
+/* The same exclusions on a materialised score matrix [R, I] (row-major): scores[r, id - col_offset] = -inf for every
+ * listed id of row r inside [col_offset, col_offset + I), CSR as above.  brk_topk_rows afterwards gives the
+ * exclusion semantics (it never selects -inf and pads with -1). */
+int brk_mask_excluded(brk_ctx* ctx, float* scores, int64_t R, int64_t I, int32_t col_offset,
+                      const int64_t* excl_indptr, const int32_t* excl_ids, void* stream);
 /* Top-k per row of a materialised score matrix [R, I] (models without a factorised scorer: NeuMF,
  * trainers/topKmetrics.py:29-33 + __topk :51-72); same ordering rule; ids are column indices,
  * -1 pads rows with fewer than k columns. */
