@@ -208,11 +208,8 @@ template <int BN, int A_MN, int B_MN>
 int launch(brk_ctx* ctx, const Params& P, int splits, cudaStream_t st) {
   const size_t pipe = size_t(STAGES) * size_t(BM * KC * 4 + BN * KC * 4), stagec = size_t(BM) * (BN + 4) * 4;
   const size_t smem = (pipe > stagec ? pipe : stagec) + 1024;
-  static bool done = false;
-  if (!done) {
-    BRK_CUDA(cudaFuncSetAttribute(gemm_tf32_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    done = true;
-  }
+  // the shared-memory opt-in is per device: set it for the current one on every call
+  BRK_CUDA(cudaFuncSetAttribute(gemm_tf32_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   dim3 grid((P.N + BN - 1) / BN, (P.M + BM - 1) / BM, splits);
   gemm_tf32_kernel<BN, A_MN, B_MN><<<grid, NT, smem, st>>>(P);
   BRK_LAUNCH_CHECK();

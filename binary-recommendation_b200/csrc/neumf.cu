@@ -669,15 +669,12 @@ int run_neumf(brk_ctx* ctx, const NeumfArgs& A, cudaStream_t st) {
                            size_t(kTile) * (pad4(H3) + 4) + size_t(kTile) * (2 * E + 4) + 4 * H2 + size_t(kTile) * (H3 + 2)) + 2 * kTile * 4;
   const size_t smD = bytes(size_t(kTile) * (pad4(H1) + 4) * 2 + H1 * pad4(H2) + size_t(kTile) * (pad4(H2) + 4) + 4 * H1 + 5 * H2);
   const size_t smE = bytes(size_t(kTile) * (2 * E + 4) + 2 * E * pad4(H1) + size_t(kTile) * (pad4(H1) + 4) + 5 * H1) + 2 * kTile * 4;
-  static bool attr_done = false;
-  if (!attr_done) {
-    BRK_CUDA(cudaFuncSetAttribute(neumf_fwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smA)));
-    BRK_CUDA(cudaFuncSetAttribute(neumf_fwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smB)));
-    BRK_CUDA(cudaFuncSetAttribute(neumf_head<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smC)));
-    BRK_CUDA(cudaFuncSetAttribute(neumf_bwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smD)));
-    BRK_CUDA(cudaFuncSetAttribute(neumf_bwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smE)));
-    attr_done = true;
-  }
+  // the shared-memory opt-in is per device: set it for the current one on every call
+  BRK_CUDA(cudaFuncSetAttribute(neumf_fwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smA)));
+  BRK_CUDA(cudaFuncSetAttribute(neumf_fwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smB)));
+  BRK_CUDA(cudaFuncSetAttribute(neumf_head<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smC)));
+  BRK_CUDA(cudaFuncSetAttribute(neumf_bwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smD)));
+  BRK_CUDA(cudaFuncSetAttribute(neumf_bwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smE)));
   neumf_fwd1<E, H1, H2, H3, ACT><<<grid, kTile, smA, st>>>(A);
   neumf_fwd2<E, H1, H2, H3, ACT><<<grid, kTile, smB, st>>>(A);
   neumf_head<E, H1, H2, H3, ACT><<<grid, kTile, smC, st>>>(A);

@@ -581,15 +581,12 @@ int run(brk_ctx* ctx, const Args& A, cudaStream_t st) {
                         size_t(TS) * v2::zpitch<H3>() + 2 * TS + 4 * H2);
   const size_t smD = by(size_t(2 * H1) * PT + H1 * H2 + size_t(H2) * PT + size_t(TS) * v2::zpitch<H2>() + 4 * H1 + 5 * H2);
   const size_t smE = by(size_t(2 * E) * PT + 2 * E * H1 + size_t(H1) * PT + size_t(TS) * v2::zpitch<H1>() + 5 * H1);
-  static bool attr_done = false;
-  if (!attr_done) {
-    BRK_CUDA(cudaFuncSetAttribute(fwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smA)));
-    BRK_CUDA(cudaFuncSetAttribute(fwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smB)));
-    BRK_CUDA(cudaFuncSetAttribute(head<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smC)));
-    BRK_CUDA(cudaFuncSetAttribute(bwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smD)));
-    BRK_CUDA(cudaFuncSetAttribute(bwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smE)));
-    attr_done = true;
-  }
+  // the shared-memory opt-in is per device: set it for the current one on every call
+  BRK_CUDA(cudaFuncSetAttribute(fwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smA)));
+  BRK_CUDA(cudaFuncSetAttribute(fwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smB)));
+  BRK_CUDA(cudaFuncSetAttribute(head<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smC)));
+  BRK_CUDA(cudaFuncSetAttribute(bwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smD)));
+  BRK_CUDA(cudaFuncSetAttribute(bwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smE)));
   fwd1<E, H1, H2, H3, ACT><<<grid, NT, smA, st>>>(A);
   fwd2<E, H1, H2, H3, ACT><<<grid, NT, smB, st>>>(A);
   head<E, H1, H2, H3, ACT><<<grid, NT, smC, st>>>(A);

@@ -1052,14 +1052,16 @@ int run(brk_ctx* ctx, const Args& A, cudaStream_t st) {
                         size_t(H3) * SP + size_t(TS) * (H3 + 1) + 2 * TS + 4 * H2);
   const size_t smD = by(size_t(TS) * pad32(H1) + 2 * size_t(TS) * pad32(H2) + H1 * pad32(H2) + size_t(H1) * SP + 4 * H1 + 5 * H2);
   const size_t smE = by(size_t(TS) * K0 + 2 * size_t(TS) * pad32(H1) + K0 * pad32(H1) + TS * (K0 / 32) + 5 * H1);
-  static bool attr_done = false;
+  // the shared-memory opt-in is per device: set it for the current one on every call; the occupancy caps below are
+  // properties of the kernels, computed once
+  BRK_CUDA(cudaFuncSetAttribute(tc_fwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smA)));
+  BRK_CUDA(cudaFuncSetAttribute(tc_fwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smB)));
+  BRK_CUDA(cudaFuncSetAttribute(tc_head<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smC)));
+  BRK_CUDA(cudaFuncSetAttribute(tc_bwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smD)));
+  BRK_CUDA(cudaFuncSetAttribute(tc_bwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smE)));
+  static bool occ_done = false;
   static int occ_d = 0, occ_e = 0, occ_c = 0;
-  if (!attr_done) {
-    BRK_CUDA(cudaFuncSetAttribute(tc_fwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smA)));
-    BRK_CUDA(cudaFuncSetAttribute(tc_fwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smB)));
-    BRK_CUDA(cudaFuncSetAttribute(tc_head<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smC)));
-    BRK_CUDA(cudaFuncSetAttribute(tc_bwd2<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smD)));
-    BRK_CUDA(cudaFuncSetAttribute(tc_bwd1<E, H1, H2, H3, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smE)));
+  if (!occ_done) {
     // persistent grids: CTAs per SM by shared memory (227 KB), registers (2 x 256 threads) and TMEM (512 columns:
     // bwd2 allocates 128, bwd1 256 per CTA)
     occ_d = int((227 * 1024) / (smD + 1024)); if (occ_d > 2) occ_d = 2;
@@ -1083,7 +1085,7 @@ int run(brk_ctx* ctx, const Args& A, cudaStream_t st) {
               fa.numRegs, fa.sharedSizeBytes, smC, occ_c, occ_d, occ_e, smD, smE);
     }
     BRK_REQUIRE(occ_d > 0 && occ_e > 0 && occ_c > 0, BRK_E_STATE, "brk_neumf_step: tensor-core kernels do not fit");
-    attr_done = true;
+    occ_done = true;
   }
   {
     static unsigned long long* trace_set = nullptr;

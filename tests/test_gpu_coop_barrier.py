@@ -72,8 +72,17 @@ def test_neumf_graph_replay_equals_eager_steps(dev, variant):
     _assert_bit_equal(_neumf_state(a, la), _neumf_state(b, lb))
 
 
-def _run_on(dev):
-    """One NeuMF tensor-core step, one BPR train_steps launch and one two-tower step on `dev`."""
+def _neumf_grads(net, loss, out):
+    """Loss, predictions and the gradients of the four tables and the dense block after forward_backward (on the host)."""
+    tabs = dict(zip(("uMLP", "iMLP", "uMF", "iMF", "dense"), net.tables() + [net.dense]))
+    return dict({f"{name}.g": t.g.cpu().numpy() for name, t in tabs.items()}, loss=loss.cpu().numpy(), out=out.cpu().numpy())
+
+
+def _run_on(dev, monkeypatch):
+    """One NeuMF tensor-core step, one BPR train_steps launch and one two-tower step on `dev`; then the multi-kernel
+    launchers whose kernels ask for more than 48 KB of shared memory: the five-kernel tensor-core NeuMF step
+    (csrc/neumf_tc.cu), the fp32 tiled one (csrc/neumf2.cu), the script spec's (csrc/neumf.cu) and the multi-kernel
+    two-tower step (csrc/gemm_tc.cu)."""
     from binrec_b200.BPRModel import BPRNet
     from binrec_b200.NeuMFModel import NeuMFNet
     from binrec_b200.twoTower import TwoTowerModel
@@ -81,6 +90,16 @@ def _run_on(dev):
         net = NeuMFNet(U, I, 32, dropout=0.2, device=dev, tensor_cores=True)
         nl, _ = net.train_on_batch(*(torch.from_numpy(x).to(dev) for x in _distinct_rows_batch(3, 2048)), first_index=7, epoch=1)
         neumf = _neumf_state(net, nl)
+
+        multi = {}
+        monkeypatch.setenv("BRK_NEUMF_NO_FUSED", "1")
+        for name, E, kw in (("five_kernel", 64, dict(tensor_cores=True)), ("fp32_tiled", 32, dict(tensor_cores=False)),
+                            ("script_spec", 10, dict(hidden=(100, 50, 10), tensor_cores=False))):
+            net = NeuMFNet(U, I, E, dropout=0.2, device=dev, **kw)
+            batch = (torch.from_numpy(x).to(dev) for x in _distinct_rows_batch(4, 2048))
+            loss, out = net.forward_backward(*batch, first_index=7, epoch=1)
+            multi[name] = _neumf_grads(net, loss, out)
+        monkeypatch.delenv("BRK_NEUMF_NO_FUSED")
 
         rng = np.random.default_rng(5)
         Ub, Ib, B = 400, 300, 512
@@ -100,21 +119,47 @@ def _run_on(dev):
         tl = tt.train_step(info)["loss"].item()
         tabs = {f"{n}.{t}": getattr(getattr(tt, n), t) for n in ("userTower", "itemTower") for t in ("emb", "dense")}
         tt_out = (tl, {f"{name}.{k}": getattr(tab, k).cpu().numpy() for name, tab in tabs.items() for k in "wm"})
+
+        # multi-kernel two-tower step: every product through gemm_tf32 (leading dimensions multiples of 4)
+        monkeypatch.setenv("BRK_TT_NO_FUSED", "1")
+        tt = TwoTowerModel(64, 200, 300, "CUSTOMER_ID", "MATERIAL", users, items, semb=64, device=dev, tensor_cores=True)
+        tt.compile("Adagrad", learningRate=0.1)
+        info = {"CUSTOMER_ID": [users[j] for j in rng.integers(0, 300, 512)],
+                "MATERIAL": [items[j] for j in (200 * rng.random(512) ** 2).astype(np.int64)]}
+        tl = tt.train_step(info)["loss"].item()
+        monkeypatch.delenv("BRK_TT_NO_FUSED")
+        tabs = {f"{n}.{t}": getattr(getattr(tt, n), t) for n in ("userTower", "itemTower") for t in ("emb", "dense")}
+        multi["twotower"] = (tl, {f"{name}.{k}": getattr(tab, k).cpu().numpy() for name, tab in tabs.items() for k in "wm"})
         torch.cuda.synchronize()
-    return neumf, bpr_out, tt_out
+    return neumf, bpr_out, tt_out, multi
 
 
-def test_cooperative_steps_on_two_devices_in_one_process():
+def _assert_twotower_close(t1, t0):
+    np.testing.assert_allclose(t1[0], t0[0], rtol=1e-5)
+    for k in t0[1]:
+        np.testing.assert_allclose(t1[1][k], t0[1][k], rtol=1e-4, atol=2e-5 if k.endswith(".w") else 1e-6, err_msg=k)
+
+
+def test_cooperative_steps_on_two_devices_in_one_process(monkeypatch):
     """Each device's context has its own barrier words and its own shared-memory opt-in of the kernels: the same steps
     on cuda:1, after cuda:0 ran them in this process, give what cuda:0 gave.  BPR and two-tower repeat rows, so they are
-    held to the tolerances of two runs of the same step (tests/test_gpu_bpr_staged.py, tests/test_gpu_twotower.py)."""
+    held to the tolerances of two runs of the same step (tests/test_gpu_bpr_staged.py, tests/test_gpu_twotower.py).  The
+    multi-kernel NeuMF steps sum their dense gradients with REDs in no fixed order: their loss and predictions are held to
+    rtol 1e-5, each gradient tensor to 1e-5 of its largest entry (compared before the optimizer: Adam would turn the
+    last-bit noise of a near-zero gradient into a step of +-lr)."""
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
-    (n0, b0, t0), (n1, b1, t1) = _run_on(torch.device("cuda:0")), _run_on(torch.device("cuda:1"))
+    (n0, b0, t0, m0), (n1, b1, t1, m1) = _run_on(torch.device("cuda:0"), monkeypatch), _run_on(torch.device("cuda:1"), monkeypatch)
     _assert_bit_equal(n1, n0)
     np.testing.assert_allclose(b1[0], b0[0], rtol=1e-5, atol=1e-7)
     for k in b0[1]:
         np.testing.assert_allclose(b1[1][k], b0[1][k], rtol=1e-5, atol=1e-7, err_msg=k)
-    np.testing.assert_allclose(t1[0], t0[0], rtol=1e-5)
-    for k in t0[1]:
-        np.testing.assert_allclose(t1[1][k], t0[1][k], rtol=1e-4, atol=2e-5 if k.endswith(".w") else 1e-6, err_msg=k)
+    _assert_twotower_close(t1, t0)
+    _assert_twotower_close(m1.pop("twotower"), m0.pop("twotower"))
+    for name in m0:
+        for k, want in m0[name].items():
+            got = m1[name][k]
+            if k.endswith(".g"):
+                assert np.abs(got - want).max() <= 1e-5 * np.abs(want).max(), (name, k)
+            else:
+                np.testing.assert_allclose(got, want, rtol=1e-5, atol=1e-7, err_msg=f"{name} {k}")

@@ -110,7 +110,7 @@ def test_bpr_batch_of_one_and_all_samples_on_one_row(dev):
 
 
 def test_lazy_adam_moves_exactly_the_batch_rows_on_a_large_table(dev):
-    rows, d, n = 2_000_000, 64, 65_536
+    rows, d, n = ROWS_SCAN, 64, 65_536
     g = torch.Generator(device=dev); g.manual_seed(3)
     tab = H().Table(torch.empty(rows, d, device=dev).uniform_(-0.05, 0.05, generator=g))
     w0 = tab.w.clone()
@@ -125,6 +125,100 @@ def test_lazy_adam_moves_exactly_the_batch_rows_on_a_large_table(dev):
     # first Adam step with g > 0: every coordinate of a hit row moves by -lr (up to rounding)
     step = (tab.w - w0)[hit]
     torch.testing.assert_close(step, torch.full_like(step, -1e-3), rtol=1e-3, atol=1e-7)
+
+
+# ---- values of the row-sparse optimizers (csrc/optim.cu rows_pass) where its bitmask scan merges slots ---------------
+# rows_pass gives each warp up to 32 bitmask words per slot, taken `stride` words apart; a warp owns several slots only
+# when the table has more than 32 words per warp of the grid (SMs x 2 CTAs x 8 warps: ~2.4 M rows on a B200).  There it
+# prefetches the next slot's words, carries a partial row list (< gpw * 4 rows) into the next slot and flushes on its
+# last slot.  6 000 017 rows is past that even at 4 CTAs per SM, and its last bitmask word holds 17 rows.
+ROWS_SCAN = 6_000_017
+
+
+def _pattern(name, rows, gen, dev):
+    n = 65_536
+    if name == "uniform":                  # sparse slots: their rows are carried into the next slot's list
+        return torch.randint(0, rows, (n,), generator=gen, device=dev, dtype=torch.int32)
+    if name == "cubic":                    # a crowded neighbourhood that the stride layout spreads over many warps
+        return (rows * torch.rand(n, generator=gen, device=dev, dtype=torch.float64) ** 3).to(torch.int32).clamp_(max=rows - 1)
+    if name == "all":                      # every slot flushes full 1024-row lists
+        return torch.arange(rows, device=dev, dtype=torch.int32)
+    if name == "last":                     # the partial last word alone
+        return torch.full((1,), rows - 1, device=dev, dtype=torch.int32)
+    if name == "uniform+last":
+        return torch.cat([_pattern("uniform", rows, gen, dev), _pattern("last", rows, gen, dev)])
+    raise ValueError(name)
+
+
+def _prepare(tab, ids, gen):
+    """Random-normal gradients scattered into the accumulator (duplicates summed, rows marked), then the touched rows'
+    w / m / v / g gathered to the host in float64 and device copies of the slots, for the untouched rows."""
+    H().scatter_add_rows(tab.g, ids, torch.randn(ids.numel(), tab.d, generator=gen, device=tab.w.device), tab.touched)
+    rows = torch.unique(ids.long())
+    slots = [k for k in "wmv" if getattr(tab, k) is not None]
+    host = {k: getattr(tab, k)[rows].double().cpu().numpy() for k in slots + ["g"]}
+    return rows, host, {k: getattr(tab, k).clone() for k in slots}
+
+
+def _check_rows(tab, rows, want, before, tag):
+    """Touched rows against the float64 reference, untouched rows bit-identical, accumulator and bitmask left zero."""
+    untouched = torch.ones(tab.rows, dtype=torch.bool, device=tab.w.device)
+    untouched[rows] = False
+    for k in before:
+        got = getattr(tab, k)[rows].double().cpu().numpy()
+        print(f"{tag} {k}: touched rows {rows.numel()}, max |err| {np.abs(got - want[k]).max():.2e}")
+        np.testing.assert_allclose(got, want[k], rtol=1e-5, atol=1e-6, err_msg=f"{tag} {k}")
+        assert torch.equal(getattr(tab, k)[untouched], before[k][untouched]), (tag, k)
+    assert not tab.g.any().item() and not tab.touched.any().item(), tag
+
+
+# the hyper-parameters as the kernels hold them (float32, as Keras does): 1 - beta_2 is then 1 - 0.999f = 0.00099998713,
+# 1.3e-5 away from 0.001 -- more than rtol 1e-5 wherever v is large
+_F32 = lambda x: float(np.float32(x))                                    # noqa: E731
+ADAM_HYPER = dict(lr=_F32(1e-3), beta1=_F32(0.9), beta2=_F32(0.999), eps=_F32(1e-7))
+ADAGRAD_HYPER = dict(lr=_F32(0.1), eps=_F32(1e-7))
+
+
+def _lazy_adam_step(opt, tabs, patterns, gen, t, tag):
+    """One Adam.apply (one brk_adam_rows call over every table) against oracle/embedding.py adam_rows_lazy at step t."""
+    from oracle import embedding as OE
+    prep = [_prepare(tab, _pattern(p, tab.rows, gen, tab.w.device), gen) for tab, p in zip(tabs, patterns)]
+    opt.apply(tabs)
+    assert int(opt.state[0].item()) == t
+    for tab, p, (rows, host, before) in zip(tabs, patterns, prep):
+        OE.adam_rows_lazy(host["w"], host["m"], host["v"], host["g"], np.arange(rows.numel()), t, **ADAM_HYPER)
+        _check_rows(tab, rows, host, before, f"{tag} d={tab.d} {p} t={t}")
+
+
+@pytest.mark.parametrize("d,first,second", [(4, "all", "last"), (10, "uniform", "cubic"), (64, "cubic", "uniform+last")])
+def test_row_sparse_optimizers_match_the_oracle_on_a_large_table(dev, d, first, second):
+    """d = 4: one lane per row (float4), a list flushed once 128 rows are waiting; d = 10: the scalar path (rows not a
+    multiple of 4 floats); d = 64: 16 lanes per row.  Two lazy-Adam steps (t = 1, 2) with different row sets, then one
+    sparse Adagrad step on a fresh table.  Touched rows: w / m / v at rtol 1e-5 / atol 1e-6 of the float64 reference
+    computed from the same float32 inputs; untouched rows bit-identical."""
+    from oracle import embedding as OE
+    gen = torch.Generator(device=dev); gen.manual_seed(d)
+    tab = H().Table(torch.empty(ROWS_SCAN, d, device=dev).uniform_(-0.05, 0.05, generator=gen))
+    opt = H().Adam(1e-3, sparse="lazy", device=dev)
+    _lazy_adam_step(opt, [tab], [first], gen, 1, "lazy Adam")
+    _lazy_adam_step(opt, [tab], [second], gen, 2, "lazy Adam")
+    del tab, opt
+    tab = H().Table(torch.empty(ROWS_SCAN, d, device=dev).uniform_(-0.05, 0.05, generator=gen), slots=1, slot_init=0.1)
+    rows, host, before = _prepare(tab, _pattern(first, ROWS_SCAN, gen, dev), gen)
+    H().Adagrad(0.1, rows_threshold_bytes=0).apply([tab])
+    OE.adagrad_rows(host["w"], host["m"], host["g"], np.arange(rows.numel()), **ADAGRAD_HYPER)
+    _check_rows(tab, rows, host, before, f"Adagrad d={d} {first}")
+
+
+def test_lazy_adam_over_three_tables_of_different_widths_in_one_call(dev):
+    """One brk_adam_rows call over three tables: the per-table state of the scan (row list, prefetch) restarts at every
+    table.  100 003 x 256: 64 float4 chunks per row, more than a warp's 32 lanes (the chunk loop of the scalar path)."""
+    gen = torch.Generator(device=dev); gen.manual_seed(17)
+    tabs = [H().Table(torch.empty(r, d, device=dev).uniform_(-0.05, 0.05, generator=gen))
+            for r, d in ((ROWS_SCAN, 4), (100_003, 256), (ROWS_SCAN, 64))]
+    opt = H().Adam(1e-3, sparse="lazy", device=dev)
+    _lazy_adam_step(opt, tabs, ["cubic", "uniform+last", "uniform"], gen, 1, "three tables")
+    _lazy_adam_step(opt, tabs, ["uniform+last", "cubic", "last"], gen, 2, "three tables")
 
 
 def test_bpr_twenty_bench_identical_steps_match_the_oracle(dev):
