@@ -67,6 +67,10 @@ class brk_twotower_workspace(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("eu", "ei", "q", "c", "dq", "dc", "scores", "ones", "acc", "deu", "dei")]
 
 
+class brk_twotower_shards(C.Structure):
+    _fields_ = [("user", brk_shards), ("item", brk_shards)]
+
+
 _P, _I32, _I64, _U32, _F32, _F64 = C.c_void_p, C.c_int32, C.c_int64, C.c_uint32, C.c_float, C.c_double
 
 # name -> (restype, argtypes); mirrors include/brk_b200.h one to one.
@@ -127,6 +131,9 @@ SIGNATURES = {
                                     C.POINTER(brk_twotower_workspace), _P, _P]),
     "brk_twotower_train_step": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), _P, _P, _P, _P, _I64, _I32,
                                           C.POINTER(brk_twotower_workspace), _F32, _F32, _I64, _P, _P]),
+    "brk_twotower_step_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards), _P,
+                                            _P, _P, _P, _I64, _I32, C.POINTER(brk_twotower_workspace), _P, _P]),
+    "brk_tower_forward_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_shards), _P, _I64, _P, _P, _P]),
     "brk_bf16_padded_dim": (C.c_int32, [_I32]),
     "brk_rows_to_bf16": (C.c_int, [_P, _P, _I64, _I32, _P, _I32, _P]),
     "brk_score_topk_workspace_bytes": (C.c_int64, [_P, _I64, _I64, _I32]),

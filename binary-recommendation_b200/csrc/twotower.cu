@@ -114,7 +114,8 @@ __global__ void __launch_bounds__(128) colsum_kernel(const float* __restrict__ X
 }  // namespace
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
-                            float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps);   // twotower_fused.cu
+                            float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
+                            const brk_twotower_shards* sh);                                                       // twotower_fused.cu
 int brk_gemm_tf32_impl(brk_ctx* ctx, const float* A, const float* B, float* C, const float* bias, int M, int N, int K, int lda,
                        int ldb, int ldc, int trans_a, int trans_b, float alpha, int accumulate, bool allow_split,
                        cudaStream_t st);
@@ -208,9 +209,11 @@ extern "C" int brk_sgemm(brk_ctx* ctx, const float* A, const float* B, float* C,
                true);
 }
 
+// sh != nullptr: the rows come from the row-sharded table sh instead of t->emb
 static int tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t* ids, int64_t n, float* emb_out, float* out,
-                         int tcore, void* stream) {
-  int rc = brk_gather_rows(ctx, t->emb.w, t->emb.rows, t->E, ids, n, emb_out, stream);
+                         int tcore, void* stream, const brk_shards* sh = nullptr) {
+  int rc = sh ? brk_gather_rows_sharded(ctx, sh, t->E, ids, n, emb_out, stream)
+              : brk_gather_rows(ctx, t->emb.w, t->emb.rows, t->E, ids, n, emb_out, stream);
   if (rc) return rc;
   const float* W = t->dense.w;                       // [E, S] Keras kernel, then bias [S]
   return gemm(ctx, (cudaStream_t)stream, tcore, emb_out, W, out, W + int64_t(t->E) * t->S, int(n), t->S, t->E, t->E, t->S,
@@ -224,27 +227,22 @@ extern "C" int brk_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t
   return tower_forward(ctx, t, ids, n, emb_out, out, 0, stream);
 }
 
-extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
-                                 const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
-                                 int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
-                                 void* stream) {
+// The step after argument checks (brk_twotower_step, brk_twotower_step_sharded).  sh != nullptr: the embedding rows are
+// gathered from and their gradients scattered into the row-sharded tables sh instead of user->emb / item->emb.
+static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
+                         const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                         int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out, void* stream) {
   // mode bit 8 (0x100): Dense / in-batch products on the tensor cores (TF32 operands, gemm_tc.cu)
   const int tcore = (mode & 0x100) ? 1 : 0;
   mode &= 0xFF;
-  BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_step: null argument");
-  BRK_REQUIRE(user->S == item->S && batch > 0 && batch < (1 << 30), BRK_E_ARG, "brk_twotower_step: S %d vs %d, batch %lld",
-              user->S, item->S, (long long)batch);
-  BRK_REQUIRE(mode == 0 || labels, BRK_E_ARG, "brk_twotower_step: rdZero mode needs labels");
-  BRK_REQUIRE(ws->eu && ws->ei && ws->q && ws->c && ws->dq && ws->dc && ws->acc && (mode != 0 || ws->scores), BRK_E_ARG,
-              "brk_twotower_step: workspace missing");
-  BRK_REQUIRE(!training || (user->emb.g && item->emb.g && user->dense.g && item->dense.g && ws->deu && ws->dei), BRK_E_ARG,
-              "brk_twotower_step: gradient accumulators / deu, dei workspace missing");
   cudaStream_t st = (cudaStream_t)stream;
   const int B = int(batch), S = user->S, Eu = user->E, Ei = item->E;
+  const brk_shards* tsh[2] = {sh ? &sh->user : nullptr, sh ? &sh->item : nullptr};
   int rc;
   if (mode == 0 && tcore) {                         // the whole step as one cooperative launch when the batch fits on chip
     int handled = 0;
-    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, training, ws, loss_out, st, &handled, 0, 0.f, 0.f))) return rc;
+    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, training, ws, loss_out, st, &handled, 0, 0.f, 0.f,
+                                      sh))) return rc;
     if (handled) return 0;
   }
   // The user chain and the item chain are independent until the score product and again after the loss gradient, and
@@ -262,9 +260,9 @@ extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_
   // towers: q = Eu[u] Wu + bu, c = Ei[i] Wi + bi
   BRK_FORK(ctx, st, 0);
   if (training && mode == 0) BRK_CUDA(cudaMemsetAsync(dz[1], 0, size_t(B) * S * sizeof(float), fk));   // RED targets of
-  if ((rc = tower_forward(ctx, item, i, batch, ws->ei, ws->c, tcore, fk))) return rc;                    // the split-K
+  if ((rc = tower_forward(ctx, item, i, batch, ws->ei, ws->c, tcore, fk, tsh[1]))) return rc;            // the split-K
   if (training && mode == 0) BRK_CUDA(cudaMemsetAsync(dz[0], 0, size_t(B) * S * sizeof(float), st));   // products below
-  if ((rc = tower_forward(ctx, user, u, batch, ws->eu, ws->q, tcore, stream))) return rc;
+  if ((rc = tower_forward(ctx, user, u, batch, ws->eu, ws->q, tcore, stream, tsh[0]))) return rc;
   BRK_JOIN(ctx, st, 0);
   if (mode == 0) {
     // scores = q c^T; softmax CE (SUM) with accidental-hit removal; in place P = softmax - I
@@ -311,13 +309,71 @@ extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_
     // de = dz W^T: W stored [E,S] = "B stored [N,K]" with N = E, K = S  (tb = 1); its own buffer: the dW product
     // beside it is still reading the gathered rows e
     if ((rc = gemm(ctx, sk, tcore, dz[k], tw[k]->dense.w, de[k], nullptr, B, E[k], S, S, S, E[k], 0, 1, 1.f, 0, false))) return rc;
-    if ((rc = brk_scatter_add_rows(ctx, tw[k]->emb.g, tw[k]->emb.rows, E[k], ids[k], batch, de[k], tw[k]->emb.touched, 0,
-                                   (void*)sk)))
-      return rc;
+    rc = tsh[k] ? brk_scatter_add_rows_sharded(ctx, tsh[k], E[k], ids[k], batch, de[k], (void*)sk)
+                : brk_scatter_add_rows(ctx, tw[k]->emb.g, tw[k]->emb.rows, E[k], ids[k], batch, de[k], tw[k]->emb.touched, 0,
+                                       (void*)sk);
+    if (rc) return rc;
     if (wide) BRK_JOIN(ctx, sk, 1 + k);
   }
   BRK_JOIN(ctx, st, 0);
   return 0;
+}
+
+extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                 const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                 int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
+                                 void* stream) {
+  BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_step: null argument");
+  BRK_REQUIRE(user->S == item->S && batch > 0 && batch < (1 << 30), BRK_E_ARG, "brk_twotower_step: S %d vs %d, batch %lld",
+              user->S, item->S, (long long)batch);
+  BRK_REQUIRE((mode & 0xFF) == 0 || labels, BRK_E_ARG, "brk_twotower_step: rdZero mode needs labels");
+  BRK_REQUIRE(ws->eu && ws->ei && ws->q && ws->c && ws->dq && ws->dc && ws->acc && ((mode & 0xFF) != 0 || ws->scores), BRK_E_ARG,
+              "brk_twotower_step: workspace missing");
+  BRK_REQUIRE(!training || (user->emb.g && item->emb.g && user->dense.g && item->dense.g && ws->deu && ws->dei), BRK_E_ARG,
+              "brk_twotower_step: gradient accumulators / deu, dei workspace missing");
+  return twotower_step(ctx, user, item, nullptr, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream);
+}
+
+static int check_shards(const brk_shards* s, int32_t E, const char* which) {
+  BRK_REQUIRE(s->world >= 1 && s->world <= BRK_MAX_PEERS, BRK_E_ARG, "brk_twotower_step_sharded: %s world=%d (1..%d)", which,
+              s->world, BRK_MAX_PEERS);
+  BRK_REQUIRE(s->rank >= 0 && s->rank < s->world, BRK_E_ARG, "brk_twotower_step_sharded: %s rank=%d world=%d", which, s->rank,
+              s->world);
+  for (int p = 0; p < s->world; ++p)
+    BRK_REQUIRE(s->w[p] && s->g[p] && s->touched[p], BRK_E_ARG, "brk_twotower_step_sharded: %s shard %d has a null w / g / touched",
+                which, p);
+  BRK_REQUIRE(E > 0 && (E & 3) == 0, BRK_E_ARG, "brk_twotower_step_sharded: %s width %d is not a positive multiple of 4", which, E);
+  return 0;
+}
+
+extern "C" int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
+                                         const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels,
+                                         int64_t batch, int32_t mode, const brk_twotower_workspace* ws, float* loss_out,
+                                         void* stream) {
+  BRK_REQUIRE(ctx && user && item && ws, BRK_E_ARG, "brk_twotower_step_sharded: null argument");
+  BRK_REQUIRE(sh, BRK_E_ARG, "brk_twotower_step_sharded: null shards");
+  int rc;
+  if ((rc = check_shards(&sh->user, user->E, "user"))) return rc;
+  if ((rc = check_shards(&sh->item, item->E, "item"))) return rc;
+  BRK_REQUIRE(sh->user.world == sh->item.world && sh->user.rank == sh->item.rank, BRK_E_ARG,
+              "brk_twotower_step_sharded: user / item shards of different worlds or ranks");
+  BRK_REQUIRE(user->S == item->S && batch >= 0 && batch < (1 << 30), BRK_E_ARG,
+              "brk_twotower_step_sharded: S %d vs %d, batch %lld", user->S, item->S, (long long)batch);
+  if (batch == 0) return 0;
+  BRK_REQUIRE(u && i, BRK_E_ARG, "brk_twotower_step_sharded: null ids");
+  BRK_REQUIRE((mode & 0xFF) == 0 || labels, BRK_E_ARG, "brk_twotower_step_sharded: rdZero mode needs labels");
+  BRK_REQUIRE(ws->eu && ws->ei && ws->q && ws->c && ws->dq && ws->dc && ws->acc && ws->deu && ws->dei &&
+              ((mode & 0xFF) != 0 || ws->scores), BRK_E_ARG, "brk_twotower_step_sharded: workspace missing");
+  BRK_REQUIRE(user->dense.w && item->dense.w && user->dense.g && item->dense.g, BRK_E_ARG,
+              "brk_twotower_step_sharded: Dense blocks or their gradients missing");
+  return twotower_step(ctx, user, item, sh, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream);
+}
+
+extern "C" int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const brk_shards* sh, const int32_t* ids, int64_t n,
+                                         float* emb_out, float* out, void* stream) {
+  BRK_REQUIRE(ctx && t && sh && ids && emb_out && out, BRK_E_ARG, "brk_tower_forward_sharded: null argument");
+  BRK_REQUIRE(t->dense.w && t->E > 0 && t->S > 0 && n > 0, BRK_E_ARG, "brk_tower_forward_sharded: bad tower");
+  return tower_forward(ctx, t, ids, n, emb_out, out, 0, stream, sh);
 }
 
 // Training step + Keras Adagrad (twoTower.py:89-102 with the optimizer of :278-279) in one call.  In-batch-softmax steps
@@ -334,7 +390,8 @@ extern "C" int brk_twotower_train_step(brk_ctx* ctx, const brk_tower* user, cons
   if ((mode & 0xFF) == 0 && (mode & 0x100) && user->S == item->S && batch > 0 && batch < (1 << 30) && ws->q && ws->c && ws->dq &&
       ws->dc && ws->acc && user->emb.g && item->emb.g && user->dense.g && item->dense.g) {
     int handled = 0;
-    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps))) return rc;
+    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps, nullptr)))
+      return rc;
     if (handled) return 0;
   }
   if ((rc = brk_twotower_step(ctx, user, item, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream))) return rc;

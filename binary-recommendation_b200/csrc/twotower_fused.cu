@@ -25,11 +25,18 @@
 // a B200); larger batches, other modes (rdZero) and widths above 128 take the multi-kernel step.
 // The grid barrier (brk_grid_barrier, common.cuh) keeps its base in device memory (bar[2]), so the launch can be captured
 // into a CUDA graph and replayed (TwoTowerModel.fit does).
+//
+// fused_step<true> is the same step on row-sharded tables (brk_twotower_step_sharded): row r of a table lives on rank
+// r % G at local row r / G.  The ids are split into (owner, local row) once, where they are staged in shared memory; the
+// gathers of phases F and G read the owner's shard (NVLink peer memory across GPUs) and phase G's row-gradient REDs and
+// touched bits go to the owner's accumulator and bitmask.  Phase O does not run: an owner's accumulator is complete only
+// after a cross-GPU barrier and the Dense gradients only after their all-reduce, so the launch ends after phase G.
 #include "common.cuh"
 #include "tc.cuh"
 #include "tc_tiles.cuh"
 #include <math_constants.h>
 #include <stdlib.h>
+#include <type_traits>
 
 namespace ttf {
 
@@ -60,6 +67,12 @@ struct Params {
   int do_opt; float lr, eps;
   brk_table dn[2];
 };
+// fused_step<true> (row-sharded tables): the same block followed by the two tables' shards.  A separate type keeps the
+// parameter block of fused_step<false> as it was (its size changes ptxas' schedule).
+struct ShardedParams : Params {
+  brk_shards su, si;
+};
+template <bool SH> using ParamsT = typename std::conditional<SH, ShardedParams, Params>::type;
 
 __device__ __forceinline__ void adagrad4(float4* w, float4* a, float4* g, float lr, float eps) {
   float4 w4 = *w, a4 = *a;
@@ -102,18 +115,25 @@ __device__ __forceinline__ void load_tile(uint8_t* dst, const float* __restrict_
     cp_async16(d + k * 1024, nb ? (const void*)(p + int64_t(8 * k) * ld) : (const void*)src, nb);
   }
 }
-template <int MN>
-__device__ __forceinline__ void gather_tile(uint8_t* dst, const float* __restrict__ table, int d_, const int32_t* ids_s, int valid) {
+// SH: ids_s holds local rows and own_s their owners; the row is read from shard own_s[.] of tower `tw`'s table (`table`
+// is then unused: the zero-byte copies past `valid` name shard 0).
+template <int MN, bool SH, class PT>
+__device__ __forceinline__ void gather_tile(uint8_t* dst, const float* __restrict__ table, const PT& P, int tw, int d_,
+                                            const int32_t* ids_s, const int32_t* own_s, int valid) {
   const int w = threadIdx.x >> 5, c4 = threadIdx.x & 31;
   int cb = (d_ - c4 * 4) * 4;
   cb = cb < 0 ? 0 : (cb > 16 ? 16 : cb);
   uint8_t* d = dst + (MN ? mn_off16(TS, w, c4) : km_off16(TS, w, c4));
+  if constexpr (SH) table = (tw == 0 ? P.su : P.si).w[0];
 #pragma unroll
   for (int k = 0; k < TS / 8; ++k) {
     const int nb = (w + 8 * k < valid) ? cb : 0;
-    cp_async16(d + k * 1024, nb ? (const void*)(table + int64_t(ids_s[w + 8 * k]) * d_ + c4 * 4) : (const void*)table, nb);
+    const float* src = table;
+    if constexpr (SH) src = (tw == 0 ? P.su : P.si).w[own_s[w + 8 * k]];
+    cp_async16(d + k * 1024, nb ? (const void*)(src + int64_t(ids_s[w + 8 * k]) * d_ + c4 * 4) : (const void*)table, nb);
   }
 }
+
 
 // 64 accumulator columns [c0, c0 + 64) of this thread's TMEM lane
 __device__ __forceinline__ void tmem_load64(uint32_t tmem, int warp, int c0, float (&v)[64]) {
@@ -143,13 +163,26 @@ __device__ __forceinline__ float4 staging_ld(const uint8_t* stg, int r, int c4) 
 
 #define TTF_OPERANDS_READY() do { cp_async_wait_all(); tc::fence_proxy_async_smem(); __syncthreads(); tc::fence_after_sync(); } while (0)
 
-__global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
+// ids_s[t] <- id r0 + t of tower k (threads t < TS); SH: the local row, and own_s[t] its owner (the one division per id)
+template <bool SH>
+__device__ __forceinline__ void stage_ids(const ParamsT<SH>& P, int k, int r0, int valid, int32_t* ids_s, int32_t* own_s) {
+  const int t = threadIdx.x;
+  if (t < TS) {
+    const int32_t id = t < valid ? __ldg(P.ids[k] + r0 + t) : 0;
+    if constexpr (SH) { ids_s[t] = id / P.su.world; own_s[t] = id % P.su.world; }
+    else ids_s[t] = id;
+  }
+}
+
+template <bool SH>
+__global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* buf0 = sm; uint8_t* buf1 = sm + TILE; uint8_t* buf2 = sm + 2 * TILE;
   __shared__ uint64_t mbar;
   __shared__ uint32_t tmem_slot;
   __shared__ int32_t ids_s[TS], cand_r[TS];
+  __shared__ int32_t own_s[SH ? TS : 1];                                // SH: owner rank of the row in ids_s
   __shared__ __align__(16) int32_t cand_c[TS];
   __shared__ float pm[2][TS], ps[2][TS], diag_s[TS], lse_s[TS];
   __shared__ double red[32];
@@ -176,10 +209,10 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
   if (b < 2 * T) {
     const int k = b / T, r0 = (b % T) * TS, valid = min(TS, B - r0), E = P.E[k];
     const brk_table& tab = k == 0 ? P.eu : P.ei;
-    if (t < TS) ids_s[t] = t < valid ? __ldg(P.ids[k] + r0 + t) : 0;
+    stage_ids<SH>(P, k, r0, valid, ids_s, own_s);
     load_tile<1>(buf1, P.W[k], S, 0, E, S);                             // W [K = E][N = S]: MN-major B operand
     __syncthreads();
-    gather_tile<0>(buf0, tab.w, E, ids_s, valid);                       // e [M = samples][K = E]: K-major A operand
+    gather_tile<0, SH>(buf0, tab.w, P, k, E, ids_s, own_s, valid);   // e [M = samples][K = E]: K-major A operand
     cp_async_commit();
     TTF_OPERANDS_READY();
     if (t == 0) {
@@ -351,12 +384,12 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
   const int gk = b / (2 * T), g_r0 = ((b % (2 * T)) >> 1) * TS, g_valid = min(TS, B - g_r0), g_job = b & 1;
   if (g_cta) {
     __syncthreads();                                                    // staging and operand tiles of the phase above are done with
-    if (t < TS) ids_s[t] = t < g_valid ? __ldg(P.ids[gk] + g_r0 + t) : 0;
+    stage_ids<SH>(P, gk, g_r0, g_valid, ids_s, own_s);
     if (g_job == 0) {
       load_tile<0>(buf1, P.W[gk], S, 0, P.E[gk], S);
     } else {
       __syncthreads();
-      gather_tile<1>(buf0, (gk == 0 ? P.eu : P.ei).w, P.E[gk], ids_s, g_valid);
+      gather_tile<1, SH>(buf0, (gk == 0 ? P.eu : P.ei).w, P, gk, P.E[gk], ids_s, own_s, g_valid);
     }
     cp_async_commit();
   }
@@ -366,7 +399,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
   if (b == 0 && t == 0) {                                               // every loss contribution was added before the barrier
     if (P.loss_out) P.loss_out[0] = float(*reinterpret_cast<volatile double*>(P.acc));
     *P.acc = 0.0;
-    if (!(P.training && P.do_opt)) P.bar[2] = bar_target;               // base of the next launch
+    if (SH || !(P.training && P.do_opt)) P.bar[2] = bar_target;         // base of the next launch
   }
 
   // ---------------- phase G: gradients of the tower parameters ----------------
@@ -389,8 +422,15 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
         const int rr = idx >> 5, c4 = idx & 31;
         if (rr < valid) {
           const int64_t row = ids_s[rr];
-          if (c4 * 4 < E) red_add_f4(tab.g + row * E + c4 * 4, staging_ld(buf2, rr, c4));
-          if (c4 == 0 && tab.touched) asm volatile("red.global.or.b32 [%0], %1;" ::"l"(tab.touched + (row >> 5)), "r"(1u << (row & 31)) : "memory");
+          if constexpr (SH) {                                           // the owner's accumulator and bitmask (never null)
+            const brk_shards& sh = k == 0 ? P.su : P.si;
+            const int o = own_s[rr];
+            if (c4 * 4 < E) red_add_f4(sh.g[o] + row * E + c4 * 4, staging_ld(buf2, rr, c4));
+            if (c4 == 0) asm volatile("red.global.or.b32 [%0], %1;" ::"l"(sh.touched[o] + (row >> 5)), "r"(1u << (row & 31)) : "memory");
+          } else {
+            if (c4 * 4 < E) red_add_f4(tab.g + row * E + c4 * 4, staging_ld(buf2, rr, c4));
+            if (c4 == 0 && tab.touched) asm volatile("red.global.or.b32 [%0], %1;" ::"l"(tab.touched + (row >> 5)), "r"(1u << (row & 31)) : "memory");
+          }
         }
       }
     } else {
@@ -419,7 +459,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
   }
   stamp(P, 7);
   // ---------------- phase O: Keras Adagrad (optim.cu AdagradOp) on what this step touched ----------------
-  if (P.training && P.do_opt) {
+  if (!SH && P.training && P.do_opt) {
     brk_grid_barrier(P.bar, bar_target);
     if (b == 0 && t == 0) P.bar[2] = bar_target;
     // rows: every warp takes a run of `per` (tower, sample) pairs, one per lane: the ids are loaded and the touched bits
@@ -486,9 +526,12 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const Params P) {
 }  // namespace ttf
 
 // Internal entry (twotower.cu): *handled = 0 when the shape is not this kernel's (the caller then takes the multi-kernel step).
+// sh != nullptr: the tables are row-sharded (brk_twotower_step_sharded, training only, do_opt = 0); the embedding
+// tables of user / item are then not read.
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
-                            float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps) {
+                            float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
+                            const brk_twotower_shards* sh) {
   using namespace ttf;
   *handled = 0;
   const int S = user->S, B = int(batch), T = (B + TS - 1) / TS;
@@ -497,16 +540,27 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
   if (getenv("BRK_TT_NO_FUSED")) return 0;
   if (S > 128 || user->E > 128 || item->E > 128 || (S & 3) || (user->E & 3) || (item->E & 3) || need > ctx->sm_count || T > 12) return 0;
   const brk_tower* tw[2] = {user, item};
+  if (sh != nullptr) {
+    if (!training || do_opt) return 0;
+    const brk_shards* s2[2] = {&sh->user, &sh->item};
+    for (int k = 0; k < 2; ++k)
+      for (int p = 0; p < s2[k]->world; ++p)
+        if (!brk_aligned16(s2[k]->w[p]) || !brk_aligned16(s2[k]->g[p])) return 0;
+  }
   for (int k = 0; k < 2; ++k)
-    if (!brk_aligned16(tw[k]->emb.w) || !brk_aligned16(tw[k]->dense.w) || (training && (!brk_aligned16(tw[k]->emb.g) || !brk_aligned16(tw[k]->dense.g))))
+    if ((!sh && !brk_aligned16(tw[k]->emb.w)) || !brk_aligned16(tw[k]->dense.w) ||
+        (training && ((!sh && !brk_aligned16(tw[k]->emb.g)) || !brk_aligned16(tw[k]->dense.g))))
       return 0;
   if (!brk_aligned16(ws->q) || !brk_aligned16(ws->c) || (training && (!brk_aligned16(ws->dq) || !brk_aligned16(ws->dc)))) return 0;
   const size_t smem = 3 * size_t(TILE) + 1024;
-  // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of the kernel, queried once
-  BRK_CUDA(cudaFuncSetAttribute(fused_step, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  static int per_sm = -1;
-  if (per_sm < 0) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fused_step, NT, smem));
-  if (grid > per_sm * ctx->sm_count) return 0;
+  const void* kern = sh ? (const void*)fused_step<true> : (const void*)fused_step<false>;
+  // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of each instantiation,
+  // queried once
+  BRK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  static int per_sm[2] = {-1, -1};
+  int& occ = per_sm[sh ? 1 : 0];
+  if (occ < 0) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
+  if (grid > occ * ctx->sm_count) return 0;
   const size_t part_floats = size_t(T) * TS * T * 2;
   if (ctx->tt_part_floats < part_floats) {
     if (ctx->tt_part) BRK_CUDA(cudaFree(ctx->tt_part));
@@ -514,7 +568,7 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
     BRK_CUDA(cudaMalloc(&ctx->tt_part, part_floats * sizeof(float)));
     ctx->tt_part_floats = part_floats;
   }
-  Params P;
+  ShardedParams P;                                    // fused_step<false> reads its Params base (at offset 0)
   memset(&P, 0, sizeof(P));
   P.eu = user->emb; P.ei = item->emb;
   for (int k = 0; k < 2; ++k) { P.W[k] = tw[k]->dense.w; P.gW[k] = tw[k]->dense.g; P.E[k] = tw[k]->E; }
@@ -535,8 +589,9 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
     P.do_opt = 1; P.lr = lr; P.eps = eps;
     P.dn[0] = user->dense; P.dn[1] = item->dense;
   }
-  void* args[] = {&P};
-  BRK_CUDA(cudaLaunchCooperativeKernel((const void*)fused_step, dim3(grid), dim3(NT), args, smem, st));
+  if (sh) { P.su = sh->user; P.si = sh->item; }
+  void* args[] = {sh ? (void*)&P : (void*)static_cast<Params*>(&P)};
+  BRK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(NT), args, smem, st));
   *handled = 1;
   return 0;
 }

@@ -33,6 +33,7 @@ import torch.distributed as dist
 from . import _native as N
 from . import distributed as D
 from . import hotpath as H
+from .twoTower import Tower, TwoTowerModel
 
 
 def shard_rows(rows, G):
@@ -84,9 +85,11 @@ def load_sharded_model(dirpath, tables, G, rank, emulate):
 
 
 class ShardedTable:
-    """One row-sharded embedding table: local shard as an H.Table plus every rank's shard pointers."""
+    """One row-sharded embedding table: local shard as an H.Table plus every rank's shard pointers.
+    slots / slot_init: optimizer slots of every shard, as H.Table (default: Adam's m and v at zero)."""
 
-    def __init__(self, rows, d, G, rank, device, full_init=None, init_seed=0, symmetric=True, emulate=False):
+    def __init__(self, rows, d, G, rank, device, full_init=None, init_seed=0, symmetric=True, emulate=False, slots=2,
+                 slot_init=0.0):
         self.rows, self.d, self.G, self.rank, self.device = int(rows), int(d), int(G), int(rank), device
         self.local_rows = shard_rows(rows, G)
         n = self.local_rows * d
@@ -120,7 +123,7 @@ class ShardedTable:
             else:                                           # Keras Embedding init U(-0.05, 0.05), generated on the device
                 gen = torch.Generator(device=device); gen.manual_seed(int(init_seed) * 1000003 + r)
                 w2.uniform_(-0.05, 0.05, generator=gen)
-            tab = H.Table(w2, touched=False, g=g)
+            tab = H.Table(w2, slots=slots, touched=False, slot_init=slot_init, g=g)
             tab.touched = t
             self.tables[r] = tab
         self.ptr_w, self.ptr_g, self.ptr_t = ptr_w, ptr_g, ptr_t
@@ -136,12 +139,13 @@ class ShardedTable:
         s.world, s.rank = self.G, self.rank
         return s
 
-    def full_weights(self):
-        """The whole table on the host (tests): all-gather of the shards, re-interleaved."""
-        if self.emulate:
-            parts = [self.tables[r].w.cpu().numpy() for r in range(self.G)]
+    def full_weights(self, which="w"):
+        """The whole table on the host (tests): all-gather of the shards, re-interleaved.  which: "w" or an optimizer
+        slot ("m", "v")."""
+        if self.emulate or self.G == 1:
+            parts = [getattr(self.tables[r], which).cpu().numpy() for r in range(self.G)]
         else:
-            mine = self.local.w.contiguous()
+            mine = getattr(self.local, which).contiguous()
             parts_t = [torch.empty_like(mine) for _ in range(self.G)]
             dist.all_gather(parts_t, mine)
             parts = [p.cpu().numpy() for p in parts_t]
@@ -417,4 +421,159 @@ class ShardedBPRNet:
     def load_checkpoint(self, dirpath):
         rep, meta = load_sharded_model(dirpath, {"user": self.user, "item": self.item}, self.G, self.rank, self.emulate)
         self.optimizer.state.copy_(torch.from_numpy(rep["opt_state"]))
+        return meta
+
+
+class ShardedTwoTowerNet:
+    """Two-tower retrieval model (twoTower.TwoTowerModel: Embedding -> linear Dense(semb) per tower, in-batch softmax or
+    rdZero BCE, Keras Adagrad) with row-sharded embedding tables, for catalogs too large to mirror on every GPU.
+
+    Semantics, per step on a global batch split over the G ranks (D.local_slice):
+      * every rank trains its slice; the in-batch softmax uses that slice's items as negatives (MirroredStrategy's
+        per-replica loss, what the mirrored TwoTowerModel.fit does); accidental hits compare global item ids within
+        the slice;
+      * each replica's loss is SUM-reduced; gradients are summed over ranks, never scaled;
+      * row r of a table (numUser + 2 / numItem + 2 rows: the StringLookup offset) lives on rank r % G at local row
+        r // G; a rank's row gradients land in the owner's accumulator as REDs and set the owner's touched bits;
+      * every owner applies row-sparse Keras Adagrad (accumulator initial value 0.1, in `m`) to the touched rows of its
+        shards.  Adagrad leaves rows with g = 0 unchanged, so this is the mirrored dense pass up to summation order;
+      * the two Dense blocks (W [E][S], then b [S]) are mirrored; their gradients are summed over ranks by
+        brk_allreduce_dense_peer (fixed order: bit-identical replicas) and every replica applies brk_adagrad_dense.
+    So G GPUs give the mirrored TwoTowerModel's result on the same global batches.  `emulate=G` holds all G shards in
+    one process on one GPU and trains the whole batch as one replica: the unsharded single-GPU TwoTowerModel's result.
+
+    Ids arrive as int32 table rows (already looked up).  full_init: {"user", "item": full tables [rows, E];
+    "user_dense", "item_dense": flat Dense blocks as Tower.init_dense lays them out}; without it the tables are
+    U(-0.05, 0.05) and the Dense blocks Glorot-uniform from Philox(seed + 77)."""
+
+    def __init__(self, numUser, numItem, embedDim, semb, learning_rate=0.1, rdZero=False, tensor_cores=True, seed=42,
+                 device=None, emulate=0, full_init=None):
+        self.device = torch.device(device or f"cuda:{torch.cuda.current_device()}")
+        self.emulate = int(emulate)
+        self.G, self.rank = (self.emulate, 0) if self.emulate else (D.world_size(), D.rank())
+        self.embedDim, self.semb = int(embedDim), int(semb)
+        self.numUser, self.numItem = int(numUser), int(numItem)
+        self.rdZero, self.tensor_cores = bool(rdZero), bool(tensor_cores)
+        self.optimizer = H.Adagrad(learning_rate)
+        dev, E, S = self.device, self.embedDim, self.semb
+        symmetric = not self.emulate and self.G > 1
+        fi = full_init or {}
+        mk = lambda name, rows, k: ShardedTable(rows, E, self.G, self.rank, dev, full_init=fi.get(name), init_seed=seed * 16 + k,
+                                                symmetric=symmetric, emulate=bool(self.emulate), slots=1,
+                                                slot_init=H.Adagrad.INITIAL_ACCUMULATOR)
+        self.user, self.item = mk("user", self.numUser + 2, 0), mk("item", self.numItem + 2, 1)
+        rng = np.random.Generator(np.random.Philox(key=seed + 77))
+        self.dense = []
+        for name in ("user_dense", "item_dense"):
+            t = Tower.__new__(Tower)
+            t.E, t.S = E, S
+            t.init_dense(rng, dev)
+            if name in fi:
+                t.dense.w.view(-1).copy_(torch.from_numpy(np.asarray(fi[name], dtype=np.float32).reshape(-1)))
+            self.dense.append(t.dense)
+        # the Dense gradients are views of ONE flat arena, summed over the ranks once per step (peer memory, no NCCL)
+        self.grad_arena = self._reducer = None
+        self.barrier = None
+        if symmetric:
+            sizes = [t.w.numel() for t in self.dense]
+            self.grad_arena, self._reducer = D.gradient_arena(sum(sizes), dev)
+            for t, v in zip(self.dense, torch.split(self.grad_arena[:sum(sizes)], sizes)):
+                t.g = v.view(t.rows, t.d)
+            self.barrier = PeerBarrier(dev)
+        self._ws_batch = 0
+
+    _workspace = TwoTowerModel._workspace               # the mirrored model's step buffers (same attribute names)
+
+    def _towers(self):
+        return [N.brk_tower(N.brk_table(), d.c_struct(), self.embedDim, self.semb) for d in self.dense]
+
+    def _shards(self):
+        return N.brk_twotower_shards(self.user.c_shards(), self.item.c_shards())
+
+    def train_on_batch(self, u, i, labels=None, loss_out=None):
+        """One step on this rank's slice (u, i: int32 table rows; labels: rdZero targets).  Every rank must call it, an
+        empty slice included.  Returns the slice's loss as a device scalar."""
+        loss_out = self.forward_backward(u, i, labels, loss_out)
+        self.apply_gradients()
+        return loss_out
+
+    def forward_backward(self, u, i, labels=None, loss_out=None):
+        """The step without the optimizer: row gradients in the owners' accumulators (touched bits set there), Dense
+        gradients in this rank's Dense blocks."""
+        B = u.numel()
+        dev = self.device
+        loss_out = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=dev)
+        lib, ctx, st = N.lib(), N.ctx(dev), N.stream_ptr()
+        if B > 0:
+            if self.rdZero and labels is None:
+                raise ValueError("rdZero training needs labels")
+            ws = self._workspace(B)
+            ut, it = self._towers()
+            sh = self._shards()
+            u, i = H._i32(u, "u"), H._i32(i, "i")
+            N.check(lib.brk_twotower_step_sharded(ctx, C.byref(ut), C.byref(it), C.byref(sh), N.ptr(u), N.ptr(i), N.ptr(i),
+                                                  N.ptr(H._f32(labels, "labels")) if self.rdZero else None, B,
+                                                  (1 if self.rdZero else 0) | (0x100 if self.tensor_cores else 0),
+                                                  C.byref(ws), N.ptr(loss_out), st), "brk_twotower_step_sharded")
+        else:
+            loss_out.zero_()
+        return loss_out
+
+    def apply_gradients(self):
+        """Row-sparse Adagrad on the owned shards, Dense gradients summed over ranks, Adagrad on the Dense blocks."""
+        lib, ctx, st = N.lib(), N.ctx(self.device), N.stream_ptr()
+        opt = self.optimizer
+        if self.barrier is None:                            # every shard lives in this process (emulation, or G == 1)
+            tabs = [t.tables[r] for t in (self.user, self.item) for r in range(self.G)]
+            for k in range(0, len(tabs), 16):
+                N.check(lib.brk_adagrad_rows(ctx, H._pack(tabs[k:k + 16]), len(tabs[k:k + 16]), opt.lr, opt.eps, st),
+                        "brk_adagrad_rows")
+            N.check(lib.brk_adagrad_dense(ctx, H._pack(self.dense), 2, opt.lr, opt.eps, st), "brk_adagrad_dense")
+            return
+        self.barrier()                                      # every rank's REDs have landed in my shards
+        mine = [self.user.local, self.item.local]
+        N.check(lib.brk_adagrad_rows(ctx, H._pack(mine), 2, opt.lr, opt.eps, st), "brk_adagrad_rows")
+        # The all-reduce also fences the next step: its entry barrier is reached by a rank only after that rank's row
+        # pass above (stream order), and nobody leaves the all-reduce before every rank has reached it.  So no rank
+        # gathers rows of the next step before every owner has updated its shards and zeroed their accumulators.
+        D.all_reduce_sum_(self.grad_arena, self._reducer)
+        N.check(lib.brk_adagrad_dense(ctx, H._pack(self.dense), 2, opt.lr, opt.eps, st), "brk_adagrad_dense")
+
+    def check(self):
+        """Raises when a cross-GPU barrier or the Dense all-reduce timed out (call at epoch ends, not per step)."""
+        if self.barrier is not None:
+            self.barrier.check()
+        if self._reducer is not None:
+            self._reducer.check()
+
+    def _tower_forward(self, k, ids):
+        ids = H._i32(ids, "ids")
+        n = ids.numel()
+        emb = torch.empty(n, self.embedDim, dtype=torch.float32, device=self.device)
+        out = torch.empty(n, self.semb, dtype=torch.float32, device=self.device)
+        if n == 0:
+            return out
+        t, sh = self._towers()[k], (self.user, self.item)[k].c_shards()
+        N.check(N.lib().brk_tower_forward_sharded(N.ctx(self.device), C.byref(t), C.byref(sh), N.ptr(ids), n, N.ptr(emb),
+                                                  N.ptr(out), N.stream_ptr()), "brk_tower_forward_sharded")
+        return out
+
+    def score_vectors(self, user_rows, item_rows):
+        """(user vectors [n, S], item vectors [m, S]) of int32 table rows, for hotpath.BruteForceIndex / topKmetrics."""
+        return self._tower_forward(0, user_rows), self._tower_forward(1, item_rows)
+
+    # ---- checkpoint: shards of the tables and their accumulators, replicated Dense blocks and theirs ------------
+    def save_checkpoint(self, dirpath):
+        rep = {}
+        for name, t in zip(("user_dense", "item_dense"), self.dense):
+            rep[name], rep[name + "_m"] = t.w.view(-1), t.m.view(-1)
+        return save_sharded_model(dirpath, {"user": self.user, "item": self.item}, rep, self.G, self.rank, self.emulate,
+                                  meta={"model": "ShardedTwoTowerNet", "E": self.embedDim, "S": self.semb,
+                                        "numUser": self.numUser, "numItem": self.numItem})
+
+    def load_checkpoint(self, dirpath):
+        rep, meta = load_sharded_model(dirpath, {"user": self.user, "item": self.item}, self.G, self.rank, self.emulate)
+        for name, t in zip(("user_dense", "item_dense"), self.dense):
+            t.w.view(-1).copy_(torch.from_numpy(rep[name]))
+            t.m.view(-1).copy_(torch.from_numpy(rep[name + "_m"]))
         return meta

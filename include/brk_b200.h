@@ -417,6 +417,26 @@ int brk_twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_tower
                             const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                             int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
                             int64_t rows_threshold_bytes, float* loss_out, void* stream);
+/* Two-tower training on row-sharded embedding tables (sharded.ShardedTwoTowerNet): row r of a table lives on
+ * rank r % world at local row r / world (brk_shards above); the Dense blocks are mirrored.
+ *   brk_twotower_step_sharded: brk_twotower_step with training = 1 on THIS rank's slice of the global batch (its
+ *     own items are the in-batch negatives); user / item carry this rank's Dense blocks (w, g), E and S, their emb
+ *     tables are not read.  Rows are gathered from the owners' shards (peer loads), row gradients go as 16-byte REDs
+ *     into the owner's g and set the owner's touched bits; Dense gradients are added into user / item dense.g.  Mode
+ *     bits as brk_twotower_step: with 0x100 and a batch that fits on chip the step is one cooperative launch, else the
+ *     multi-kernel step.  No optimizer runs.  batch == 0 does nothing (a rank with an empty slice still joins the
+ *     exchanges that follow).  Ordering: after it, every rank must pass brk_peer_barrier before an owner applies
+ *     brk_adagrad_rows to its shards, the Dense gradients are summed over ranks (brk_allreduce_dense_peer) before
+ *     brk_adagrad_dense, and every rank must pass a cross-GPU barrier after its row pass before the next step
+ *     gathers rows (the all-reduce's entry barrier does it when it is issued after the row pass).
+ *   brk_tower_forward_sharded: brk_tower_forward with the rows gathered from the shards (inference, evaluation). */
+typedef struct brk_twotower_shards { brk_shards user, item; } brk_twotower_shards;
+int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
+                              const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels,
+                              int64_t batch, int32_t mode, const brk_twotower_workspace* ws, float* loss_out,
+                              void* stream);
+int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const brk_shards* sh, const int32_t* ids, int64_t n,
+                              float* emb_out, float* out, void* stream);
 
 /* ---- K7/K8: full-catalog scoring + top-K ------------------------------------------------------
  * Stands in for tfrs.layers.factorized_top_k.BruteForce(k).index(candidates) + call(queries)
