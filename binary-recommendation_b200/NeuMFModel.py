@@ -350,6 +350,11 @@ class NeuMFNet:
             vals.append(v); idxs.append(ix)
         return torch.cat(vals), torch.cat(idxs)
 
+    def topk_index(self, itemsId=None, id_offset=0):
+        """Full-catalog top-k index over itemsId (default: every item): see NeuMFTopKIndex.  It snapshots the item side
+        of the model, so rebuild it after training."""
+        return NeuMFTopKIndex(self, itemsId, id_offset)
+
     def state_dict(self):
         sd = {"bn_moving": self.bn_moving.cpu(), "opt_state": self.optimizer.state.cpu()}
         for name, t in zip(("uMLP", "iMLP", "uMF", "iMF", "dense"), self.tables() + [self.dense]):
@@ -364,6 +369,116 @@ class NeuMFNet:
                 if tuple(sd[key].reshape(-1).shape) != tuple(slot.reshape(-1).shape):
                     raise ValueError(f"checkpoint tensor {key!r} has {sd[key].numel()} elements, the model needs {slot.numel()}")
                 slot.copy_(sd[key].reshape(slot.shape))
+
+
+def _gemm_tf32(a, w, out, bias=None):
+    """out [M, N] = a [M, K] @ w [K, N] (+ bias) with TF32 operands and fp32 accumulation (brk_gemm_tf32)."""
+    M, K = a.shape
+    Nn = w.shape[1]
+    N.check(N.lib().brk_gemm_tf32(N.ctx(a.device), N.ptr(a), C.c_void_p(w.data_ptr()), N.ptr(out),
+                                  C.c_void_p(bias.data_ptr()) if bias is not None else None, M, Nn, K, K, Nn, Nn, 0, 0,
+                                  1.0, 0, N.stream_ptr()), "brk_gemm_tf32")
+    return out
+
+
+class NeuMFTopKIndex:
+    """Full-catalog NeuMF top-k in one kernel launch (brk_neumf_score_topk): for each queried user, the k items of the
+    index with the highest prediction -- the value predict_on_batch returns for the pair, to TF32 rounding -- sorted
+    by score, ties to the lower position, scores never materialised.  Shaped like hotpath.BruteForceIndex:
+
+        index = net.topk_index(itemsId)            # item side: iMLP[items] W1[E:2E] + b1 and the items' iMF rows
+        scores, ids = index(usersId, k=10)         # ids: positions in itemsId plus id_offset
+        scores, ids = index.query_with_exclusions(usersId, hotpath.exclusion_csr(rows, ids, len(usersId), dev))
+
+    The first Dense layer factors over [uMLP[u], iMLP[i]], so building the index computes the item half once and a
+    query the user half once; the kernel runs the rest of the network per pair on the tensor cores.  The index is a
+    snapshot of the item tables and keeps the model for the dense block, the BatchNorm statistics and the user tables:
+    rebuild it after training.  Built for the tensor-core class graph (numFactor 32 or 64, relu) and the He et al.
+    variant (E 32, mf_dim 8, hadamard, no BatchNorm); other models, and k > 32, raise ValueError -- rank them with
+    NeuMFNet.score_all.
+
+    Item-range shards: rank r indexes its range [lo, hi) with id_offset = lo; the merged lists equal the unsharded
+    index's bit for bit:
+
+        index = net.topk_index(np.arange(lo, hi), id_offset=lo)
+        scores, ids = distributed.sharded_topk(usersId, None, lo, k, local_topk=lambda q, c, off: index(q, k))
+
+    (or hotpath.topk_merge over the stacked [shards, U, k] lists in one process)."""
+
+    K_MAX = H.MAX_FUSED_K
+
+    def __init__(self, net, itemsId=None, id_offset=0):
+        h1, h2, h3 = net.hidden
+        ok = net.act == "relu" and (
+            (not net.variant and net.tensor_cores and (net.E, h1, h2, h3) in TC_SPECS) or
+            (net.variant and net.mf_mode == "hadamard" and not net.batch_norm and
+             (net.E, net.EMF, net.hidden) in FUSED_VARIANTS))
+        if not ok:
+            raise ValueError(f"no fused top-k instance for E={net.E}, mf_dim={net.EMF}, hidden={net.hidden}, act={net.act}, "
+                             f"mf_mode={net.mf_mode}, batch_norm={net.batch_norm}, tensor_cores={net.tensor_cores}; built: "
+                             f"tensor-core class graph {sorted(TC_SPECS)} and the He et al. variant {sorted(FUSED_VARIANTS)} "
+                             "-- use NeuMFNet.score_all")
+        self.net = net
+        dev = net.device
+        if itemsId is None:
+            items = torch.arange(net.numItem, dtype=torch.int32, device=dev)
+        else:
+            items = torch.as_tensor(np.asarray(itemsId, dtype=np.int32)).to(dev)
+        if items.numel() == 0:
+            raise ValueError("NeuMFTopKIndex: no items")
+        self.num_candidates = items.numel()
+        self.id_offset = int(id_offset)
+        E = net.E
+        W1 = net.param("W1")                                 # [2E, H1]: rows [0, E) act on uMLP, [E, 2E) on iMLP
+        self._W1u, self._W1i = W1[:E], W1[E:]
+        self.item_side = _gemm_tf32(H.gather_rows(net.iMLP.w, items), self._W1i,
+                                    torch.empty((items.numel(), h1), dtype=torch.float32, device=dev), net.param("b1"))
+        self.item_mf = H.gather_rows(net.iMF.w, items)
+
+    def _check_k(self, k):
+        k = 10 if k is None else int(k)
+        if k < 1 or k > self.K_MAX:
+            raise ValueError(f"k={k}: the fused NeuMF top-k keeps 1..{self.K_MAX} entries per user; use NeuMFNet.score_all")
+        return min(k, self.num_candidates)
+
+    def _run(self, usersId, k, exclusions):
+        net = self.net
+        dev = net.device
+        k = self._check_k(k)
+        users = torch.as_tensor(np.asarray(usersId, dtype=np.int32) if not isinstance(usersId, torch.Tensor) else usersId)
+        users = H._i32(users.to(dev).reshape(-1), "usersId")
+        U = users.numel()
+        vals = torch.empty((U, k), dtype=torch.float32, device=dev)
+        ids = torch.empty((U, k), dtype=torch.int32, device=dev)
+        if U == 0:
+            return vals, ids
+        user_side = _gemm_tf32(H.gather_rows(net.uMLP.w, users), self._W1u,
+                               torch.empty((U, net.hidden[0]), dtype=torch.float32, device=dev))
+        lib, ctx = N.lib(), N.ctx(dev)
+        ws_bytes = lib.brk_neumf_topk_workspace_bytes(ctx, U, self.num_candidates, k)
+        ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
+        m = net._c_model()
+        if exclusions is None:
+            N.check(lib.brk_neumf_score_topk(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U, N.ptr(self.item_side),
+                                             N.ptr(self.item_mf), self.num_candidates, k, self.id_offset, N.ptr(vals),
+                                             N.ptr(ids), N.ptr(ws), ws_bytes, N.stream_ptr()), "brk_neumf_score_topk")
+        else:
+            indptr, xids = H._check_csr(exclusions, U, dev)
+            N.check(lib.brk_neumf_score_topk_excl(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U, N.ptr(self.item_side),
+                                                  N.ptr(self.item_mf), self.num_candidates, k, self.id_offset, N.ptr(indptr),
+                                                  N.ptr(xids), N.ptr(vals), N.ptr(ids), N.ptr(ws), ws_bytes, N.stream_ptr()),
+                    "brk_neumf_score_topk_excl")
+        return vals, ids
+
+    def __call__(self, usersId, k=None):
+        """(scores [U, k], ids [U, k]) for the users usersId (rows of the user tables)."""
+        return self._run(usersId, k, None)
+
+    def query_with_exclusions(self, usersId, exclusions, k=None):
+        """As the call, with row r's listed ids left out: `exclusions` is an (indptr int64 [>= U+1], ids int32) CSR of
+        global ids (position + id_offset), ascending within each row (hotpath.exclusion_csr).  Rows with fewer than k
+        remaining items are padded with (-inf, -1)."""
+        return self._run(usersId, k, exclusions)
 
 
 class NeuMFDataset:

@@ -23,6 +23,7 @@
 // per m-tile pass (L2-resident item index) + 8k B of results per user.
 #include "common.cuh"
 #include "tc.cuh"
+#include "topk_select.cuh"
 #include <cuda_bf16.h>
 #include <limits.h>
 #include <math_constants.h>
@@ -59,19 +60,6 @@ struct TopkParams {
 // there and the id it points at.  Static shared memory, not registers -- the kernel sits at the 168-register cap of two
 // CTAs per SM -- touched only on the candidate path.  Budgeted as 4 KB (ptxas places 3 KB).
 constexpr size_t kExclCursorBytes = 4096;
-
-template <int K>
-__device__ __forceinline__ void topk_insert(float (&vals)[K], int32_t (&ids)[K], float v, int32_t id) {
-  // precondition: v > vals[K-1].  vals sorted descending; strict '>' keeps earlier (lower id) on ties.
-#pragma unroll
-  for (int j = K - 1; j > 0; --j) {
-    const bool up = v > vals[j - 1];
-    const bool here = v > vals[j];
-    ids[j] = up ? ids[j - 1] : (here ? id : ids[j]);
-    vals[j] = up ? vals[j - 1] : fmaxf(v, vals[j]);
-  }
-  if (v > vals[0]) { vals[0] = v; ids[0] = id; }
-}
 
 template <int K_CAP, bool EXCL>
 __global__ void __launch_bounds__(kThreadsTopk, 2)

@@ -485,6 +485,33 @@ int brk_topk_rows(brk_ctx* ctx, const float* scores, int64_t R, int64_t I, int32
                   int32_t* out_ids, void* stream);
 int brk_topk_merge(brk_ctx* ctx, const float* part_vals, const int32_t* part_ids, int32_t n_parts,
                    int64_t U, int32_t k, float* out_vals, int32_t* out_ids, void* stream);
+/* Full-catalog NeuMF top-k in one tcgen05 launch (csrc/neumf_topk.cu): per user, the k best items by the model's
+ * inference prediction, scores never written to HBM.  The first layer factors, x0 W1 + b1 = A_u + B_i, and the caller
+ * supplies both halves:
+ *   user_side  A [U, H1]  = uMLP[users] W1[0:E]             (TF32 operands, fp32 accumulation: brk_gemm_tf32)
+ *   item_side  B [I, H1]  = iMLP[items] W1[E:2E] + b1       (the same)
+ *   item_mf    [I, EMF]   = iMF[items], the indexed items' MF rows;  users [U]: rows of m->uMF.
+ * Per pair the kernel computes y1 = BN1(relu(A_u + B_i)) with the moving statistics (no BN in the He et al. variant),
+ * y2 = BN2(relu(y1 W2 + b2)), h3 = relu(y2 W3 + b3) -- both products tcgen05.mma kind::tf32, fp32 accumulation --
+ * then logit = h3 W4[0:H3] + gmf + b4 in fp32 (gmf = <uMF[u], iMF[i]> W4[H3] for the scalar Dot, sum of
+ * uMF[u] * W4[H3:H3+EMF] * iMF[i] for the Hadamard GMF) and out = 1 / (1 + expf(-logit)), the value brk_neumf_step
+ * returns for the pair (to TF32 rounding).  Selection on out: score desc, ties -> lower item id; ids are local
+ * positions plus id_offset; rows with fewer than k candidates are padded with (-inf, -1).  A pair's score does not
+ * depend on which other users or items share the call.  k <= 32.  Built instances (relu): the class graph
+ * (32;32,16,8) and (64;64,32,16) with tensor_cores = 1, and the He et al. variant E 32, EMF 8, (32,16,8), Hadamard,
+ * no BatchNorm; any other model is BRK_E_ARG.  Operands 16-byte aligned.  Workspace: brk_neumf_topk_workspace_bytes.
+ * _excl: per-row exclusions with the contract of brk_score_topk_bf16_excl (global ids, ascending per row; ids outside
+ * [id_offset, id_offset + I) ignored; empty lists give brk_neumf_score_topk's result bit for bit). */
+int64_t brk_neumf_topk_workspace_bytes(brk_ctx* ctx, int64_t U, int64_t I, int32_t k);
+int brk_neumf_score_topk(brk_ctx* ctx, const brk_neumf_model* m, const float* user_side, const int32_t* users,
+                         int64_t U, const float* item_side, const float* item_mf, int64_t I, int32_t k,
+                         int32_t id_offset, float* out_vals, int32_t* out_ids, void* workspace,
+                         int64_t workspace_bytes, void* stream);
+int brk_neumf_score_topk_excl(brk_ctx* ctx, const brk_neumf_model* m, const float* user_side, const int32_t* users,
+                              int64_t U, const float* item_side, const float* item_mf, int64_t I, int32_t k,
+                              int32_t id_offset, const int64_t* excl_indptr, const int32_t* excl_ids,
+                              float* out_vals, int32_t* out_ids, void* workspace, int64_t workspace_bytes,
+                              void* stream);
 
 /* ---- K9: ranking metrics ----------------------------------------------------------------------
  * Stands in for topKMetrics (trainers/topKmetrics.py:74-99): ids [U,k] are the recommended item ids
