@@ -16,7 +16,6 @@ Differences from the reference, stated once:
   * ids are int32 (the reference casts them to float32, BPRModel.py:101-103).
 """
 import ctypes as C
-import os
 
 import numpy as np
 import torch
@@ -180,7 +179,7 @@ class BPRNet:
         trains its own slice, gradients are scaled by 1/(world * batch) and summed by one all-reduce,
         every rank applies the same Adam step."""
         w = D.world_size()
-        if self.peer is not None and os.environ.get("BRK_DP_FUSED", "1") == "1":
+        if self.peer is not None:
             # one cooperative launch: fused fwd/bwd + cross-GPU reduce-scatter / Adam / all-gather
             if loss_out is None:
                 loss_out = torch.empty(1, dtype=torch.float32, device=self.device)

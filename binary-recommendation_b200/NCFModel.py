@@ -4,7 +4,7 @@ from a checkpoint and queried per user over ALL product ids of its training file
 
 The reference's predictForUser (:42-51) runs model.predict over one (customer, product) frame, drops predictions
 >= 1.0, sorts the rest descending and returns {product: '%.9f' % score} for the best numberOfItem.  Here the frame is
-one fused-forward launch over the catalog (csrc/neumf2.cu, inference mode) and the selection a device top-k
+the forward kernels of csrc/neumf.cu over the catalog (inference mode) and the selection a device top-k
 (predictions >= 1.0 masked out first); several users go through predictForUsers in one pass.
 """
 import numpy as np

@@ -32,7 +32,6 @@ from . import synth
 from .RModel import RModel
 
 TC_SPECS = {(64, 64, 32, 16), (32, 32, 16, 8)}
-BUILT_SPECS = {(32, 32, 16, 8), (64, 64, 32, 16), (16, 16, 8, 4), (8, 8, 4, 2), (10, 100, 50, 10)}
 # He et al. variant instances of the one-launch tensor-core kernel (csrc/neumf_fused.cu): (E, EMF, hidden)
 FUSED_VARIANTS = {(32, 8, (32, 16, 8))}
 

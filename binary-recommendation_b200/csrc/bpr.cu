@@ -261,7 +261,6 @@ struct BprCoopParams {
   // and, in word 4, 1 if the Adam ran from shared memory (0: global memory).  world > 1: see profiles/dp_trace.py.
   unsigned long long* dbg;
   long long spin_budget;          // clock64 budget of one cross-GPU wait (default ~30 s; BRK_PEER_SPIN_MS)
-  int32_t prefetch;               // bulk L2 prefetch of the table state at kernel entry (BRK_BPR_NO_PREFETCH=1 turns it off)
   unsigned int* bar;              // grid-barrier words {count, error, base} (common.cuh)
   // Adam operands in shared memory (world == 1): CTA b owns float4 [b * slice4[k], (b + 1) * slice4[k]) of table k's
   // w / m / v / g; 0 = Adam straight from global memory (slices too large, or BRK_BPR_NO_SMEM_ADAM=1)
@@ -397,7 +396,7 @@ __global__ void __launch_bounds__(kThreads, 4) bpr_steps_coop(const BprCoopParam
           const uint32_t dst = uint32_t(__cvta_generic_to_shared(adam_smem)) + (a - 1) * tx + (k ? nb[0] : 0u);
           asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                        ::"r"(dst), "l"(src), "r"(nb[k]), "r"(bar) : "memory");
-        } else if (P.prefetch && arrs[a] != nullptr && brk_aligned16(arrs[a])) {
+        } else if (arrs[a] != nullptr && brk_aligned16(arrs[a])) {
           asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(nb[k]) : "memory");
         }
       }
@@ -767,7 +766,6 @@ static int launch_coop_steps(brk_ctx* ctx, const brk_table* user, const brk_tabl
     BRK_CUDA(cudaMemset(g_coop_trace, 0, 4096 * 8 * sizeof(unsigned long long)));
   }
   P.dbg = (g_coop_trace && n_steps <= 4096) ? g_coop_trace : nullptr;
-  P.prefetch = getenv("BRK_BPR_NO_PREFETCH") ? 0 : 1;
   P.bar = ctx->bar[BRK_BAR_BPR];
   {
     const char* e = getenv("BRK_PEER_SPIN_MS");              // budget of one cross-GPU wait; default ~30 s at 2 GHz

@@ -21,33 +21,21 @@
 //   * dropout masks are regenerated from Philox (never stored): stream defined in oracle/neumf.py.
 // Algorithmic HBM/L2 traffic per interaction at E=32: 4 rows gathered (512 B) + 12 B ids/label +
 // 4 B prediction (528 B, SURVEY.md 8d) + 4 row gradients (512 B) + 2x re-gather in the backward.
+//
+// These kernels serve the script spec (10;100,50,10): the tiled kernels of neumf2.cu need power-of-two widths.
 #include "common.cuh"
+#include "neumf_common.cuh"   // parameter / accumulator layouts, BatchNorm and dropout constants, activations
 #include <math_constants.h>
-#include <stdlib.h>
 
 namespace {
 
+using v2::Acc; using v2::Layout;
+using v2::act_f; using v2::act_grad; using v2::drop16;
+using v2::kBnEps; using v2::kBnMomentum;
+
 constexpr int kTile = 128;            // samples per CTA = threads per CTA
-constexpr float kBnEps = 1e-3f;       // Keras BatchNormalization default epsilon
-constexpr float kBnMomentum = 0.99f;  // Keras default momentum
-constexpr uint32_t kDropThreshold = 51;               // byte < 51 -> dropped (keep prob 205/256)
-constexpr float kDropScale = 256.0f / 205.0f;
 
 __host__ __device__ constexpr int pad4(int x) { return (x + 3) & ~3; }
-
-template <int E, int H1, int H2, int H3>
-struct Layout {   // offsets (floats) inside the flat dense parameter block -- mirrored in hotpath.py
-  static constexpr int W1 = 0, b1 = W1 + 2 * E * H1, g1 = b1 + H1, be1 = g1 + H1;
-  static constexpr int W2 = be1 + H1, b2 = W2 + H1 * H2, g2 = b2 + H2, be2 = g2 + H2;
-  static constexpr int W3 = be2 + H2, b3 = W3 + H2 * H3, W4 = b3 + H3;   // b4 = W4 + H3 + 1
-};
-// accumulator block (doubles): forward sums, backward sums, loss
-template <int H1, int H2>
-struct Acc {
-  static constexpr int s1 = 0, q1 = s1 + H1, s2 = q1 + H1, q2 = s2 + H2;        // sum h, sum h^2
-  static constexpr int d2 = q2 + H2, e2 = d2 + H2, d1 = e2 + H2, e1 = d1 + H1;  // sum dy, sum dy*xhat
-  static constexpr int loss = e1 + H1, total = loss + 1;
-};
 
 struct NeumfArgs {
   brk_table uMLP, iMLP, uMF, iMF, dense;
@@ -63,22 +51,6 @@ struct NeumfArgs {
   int32_t training;
 };
 
-template <int ACT> __device__ __forceinline__ float act_f(float x) {
-  return ACT == 0 ? fmaxf(x, 0.f) : 1.0f / (1.0f + expf(-x));
-}
-template <int ACT> __device__ __forceinline__ float act_grad_from_out(float h) {
-  return ACT == 0 ? (h > 0.f ? 1.f : 0.f) : h * (1.f - h);
-}
-
-// Dropout multipliers for features [16c, 16c+16) of sample idx in `layer`.
-__device__ __forceinline__ void drop16(uint64_t idx, int c, int layer, uint32_t seed, uint32_t epoch, float (&m)[16]) {
-  const uint4 w = philox4x32_10(make_uint4(uint32_t(idx), uint32_t(idx >> 32), uint32_t(c), 0xD0u + layer), seed, epoch);
-  const uint32_t ww[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-  for (int q = 0; q < 4; ++q)
-#pragma unroll
-    for (int b = 0; b < 4; ++b) m[q * 4 + b] = ((ww[q] >> (8 * b)) & 0xFFu) >= kDropThreshold ? kDropScale : 0.f;
-}
 // In-place dropout on a shared-memory row of n features.
 template <int N>
 __device__ __forceinline__ void drop_row(float* row, uint64_t idx, int layer, uint32_t seed, uint32_t epoch) {
@@ -392,7 +364,7 @@ __global__ void __launch_bounds__(kTile) neumf_head(const NeumfArgs A) {
       hz[t * (H3 + 2) + H3 + 1] = dlogit;
 #pragma unroll
       for (int j = 0; j < pad4(H3); ++j)
-        dz[j] = j < H3 ? dlogit * w4[j] * act_grad_from_out<ACT>(h3[j]) : 0.f;
+        dz[j] = j < H3 ? dlogit * w4[j] * act_grad<ACT>(h3[j]) : 0.f;
     }
   } else {
 #pragma unroll
@@ -500,7 +472,7 @@ __global__ void __launch_bounds__(kTile) neumf_bwd2(const NeumfArgs A) {
         const float xh = (h - mean2[j]) * rstd2[j];
         const float dy = A.dy2[int64_t(j) * A.B + b0 + t];
         const float dh = gam2[j] * rstd2[j] * (dy - sdy[j] - xh * sdyx[j]);
-        dz[j] = dh * act_grad_from_out<ACT>(h);
+        dz[j] = dh * act_grad<ACT>(h);
       } else dz[j] = 0.f;
     }
   } else {
@@ -576,7 +548,7 @@ __global__ void __launch_bounds__(kTile) neumf_bwd1(const NeumfArgs A, unsigned 
         const float xh = (h - mean1[j]) * rstd1[j];
         const float dy = A.dy1[int64_t(j) * A.B + b0 + t];
         const float dh = gam1[j] * rstd1[j] * (dy - sdy[j] - xh * sdyx[j]);
-        dz[j] = dh * act_grad_from_out<ACT>(h);
+        dz[j] = dh * act_grad<ACT>(h);
       } else dz[j] = 0.f;
     }
   } else {
@@ -750,12 +722,10 @@ extern "C" int brk_neumf_step(brk_ctx* ctx, const brk_neumf_model* m, const int3
                   m->E, m->H1, m->H2, m->H3);
     return BRK_E_ARG;
   }
-  if (getenv("BRK_NEUMF_V1") == nullptr) {
-    int rc2 = 0;
-    if (brk_neumf_step_v2(ctx, m, nullptr, u, i, y, batch, global_batch, first_index, training, dropout_seed,
-                          dropout_epoch, ws, out, loss_out, (cudaStream_t)stream, &rc2) == 0)
-      return rc2;
-  }
+  int rc2 = 0;
+  if (brk_neumf_step_v2(ctx, m, nullptr, u, i, y, batch, global_batch, first_index, training, dropout_seed, dropout_epoch,
+                        ws, out, loss_out, (cudaStream_t)stream, &rc2) == 0)
+    return rc2;
   NeumfArgs A;
   A.uMLP = m->uMLP; A.iMLP = m->iMLP; A.uMF = m->uMF; A.iMF = m->iMF; A.dense = m->dense;
   A.u = u; A.i = i; A.y = y ? y : out; A.B = batch; A.first_index = first_index; A.global_B = global_batch > 0 ? global_batch : batch;
@@ -765,16 +735,8 @@ extern "C" int brk_neumf_step(brk_ctx* ctx, const brk_neumf_model* m, const int3
   A.dropout = (m->dropout != 0 && training) ? 1 : 0;
   A.loss_kind = m->loss; A.training = training;
   cudaStream_t st = (cudaStream_t)stream;
-#define BRK_NEUMF_CASE(E_, A_, B_, C_)                                                             \
-  if (m->E == E_ && m->H1 == A_ && m->H2 == B_ && m->H3 == C_) {                                    \
-    return m->act == 0 ? run_neumf<E_, A_, B_, C_, 0>(ctx, A, st) : run_neumf<E_, A_, B_, C_, 1>(ctx, A, st); \
-  }
-  BRK_NEUMF_CASE(32, 32, 16, 8)      // reference class spec, numFactor 32 (RModel.py:35): MLP 64-32-16-8
-  BRK_NEUMF_CASE(64, 64, 32, 16)     // BASELINE.json configs[3]: 64-dim tables
-  BRK_NEUMF_CASE(8, 8, 4, 2)         // small spec used by the tests
-  BRK_NEUMF_CASE(16, 16, 8, 4)
-  BRK_NEUMF_CASE(10, 100, 50, 10)    // script spec trainers/NFC_plain.py:109-152
-#undef BRK_NEUMF_CASE
+  if (m->E == 10 && m->H1 == 100 && m->H2 == 50 && m->H3 == 10)    // script spec trainers/NFC_plain.py:109-152
+    return m->act == 0 ? run_neumf<10, 100, 50, 10, 0>(ctx, A, st) : run_neumf<10, 100, 50, 10, 1>(ctx, A, st);
   // numFactor is a free attribute of the reference model (RModel.py:35): every other width runs on the any-width kernels
   return brk_neumf_step_generic(ctx, m, u, i, y, batch, global_batch, first_index, training, dropout_seed, dropout_epoch, ws, out,
                                 y ? loss_out : nullptr, st);

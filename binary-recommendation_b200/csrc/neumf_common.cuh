@@ -1,4 +1,4 @@
-// Shared by the tiled SIMT NeuMF kernels (neumf2.cu) and the tensor-core ones (neumf_tc.cu): parameter
+// Shared by the NeuMF kernels (neumf.cu, neumf2.cu, neumf_tc.cu, neumf_fused.cu, neumf_generic.cu): parameter
 // layout, accumulator layout, sharded-table addressing, kernel arguments, activations, dropout bits.
 #pragma once
 #include "common.cuh"
@@ -11,15 +11,16 @@ constexpr uint32_t kDropThreshold = 51;
 constexpr float kDropScale = 256.0f / 205.0f;
 
 template <int E, int H1, int H2, int H3>
-struct Layout {
+struct Layout {   // offsets (floats) inside the flat dense parameter block -- mirrored in hotpath.py
   static constexpr int W1 = 0, b1 = W1 + 2 * E * H1, g1 = b1 + H1, be1 = g1 + H1;
   static constexpr int W2 = be1 + H1, b2 = W2 + H1 * H2, g2 = b2 + H2, be2 = g2 + H2;
-  static constexpr int W3 = be2 + H2, b3 = W3 + H2 * H3, W4 = b3 + H3;
+  static constexpr int W3 = be2 + H2, b3 = W3 + H2 * H3, W4 = b3 + H3;   // b4 = W4 + H3 + 1
 };
+// accumulator block (doubles): forward sums, backward sums, loss
 template <int H1, int H2>
 struct Acc {
-  static constexpr int s1 = 0, q1 = s1 + H1, s2 = q1 + H1, q2 = s2 + H2;
-  static constexpr int d2 = q2 + H2, e2 = d2 + H2, d1 = e2 + H2, e1 = d1 + H1;
+  static constexpr int s1 = 0, q1 = s1 + H1, s2 = q1 + H1, q2 = s2 + H2;        // sum h, sum h^2
+  static constexpr int d2 = q2 + H2, e2 = d2 + H2, d1 = e2 + H2, e1 = d1 + H1;  // sum dy, sum dy*xhat
   static constexpr int loss = e1 + H1, total = loss + 1;
 };
 

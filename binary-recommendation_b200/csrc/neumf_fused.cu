@@ -1114,7 +1114,7 @@ int run(brk_ctx* ctx, const Args& A, const AdamReq* adam, cudaStream_t st, int* 
   // onto one SM and leave others idle, and every barrier then waits for the slow pairs.  Asking for more than half of the
   // SM's shared memory forces the spread.
   size_t smem = S::smem;
-  if (int(grid) <= ctx->sm_count && smem < size_t(120) * 1024 && getenv("BRK_NEUMF_PACK") == nullptr) smem = size_t(120) * 1024;
+  if (int(grid) <= ctx->sm_count && smem < size_t(120) * 1024) smem = size_t(120) * 1024;
   BRK_CUDA(cudaLaunchCooperativeKernel((const void*)fn, dim3(grid), dim3(NT), args, smem, st));
   return 0;
 }

@@ -1078,12 +1078,6 @@ int run(brk_ctx* ctx, const Args& A, cudaStream_t st) {
       if (occ_c > 4) occ_c = 4;
       if (occ_c < 1) occ_c = 1;
     }
-    if (getenv("BRK_NTC_DEBUG")) {
-      cudaFuncAttributes fa;
-      BRK_CUDA(cudaFuncGetAttributes(&fa, tc_head<E, H1, H2, H3, ACT>));
-      fprintf(stderr, "[brk] tc_head: regs %d static smem %zu dynamic %zu -> %d CTAs/SM; bwd2 %d, bwd1 %d (smem %zu / %zu)\n",
-              fa.numRegs, fa.sharedSizeBytes, smC, occ_c, occ_d, occ_e, smD, smE);
-    }
     BRK_REQUIRE(occ_d > 0 && occ_e > 0 && occ_c > 0, BRK_E_STATE, "brk_neumf_step: tensor-core kernels do not fit");
     occ_done = true;
   }

@@ -5,19 +5,19 @@
 // The sequential pass only orders ratings that share a user or an item: rating k reads and writes row P[u_k],
 // row Q[i_k], bu[u_k], bi[i_k] and nothing else.  brk_svd_schedule gives every rating two tickets,
 //   tu[k] = number of earlier ratings of the same user,  ti[k] = number of earlier ratings of the same item,
-// and the epoch kernel keeps one version counter per user row and per item row.  A warp owns rating k, waits
-// until ver_u[u] == tu[k] and ver_i[i] == ti[k] (every earlier rating touching either row has been applied),
-// applies the update and bumps both counters with release stores.  Ratings are dealt to the resident warps
-// round-robin in file order, so the oldest unfinished rating is always held by a running warp whose tickets are
-// already satisfied: no deadlock (the launch is cooperative, which guarantees co-residency), no global barrier,
-// and the result equals the sequential pass up to the summation order inside the 'np.dot' (a 5-step butterfly
-// over the lanes here; the element-wise updates are not contracted into FMAs, like NumPy).
+// and every word of a parameter row carries the version of the row (self-validating rows, below).  A warp owns
+// rating k, polls its user's and its item's rows until they carry versions tu[k] and ti[k] (every earlier rating
+// touching either row has been applied), applies the update and writes the new rows with versions tu[k] + 1 and
+// ti[k] + 1.  Ratings are dealt to the resident warps round-robin in file order, so the oldest unfinished rating is
+// always held by a running warp whose tickets are already satisfied: no deadlock (the launch is cooperative, which
+// guarantees co-residency), no global barrier, and the result equals the sequential pass up to the summation order
+// inside the 'np.dot' (a 5-step butterfly over the lanes here; the element-wise updates are not contracted into FMAs,
+// like NumPy).
 //
 // Bound: not HBM, not the tensor pipe -- the longest dependency chain (>= the rating count of the most popular
 // item) times one L2 hand-over of a row between two SMs.  DESIGN.md section 4.5.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace {
@@ -25,11 +25,6 @@ namespace {
 constexpr int kSvdThreads = 256;
 constexpr int kSvdWarps = kSvdThreads / 32;
 
-__device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
 __device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
   uint32_t v;
   asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
@@ -37,15 +32,6 @@ __device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
 }
 __device__ __forceinline__ void st_relaxed_u32(uint32_t* p, uint32_t v) {
   asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" :: "l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void fence_acq_rel_gpu() { asm volatile("fence.acq_rel.gpu;" ::: "memory"); }
-__device__ __forceinline__ double ld_l2_f64(const double* p) {     // rows are handed over between SMs: L2 only
-  double v;
-  asm volatile("ld.relaxed.gpu.global.f64 %0, [%1];" : "=d"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_l2_f64(double* p, double v) {
-  asm volatile("st.relaxed.gpu.global.f64 [%0], %1;" :: "l"(p), "d"(v) : "memory");
 }
 __device__ __forceinline__ double warp_sum_f64(double x) {
 #pragma unroll
@@ -58,107 +44,21 @@ __device__ __forceinline__ double svd_rule(double w, double other, double e, dou
   return __dadd_rn(w, __dmul_rn(lr, __dsub_rn(__dmul_rn(e, other), __dmul_rn(reg, w))));
 }
 
-struct SvdFit {
+// Self-validating rows.  Every 8-byte word of a row carries its own version: a float64 element is two words
+// {low half | version << 32} {high half | version << 32} written by one st.v2.b64 (two 8-byte accesses, each
+// single-copy atomic).  The consumer polls the row itself and accepts a word when its version equals the ticket;
+// version t of a row is written once (by the rating with ticket t - 1), read by exactly one warp (the rating with
+// ticket t) and then overwritten by that same warp -- no fence, no separate flag, no reader that could see a torn row.
+// A separate version counter per row costs, per hand-over of a row from one warp to the next, row stores -> fence ->
+// flag store, then on the other side flag poll -> row loads (about 3.5 L2 round trips): it measured half the speed of
+// this form (profiles/r01m_svd_sweep.txt).  Parameters are packed into this form at the start of the epoch and
+// unpacked at its end (two streaming passes over the tables).
+struct SvdLL {
   const int4* sched;          // [n] (user, item, user ticket, item ticket)
   const double* ratings;      // [n]
   int64_t n;
-  double *P, *Q, *bu, *bi;
-  uint32_t *ver_u, *ver_i;    // zero at launch
-  uint32_t* abort;            // set when a wait exceeds kSvdSpinLimit polls (inconsistent schedule): every warp leaves
-  double mu, lr, ereg, breg;
-  int32_t d;
-};
-
-// A wait is bounded: a schedule that does not belong to the rating arrays would otherwise spin for ever.
-constexpr uint32_t kSvdSpinLimit = 1u << 25;
-template <int POLL>
-__device__ __forceinline__ bool svd_wait(const uint32_t* flag, uint32_t want, uint32_t* abort) {
-  uint32_t spins = 0;
-  while ((POLL == 0 ? ld_acquire_u32(flag) : ld_relaxed_u32(flag)) != want) {
-    if ((++spins & 1023u) == 0) {
-      if (spins >= kSvdSpinLimit) st_relaxed_u32(abort, 1u);
-      if (ld_relaxed_u32(abort) != 0u) return false;
-    }
-  }
-  return true;
-}
-
-// EPL = row elements per lane (d <= 32 * EPL).
-// POLL 0: acquire loads in the spin loop; POLL 1: relaxed loads, then one acquire fence.
-template <int EPL, int POLL>
-__global__ void __launch_bounds__(kSvdThreads) svd_epoch_kernel(SvdFit a) {
-  const int lane = threadIdx.x & 31;
-  const int64_t W = int64_t(gridDim.x) * kSvdWarps;
-  // consecutive ratings go to different SMs: warp slot = (warp in block) * grid + block
-  int64_t k = int64_t(threadIdx.x >> 5) * gridDim.x + blockIdx.x;
-  if (k >= a.n) return;
-  int4 s = __ldg(a.sched + k);
-  double r = __ldg(a.ratings + k);
-  while (true) {
-    const int64_t kn = k + W;
-    int4 sn = s;
-    double rn = r;
-    if (kn < a.n) { sn = __ldg(a.sched + kn); rn = __ldg(a.ratings + kn); }   // in flight while this one waits
-
-    const uint32_t* vu = a.ver_u + s.x;
-    const uint32_t* vi = a.ver_i + s.y;
-    if (!svd_wait<POLL>(vu, uint32_t(s.z), a.abort) || !svd_wait<POLL>(vi, uint32_t(s.w), a.abort)) return;
-    if (POLL == 1) fence_acq_rel_gpu();
-
-    double* prow = a.P + int64_t(s.x) * a.d;
-    double* qrow = a.Q + int64_t(s.y) * a.d;
-    double p[EPL], q[EPL];
-#pragma unroll
-    for (int e = 0; e < EPL; ++e) {
-      const int c = lane + 32 * e;
-      p[e] = 0.0; q[e] = 0.0;
-      if (c < a.d) { p[e] = ld_l2_f64(prow + c); q[e] = ld_l2_f64(qrow + c); }
-    }
-    const double b_u = ld_l2_f64(a.bu + s.x), b_i = ld_l2_f64(a.bi + s.y);
-    double dot = 0.0;
-#pragma unroll
-    for (int e = 0; e < EPL; ++e) dot = __dadd_rn(dot, __dmul_rn(q[e], p[e]));
-    dot = warp_sum_f64(dot);
-    // error = rating - (user_bias + item_bias + global_bias + dot)                           SVD.py:198
-    const double err = __dsub_rn(r, __dadd_rn(__dadd_rn(__dadd_rn(b_u, b_i), a.mu), dot));
-#pragma unroll
-    for (int e = 0; e < EPL; ++e) {
-      const int c = lane + 32 * e;
-      if (c < a.d) {
-        const double qn = svd_rule(q[e], p[e], err, a.lr, a.ereg);        // item vector first           :203
-        const double pn = svd_rule(p[e], qn, err, a.lr, a.ereg);          // user vector from the NEW q  :204
-        st_l2_f64(qrow + c, qn);
-        st_l2_f64(prow + c, pn);
-      }
-    }
-    if (lane == 0) st_l2_f64(a.bu + s.x, svd_rule(b_u, b_u, err, a.lr, a.breg));   // error * bias itself :205
-    if (lane == 1) st_l2_f64(a.bi + s.y, svd_rule(b_i, b_i, err, a.lr, a.breg));   //                     :206
-    __syncwarp();
-    if (lane == 0) {                     // release: the fence is cumulative over the row stores of the other lanes
-      fence_acq_rel_gpu();
-      st_relaxed_u32(a.ver_u + s.x, uint32_t(s.z) + 1u);
-      st_relaxed_u32(a.ver_i + s.y, uint32_t(s.w) + 1u);
-    }
-    if (kn >= a.n) break;
-    k = kn; s = sn; r = rn;
-  }
-}
-
-// ---- second form: self-validating rows ------------------------------------------------------------------------------
-// The flag form above pays, per hand-over of a row from one warp to the next: row stores -> fence -> flag store, then
-// on the other side flag poll -> row loads (about 3.5 L2 round trips).  Here every 8-byte word of a row carries its own
-// version: a float64 element is two words {low half | version << 32} {high half | version << 32} written by one
-// st.v2.b64 (two 8-byte accesses, each single-copy atomic).  The consumer polls the row itself and accepts a word
-// when its version equals the ticket; version t of a row is written once (by the rating with ticket t - 1), read by
-// exactly one warp (the rating with ticket t) and then overwritten by that same warp -- no fence, no separate flag,
-// no reader that could see a torn row.  Parameters are packed into this form at the start of the epoch and unpacked
-// at its end (two streaming passes over the tables).
-struct SvdLL {
-  const int4* sched;
-  const double* ratings;
-  int64_t n;
   ulonglong2 *P, *Q, *bu, *bi;
-  uint32_t* abort;
+  uint32_t* abort;            // set when a wait exceeds kSvdSpinLimit polls (inconsistent schedule): every warp leaves
   double mu, lr, ereg, breg;
   int32_t d;
 };
@@ -182,6 +82,10 @@ __device__ __forceinline__ double ll_value(const ulonglong2& v) {
   return __longlong_as_double((long long)((v.y << 32) | (v.x & 0xffffffffull)));
 }
 
+// A wait is bounded: a schedule that does not belong to the rating arrays would otherwise spin for ever.
+constexpr uint32_t kSvdSpinLimit = 1u << 25;
+
+// EPL = row elements per lane (d <= 32 * EPL).
 template <int EPL>
 __global__ void __launch_bounds__(kSvdThreads) svd_epoch_ll_kernel(SvdLL a) {
   const int lane = threadIdx.x & 31;
@@ -493,14 +397,9 @@ extern "C" int brk_svd_schedule(brk_ctx* ctx, const int32_t* users, const int32_
 }
 
 template <int EPL>
-static int svd_launch_epoch(brk_ctx* ctx, SvdFit& a, SvdLL& b, int warps_per_sm, cudaStream_t st) {
-  // BRK_SVD_FORM=flags selects the first form (version counters + fences); a measurement knob, not part of the ABI
-  const char* env = getenv("BRK_SVD_FORM");
-  const bool flags = env && env[0] == 'f';
-  const void* fn = flags ? (const void*)svd_epoch_kernel<EPL, 0> : (const void*)svd_epoch_ll_kernel<EPL>;
+static int svd_launch_epoch(brk_ctx* ctx, SvdLL& a, int warps_per_sm, cudaStream_t st) {
   int occ = 0;
-  if (flags) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, svd_epoch_kernel<EPL, 0>, kSvdThreads, 0));
-  else BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, svd_epoch_ll_kernel<EPL>, kSvdThreads, 0));
+  BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, svd_epoch_ll_kernel<EPL>, kSvdThreads, 0));
   BRK_REQUIRE(occ >= 1, BRK_E_STATE, "brk_svd_fit_epoch: kernel does not fit an SM");
   int per_sm = occ;
   if (warps_per_sm > 0) {
@@ -510,15 +409,15 @@ static int svd_launch_epoch(brk_ctx* ctx, SvdFit& a, SvdLL& b, int warps_per_sm,
   int64_t grid = int64_t(ctx->sm_count) * per_sm;
   const int64_t need = (a.n + kSvdWarps - 1) / kSvdWarps;
   if (grid > need) grid = need;
-  void* args[] = {flags ? (void*)&a : (void*)&b};
-  BRK_CUDA(cudaLaunchCooperativeKernel(fn, dim3((unsigned)grid), dim3(kSvdThreads), args, 0, st));
+  void* args[] = {&a};
+  BRK_CUDA(cudaLaunchCooperativeKernel((const void*)svd_epoch_ll_kernel<EPL>, dim3((unsigned)grid), dim3(kSvdThreads),
+                                       args, 0, st));
   return 0;
 }
 
-// workspace: [abort flag, 256 B] [P, Q, bu, bi in self-validating form, 16 B per element] [version counters of the
-// flag form, 4 B per row]
+// workspace: [abort flag, 256 B] [P, Q, bu, bi in self-validating form, 16 B per element]
 static int64_t svd_fit_ws_bytes(int64_t U, int64_t I, int64_t d) {
-  return 256 + int64_t(align256(size_t((U + I) * (d + 1)) * 16)) + int64_t(align256(size_t(U + I) * 4));
+  return 256 + int64_t(align256(size_t((U + I) * (d + 1)) * 16));
 }
 extern "C" int64_t brk_svd_fit_workspace_bytes(int64_t num_users, int64_t num_items, int32_t d) {
   if (num_users < 1 || num_items < 1 || d < 1 || d > 512) return BRK_E_ARG;
@@ -541,35 +440,28 @@ extern "C" int brk_svd_fit_epoch(brk_ctx* ctx, const int32_t* sched, const doubl
   if (n == 0) return 0;
   BRK_REQUIRE(sched && ratings, BRK_E_ARG, "brk_svd_fit_epoch: null schedule / ratings");
   BRK_REQUIRE(brk_aligned16(sched), BRK_E_ALIGN, "brk_svd_fit_epoch: sched not 16-byte aligned");
-  const char* env = getenv("BRK_SVD_FORM");
-  const bool flags = env && env[0] == 'f';
-  ulonglong2* ll = reinterpret_cast<ulonglong2*>(ws + 256);
-  uint32_t* versions = reinterpret_cast<uint32_t*>(ws + 256 + align256(size_t((num_users + num_items) * (int64_t(d) + 1)) * 16));
-  SvdFit a;
+  SvdLL a;
   a.sched = reinterpret_cast<const int4*>(sched); a.ratings = ratings; a.n = n;
-  a.P = P; a.Q = Q; a.bu = bu; a.bi = bi;
-  a.ver_u = versions; a.ver_i = versions + num_users; a.abort = reinterpret_cast<uint32_t*>(ws);
-  a.mu = mu; a.lr = lr; a.ereg = emb_reg; a.breg = bias_reg; a.d = d;
-  SvdLL b;
-  b.sched = a.sched; b.ratings = ratings; b.n = n;
-  b.P = ll; b.Q = b.P + num_users * int64_t(d); b.bu = b.Q + num_items * int64_t(d); b.bi = b.bu + num_users;
-  b.abort = a.abort; b.mu = mu; b.lr = lr; b.ereg = emb_reg; b.breg = bias_reg; b.d = d;
+  a.P = reinterpret_cast<ulonglong2*>(ws + 256); a.Q = a.P + num_users * int64_t(d); a.bu = a.Q + num_items * int64_t(d);
+  a.bi = a.bu + num_users;
+  a.abort = reinterpret_cast<uint32_t*>(ws); a.mu = mu; a.lr = lr; a.ereg = emb_reg; a.breg = bias_reg; a.d = d;
   SvdTables t;
   t.plain[0] = P; t.plain[1] = Q; t.plain[2] = bu; t.plain[3] = bi;
-  t.ll[0] = b.P; t.ll[1] = b.Q; t.ll[2] = b.bu; t.ll[3] = b.bi;
+  t.ll[0] = a.P; t.ll[1] = a.Q; t.ll[2] = a.bu; t.ll[3] = a.bi;
   t.end[0] = num_users * int64_t(d); t.end[1] = t.end[0] + num_items * int64_t(d);
   t.end[2] = t.end[1] + num_users; t.end[3] = t.end[2] + num_items;
   const int pack_grid = grid_for(t.end[3], ctx->sm_count, 256);
-  if (flags) BRK_CUDA(cudaMemsetAsync(versions, 0, size_t(num_users + num_items) * 4, st));
-  else { svd_pack_kernel<<<pack_grid, 256, 0, st>>>(t, 0); BRK_LAUNCH_CHECK(); }
+  svd_pack_kernel<<<pack_grid, 256, 0, st>>>(t, 0);
+  BRK_LAUNCH_CHECK();
   int rc;
-  if (d <= 32) rc = svd_launch_epoch<1>(ctx, a, b, warps_per_sm, st);
-  else if (d <= 64) rc = svd_launch_epoch<2>(ctx, a, b, warps_per_sm, st);
-  else if (d <= 128) rc = svd_launch_epoch<4>(ctx, a, b, warps_per_sm, st);
-  else if (d <= 256) rc = svd_launch_epoch<8>(ctx, a, b, warps_per_sm, st);
-  else rc = svd_launch_epoch<16>(ctx, a, b, warps_per_sm, st);
+  if (d <= 32) rc = svd_launch_epoch<1>(ctx, a, warps_per_sm, st);
+  else if (d <= 64) rc = svd_launch_epoch<2>(ctx, a, warps_per_sm, st);
+  else if (d <= 128) rc = svd_launch_epoch<4>(ctx, a, warps_per_sm, st);
+  else if (d <= 256) rc = svd_launch_epoch<8>(ctx, a, warps_per_sm, st);
+  else rc = svd_launch_epoch<16>(ctx, a, warps_per_sm, st);
   if (rc) return rc;
-  if (!flags) { svd_pack_kernel<<<pack_grid, 256, 0, st>>>(t, 1); BRK_LAUNCH_CHECK(); }
+  svd_pack_kernel<<<pack_grid, 256, 0, st>>>(t, 1);
+  BRK_LAUNCH_CHECK();
   return 0;
 }
 

@@ -27,7 +27,6 @@
 #include <cuda_bf16.h>
 #include <limits.h>
 #include <math_constants.h>
-#include <stdlib.h>
 
 namespace {
 
@@ -49,7 +48,6 @@ struct TopkParams {
   int32_t tiles_per_split;
   int32_t stages;
   int32_t id_offset;     // added to local item ids (item-range shards)
-  int32_t probe;         // diagnostics: 1 = epilogue only drains TMEM (measures the TMEM-read ceiling)
   float* out_vals;       // [n_splits * kHalves, U, k]
   int32_t* out_ids;
   const int64_t* excl_indptr;   // EXCL only: [U + 1] absolute offsets into excl_ids
@@ -205,36 +203,29 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
       return bits;
     };
 
-    auto process = [&](uint32_t (&r)[32], int64_t col0, bool ragged) {
-      if (P.probe == 1) {                               // keep the loads alive, do nothing else
-        uint32_t x = 0;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) x ^= r[j];
-        if (x == 0x7fc12345u) thr = 0.f;
-        return;
-      }
-      // The scores are used straight out of the registers tcgen05.ld filled: copying them into a float array cost 32
-      // moves per 32 scores, more than the max-tree itself.  Only the last item tile can be ragged; it takes the
-      // generic path below.
 #define V(j) __uint_as_float(r[(j)])
-      if (ragged) {
+    // A chunk of the last item tile, which can be ragged: every column is bounds-checked on its own.
+    auto process_ragged = [&](uint32_t (&r)[32], int64_t col0) {
 #pragma unroll
-        for (int j = 0; j < 32; ++j) scratch[j * kScratchStride] = V(j);
-        uint32_t live = 0xffffffffu;                      // EXCL: columns not listed
-        if constexpr (EXCL) live = ~excluded_bits(int32_t(col0) + P.id_offset);
+      for (int j = 0; j < 32; ++j) scratch[j * kScratchStride] = V(j);
+      uint32_t live = 0xffffffffu;                        // EXCL: columns not listed
+      if constexpr (EXCL) live = ~excluded_bits(int32_t(col0) + P.id_offset);
 #pragma unroll 1
-        for (int j = 0; j < 32; ++j) {
-          const float x = scratch[j * kScratchStride];
-          if (col0 + j < P.I && x > thr) {
-            if constexpr (EXCL) {
-              if (!((live >> j) & 1u)) continue;
-            }
-            topk_insert<K_CAP>(vals, ids, x, int32_t(col0 + j) + P.id_offset);
-            thr = vals[K_CAP - 1];
+      for (int j = 0; j < 32; ++j) {
+        const float x = scratch[j * kScratchStride];
+        if (col0 + j < P.I && x > thr) {
+          if constexpr (EXCL) {
+            if (!((live >> j) & 1u)) continue;
           }
+          topk_insert<K_CAP>(vals, ids, x, int32_t(col0 + j) + P.id_offset);
+          thr = vals[K_CAP - 1];
         }
-        return;
       }
+    };
+
+    // A flagged chunk of a full tile.  The scores are used straight out of the registers tcgen05.ld filled: copying them
+    // into a float array cost 32 moves per 32 scores, more than the max-tree itself.
+    auto process_flagged = [&](uint32_t (&r)[32], int64_t col0) {
       // 4 independent FMNMX3 chains, one per group of 8 columns
       float gm[4];
 #pragma unroll
@@ -271,8 +262,8 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
           }
         }
       }
-#undef V
     };
+#undef V
 
     // max of a 32-score chunk: 4 independent FMNMX3 chains (one per group of 8 columns), no branch
     auto chunk_max = [&](const uint32_t (&r)[32]) -> float {
@@ -297,33 +288,25 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
       const bool ragged = col_half + kBN / kHalves > P.I;   // only in the last item tile
       const uint32_t taddr = tmem_base + (uint32_t(quad * 32) << 16) + buf * kBN + half * (kBN / kHalves);
       uint32_t ra[32], rb[32];
-      if (P.probe == 2) {                                 // diagnostics: the half-tile as 2 x 64 packed 16-bit columns
-        tc::tmem_ld_32x32_pack16_issue(taddr, ra);
-        tc::tmem_ld_32x32_pack16_issue(taddr + 64, rb);
-        tc::tmem_ld_wait(ra);
-        tc::tmem_ld_wait(rb);
-        uint32_t x = 0;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) x ^= ra[j] ^ rb[j];
-        if (x == 0x7fc12345u) thr = 0.f;
-      } else if (ragged || P.probe != 0) {                // last item tile / diagnostics: chunk by chunk
+      if (ragged) {                                       // last item tile: chunk by chunk
         tc::tmem_ld_32x32_issue(taddr, ra);
         tc::tmem_ld_wait(ra);
 #pragma unroll 1
         for (int c = 0; c < kChunks; c += 2) {
           tc::tmem_ld_32x32_issue(taddr + (c + 1) * 32, rb);     // in flight while chunk c is processed
-          process(ra, col_half + c * 32, ragged);
+          process_ragged(ra, col_half + c * 32);
           tc::tmem_ld_wait(rb);
           if (c + 2 < kChunks) tc::tmem_ld_32x32_issue(taddr + (c + 2) * 32, ra);
-          process(rb, col_half + (c + 1) * 32, ragged);
+          process_ragged(rb, col_half + (c + 1) * 32);
           if (c + 2 < kChunks) tc::tmem_ld_wait(ra);
         }
       } else {
         // The common case has NO branch per chunk: the four chunk maxima are compared with the row's k-th best (as it
         // stood at the start of the tile: it only rises, so this flags a superset) into a 4-bit mask, and ONE warp-wide
-        // vote per tile decides whether anything has to be looked at again.  (With a compare-and-branch, a probe check
-        // and a ragged check per chunk the epilogue ran at 15-17 scores/clk/SM against 29 for the bare TMEM drain: the
-        // ~5 branches per chunk, not the max-tree, were the cost -- profiles/r02_topk_probe.txt.)
+        // vote per tile decides whether anything has to be looked at again.  (With a compare-and-branch and two uniform
+        // checks per chunk the epilogue ran at 15-17 scores/clk/SM against 29 for the bare TMEM drain: the ~5 branches per
+        // chunk, not the max-tree, were the cost, and one extra uniform branch per chunk alone cost 11 % --
+        // profiles/r02_topk_probe.txt.)
         static_assert(kChunks == 4, "the tile epilogue is written out for four 32-column chunks per warp");
         uint32_t flagged = 0u;
         tc::tmem_ld_32x32_issue(taddr, ra);
@@ -348,7 +331,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
           todo &= todo - 1;
           tc::tmem_ld_32x32_issue(taddr + c * 32, ra);
           tc::tmem_ld_wait(ra);
-          process(ra, col_half + c * 32, false);
+          process_flagged(ra, col_half + c * 32);
         }
       }
       tc::fence_before_sync();
@@ -525,7 +508,6 @@ int score_topk(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* 
   TopkParams P;
   P.U = U; P.I = I; P.KB = dpad / kKBlock; P.k = k; P.id_offset = id_offset;
   P.excl_indptr = excl_indptr; P.excl_ids = excl_ids;
-  P.probe = getenv("BRK_TOPK_PROBE") ? atoi(getenv("BRK_TOPK_PROBE")) : 0;
   int S, tps;
   P.n_tiles = plan_splits(ctx->sm_count * (dpad <= 128 ? 2 : 1), U, I, &S, &tps);
   P.tiles_per_split = tps;

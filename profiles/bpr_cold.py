@@ -1,6 +1,5 @@
 """BPR step (headline workload: ML-1M shape, d = 64, batch 16 384) timed the way bench.py's `value` is: L2 flushed before
-every step (256 MiB written and read back), CUDA events around the step's one launch -- and back to back (hot L2).
-  BRK_BPR_NO_PREFETCH=1 python profiles/bpr_cold.py     # without the bulk L2 prefetch at kernel entry"""
+every step (256 MiB written and read back), CUDA events around the step's one launch -- and back to back (hot L2)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT)
 import torch

@@ -1,6 +1,6 @@
-"""Biased-SVD epoch kernel (csrc/svd.cu): epoch time against residency (warps per SM) and the hand-over form (self-validating rows / flags + fences), on the
-ML-1M-shaped file (power-law head) and on a uniform file of the same size; prints the critical path so that the time
-per chain link can be read off.   python profiles/svd_case.py [once]      (once: a single epoch, for ncu)"""
+"""Biased-SVD epoch kernel (csrc/svd.cu): epoch time against residency (warps per SM), on the ML-1M-shaped file
+(power-law head) and on a uniform file of the same size; prints the critical path so that the time per chain link can
+be read off.   python profiles/svd_case.py [once]      (once: a single epoch, for ncu)"""
 import os
 import sys
 import time
@@ -43,13 +43,10 @@ def main():
         chain = frame.critical_path()
         print(f"skew={skew}: n={len(u)} critical path {chain} (max item count {np.bincount(i).max()}, max user count "
               f"{np.bincount(u).max()}), schedule build {t_sched * 1e3:.1f} ms (incl. H2D)", flush=True)
-        for form in ("rows", "flags"):
-            os.environ["BRK_SVD_FORM"] = form
-            for warps in (0, 24, 16, 8):
-                ms = epoch_ms(frame, P, Q, bu, bi, mu, warps)
-                print(f"  form={form:5s} warps_per_sm={warps:2d}: {ms:8.3f} ms/epoch  {len(u) / ms / 1e3:8.2f} M ratings/s  "
-                      f"{ms * 1e6 / chain:7.1f} ns per chain link", flush=True)
-        os.environ.pop("BRK_SVD_FORM", None)
+        for warps in (0, 24, 16, 8):
+            ms = epoch_ms(frame, P, Q, bu, bi, mu, warps)
+            print(f"  warps_per_sm={warps:2d}: {ms:8.3f} ms/epoch  {len(u) / ms / 1e3:8.2f} M ratings/s  "
+                  f"{ms * 1e6 / chain:7.1f} ns per chain link", flush=True)
 
 
 if __name__ == "__main__":
