@@ -354,6 +354,11 @@ class NeuMFNet:
         of the model, so rebuild it after training."""
         return NeuMFTopKIndex(self, itemsId, id_offset)
 
+    def topk_index_fp32(self, itemsId=None, id_offset=0):
+        """Full-catalog top-k index of an fp32 model (tensor_cores=False) over itemsId (default: every item): see
+        NeuMFTopKIndexFP32.  It snapshots the item side of the model, so rebuild it after training."""
+        return NeuMFTopKIndexFP32(self, itemsId, id_offset)
+
     def state_dict(self):
         sd = {"bn_moving": self.bn_moving.cpu(), "opt_state": self.optimizer.state.cpu()}
         for name, t in zip(("uMLP", "iMLP", "uMF", "iMF", "dense"), self.tables() + [self.dense]):
@@ -380,43 +385,24 @@ def _gemm_tf32(a, w, out, bias=None):
     return out
 
 
-class NeuMFTopKIndex:
-    """Full-catalog NeuMF top-k in one kernel launch (brk_neumf_score_topk): for each queried user, the k items of the
-    index with the highest prediction -- the value predict_on_batch returns for the pair, to TF32 rounding -- sorted
-    by score, ties to the lower position, scores never materialised.  Shaped like hotpath.BruteForceIndex:
+def _sgemm(a, w, out, bias=None):
+    """out [M, N] = a [M, K] @ w [K, N] (+ bias) in fp32 on the CUDA cores (brk_sgemm); a row of out depends on that row
+    of a alone (no split K)."""
+    M, K = a.shape
+    Nn = w.shape[1]
+    N.check(N.lib().brk_sgemm(N.ctx(a.device), N.ptr(a), C.c_void_p(w.data_ptr()), N.ptr(out),
+                              C.c_void_p(bias.data_ptr()) if bias is not None else None, M, Nn, K, K, Nn, Nn, 0, 0, 1.0, 0,
+                              N.stream_ptr()), "brk_sgemm")
+    return out
 
-        index = net.topk_index(itemsId)            # item side: iMLP[items] W1[E:2E] + b1 and the items' iMF rows
-        scores, ids = index(usersId, k=10)         # ids: positions in itemsId plus id_offset
-        scores, ids = index.query_with_exclusions(usersId, hotpath.exclusion_csr(rows, ids, len(usersId), dev))
 
-    The first Dense layer factors over [uMLP[u], iMLP[i]], so building the index computes the item half once and a
-    query the user half once; the kernel runs the rest of the network per pair on the tensor cores.  The index is a
-    snapshot of the item tables and keeps the model for the dense block, the BatchNorm statistics and the user tables:
-    rebuild it after training.  Built for the tensor-core class graph (numFactor 32 or 64, relu) and the He et al.
-    variant (E 32, mf_dim 8, hadamard, no BatchNorm); other models, and k > 32, raise ValueError -- rank them with
-    NeuMFNet.score_all.
-
-    Item-range shards: rank r indexes its range [lo, hi) with id_offset = lo; the merged lists equal the unsharded
-    index's bit for bit:
-
-        index = net.topk_index(np.arange(lo, hi), id_offset=lo)
-        scores, ids = distributed.sharded_topk(usersId, None, lo, k, local_topk=lambda q, c, off: index(q, k))
-
-    (or hotpath.topk_merge over the stacked [shards, U, k] lists in one process)."""
+class _FactoredTopKIndex:
+    """What the NeuMF top-k indexes share: the item half of the factored first layer computed once, the user half per
+    query, then one scoring + selection launch.  Subclasses name the product and the C entry points."""
 
     K_MAX = H.MAX_FUSED_K
 
     def __init__(self, net, itemsId=None, id_offset=0):
-        h1, h2, h3 = net.hidden
-        ok = net.act == "relu" and (
-            (not net.variant and net.tensor_cores and (net.E, h1, h2, h3) in TC_SPECS) or
-            (net.variant and net.mf_mode == "hadamard" and not net.batch_norm and
-             (net.E, net.EMF, net.hidden) in FUSED_VARIANTS))
-        if not ok:
-            raise ValueError(f"no fused top-k instance for E={net.E}, mf_dim={net.EMF}, hidden={net.hidden}, act={net.act}, "
-                             f"mf_mode={net.mf_mode}, batch_norm={net.batch_norm}, tensor_cores={net.tensor_cores}; built: "
-                             f"tensor-core class graph {sorted(TC_SPECS)} and the He et al. variant {sorted(FUSED_VARIANTS)} "
-                             "-- use NeuMFNet.score_all")
         self.net = net
         dev = net.device
         if itemsId is None:
@@ -424,15 +410,25 @@ class NeuMFTopKIndex:
         else:
             items = torch.as_tensor(np.asarray(itemsId, dtype=np.int32)).to(dev)
         if items.numel() == 0:
-            raise ValueError("NeuMFTopKIndex: no items")
+            raise ValueError(f"{type(self).__name__}: no items")
         self.num_candidates = items.numel()
         self.id_offset = int(id_offset)
         E = net.E
         W1 = net.param("W1")                                 # [2E, H1]: rows [0, E) act on uMLP, [E, 2E) on iMLP
         self._W1u, self._W1i = W1[:E], W1[E:]
-        self.item_side = _gemm_tf32(H.gather_rows(net.iMLP.w, items), self._W1i,
-                                    torch.empty((items.numel(), h1), dtype=torch.float32, device=dev), net.param("b1"))
+        self.item_side = self._product(H.gather_rows(net.iMLP.w, items), self._W1i,
+                                       torch.empty((items.numel(), net.hidden[0]), dtype=torch.float32, device=dev),
+                                       net.param("b1"))
         self.item_mf = H.gather_rows(net.iMF.w, items)
+
+    @staticmethod
+    def _product(a, w, out, bias=None):
+        raise NotImplementedError
+
+    def _workspace_bytes(self, lib, ctx, m, U, k):
+        raise NotImplementedError
+
+    _SCORE = _SCORE_EXCL = None                              # names of the C entry points
 
     def _check_k(self, k):
         k = 10 if k is None else int(k)
@@ -451,22 +447,22 @@ class NeuMFTopKIndex:
         ids = torch.empty((U, k), dtype=torch.int32, device=dev)
         if U == 0:
             return vals, ids
-        user_side = _gemm_tf32(H.gather_rows(net.uMLP.w, users), self._W1u,
-                               torch.empty((U, net.hidden[0]), dtype=torch.float32, device=dev))
+        user_side = self._product(H.gather_rows(net.uMLP.w, users), self._W1u,
+                                  torch.empty((U, net.hidden[0]), dtype=torch.float32, device=dev))
         lib, ctx = N.lib(), N.ctx(dev)
-        ws_bytes = lib.brk_neumf_topk_workspace_bytes(ctx, U, self.num_candidates, k)
-        ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         m = net._c_model()
+        ws_bytes = self._workspace_bytes(lib, ctx, m, U, k)
+        ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         if exclusions is None:
-            N.check(lib.brk_neumf_score_topk(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U, N.ptr(self.item_side),
-                                             N.ptr(self.item_mf), self.num_candidates, k, self.id_offset, N.ptr(vals),
-                                             N.ptr(ids), N.ptr(ws), ws_bytes, N.stream_ptr()), "brk_neumf_score_topk")
+            N.check(getattr(lib, self._SCORE)(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U, N.ptr(self.item_side),
+                                              N.ptr(self.item_mf), self.num_candidates, k, self.id_offset, N.ptr(vals),
+                                              N.ptr(ids), N.ptr(ws), ws_bytes, N.stream_ptr()), self._SCORE)
         else:
             indptr, xids = H._check_csr(exclusions, U, dev)
-            N.check(lib.brk_neumf_score_topk_excl(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U, N.ptr(self.item_side),
-                                                  N.ptr(self.item_mf), self.num_candidates, k, self.id_offset, N.ptr(indptr),
-                                                  N.ptr(xids), N.ptr(vals), N.ptr(ids), N.ptr(ws), ws_bytes, N.stream_ptr()),
-                    "brk_neumf_score_topk_excl")
+            N.check(getattr(lib, self._SCORE_EXCL)(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U,
+                                                   N.ptr(self.item_side), N.ptr(self.item_mf), self.num_candidates, k,
+                                                   self.id_offset, N.ptr(indptr), N.ptr(xids), N.ptr(vals), N.ptr(ids),
+                                                   N.ptr(ws), ws_bytes, N.stream_ptr()), self._SCORE_EXCL)
         return vals, ids
 
     def __call__(self, usersId, k=None):
@@ -478,6 +474,94 @@ class NeuMFTopKIndex:
         global ids (position + id_offset), ascending within each row (hotpath.exclusion_csr).  Rows with fewer than k
         remaining items are padded with (-inf, -1)."""
         return self._run(usersId, k, exclusions)
+
+
+class NeuMFTopKIndex(_FactoredTopKIndex):
+    """Full-catalog NeuMF top-k in one kernel launch (brk_neumf_score_topk): for each queried user, the k items of the
+    index with the highest prediction -- the value predict_on_batch returns for the pair, to TF32 rounding -- sorted
+    by score, ties to the lower position, scores never materialised.  Shaped like hotpath.BruteForceIndex:
+
+        index = net.topk_index(itemsId)            # item side: iMLP[items] W1[E:2E] + b1 and the items' iMF rows
+        scores, ids = index(usersId, k=10)         # ids: positions in itemsId plus id_offset
+        scores, ids = index.query_with_exclusions(usersId, hotpath.exclusion_csr(rows, ids, len(usersId), dev))
+
+    The first Dense layer factors over [uMLP[u], iMLP[i]], so building the index computes the item half once and a
+    query the user half once; the kernel runs the rest of the network per pair on the tensor cores.  The index is a
+    snapshot of the item tables and keeps the model for the dense block, the BatchNorm statistics and the user tables:
+    rebuild it after training.  Built for the tensor-core class graph (numFactor 32 or 64, relu) and the He et al.
+    variant (E 32, mf_dim 8, hadamard, no BatchNorm); other models, and k > 32, raise ValueError -- rank them with
+    NeuMFNet.score_all (the fp32 models: NeuMFNet.topk_index_fp32).
+
+    Item-range shards: rank r indexes its range [lo, hi) with id_offset = lo; the merged lists equal the unsharded
+    index's bit for bit:
+
+        index = net.topk_index(np.arange(lo, hi), id_offset=lo)
+        scores, ids = distributed.sharded_topk(usersId, None, lo, k, local_topk=lambda q, c, off: index(q, k))
+
+    (or hotpath.topk_merge over the stacked [shards, U, k] lists in one process)."""
+
+    _SCORE, _SCORE_EXCL = "brk_neumf_score_topk", "brk_neumf_score_topk_excl"
+    _product = staticmethod(_gemm_tf32)
+
+    def __init__(self, net, itemsId=None, id_offset=0):
+        h1, h2, h3 = net.hidden
+        ok = net.act == "relu" and (
+            (not net.variant and net.tensor_cores and (net.E, h1, h2, h3) in TC_SPECS) or
+            (net.variant and net.mf_mode == "hadamard" and not net.batch_norm and
+             (net.E, net.EMF, net.hidden) in FUSED_VARIANTS))
+        if not ok:
+            raise ValueError(f"no fused top-k instance for E={net.E}, mf_dim={net.EMF}, hidden={net.hidden}, act={net.act}, "
+                             f"mf_mode={net.mf_mode}, batch_norm={net.batch_norm}, tensor_cores={net.tensor_cores}; built: "
+                             f"tensor-core class graph {sorted(TC_SPECS)} and the He et al. variant {sorted(FUSED_VARIANTS)} "
+                             "-- use NeuMFNet.score_all")
+        super().__init__(net, itemsId, id_offset)
+
+    def _workspace_bytes(self, lib, ctx, m, U, k):
+        return lib.brk_neumf_topk_workspace_bytes(ctx, U, self.num_candidates, k)
+
+
+class NeuMFTopKIndexFP32(_FactoredTopKIndex):
+    """Full-catalog top-k for the fp32 NeuMF models in one kernel launch on the CUDA cores (brk_neumf_score_topk_fp32):
+    for each queried user, the k items of the index with the highest prediction -- the value predict_on_batch returns
+    for the pair, to fp32 rounding -- sorted by score, ties to the lower position, scores never materialised.  The
+    surface is NeuMFTopKIndex's:
+
+        index = net.topk_index_fp32(itemsId)       # item side: iMLP[items] W1[E:2E] + b1 (fp32) and the items' iMF rows
+        scores, ids = index(usersId, k=10)         # ids: positions in itemsId plus id_offset
+        scores, ids = index.query_with_exclusions(usersId, hotpath.exclusion_csr(rows, ids, len(usersId), dev))
+
+    Both halves of the factored first layer are fp32 products (brk_sgemm), and the kernel runs the rest of the network
+    per pair in fp32.  Covers every fp32 model (tensor_cores=False) up to H1 <= 128, H2 <= 64, H3 <= 32 and
+    mf_dim <= 128 (numFactor free): the class graph NeuMFModel builds at any numFactor <= 128, the NFC_plain network of
+    NCFModel / fit_nfc_plain (sigmoid, hidden (100, 50, 10)) and the fp32 He-style variants (Hadamard head, with or
+    without BatchNorm).  Tensor-core models raise ValueError (use NeuMFNet.topk_index), as do wider models and k > 32
+    (use NeuMFNet.score_all).  Like NeuMFTopKIndex the index is a snapshot of the item tables: rebuild it after training.
+
+    Item-range shards: rank r indexes its range [lo, hi) with id_offset = lo; the merged lists equal the unsharded
+    index's bit for bit:
+
+        index = net.topk_index_fp32(np.arange(lo, hi), id_offset=lo)
+        scores, ids = distributed.sharded_topk(usersId, None, lo, k, local_topk=lambda q, c, off: index(q, k))
+
+    (or hotpath.topk_merge over the stacked [shards, U, k] lists in one process)."""
+
+    MAX_WIDTHS = dict(H1=128, H2=64, H3=32, mf_dim=128)
+    _SCORE, _SCORE_EXCL = "brk_neumf_score_topk_fp32", "brk_neumf_score_topk_fp32_excl"
+    _product = staticmethod(_sgemm)
+
+    def __init__(self, net, itemsId=None, id_offset=0):
+        if net.tensor_cores:
+            raise ValueError("the model computes with TF32 tensor-core products (tensor_cores=True): rank it with "
+                             "NeuMFNet.topk_index")
+        h1, h2, h3 = net.hidden
+        cap = self.MAX_WIDTHS
+        if h1 > cap["H1"] or h2 > cap["H2"] or h3 > cap["H3"] or net.EMF > cap["mf_dim"]:
+            raise ValueError(f"no fp32 top-k instance for hidden={net.hidden}, mf_dim={net.EMF}; built up to hidden "
+                             f"({cap['H1']}, {cap['H2']}, {cap['H3']}) and mf_dim {cap['mf_dim']} -- use NeuMFNet.score_all")
+        super().__init__(net, itemsId, id_offset)
+
+    def _workspace_bytes(self, lib, ctx, m, U, k):
+        return lib.brk_neumf_topk_fp32_workspace_bytes(ctx, C.byref(m), U, self.num_candidates, k)
 
 
 class NeuMFDataset:

@@ -149,7 +149,12 @@ SIGNATURES = {
                                        _I64, _P]),
     "brk_neumf_score_topk_excl": (C.c_int, [_P, C.POINTER(brk_neumf_model), _P, _P, _I64, _P, _P, _I64, _I32, _I32, _P, _P,
                                             _P, _P, _P, _I64, _P]),
-    "brk_epoch_permutation": (C.c_int, [_P, _I64, _I64, _I64, _U32, _U32, _U32, _P, _P]),
+    "brk_neumf_topk_fp32_workspace_bytes": (C.c_int64, [_P, C.POINTER(brk_neumf_model), _I64, _I64, _I32]),
+    "brk_neumf_score_topk_fp32": (C.c_int, [_P, C.POINTER(brk_neumf_model), _P, _P, _I64, _P, _P, _I64, _I32, _I32, _P, _P,
+                                            _P, _I64, _P]),
+    "brk_neumf_score_topk_fp32_excl": (C.c_int, [_P, C.POINTER(brk_neumf_model), _P, _P, _I64, _P, _P, _I64, _I32, _I32,
+                                                 _P, _P, _P, _P, _P, _I64, _P]),
+    "brk_epoch_permutation":(C.c_int, [_P, _I64, _I64, _I64, _U32, _U32, _U32, _P, _P]),
     "brk_epoch_permutation_host": (C.c_int, [_I64, _I64, _I64, _U32, _U32, _U32, _P]),
     "brk_neumf_epoch_build": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _U32, _U32, _I32, _P, _P, _P, _P, _P, _P]),
     "brk_vocab_capacity": (C.c_int64, [_I64]),

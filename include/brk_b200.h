@@ -512,6 +512,33 @@ int brk_neumf_score_topk_excl(brk_ctx* ctx, const brk_neumf_model* m, const floa
                               int32_t id_offset, const int64_t* excl_indptr, const int32_t* excl_ids,
                               float* out_vals, int32_t* out_ids, void* workspace, int64_t workspace_bytes,
                               void* stream);
+/* Full-catalog NeuMF top-k for the fp32 models (tensor_cores = 0) in one launch on the CUDA cores
+ * (csrc/neumf_topk_fp32.cu).  Arguments and outputs as brk_neumf_score_topk / _excl; both halves of the first layer
+ * are fp32 products here:
+ *   user_side  A [U, H1]  = uMLP[users] W1[0:E]             (brk_sgemm)
+ *   item_side  B [I, H1]  = iMLP[items] W1[E:2E] + b1       (brk_sgemm with bias)
+ *   item_mf    [I, EMF]   = iMF[items];  users [U]: rows of m->uMF.
+ * Per pair, in fp32 with the sums in the order of the any-width forward: y1 = BN1(act(A_u + B_i)),
+ * y2 = BN2(act(y1 W2 + b2)), h3 = act(y2 W3 + b3), logit = h3 W4[0:H3] + gmf + b4 (gmf = W4[H3] <uMF[u], iMF[i]> for
+ * the Dot head, sum_f (uMF[u][f] iMF[i][f]) W4[H3 + f] for the Hadamard head), out = 1 / (1 + expf(-logit)); act is
+ * m->act (relu or sigmoid), BatchNorm uses the moving statistics (eps 1e-3) and is skipped with no_batch_norm.  out
+ * agrees with brk_neumf_step's prediction for the pair to fp32 rounding.  Selection on out: score desc, ties -> lower
+ * item id; ids are local positions plus id_offset; rows with fewer than k candidates are padded with (-inf, -1).  A
+ * pair's score does not depend on which other users or items share the call.  Any width up to H1 <= 128, H2 <= 64,
+ * H3 <= 32, EMF <= 128 (E free), 1 <= k <= 32, U >= 0 (U = 0 does nothing), I >= 1.  BRK_E_ARG for tensor_cores != 0
+ * (those models rank through brk_neumf_score_topk), widths beyond the caps, k out of range, null operands and a
+ * workspace smaller than brk_neumf_topk_fp32_workspace_bytes (which depends on the model's widths, U and k).
+ * _excl: per-row exclusions with the contract of brk_neumf_score_topk_excl. */
+int64_t brk_neumf_topk_fp32_workspace_bytes(brk_ctx* ctx, const brk_neumf_model* m, int64_t U, int64_t I, int32_t k);
+int brk_neumf_score_topk_fp32(brk_ctx* ctx, const brk_neumf_model* m, const float* user_side, const int32_t* users,
+                              int64_t U, const float* item_side, const float* item_mf, int64_t I, int32_t k,
+                              int32_t id_offset, float* out_vals, int32_t* out_ids, void* workspace,
+                              int64_t workspace_bytes, void* stream);
+int brk_neumf_score_topk_fp32_excl(brk_ctx* ctx, const brk_neumf_model* m, const float* user_side,
+                                   const int32_t* users, int64_t U, const float* item_side, const float* item_mf,
+                                   int64_t I, int32_t k, int32_t id_offset, const int64_t* excl_indptr,
+                                   const int32_t* excl_ids, float* out_vals, int32_t* out_ids, void* workspace,
+                                   int64_t workspace_bytes, void* stream);
 
 /* ---- K9: ranking metrics ----------------------------------------------------------------------
  * Stands in for topKMetrics (trainers/topKmetrics.py:74-99): ids [U,k] are the recommended item ids
