@@ -59,8 +59,15 @@ struct TopkParams {
 // CTAs per SM -- touched only on the candidate path.  Budgeted as 4 KB (ptxas places 3 KB).
 constexpr size_t kExclCursorBytes = 4096;
 
+// Longest fused lists: 128 entries while dpad <= 128, 64 at dpad 192 and 256, where a 128-entry heap (128 KB) beside
+// the 48 / 64 KB query tile leaves no room for two pipeline stages.  hotpath.fused_k_cap states the same caps.
+constexpr int kHeapCap = 128;
+constexpr int kHeapCapWide = 64;
+
+// Lists longer than 32 (K_CAP = kHeapCap) keep a heap of k entries per row in dynamic shared memory, 128 x k x 8 B, so
+// those instantiations run one CTA per SM.
 template <int K_CAP, bool EXCL>
-__global__ void __launch_bounds__(kThreadsTopk, 2)
+__global__ void __launch_bounds__(kThreadsTopk, K_CAP > 32 ? 1 : 2)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_c,
                   const TopkParams P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -150,10 +157,28 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
     const int quad = warp & 3;                          // TMEM lane quadrant this warp may read
     const int half = (warp - 2) >> 2;                   // which 128-column half of each tile
     const int64_t row = int64_t(m_tile) * kBM + quad * 32 + lane;
-    float vals[K_CAP]; int32_t ids[K_CAP];
+    // The row's running list.  K_CAP <= 32: K_CAP entries in registers, sorted (topk_insert).  Longer lists: a min-heap
+    // of exactly k entries in shared memory behind the barriers (topk_heap_*), so that `thr` is the row's k-th best.
+    constexpr bool kHeap = K_CAP > 32;
+    float vals[kHeap ? 1 : K_CAP]; int32_t ids[kHeap ? 1 : K_CAP];
+    // (addressed from smem_raw, not through `smem`, so that the compiler emits LDS / STS rather than generic loads)
+    TopkEntry* heap = reinterpret_cast<TopkEntry*>(smem_raw + (smem - smem_raw) + P.KB * kABytesPerKB + P.stages * kBBytes + 256) +
+                      (threadIdx.x - 64);
+    if constexpr (kHeap) {
+      topk_heap_init(heap, kBM, P.k);
+    } else {
 #pragma unroll
-    for (int j = 0; j < K_CAP; ++j) { vals[j] = -CUDART_INF_F; ids[j] = -1; }
+      for (int j = 0; j < K_CAP; ++j) { vals[j] = -CUDART_INF_F; ids[j] = -1; }
+    }
     float thr = -CUDART_INF_F;
+    auto insert = [&](float x, int32_t id) {              // precondition: x > thr
+      if constexpr (kHeap) {
+        thr = topk_heap_replace_root(heap, kBM, P.k, TopkEntry{x, id});
+      } else {
+        topk_insert<K_CAP>(vals, ids, x, id);
+        thr = vals[K_CAP - 1];
+      }
+    };
     constexpr int kChunks = kBN / kHalves / 32;         // 4 chunks of 32 columns per tile per warp
 
     // Slow-path scratch: 32 floats per epilogue thread, column-major so that lane i of a warp hits
@@ -217,8 +242,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
           if constexpr (EXCL) {
             if (!((live >> j) & 1u)) continue;
           }
-          topk_insert<K_CAP>(vals, ids, x, int32_t(col0 + j) + P.id_offset);
-          thr = vals[K_CAP - 1];
+          insert(x, int32_t(col0 + j) + P.id_offset);
         }
       }
     };
@@ -257,8 +281,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
           mask &= mask - 1;
           const float x = scratch[j * kScratchStride];
           if (x > thr) {
-            topk_insert<K_CAP>(vals, ids, x, int32_t(col0 + j) + P.id_offset);
-            thr = vals[K_CAP - 1];
+            insert(x, int32_t(col0 + j) + P.id_offset);
           }
         }
       }
@@ -342,9 +365,15 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
       const int64_t part = int64_t(split) * kHalves + half;
       float* ov = P.out_vals + (part * P.U + row) * P.k;
       int32_t* oi = P.out_ids + (part * P.U + row) * P.k;
+      if constexpr (kHeap) {
+        topk_heap_sort(heap, kBM, P.k);
+#pragma unroll 1
+        for (int j = 0; j < P.k; ++j) { const TopkEntry e = heap[j * kBM]; ov[j] = e.v; oi[j] = e.id; }
+      } else {
 #pragma unroll
-      for (int j = 0; j < K_CAP; ++j)
-        if (j < P.k) { ov[j] = vals[j]; oi[j] = ids[j]; }
+        for (int j = 0; j < K_CAP; ++j)
+          if (j < P.k) { ov[j] = vals[j]; oi[j] = ids[j]; }
+      }
     }
   }
 
@@ -375,6 +404,37 @@ topk_merge_kernel(const float* __restrict__ pv, const int32_t* __restrict__ pi, 
     }
     if (best < 0) { ov[u * k + j] = -CUDART_INF_F; oi[u * k + j] = -1; }
     else { ov[u * k + j] = bv; oi[u * k + j] = bi; ++head[best]; }
+  }
+}
+
+// The same merge for the long lists of the heap form (k > 32, S <= 32 item splits): one warp per user, lane s holding
+// the head of list s.  Each output entry is one warp arg-max (score desc, id asc; ids are distinct across splits) and
+// the winning lane steps its list.  topk_merge_kernel's thread per user walks S*k entries one dependent load after the
+// other: 2.09 ms at S = 32, k = 128 for 128 users, against 0.048 ms here (B200 at 1000 W, profiles/r08_topk_long.json).
+__global__ void __launch_bounds__(256)
+topk_merge_warp_kernel(const float* __restrict__ pv, const int32_t* __restrict__ pi, int S, int64_t U, int k,
+                       float* __restrict__ ov, int32_t* __restrict__ oi) {
+  const int lane = threadIdx.x & 31;
+  const int64_t u = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  if (u >= U) return;
+  const int64_t base = (int64_t(lane) * U + u) * k;   // list `lane` of user u (lane < S)
+  int h = 0;
+  float v = -CUDART_INF_F; int32_t id = -1;           // the lane's head; id < 0: no list or exhausted
+  auto load = [&]() {
+    id = (lane < S && h < k) ? pi[base + h] : -1;
+    v = id >= 0 ? pv[base + h] : -CUDART_INF_F;
+  };
+  load();
+  for (int j = 0; j < k; ++j) {
+    float bv = v; int32_t bi = id;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float v2 = __shfl_xor_sync(0xffffffffu, bv, o);
+      const int32_t i2 = __shfl_xor_sync(0xffffffffu, bi, o);
+      if (i2 >= 0 && (bi < 0 || v2 > bv || (v2 == bv && i2 < bi))) { bv = v2; bi = i2; }
+    }
+    if (lane == 0) { ov[u * k + j] = bi < 0 ? -CUDART_INF_F : bv; oi[u * k + j] = bi; }
+    if (bi >= 0 && id == bi) { ++h; load(); }
   }
 }
 
@@ -443,6 +503,11 @@ template <int K_CAP, bool EXCL>
 int launch_topk(const CUtensorMap& tq, const CUtensorMap& tcm, const TopkParams& P, dim3 grid, size_t smem,
                 cudaStream_t st) {
   BRK_CUDA(cudaFuncSetAttribute(score_topk_kernel<K_CAP, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  if constexpr (K_CAP > 32) {                         // the heap form is planned for one resident CTA per SM
+    int per_sm = 0;
+    BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, score_topk_kernel<K_CAP, EXCL>, kThreadsTopk, smem));
+    BRK_REQUIRE(per_sm >= 1, BRK_E_STATE, "brk_score_topk_bf16: %zu bytes of shared memory do not fit an SM", smem);
+  }
   score_topk_kernel<K_CAP, EXCL><<<grid, kThreadsTopk, smem, st>>>(tq, tcm, P);
   BRK_LAUNCH_CHECK();
   return 0;
@@ -501,27 +566,33 @@ int score_topk(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* 
               "brk_score_topk_bf16: U=%lld I=%lld", (long long)U, (long long)I);
   BRK_REQUIRE(dpad > 0 && dpad % kKBlock == 0 && dpad / kKBlock <= kMaxKB, BRK_E_ARG,
               "brk_score_topk_bf16: dpad=%d must be a multiple of %d and <= %d", dpad, kKBlock, kKBlock * kMaxKB);
-  BRK_REQUIRE(k >= 1 && k <= 32, BRK_E_ARG, "brk_score_topk_bf16: k=%d (1..32)", k);
+  BRK_REQUIRE(k >= 1 && k <= kHeapCap, BRK_E_ARG, "brk_score_topk_bf16: k=%d (1..%d)", k, kHeapCap);
+  BRK_REQUIRE(dpad <= 128 || k <= kHeapCapWide, BRK_E_ARG, "brk_score_topk_bf16: k=%d at dpad=%d (k <= %d above dpad 128)",
+              k, dpad, kHeapCapWide);
   BRK_REQUIRE(brk_aligned16(q_bf16) && brk_aligned16(c_bf16), BRK_E_ALIGN, "brk_score_topk_bf16: operands must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
 
   TopkParams P;
   P.U = U; P.I = I; P.KB = dpad / kKBlock; P.k = k; P.id_offset = id_offset;
   P.excl_indptr = excl_indptr; P.excl_ids = excl_ids;
-  int S, tps;
-  P.n_tiles = plan_splits(ctx->sm_count * (dpad <= 128 ? 2 : 1), U, I, &S, &tps);
-  P.tiles_per_split = tps;
+  const bool heap = k > 32;
   const size_t a_bytes = size_t(P.KB) * kABytesPerKB;
-  constexpr size_t kScratchBytes = size_t(kEpiWarps) * 32 * 32 * sizeof(float);   // 32 KB
-  // two CTAs per SM (each with its own pair of TMEM accumulators) when the query tile leaves room: while one CTA's epilogue
-  // warps wait for their next accumulator the other's keep the SM busy
-  const size_t budget = a_bytes <= 32 * 1024 ? size_t(113) * 1024 : size_t(227) * 1024;
-  int stages = int((budget - 1024 - 256 - kScratchBytes - (excl ? kExclCursorBytes : 0) - a_bytes) / kBBytes);
+  const size_t heap_bytes = heap ? size_t(kBM) * k * sizeof(TopkEntry) : 0;
+  constexpr size_t kScratchBytes = size_t(kEpiWarps) * 32 * 32 * sizeof(float);   // 16 KB
+  // two CTAs per SM (each with its own pair of TMEM accumulators) when the query tile and the lists leave room: while one
+  // CTA's epilogue warps wait for their next accumulator the other's keep the SM busy
+  const bool two_ctas = a_bytes <= 32 * 1024 && !heap;
+  int S, tps;
+  P.n_tiles = plan_splits(ctx->sm_count * (two_ctas ? 2 : 1), U, I, &S, &tps);
+  P.tiles_per_split = tps;
+  const int64_t budget = two_ctas ? int64_t(113) * 1024 : int64_t(227) * 1024;
+  int stages = int((budget - 1024 - 256 - int64_t(kScratchBytes) - (excl ? int64_t(kExclCursorBytes) : 0) - int64_t(a_bytes) -
+                    int64_t(heap_bytes)) / int64_t(kBBytes));
   if (stages > 6) stages = 6;
-  BRK_REQUIRE(stages >= 2, BRK_E_ARG, "brk_score_topk_bf16: no room for a 2-stage pipeline at dpad=%d", dpad);
+  BRK_REQUIRE(stages >= 2, BRK_E_ARG, "brk_score_topk_bf16: no room for a 2-stage pipeline at dpad=%d k=%d", dpad, k);
   P.stages = stages;
-  // + kScratchBytes (+ kExclCursorBytes) of static shared memory
-  const size_t smem = 1024 + a_bytes + size_t(stages) * kBBytes + 256;
+  // + kScratchBytes (+ kExclCursorBytes) of static shared memory; the heaps follow the 256 bytes of barriers
+  const size_t smem = 1024 + a_bytes + size_t(stages) * kBBytes + 256 + heap_bytes;
 
   const int parts = S * kHalves;                       // partial lists per user row
   const int64_t need = int64_t(parts) * U * k * 8;
@@ -530,7 +601,10 @@ int score_topk(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* 
               (long long)workspace_bytes);
   float* pv = reinterpret_cast<float*>(workspace);
   int32_t* pi = reinterpret_cast<int32_t*>(pv + int64_t(parts) * U * k);
-  P.out_vals = pv; P.out_ids = pi;
+  // a heap-form launch without item splits writes the final lists: merging one list is a copy, 1.05 ms of a 28.8 ms call
+  // at 65 536 x 250 000, k = 128 on a B200
+  const bool direct = heap && parts == 1;
+  P.out_vals = direct ? out_vals : pv; P.out_ids = direct ? out_ids : pi;
 
   CUtensorMap tq, tcm;
   BRK_REQUIRE(tc::make_tmap_bf16_sw128(&tq, q_bf16, uint64_t(U), uint64_t(dpad), kBM) == 0, BRK_E_STATE,
@@ -542,9 +616,13 @@ int score_topk(brk_ctx* ctx, const uint16_t* q_bf16, int64_t U, const uint16_t* 
   int rc;
   if (k <= 10) rc = excl ? launch_topk<10, true>(tq, tcm, P, grid, smem, st) : launch_topk<10, false>(tq, tcm, P, grid, smem, st);
   else if (k <= 16) rc = excl ? launch_topk<16, true>(tq, tcm, P, grid, smem, st) : launch_topk<16, false>(tq, tcm, P, grid, smem, st);
-  else rc = excl ? launch_topk<32, true>(tq, tcm, P, grid, smem, st) : launch_topk<32, false>(tq, tcm, P, grid, smem, st);
-  if (rc) return rc;
-  topk_merge_kernel<<<unsigned((U + 255) / 256), 256, 0, st>>>(pv, pi, parts, U, k, out_vals, out_ids);
+  else if (k <= 32) rc = excl ? launch_topk<32, true>(tq, tcm, P, grid, smem, st) : launch_topk<32, false>(tq, tcm, P, grid, smem, st);
+  else rc = excl ? launch_topk<kHeapCap, true>(tq, tcm, P, grid, smem, st) : launch_topk<kHeapCap, false>(tq, tcm, P, grid, smem, st);
+  if (rc || direct) return rc;
+  if (heap)
+    topk_merge_warp_kernel<<<unsigned((U * 32 + 255) / 256), 256, 0, st>>>(pv, pi, parts, U, k, out_vals, out_ids);
+  else
+    topk_merge_kernel<<<unsigned((U + 255) / 256), 256, 0, st>>>(pv, pi, parts, U, k, out_vals, out_ids);
   BRK_LAUNCH_CHECK();
   return 0;
 }

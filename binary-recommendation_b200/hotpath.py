@@ -270,7 +270,14 @@ def rows_to_bf16(x):
     return out
 
 
-MAX_FUSED_K = 32          # list length the selection kernels keep per row (csrc/topk.cu)
+MAX_FUSED_K = 32          # longest list of topk_rows and of the NeuMF top-K indexes (register lists per row)
+
+
+def fused_k_cap(dpad):
+    """Longest list the fused scorer (brk_score_topk_bf16 / _excl) selects for candidates of padded width `dpad`: 128
+    up to dpad 128, 64 at dpad 192 and 256 (csrc/topk.cu kHeapCap / kHeapCapWide: lists beyond 32 keep a heap per row
+    in shared memory beside the query tile).  BruteForceIndex takes longer lists through _call_materialised."""
+    return 128 if dpad <= 128 else 64
 
 
 class BruteForceIndex:
@@ -301,9 +308,9 @@ class BruteForceIndex:
         if self._c is None:
             raise RuntimeError("BruteForceIndex: call index(candidates) first")
         k = min(int(k or self.k), self.num_candidates)
-        if k > MAX_FUSED_K:
-            # the selection epilogue keeps at most 32 entries per row in registers; longer lists take the materialised
-            # route: fp32 scores of a chunk of users (brk_sgemm) + the multi-pass row top-k below
+        if k > fused_k_cap(self._c.shape[1]):
+            # lists beyond the fused kernel's cap take the materialised route: fp32 scores of a chunk of users
+            # (brk_sgemm) + the multi-pass row top-k below
             return self._call_materialised(queries, k)
         if queries.shape[1] != self.dim:
             raise ValueError(f"query dim {queries.shape[1]} != candidate dim {self.dim}")
@@ -340,7 +347,7 @@ class BruteForceIndex:
         if isinstance(exclusions, torch.Tensor):
             exclusions = self._dense_exclusions(exclusions, U)
         indptr, xids = _check_csr(exclusions, U, dev)
-        if k > MAX_FUSED_K:
+        if k > fused_k_cap(self._c.shape[1]):
             return self._call_materialised(queries, k, (indptr, xids))
         vals = torch.empty((U, k), dtype=torch.float32, device=dev)
         ids = torch.empty((U, k), dtype=torch.int32, device=dev)
@@ -396,8 +403,8 @@ def sgemm(a, b, trans_b=False):
 
 
 def _bruteforce_materialised(self, queries, k, exclusions=None):
-    """k > 32: bf16-rounded operands like the fused kernel (so shorter and longer lists agree on their common prefix up
-    to fp32 summation order), scores of <= 2^24 pairs at a time, multi-pass top-k.  `exclusions`: a checked CSR of
+    """k above the fused cap (fused_k_cap): bf16-rounded operands like the fused kernel (so shorter and longer lists
+    agree on their common prefix up to fp32 summation order), scores of <= 2^24 pairs at a time, multi-pass top-k.  `exclusions`: a checked CSR of
     global ids, masked out of each chunk's scores."""
     U, I = queries.shape[0], self.num_candidates
     dev = queries.device

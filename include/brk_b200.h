@@ -448,7 +448,12 @@ int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const brk_shards
  *   brk_bf16_padded_dim(d)      row width of the bf16 operand copies (d rounded up to 64)
  *   brk_rows_to_bf16            fp32 [rows,d] -> bf16 [rows,dpad], zero padded (the "index" step)
  *   brk_score_topk_bf16         out_vals/out_ids [U,k]; id_offset is added to every item id (item-
- *                               range shards); workspace: brk_score_topk_workspace_bytes(...) bytes
+ *                               range shards); workspace: brk_score_topk_workspace_bytes(...) bytes.
+ *                               1 <= k <= 128 for dpad <= 128, k <= 64 for dpad 192 and 256 (BRK_E_ARG
+ *                               beyond).  k <= 32 keeps each row's list in registers, longer lists a
+ *                               heap per row in shared memory (one CTA per SM); the scores, the order
+ *                               and the tie rule are the same, so a longer list's first entries equal
+ *                               a shorter call's bit for bit
  *   brk_topk_merge              merges n_parts partial lists [n_parts,U,k] (score desc, id asc) --
  *                               the result is identical to an unsharded scan. */
 int32_t brk_bf16_padded_dim(int32_t d);
