@@ -416,10 +416,15 @@ class _FactoredTopKIndex:
         E = net.E
         W1 = net.param("W1")                                 # [2E, H1]: rows [0, E) act on uMLP, [E, 2E) on iMLP
         self._W1u, self._W1i = W1[:E], W1[E:]
-        self.item_side = self._product(H.gather_rows(net.iMLP.w, items), self._W1i,
+        self.item_side = self._product(self._rows("iMLP", items), self._W1i,
                                        torch.empty((items.numel(), net.hidden[0]), dtype=torch.float32, device=dev),
                                        net.param("b1"))
-        self.item_mf = H.gather_rows(net.iMF.w, items)
+        self.item_mf = self._rows("iMF", items)
+
+    def _rows(self, table, ids):
+        """Rows `ids` (int32, device) of the model's table `table` ("uMLP", "iMLP", "uMF", "iMF"); the indexes of
+        sharded.ShardedNeuMFNet gather them from the shards instead."""
+        return H.gather_rows(getattr(self.net, table).w, ids)
 
     @staticmethod
     def _product(a, w, out, bias=None):
@@ -437,20 +442,35 @@ class _FactoredTopKIndex:
         return min(k, self.num_candidates)
 
     def _run(self, usersId, k, exclusions):
-        net = self.net
-        dev = net.device
         k = self._check_k(k)
-        users = torch.as_tensor(np.asarray(usersId, dtype=np.int32) if not isinstance(usersId, torch.Tensor) else usersId)
-        users = H._i32(users.to(dev).reshape(-1), "usersId")
+        users = self._users(usersId)
         U = users.numel()
+        if U == 0:
+            dev = self.net.device
+            return torch.empty((0, k), dtype=torch.float32, device=dev), torch.empty((0, k), dtype=torch.int32, device=dev)
+        if exclusions is not None:
+            exclusions = H._check_csr(exclusions, U, self.net.device)
+        return self._score(self._query(users), U, k, exclusions)
+
+    def _users(self, usersId):
+        users = torch.as_tensor(np.asarray(usersId, dtype=np.int32) if not isinstance(usersId, torch.Tensor) else usersId)
+        return H._i32(users.to(self.net.device).reshape(-1), "usersId")
+
+    def _query(self, users):
+        """The user half of a query: (user_side [U, H1], brk_neumf_model, the kernel's user rows)."""
+        net = self.net
+        user_side = self._product(self._rows("uMLP", users), self._W1u,
+                                  torch.empty((users.numel(), net.hidden[0]), dtype=torch.float32, device=net.device))
+        return user_side, net._c_model(), users
+
+    def _score(self, query, U, k, exclusions):
+        """One scoring + selection launch over this index's items for a prepared query; `exclusions`: a checked CSR or
+        None.  Returns (vals, ids) [U, k]."""
+        user_side, m, users = query
+        dev = self.net.device
         vals = torch.empty((U, k), dtype=torch.float32, device=dev)
         ids = torch.empty((U, k), dtype=torch.int32, device=dev)
-        if U == 0:
-            return vals, ids
-        user_side = self._product(H.gather_rows(net.uMLP.w, users), self._W1u,
-                                  torch.empty((U, net.hidden[0]), dtype=torch.float32, device=dev))
         lib, ctx = N.lib(), N.ctx(dev)
-        m = net._c_model()
         ws_bytes = self._workspace_bytes(lib, ctx, m, U, k)
         ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         if exclusions is None:
@@ -458,7 +478,7 @@ class _FactoredTopKIndex:
                                               N.ptr(self.item_mf), self.num_candidates, k, self.id_offset, N.ptr(vals),
                                               N.ptr(ids), N.ptr(ws), ws_bytes, N.stream_ptr()), self._SCORE)
         else:
-            indptr, xids = H._check_csr(exclusions, U, dev)
+            indptr, xids = exclusions
             N.check(getattr(lib, self._SCORE_EXCL)(ctx, C.byref(m), N.ptr(user_side), N.ptr(users), U,
                                                    N.ptr(self.item_side), N.ptr(self.item_mf), self.num_candidates, k,
                                                    self.id_offset, N.ptr(indptr), N.ptr(xids), N.ptr(vals), N.ptr(ids),
@@ -504,6 +524,12 @@ class NeuMFTopKIndex(_FactoredTopKIndex):
     _product = staticmethod(_gemm_tf32)
 
     def __init__(self, net, itemsId=None, id_offset=0):
+        self.check_model(net)
+        super().__init__(net, itemsId, id_offset)
+
+    @staticmethod
+    def check_model(net):
+        """Raises ValueError unless a fused top-k instance covers the model."""
         h1, h2, h3 = net.hidden
         ok = net.act == "relu" and (
             (not net.variant and net.tensor_cores and (net.E, h1, h2, h3) in TC_SPECS) or
@@ -514,7 +540,6 @@ class NeuMFTopKIndex(_FactoredTopKIndex):
                              f"mf_mode={net.mf_mode}, batch_norm={net.batch_norm}, tensor_cores={net.tensor_cores}; built: "
                              f"tensor-core class graph {sorted(TC_SPECS)} and the He et al. variant {sorted(FUSED_VARIANTS)} "
                              "-- use NeuMFNet.score_all")
-        super().__init__(net, itemsId, id_offset)
 
     def _workspace_bytes(self, lib, ctx, m, U, k):
         return lib.brk_neumf_topk_workspace_bytes(ctx, U, self.num_candidates, k)
@@ -550,15 +575,20 @@ class NeuMFTopKIndexFP32(_FactoredTopKIndex):
     _product = staticmethod(_sgemm)
 
     def __init__(self, net, itemsId=None, id_offset=0):
+        self.check_model(net)
+        super().__init__(net, itemsId, id_offset)
+
+    @classmethod
+    def check_model(cls, net):
+        """Raises ValueError unless the fp32 kernel covers the model."""
         if net.tensor_cores:
             raise ValueError("the model computes with TF32 tensor-core products (tensor_cores=True): rank it with "
                              "NeuMFNet.topk_index")
         h1, h2, h3 = net.hidden
-        cap = self.MAX_WIDTHS
+        cap = cls.MAX_WIDTHS
         if h1 > cap["H1"] or h2 > cap["H2"] or h3 > cap["H3"] or net.EMF > cap["mf_dim"]:
             raise ValueError(f"no fp32 top-k instance for hidden={net.hidden}, mf_dim={net.EMF}; built up to hidden "
                              f"({cap['H1']}, {cap['H2']}, {cap['H3']}) and mf_dim {cap['mf_dim']} -- use NeuMFNet.score_all")
-        super().__init__(net, itemsId, id_offset)
 
     def _workspace_bytes(self, lib, ctx, m, U, k):
         return lib.brk_neumf_topk_fp32_workspace_bytes(ctx, C.byref(m), U, self.num_candidates, k)

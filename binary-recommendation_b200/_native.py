@@ -144,6 +144,7 @@ SIGNATURES = {
     "brk_rank_eval_rows": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _P, _I32, _P, _P, _P, _P]),
     "brk_topk_rows": (C.c_int, [_P, _P, _I64, _I64, _I32, _P, _P, _P]),
     "brk_topk_merge": (C.c_int, [_P, _P, _P, _I32, _I64, _I32, _P, _P, _P]),
+    "brk_topk_merge_peer": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _I32, _P, _P, _P, _P]),
     "brk_neumf_topk_workspace_bytes": (C.c_int64, [_P, _I64, _I64, _I32]),
     "brk_neumf_score_topk": (C.c_int, [_P, C.POINTER(brk_neumf_model), _P, _P, _I64, _P, _P, _I64, _I32, _I32, _P, _P, _P,
                                        _I64, _P]),

@@ -438,6 +438,86 @@ topk_merge_warp_kernel(const float* __restrict__ pv, const int32_t* __restrict__
   }
 }
 
+// The merge of item-range lists that live in other GPUs' memory (brk_topk_merge_peer).  A peer's list is read in bulk:
+// each CTA copies the [users, k] rows of its block of kMergeUsers users from every part into shared memory with 16-byte
+// loads (one contiguous span per part and array), then one warp per user merges on chip, lane s holding the head of
+// part s.  Each output entry scans the heads in part order with topk_merge_kernel's comparison, so the result equals
+// that kernel's for any input, duplicate ids and equal scores across parts included.  Before anything is written every
+// CTA checks each part's header {seq, U, k} against part 0's seq and the caller's U and k; on a mismatch it returns,
+// and CTA 0 reports it in *err.
+constexpr int kMergeUsers = 8;                         // users (= warps) per CTA
+
+__device__ __forceinline__ void stage_span(void* dst, const void* src, int64_t n_words) {
+  const int t = threadIdx.x, nt = blockDim.x;
+  uint32_t* d = static_cast<uint32_t*>(dst);
+  const uint32_t* s = static_cast<const uint32_t*>(src);
+  int64_t head = 0;
+  if ((reinterpret_cast<uintptr_t>(s) & 15) == 0 && (reinterpret_cast<uintptr_t>(d) & 15) == 0) {
+    const int64_t n4 = n_words >> 2;
+    for (int64_t q = t; q < n4; q += nt) reinterpret_cast<uint4*>(d)[q] = reinterpret_cast<const uint4*>(s)[q];
+    head = n4 << 2;
+  }
+  for (int64_t q = head + t; q < n_words; q += nt) d[q] = s[q];
+}
+
+__global__ void __launch_bounds__(kMergeUsers * 32)
+topk_merge_peer_kernel(const float* const* __restrict__ part_vals, const int32_t* const* __restrict__ part_ids,
+                       const int32_t* const* __restrict__ part_hdr, int S, int64_t U, int k, float* __restrict__ ov,
+                       int32_t* __restrict__ oi, int32_t* __restrict__ err) {
+  extern __shared__ __align__(16) unsigned char merge_smem[];
+  __shared__ int bad;
+  if (threadIdx.x == 0) {
+    bad = 0;
+    const int32_t seq = part_hdr[0][0];
+    for (int s = 0; s < S; ++s) {
+      const int32_t* h = part_hdr[s];
+      if (!bad && (h[0] != seq || int64_t(h[1]) != U || h[2] != k)) bad = 1 + s;
+    }
+    if (bad && blockIdx.x == 0) *err = bad;
+  }
+  __syncthreads();
+  if (bad) return;
+
+  const int64_t u0 = int64_t(blockIdx.x) * kMergeUsers;
+  const int nb = int(U - u0 < kMergeUsers ? U - u0 : kMergeUsers);
+  const int span = nb * k;                             // entries of one part for this block
+  const int stride = kMergeUsers * k;                  // shared-memory stride between parts (a multiple of 8 entries)
+  float* sv = reinterpret_cast<float*>(merge_smem);
+  int32_t* si = reinterpret_cast<int32_t*>(sv + int64_t(S) * stride);
+  for (int s = 0; s < S; ++s) {
+    stage_span(sv + s * stride, part_vals[s] + u0 * k, span);
+    stage_span(si + s * stride, part_ids[s] + u0 * k, span);
+  }
+  __syncthreads();
+
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  if (w >= nb) return;
+  const float* lv = sv + lane * stride + w * k;        // lane < S: part `lane`'s list of user u0 + w
+  const int32_t* li = si + lane * stride + w * k;
+  int h = 0;
+  float v = -CUDART_INF_F; int32_t id = -1;            // the lane's head; id < 0: no part or exhausted
+  if (lane < S) { id = li[0]; v = lv[0]; }
+  const int64_t o = (u0 + w) * k;
+  for (int j = 0; j < k; ++j) {
+    int best = -1; float bv = 0.f; int32_t bi = 0;
+    for (int s = 0; s < S; ++s) {
+      const float v2 = __shfl_sync(0xffffffffu, v, s);
+      const int32_t i2 = __shfl_sync(0xffffffffu, id, s);
+      if (i2 < 0) continue;
+      if (best < 0 || v2 > bv || (v2 == bv && i2 < bi)) { best = s; bv = v2; bi = i2; }
+    }
+    if (lane == 0) {
+      if (best < 0) { ov[o + j] = -CUDART_INF_F; oi[o + j] = -1; }
+      else { ov[o + j] = bv; oi[o + j] = bi; }
+    }
+    if (lane == best) {
+      ++h;
+      if (h < k) { id = li[h]; v = lv[h]; } else id = -1;
+      if (id < 0) v = -CUDART_INF_F;
+    }
+  }
+}
+
 __global__ void __launch_bounds__(256)
 rows_to_bf16_kernel(const float* __restrict__ src, int64_t rows, int d, __nv_bfloat16* __restrict__ dst, int dpad) {
   const int64_t n = rows * dpad;
@@ -667,6 +747,24 @@ extern "C" int brk_topk_merge(brk_ctx* ctx, const float* part_vals, const int32_
               n_parts, (long long)U, k);
   topk_merge_kernel<<<unsigned((U + 255) / 256), 256, 0, (cudaStream_t)stream>>>(part_vals, part_ids, n_parts, U, k,
                                                                                out_vals, out_ids);
+  BRK_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int brk_topk_merge_peer(brk_ctx* ctx, const float* const* part_vals, const int32_t* const* part_ids,
+                                   const int32_t* const* part_hdr, int32_t n_parts, int64_t U, int32_t k, float* out_vals,
+                                   int32_t* out_ids, int32_t* err, void* stream) {
+  BRK_REQUIRE(ctx && part_vals && part_ids && part_hdr && out_vals && out_ids && err, BRK_E_ARG,
+              "brk_topk_merge_peer: null argument");
+  BRK_REQUIRE(n_parts >= 1 && n_parts <= BRK_MAX_PEERS && k >= 1 && k <= kHeapCap && U >= 0 &&
+                  (U + kMergeUsers - 1) / kMergeUsers <= INT_MAX,
+              BRK_E_ARG, "brk_topk_merge_peer: n_parts=%d (1..%d) U=%lld k=%d (1..%d)", n_parts, BRK_MAX_PEERS,
+              (long long)U, k, kHeapCap);
+  if (U == 0) return 0;
+  const size_t smem = size_t(n_parts) * kMergeUsers * k * 8;
+  BRK_CUDA(cudaFuncSetAttribute(topk_merge_peer_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  topk_merge_peer_kernel<<<unsigned((U + kMergeUsers - 1) / kMergeUsers), kMergeUsers * 32, smem, (cudaStream_t)stream>>>(
+      part_vals, part_ids, part_hdr, n_parts, U, k, out_vals, out_ids, err);
   BRK_LAUNCH_CHECK();
   return 0;
 }

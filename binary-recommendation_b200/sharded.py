@@ -33,6 +33,7 @@ import torch.distributed as dist
 from . import _native as N
 from . import distributed as D
 from . import hotpath as H
+from .NeuMFModel import NeuMFTopKIndex, NeuMFTopKIndexFP32
 from .twoTower import Tower, TwoTowerModel
 
 
@@ -159,6 +160,9 @@ class ShardedTable:
 class ShardedNeuMFNet:
     """NeuMF (class spec, src/models/NeuMFModel.py:53-100) with row-sharded tables; see the module docstring."""
 
+    # the reference class graph: NeuMFNet's attributes of the same names (the top-k indexes read them)
+    variant, mf_mode, batch_norm = False, "dot", True
+
     def __init__(self, numUser, numItem, numFactor, act="relu", loss="mse", learning_rate=1e-3, dropout=0.0,
                  seed=42, dropout_seed=11, device=None, mode="peer", emulate=0, full_init=None, tensor_cores=False):
         from .NeuMFModel import NeuMFNet
@@ -172,6 +176,7 @@ class ShardedNeuMFNet:
             self.G, self.rank = D.world_size(), D.rank()
         E = int(numFactor)
         self.E, self.hidden = E, (E, E // 2, E // 4)
+        self.EMF = E
         self.numUser, self.numItem = int(numUser), int(numItem)
         self.act, self.loss, self.dropout, self.dropout_seed = act, loss, float(dropout), dropout_seed
         dev, G, r = self.device, self.G, self.rank
@@ -224,6 +229,51 @@ class ShardedNeuMFNet:
 
     def _c_shards(self):
         return N.brk_neumf_shards(*[t.c_shards() for t in self._tables()])
+
+    def param(self, name):
+        """View of the dense block's parameter `name` (NeuMFNet.DENSE_ORDER, NeuMFNet's layout)."""
+        E, (h1, h2, h3) = self.E, self.hidden
+        shapes = dict(W1=(2 * E, h1), b1=(h1,), g1=(h1,), be1=(h1,), W2=(h1, h2), b2=(h2,), g2=(h2,), be2=(h2,),
+                      W3=(h2, h3), b3=(h3,), W4=(h3 + 1, 1), b4=(1,))
+        off = 0
+        for key in self._net_cls.DENSE_ORDER:
+            n = int(np.prod(shapes[key]))
+            if key == name:
+                return self.dense.w.view(-1)[off:off + n].view(*shapes[key])
+            off += n
+        raise KeyError(name)
+
+    def _gather_rows(self, names, ids):
+        """Rows `ids` (global row ids, int32 on this device) of the tables `names`: peer loads from the owners' shards, or
+        in mode "nccl" the all-to-all of distributed.ShardedLookup (collective: every rank calls it)."""
+        tabs = [getattr(self, n) for n in names]
+        if self.mode == "peer" or self.emulate or self.G == 1:
+            return [_gather_rows_sharded(t, ids) for t in tabs]
+        lk = D.ShardedLookup(ids, self.G)
+        gather = lambda w: (lambda x: H.gather_rows(w, x.to(torch.int32)) if x.numel() else w.new_empty((0, self.E)))
+        return [lk.forward(gather(t.local.w)) for t in tabs]
+
+    # ---- full-catalog top-k (collective: every rank calls with the same arguments) ---------------------------------
+    def topk_index(self, itemsId=None):
+        """Top-k index of a tensor-core model (tensor_cores=True) over itemsId (default: every item): see
+        ShardedTopKIndex.  Per query 1 <= k <= 32; the lists equal NeuMFNet.topk_index's over the full tables."""
+        if not self.tensor_cores:
+            raise ValueError("the model computes in fp32 (tensor_cores=False): rank it with ShardedNeuMFNet.topk_index_fp32")
+        return ShardedNeuMFTopKIndex(self, itemsId, NeuMFTopKIndex)
+
+    def topk_index_fp32(self, itemsId=None):
+        """Top-k index of an fp32 model (tensor_cores=False) over itemsId: see ShardedTopKIndex.  The lists equal
+        NeuMFNet.topk_index_fp32's over the full tables."""
+        if self.tensor_cores:
+            raise ValueError("the model computes with TF32 tensor-core products (tensor_cores=True): rank it with "
+                             "ShardedNeuMFNet.topk_index")
+        return ShardedNeuMFTopKIndex(self, itemsId, NeuMFTopKIndexFP32)
+
+    def score_all(self, usersId, itemsId, k, exclude=None):
+        """(scores [U, k], positions in itemsId [U, k]) for topKRatings: a one-off top-k index over itemsId.  `exclude`:
+        an (indptr, ids) CSR of positions per user (hotpath.exclusion_csr).  Collective."""
+        index = self.topk_index(itemsId) if self.tensor_cores else self.topk_index_fp32(itemsId)
+        return index(usersId, k) if exclude is None else index.query_with_exclusions(usersId, exclude, k)
 
     def _workspace(self, batch):
         if batch > self._ws_batch:
@@ -414,6 +464,19 @@ class ShardedBPRNet:
         if self.barrier is not None:
             self.barrier.check()
 
+    def topk_index(self, itemsId=None, k=10):
+        """Top-k index over itemsId (default: every item) by the dot product of user and item rows: see ShardedTopKIndex.
+        The lists equal BruteForceIndex(k).index(item_w[itemsId])(user_w[usersId]) over the full tables; k up to
+        hotpath.fused_k_cap of the row width."""
+        return ShardedDotTopKIndex(self, itemsId, k, lambda which, ids: _gather_rows_sharded((self.user, self.item)[which], ids),
+                                   self.d, self.item.rows)
+
+    def score_all(self, usersId, itemsId, k, exclude=None):
+        """(scores [U, k], positions in itemsId [U, k]) for topKRatings: a one-off top-k index over itemsId.  `exclude`:
+        an (indptr, ids) CSR of positions per user (hotpath.exclusion_csr).  Collective."""
+        index = self.topk_index(itemsId, k)
+        return index(usersId, k) if exclude is None else index.query_with_exclusions(usersId, exclude, k)
+
     def save_checkpoint(self, dirpath):
         return save_sharded_model(dirpath, {"user": self.user, "item": self.item}, {"opt_state": self.optimizer.state},
                                   self.G, self.rank, self.emulate, meta={"model": "ShardedBPRNet", "d": self.d})
@@ -562,6 +625,12 @@ class ShardedTwoTowerNet:
         """(user vectors [n, S], item vectors [m, S]) of int32 table rows, for hotpath.BruteForceIndex / topKmetrics."""
         return self._tower_forward(0, user_rows), self._tower_forward(1, item_rows)
 
+    def topk_index(self, itemsId=None, k=10):
+        """Top-k index over the item table rows itemsId (default: every row) by the dot product of the tower outputs: see
+        ShardedTopKIndex.  The lists equal a BruteForceIndex over score_vectors' outputs; k up to hotpath.fused_k_cap
+        of semb."""
+        return ShardedDotTopKIndex(self, itemsId, k, self._tower_forward, self.semb, self.item.rows)
+
     # ---- checkpoint: shards of the tables and their accumulators, replicated Dense blocks and theirs ------------
     def save_checkpoint(self, dirpath):
         rep = {}
@@ -577,3 +646,299 @@ class ShardedTwoTowerNet:
             t.w.view(-1).copy_(torch.from_numpy(rep[name]))
             t.m.view(-1).copy_(torch.from_numpy(rep[name + "_m"]))
         return meta
+
+
+# ---- full-catalog top-k over item ranges of the row-sharded models ------------------------------------------------------
+def _gather_rows_sharded(table, ids):
+    """Rows `ids` (global row ids, int32 on the device) of a ShardedTable: peer loads from the owners' shards (plain local
+    loads under emulation or with one GPU)."""
+    if ids.numel() == 0:
+        return torch.empty((0, table.d), dtype=torch.float32, device=ids.device)
+    return H.gather_rows_sharded(table.c_shards(), table.d, ids)
+
+
+class _ListBuffers:
+    """The exchange buffers of ShardedTopKIndex: two alternating slots per range, each [header: 4 int32][scores: cap fp32]
+    [ids: cap int32], and per slot the DEVICE pointer arrays (scores, ids, headers of every range) that
+    brk_topk_merge_peer reads.  Symmetric (NVLink peer-mapped) memory with one slot pair per rank in a multi-GPU run,
+    `G` plain local buffers in one process."""
+
+    def __init__(self, G, device, cap, symmetric):
+        self.cap = int(cap)
+        self.slot = 4 + 2 * self.cap
+        n = 2 * self.slot
+        if symmetric:
+            import torch.distributed._symmetric_memory as symm_mem
+            buf = symm_mem.empty(n, dtype=torch.float32, device=device)
+            self._handle = symm_mem.rendezvous(buf, dist.group.WORLD.group_name)
+            self.mine = {D.rank(): buf}
+            bases = list(self._handle.buffer_ptrs)
+        else:
+            self.mine = {r: torch.empty(n, dtype=torch.float32, device=device) for r in range(G)}
+            bases = [self.mine[r].data_ptr() for r in range(G)]
+        for b in self.mine.values():
+            b.zero_()
+        self.ptrs = []
+        for s in (0, 1):
+            o = s * self.slot
+            self.ptrs.append(torch.tensor([[p + 4 * (o + 4) for p in bases], [p + 4 * (o + 4 + self.cap) for p in bases],
+                                           [p + 4 * o for p in bases]], dtype=torch.int64, device=device))
+
+    def views(self, r, s, U, k):
+        """(header int32 [4], scores [U, k], ids [U, k]) of range r's slot s."""
+        b, o = self.mine[r], s * self.slot
+        return (b[o:o + 4].view(torch.int32), b[o + 4:o + 4 + U * k].view(U, k),
+                b[o + 4 + self.cap:o + 4 + self.cap + U * k].view(torch.int32).view(U, k))
+
+
+class ShardedTopKIndex:
+    """Full-catalog top-k of a row-sharded model (ShardedNeuMFNet, ShardedBPRNet, ShardedTwoTowerNet) over item ranges.
+
+        index = net.topk_index(itemsId)                  # collective: every rank passes the same itemsId
+        scores, ids = index(usersId, k=10)               # collective; ids: positions in itemsId
+        scores, ids = index.query_with_exclusions(usersId, hotpath.exclusion_csr(rows, ids, len(usersId), dev))
+
+    Rank r of G indexes the positions [lo, hi) = distributed.local_slice(len(itemsId), r, G): it gathers those items'
+    rows from their owners (row-sharded tables: row i on rank i % G) and builds its item side as the unsharded index
+    does, with id_offset = lo.  A query gathers the users' rows from the shards, scores them against the local range with
+    the model's fused top-k kernel, pads the list to exactly k entries with (-inf, -1), publishes it in a symmetric
+    buffer and merges every rank's list from the peers' memory (brk_topk_merge_peer).  Every rank gets the same
+    [U, min(k, len(itemsId))] lists, equal bit for bit to the single-GPU index over the full tables.
+
+    Protocol (mode "peer"): the build and every query start with a cross-GPU barrier, so that no rank reads a shard
+    while its owner's optimizer pass may still be running.  Users go in chunks of CHUNK_ENTRIES // k; chunk c is
+    published in slot c % 2 with a header {seq, U, k}, then a barrier, then the merge.  A rank reaches chunk c + 1's
+    barrier only after its merge of chunk c (stream order), so nobody overwrites a slot a peer may still read, with one
+    barrier per chunk.  The merge checks every rank's header against its own and the query raises ValueError when they
+    differ (a rank skipped a call, or the ranks passed different users or k).  ShardedNeuMFNet(mode="nccl") gathers
+    rows with the all-to-all of distributed.ShardedLookup and exchanges the lists with an NCCL all-gather +
+    brk_topk_merge, as does a run where symmetric memory is unavailable.  `emulate=G` (and G = 1) scores all ranges in
+    one process into local buffers and runs the same merge kernel.
+
+    The index is a snapshot of the item rows: rebuild it after training."""
+
+    CHUNK_ENTRIES = 1 << 21          # list entries (score + id, 8 B) per exchange slot: 16 MB, two slots
+
+    def __init__(self, net, itemsId, k_cap, k=10):
+        self.net, self.device = net, net.device
+        self.G, self.rank = net.G, net.rank
+        self.multi = not net.emulate and self.G > 1
+        self.k_cap = int(k_cap)
+        self.k = self._check_k(k)
+        if itemsId is None:
+            items = np.arange(self._num_items(), dtype=np.int32)
+        else:
+            items = (itemsId.cpu().numpy() if isinstance(itemsId, torch.Tensor) else np.asarray(itemsId)).astype(np.int32).reshape(-1)
+        if items.size == 0:
+            raise ValueError(f"{type(self).__name__}: no items")
+        self.num_candidates = int(items.size)
+        self._bufs, self._barrier, self._nccl = None, None, False
+        if not self.multi:
+            self._bufs = _ListBuffers(self.G, self.device, self.CHUNK_ENTRIES, symmetric=False)
+        elif self._peer_rows():
+            try:
+                self._bufs = _ListBuffers(self.G, self.device, self.CHUNK_ENTRIES, symmetric=True)
+                self._barrier = PeerBarrier(self.device)
+            except Exception as e:                # pragma: no cover - depends on the box
+                self._bufs, self._nccl = None, True
+                if self.rank == 0:
+                    print(f"[binrec_b200] symmetric memory unavailable ({e!r}); exchanging top-k lists over NCCL", flush=True)
+        else:
+            self._nccl = True
+        self._err = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._seq = 0
+        self._sync()
+        self.parts = {}                                    # range -> (lo, scorer or None for an empty range)
+        for r in (range(self.G) if not self.multi else [self.rank]):
+            lo, hi = D.local_slice(self.num_candidates, r, self.G)
+            self.parts[r] = (lo, self._build_part(items[lo:hi], lo))
+
+    # ---- model-specific hooks ----------------------------------------------------------------------------------------
+    def _num_items(self):
+        raise NotImplementedError
+
+    def _peer_rows(self):
+        """True when rows are gathered with peer loads (the tables live in symmetric memory)."""
+        return True
+
+    def _build_part(self, items, lo):
+        """Scorer of the positions [lo, lo + len(items)) (items: table rows, host int32; may be empty)."""
+        raise NotImplementedError
+
+    def _query(self, users):
+        """The user side of a chunk of users (int32 table rows on the device); collective in a multi-GPU run."""
+        raise NotImplementedError
+
+    def _score(self, part, query, U, k, exclusions):
+        """(scores, ids) [U, min(k, part's items)] of one range; ids are global positions."""
+        raise NotImplementedError
+
+    # ---- collective query --------------------------------------------------------------------------------------------
+    def _check_k(self, k):
+        k = self.k if k is None else int(k)
+        if k < 1 or k > self.k_cap:
+            raise ValueError(f"k={k}: the sharded top-k of {type(self.net).__name__} keeps 1..{self.k_cap} entries per user")
+        return k
+
+    def _sync(self):
+        """Cross-GPU barrier: in stream order on the peer path, a host rendezvous after a device synchronise otherwise."""
+        if self._barrier is not None:
+            self._barrier()
+        elif self.multi:
+            torch.cuda.synchronize(self.device)
+            dist.barrier()
+
+    def __call__(self, usersId, k=None):
+        """(scores [U, k], ids [U, k]) for the users usersId (rows of the user tables); ids are positions in itemsId, best
+        first, ties to the lower position.  Collective: every rank passes the same users and k."""
+        return self._run(usersId, k, None)
+
+    def query_with_exclusions(self, usersId, exclusions, k=None):
+        """As the call, with row r's listed positions left out: `exclusions` is an (indptr int64 [>= U+1], ids int32) CSR
+        of global positions, ascending within each row (hotpath.exclusion_csr), the same on every rank.  Rows with
+        fewer than k remaining items are padded with (-inf, -1)."""
+        return self._run(usersId, k, exclusions)
+
+    def _run(self, usersId, k, exclusions):
+        k = min(self._check_k(k), self.num_candidates)
+        dev = self.device
+        users = torch.as_tensor(np.asarray(usersId, dtype=np.int32) if not isinstance(usersId, torch.Tensor) else usersId)
+        users = H._i32(users.to(dev).reshape(-1), "usersId")
+        U = users.numel()
+        vals = torch.empty((U, k), dtype=torch.float32, device=dev)
+        ids = torch.empty((U, k), dtype=torch.int32, device=dev)
+        if U == 0:
+            return vals, ids
+        if exclusions is not None:
+            exclusions = H._check_csr(exclusions, U, dev)
+        self._sync()
+        step = max(1, self.CHUNK_ENTRIES // k)
+        for s0 in range(0, U, step):
+            n = min(U, s0 + step) - s0
+            q = self._query(users[s0:s0 + n])
+            ex = None if exclusions is None else (exclusions[0][s0:], exclusions[1])
+            lists = {r: (self._score(part, q, n, k, ex) if part is not None else None) for r, (lo, part) in self.parts.items()}
+            self._exchange(lists, n, k, vals[s0:s0 + n], ids[s0:s0 + n])
+        if self._bufs is not None:
+            err = int(self._err.item())
+            if self._barrier is not None:
+                self._barrier.check()
+            if err:
+                self._err.zero_()
+                raise ValueError(f"sharded top-k: rank {err - 1}'s list header differs from this rank's (a rank skipped a "
+                                 "query, or the ranks passed different users or k); no result was written")
+        return vals, ids
+
+    @staticmethod
+    def _pad(lst, dst_v, dst_i):
+        """Writes a range's list into [n, k] buffers, padded with (-inf, -1) (a range shorter than k, or empty)."""
+        if lst is None or lst[0].shape[1] < dst_v.shape[1]:
+            dst_v.fill_(float("-inf")); dst_i.fill_(-1)
+        if lst is not None:
+            w = lst[0].shape[1]
+            dst_v[:, :w].copy_(lst[0]); dst_i[:, :w].copy_(lst[1])
+
+    def _exchange(self, lists, n, k, out_v, out_i):
+        dev = self.device
+        if self._nccl:
+            v = torch.empty((n, k), dtype=torch.float32, device=dev)
+            i = torch.empty((n, k), dtype=torch.int32, device=dev)
+            self._pad(lists[self.rank], v, i)
+            mv, mi = H.topk_merge(*D.gather_topk_parts(v, i))
+            out_v.copy_(mv); out_i.copy_(mi)
+            return
+        slot, seq = self._seq & 1, self._seq & 0x7FFFFFFF
+        self._seq += 1
+        for r, lst in lists.items():
+            hdr, bv, bi = self._bufs.views(r, slot, n, k)
+            self._pad(lst, bv, bi)
+            hdr[0].fill_(seq); hdr[1].fill_(n); hdr[2].fill_(k)
+        if self._barrier is not None:
+            self._barrier()                               # every rank's list of this chunk is in its slot
+        p = self._bufs.ptrs[slot]
+        N.check(N.lib().brk_topk_merge_peer(N.ctx(dev), N.ptr(p[0]), N.ptr(p[1]), N.ptr(p[2]), self.G, n, k, N.ptr(out_v),
+                                            N.ptr(out_i), N.ptr(self._err), N.stream_ptr()), "brk_topk_merge_peer")
+
+
+class ShardedNeuMFTopKIndex(ShardedTopKIndex):
+    """ShardedNeuMFNet.topk_index / topk_index_fp32: each range is a NeuMFTopKIndex / NeuMFTopKIndexFP32 whose rows come
+    from the shards; a query computes the user half of the factored first layer once (uMLP rows gathered from the
+    shards) and hands the kernel a model whose uMF table is the gathered rows.  BatchNorm statistics are per replica in
+    sharded training; the index uses rank 0's, broadcast at build time -- those save_checkpoint keeps, so the index
+    equals the single-GPU index of the restored checkpoint."""
+
+    def __init__(self, net, itemsId, part_cls):
+        part_cls.check_model(net)                      # on every rank, whether or not its range is empty
+        self._part_cls = part_cls
+        self.bn = D.broadcast_(net.bn_moving.clone(), 0) if (not net.emulate and net.G > 1) else net.bn_moving.clone()
+        super().__init__(net, itemsId, H.MAX_FUSED_K)
+
+    def _num_items(self):
+        return self.net.numItem
+
+    def _peer_rows(self):
+        return self.net.mode == "peer"
+
+    def _build_part(self, items, lo):
+        if items.size == 0:
+            if self._nccl:                               # join the all-to-all lookups of the ranks that do have items
+                self.net._gather_rows(["iMLP"], torch.empty(0, dtype=torch.int32, device=self.device))
+                self.net._gather_rows(["iMF"], torch.empty(0, dtype=torch.int32, device=self.device))
+            return None
+        return _RANGE_CLS[self._part_cls](self.net, items, lo)
+
+    def _query(self, users):
+        net = self.net
+        uMLP, uMF = net._gather_rows(["uMLP", "uMF"], users)
+        n, h1 = users.numel(), net.hidden[0]
+        user_side = self._part_cls._product(uMLP, net.param("W1")[:net.E], torch.empty((n, h1), dtype=torch.float32,
+                                                                                       device=self.device))
+        m = net._c_model()
+        m.uMF = N.brk_table(uMF.data_ptr(), None, None, None, None, n, uMF.shape[1], 0)
+        m.bn_moving = self.bn.data_ptr()
+        return user_side, m, torch.arange(n, dtype=torch.int32, device=self.device), uMF
+
+    def _score(self, part, query, U, k, exclusions):
+        return part._score(query[:3], U, min(k, part.num_candidates), exclusions)
+
+
+class _ShardRows:
+    """Row source of a NeuMF index over one item range: the rows are gathered from the shards of ShardedNeuMFNet."""
+
+    def _rows(self, table, ids):
+        return self.net._gather_rows([table], ids)[0]
+
+
+class _NeuMFRange(_ShardRows, NeuMFTopKIndex):
+    pass
+
+
+class _NeuMFRangeFP32(_ShardRows, NeuMFTopKIndexFP32):
+    pass
+
+
+_RANGE_CLS = {NeuMFTopKIndex: _NeuMFRange, NeuMFTopKIndexFP32: _NeuMFRangeFP32}
+
+
+class ShardedDotTopKIndex(ShardedTopKIndex):
+    """ShardedBPRNet.topk_index / ShardedTwoTowerNet.topk_index: each range is a hotpath.BruteForceIndex over the bf16
+    candidates of its items (BPR: the item rows; two-tower: the item tower's outputs), queried with the users' rows
+    (two-tower: user tower outputs), all gathered from the shards."""
+
+    def __init__(self, net, itemsId, k, vectors, dim, num_items):
+        self._vectors, self._num = vectors, num_items
+        super().__init__(net, itemsId, H.fused_k_cap(int(N.lib().brk_bf16_padded_dim(dim))), k)
+
+    def _num_items(self):
+        return self._num
+
+    def _build_part(self, items, lo):
+        if items.size == 0:
+            return None
+        return H.BruteForceIndex(self.k).index(self._vectors(1, torch.from_numpy(items).to(self.device)), id_offset=lo)
+
+    def _query(self, users):
+        return self._vectors(0, users)
+
+    def _score(self, part, query, U, k, exclusions):
+        return part(query, k) if exclusions is None else part.query_with_exclusions(query, exclusions, k)

@@ -490,6 +490,19 @@ int brk_topk_rows(brk_ctx* ctx, const float* scores, int64_t R, int64_t I, int32
                   int32_t* out_ids, void* stream);
 int brk_topk_merge(brk_ctx* ctx, const float* part_vals, const int32_t* part_ids, int32_t n_parts,
                    int64_t U, int32_t k, float* out_vals, int32_t* out_ids, void* stream);
+/* The merge of brk_topk_merge over lists held in other GPUs' memory: the exchange step of a full-catalog top-k over
+ * item-range shards (sharded.ShardedTopKIndex).  part_vals / part_ids / part_hdr are DEVICE arrays of n_parts pointers
+ * (1 <= n_parts <= BRK_MAX_PEERS), typically NVLink peer mappings of every rank's symmetric buffer: part s is one
+ * rank's list [U, k] (score desc, id asc, (-inf, -1) padded) and its header, 3 int32 {seq, U, k} that the rank wrote
+ * before a cross-GPU barrier (brk_peer_barrier) that precedes this call.  Every CTA copies its block of users from all
+ * parts into shared memory with 16-byte loads and merges on chip; out_vals / out_ids [U, k] equal brk_topk_merge over
+ * the same parts stacked, bit for bit.  If any header differs from {part 0's seq, U, k} -- a rank skipped a call, or
+ * the ranks passed different users or a different k -- *err (device int32, left untouched otherwise) receives
+ * 1 + the first such part and no result is written.  BRK_E_ARG for null pointers, n_parts outside 1..BRK_MAX_PEERS,
+ * k outside 1..128 and U < 0; U = 0 does nothing. */
+int brk_topk_merge_peer(brk_ctx* ctx, const float* const* part_vals, const int32_t* const* part_ids,
+                        const int32_t* const* part_hdr, int32_t n_parts, int64_t U, int32_t k, float* out_vals,
+                        int32_t* out_ids, int32_t* err, void* stream);
 /* Full-catalog NeuMF top-k in one tcgen05 launch (csrc/neumf_topk.cu): per user, the k best items by the model's
  * inference prediction, scores never written to HBM.  The first layer factors, x0 W1 + b1 = A_u + B_i, and the caller
  * supplies both halves:
