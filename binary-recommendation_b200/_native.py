@@ -71,6 +71,13 @@ class brk_twotower_shards(C.Structure):
     _fields_ = [("user", brk_shards), ("item", brk_shards)]
 
 
+class brk_twotower_global(C.Structure):
+    _fields_ = [("cand", C.c_void_p * BRK_MAX_PEERS), ("ids", C.c_void_p * BRK_MAX_PEERS),
+                ("slot", C.c_void_p * BRK_MAX_PEERS), ("offset", C.c_int64 * BRK_MAX_PEERS),
+                ("count", C.c_int64 * BRK_MAX_PEERS), ("cap", C.c_int64), ("n_cap", C.c_int64), ("c_all", C.c_void_p),
+                ("ids_all", C.c_void_p), ("err", C.c_void_p), ("world", C.c_int32), ("rank", C.c_int32)]
+
+
 _P, _I32, _I64, _U32, _F32, _F64 = C.c_void_p, C.c_int32, C.c_int64, C.c_uint32, C.c_float, C.c_double
 
 # name -> (restype, argtypes); mirrors include/brk_b200.h one to one.
@@ -134,6 +141,9 @@ SIGNATURES = {
     "brk_twotower_step_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards), _P,
                                             _P, _P, _P, _I64, _I32, C.POINTER(brk_twotower_workspace), _P, _P]),
     "brk_tower_forward_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_shards), _P, _I64, _P, _P, _P]),
+    "brk_twotower_step_global": (C.c_int, [_P, _I32, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards),
+                                           C.POINTER(brk_twotower_global), _P, _P, _I32, C.POINTER(brk_twotower_workspace), _P,
+                                           _P]),
     "brk_bf16_padded_dim": (C.c_int32, [_I32]),
     "brk_rows_to_bf16": (C.c_int, [_P, _P, _I64, _I32, _P, _I32, _P]),
     "brk_score_topk_workspace_bytes": (C.c_int64, [_P, _I64, _I64, _I32]),

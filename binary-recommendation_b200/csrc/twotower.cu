@@ -334,15 +334,13 @@ extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_
   return twotower_step(ctx, user, item, nullptr, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream);
 }
 
-static int check_shards(const brk_shards* s, int32_t E, const char* which) {
-  BRK_REQUIRE(s->world >= 1 && s->world <= BRK_MAX_PEERS, BRK_E_ARG, "brk_twotower_step_sharded: %s world=%d (1..%d)", which,
-              s->world, BRK_MAX_PEERS);
-  BRK_REQUIRE(s->rank >= 0 && s->rank < s->world, BRK_E_ARG, "brk_twotower_step_sharded: %s rank=%d world=%d", which, s->rank,
-              s->world);
+static int check_shards(const brk_shards* s, int32_t E, const char* which, const char* fn = "brk_twotower_step_sharded") {
+  BRK_REQUIRE(s->world >= 1 && s->world <= BRK_MAX_PEERS, BRK_E_ARG, "%s: %s world=%d (1..%d)", fn, which, s->world,
+              BRK_MAX_PEERS);
+  BRK_REQUIRE(s->rank >= 0 && s->rank < s->world, BRK_E_ARG, "%s: %s rank=%d world=%d", fn, which, s->rank, s->world);
   for (int p = 0; p < s->world; ++p)
-    BRK_REQUIRE(s->w[p] && s->g[p] && s->touched[p], BRK_E_ARG, "brk_twotower_step_sharded: %s shard %d has a null w / g / touched",
-                which, p);
-  BRK_REQUIRE(E > 0 && (E & 3) == 0, BRK_E_ARG, "brk_twotower_step_sharded: %s width %d is not a positive multiple of 4", which, E);
+    BRK_REQUIRE(s->w[p] && s->g[p] && s->touched[p], BRK_E_ARG, "%s: %s shard %d has a null w / g / touched", fn, which, p);
+  BRK_REQUIRE(E > 0 && (E & 3) == 0, BRK_E_ARG, "%s: %s width %d is not a positive multiple of 4", fn, which, E);
   return 0;
 }
 
@@ -374,6 +372,24 @@ extern "C" int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const
   BRK_REQUIRE(ctx && t && sh && ids && emb_out && out, BRK_E_ARG, "brk_tower_forward_sharded: null argument");
   BRK_REQUIRE(t->dense.w && t->E > 0 && t->S > 0 && n > 0, BRK_E_ARG, "brk_tower_forward_sharded: bad tower");
   return tower_forward(ctx, t, ids, n, emb_out, out, 0, stream, sh);
+}
+
+// Pieces of the step that the global-negatives phases (twotower_global.cu) run in their own order.
+int brk_tt_gemm(brk_ctx* ctx, cudaStream_t st, int tcore, const float* A, const float* B, float* C, int M, int N, int K, int lda,
+                int ldb, int ldc, int ta, int tb, int accumulate, bool allow_split) {
+  return gemm(ctx, st, tcore, A, B, C, nullptr, M, N, K, lda, ldb, ldc, ta, tb, 1.f, accumulate, allow_split);
+}
+int brk_tt_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t* ids, int64_t n, float* emb_out, float* out, int tcore,
+                         cudaStream_t st, const brk_shards* sh) {
+  return tower_forward(ctx, t, ids, n, emb_out, out, tcore, st, sh);
+}
+int brk_tt_colsum(cudaStream_t st, const float* X, int M, int N, float* out) {
+  colsum_kernel<<<dim3((N + 127) / 128, (M + 63) / 64), 128, 0, st>>>(X, M, N, N, out);
+  BRK_LAUNCH_CHECK();
+  return 0;
+}
+int brk_tt_check_shards(const brk_shards* s, int32_t E, const char* which, const char* fn) {
+  return check_shards(s, E, which, fn);
 }
 
 // Training step + Keras Adagrad (twoTower.py:89-102 with the optimizer of :278-279) in one call.  In-batch-softmax steps

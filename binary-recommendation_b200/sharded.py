@@ -34,7 +34,7 @@ from . import _native as N
 from . import distributed as D
 from . import hotpath as H
 from .NeuMFModel import NeuMFTopKIndex, NeuMFTopKIndexFP32
-from .twoTower import Tower, TwoTowerModel
+from .twoTower import GlobalNegatives, Tower, TwoTowerModel
 
 
 def shard_rows(rows, G):
@@ -494,7 +494,9 @@ class ShardedTwoTowerNet:
     Semantics, per step on a global batch split over the G ranks (D.local_slice):
       * every rank trains its slice; the in-batch softmax uses that slice's items as negatives (MirroredStrategy's
         per-replica loss, what the mirrored TwoTowerModel.fit does); accidental hits compare global item ids within
-        the slice;
+        the slice.  With global_negatives=True every rank's queries are scored against the items of the whole global
+        batch instead (GlobalNegatives, brk_twotower_step_global): the label of global row o is column o, accidental
+        hits are masked across slices, and the ranks' losses sum to the one-GPU loss of the global batch;
       * each replica's loss is SUM-reduced; gradients are summed over ranks, never scaled;
       * row r of a table (numUser + 2 / numItem + 2 rows: the StringLookup offset) lives on rank r % G at local row
         r // G; a rank's row gradients land in the owner's accumulator as REDs and set the owner's touched bits;
@@ -504,16 +506,21 @@ class ShardedTwoTowerNet:
         brk_allreduce_dense_peer (fixed order: bit-identical replicas) and every replica applies brk_adagrad_dense.
     So G GPUs give the mirrored TwoTowerModel's result on the same global batches.  `emulate=G` holds all G shards in
     one process on one GPU and trains the whole batch as one replica: the unsharded single-GPU TwoTowerModel's result.
+    With global_negatives=True, `emulate=G` splits each batch with local_slice over the G emulated ranks and runs the
+    three phases of brk_twotower_step_global rank by rank; with one rank (G = 1) the flag changes nothing.
 
     Ids arrive as int32 table rows (already looked up).  full_init: {"user", "item": full tables [rows, E];
     "user_dense", "item_dense": flat Dense blocks as Tower.init_dense lays them out}; without it the tables are
     U(-0.05, 0.05) and the Dense blocks Glorot-uniform from Philox(seed + 77)."""
 
     def __init__(self, numUser, numItem, embedDim, semb, learning_rate=0.1, rdZero=False, tensor_cores=True, seed=42,
-                 device=None, emulate=0, full_init=None):
+                 device=None, emulate=0, full_init=None, global_negatives=False):
+        if global_negatives and rdZero:
+            raise ValueError("global_negatives needs the in-batch softmax: rdZero has no in-batch negatives")
         self.device = torch.device(device or f"cuda:{torch.cuda.current_device()}")
         self.emulate = int(emulate)
         self.G, self.rank = (self.emulate, 0) if self.emulate else (D.world_size(), D.rank())
+        self.global_negatives = bool(global_negatives)
         self.embedDim, self.semb = int(embedDim), int(semb)
         self.numUser, self.numItem = int(numUser), int(numItem)
         self.rdZero, self.tensor_cores = bool(rdZero), bool(tensor_cores)
@@ -543,6 +550,8 @@ class ShardedTwoTowerNet:
             for t, v in zip(self.dense, torch.split(self.grad_arena[:sum(sizes)], sizes)):
                 t.g = v.view(t.rows, t.d)
             self.barrier = PeerBarrier(dev)
+        self._global = GlobalNegatives(self.G, self.rank, E, S, dev, emulate=bool(self.emulate), barrier=self.barrier) \
+            if self.global_negatives and self.G > 1 else None
         self._ws_batch = 0
 
     _workspace = TwoTowerModel._workspace               # the mirrored model's step buffers (same attribute names)
@@ -553,21 +562,39 @@ class ShardedTwoTowerNet:
     def _shards(self):
         return N.brk_twotower_shards(self.user.c_shards(), self.item.c_shards())
 
-    def train_on_batch(self, u, i, labels=None, loss_out=None):
+    def train_on_batch(self, u, i, labels=None, loss_out=None, split=None):
         """One step on this rank's slice (u, i: int32 table rows; labels: rdZero targets).  Every rank must call it, an
-        empty slice included.  Returns the slice's loss as a device scalar."""
-        loss_out = self.forward_backward(u, i, labels, loss_out)
+        empty slice included.  Returns the slice's loss as a device scalar.  With global_negatives on real ranks, `split`
+        lists the slice sizes of all G ranks (default: every slice has this one's size); under emulation u, i are the
+        global batch and the loss is the sum over the emulated ranks."""
+        loss_out = self.forward_backward(u, i, labels, loss_out, split)
         self.apply_gradients()
         return loss_out
 
-    def forward_backward(self, u, i, labels=None, loss_out=None):
+    def forward_backward(self, u, i, labels=None, loss_out=None, split=None):
         """The step without the optimizer: row gradients in the owners' accumulators (touched bits set there), Dense
         gradients in this rank's Dense blocks."""
         B = u.numel()
         dev = self.device
         loss_out = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=dev)
         lib, ctx, st = N.lib(), N.ctx(dev), N.stream_ptr()
-        if B > 0:
+        if self._global is not None:
+            u, i = H._i32(u, "u"), H._i32(i, "i")
+            if self.emulate:
+                bounds = {r: D.local_slice(B, r, self.G) for r in range(self.G)}
+                parts = {r: (u[lo:hi], i[lo:hi]) for r, (lo, hi) in bounds.items()}
+                split = [hi - lo for lo, hi in bounds.values()]
+            else:
+                parts = {self.rank: (u, i)}
+                split = split if split is not None else [B] * self.G
+
+            def shards(r):
+                sh = self._shards()
+                sh.user.rank = sh.item.rank = r
+                return sh
+            ut, it = self._towers()
+            self._global.step(ut, it, shards, parts, split, self.tensor_cores, loss_out)
+        elif B > 0:
             if self.rdZero and labels is None:
                 raise ValueError("rdZero training needs labels")
             ws = self._workspace(B)
@@ -608,6 +635,8 @@ class ShardedTwoTowerNet:
             self.barrier.check()
         if self._reducer is not None:
             self._reducer.check()
+        if self._global is not None:
+            self._global.check()
 
     def _tower_forward(self, k, ids):
         ids = H._i32(ids, "ids")

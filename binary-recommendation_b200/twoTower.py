@@ -91,15 +91,133 @@ class Tower:
         return self.dense.w.view(-1)[self.E * self.S:self.E * self.S + self.S]
 
 
+class GlobalNegatives:
+    """Global in-batch negatives for data-parallel two-tower training (brk_twotower_step_global): every rank's queries
+    are scored against the candidates of the whole global batch, so G GPUs on a global batch compute the one-GPU loss
+    and gradients of that batch, up to summation order.
+
+    Holds every rank's candidate block [cap, S], id block [4 + cap] (header {count, S}, then ids) and dc-partial slot
+    [n_cap, S]: symmetric (NVLink peer-mapped) buffers with a PeerBarrier between the phases in a multi-GPU run, or G
+    local buffers when one process emulates G ranks on one GPU.  Buffers grow on demand; a growth is collective, and
+    every rank sees the same split, so all ranks grow at the same step."""
+
+    def __init__(self, G, rank, E, S, device, emulate, barrier=None):
+        self.G, self.rank, self.E, self.S, self.device, self.emulate = int(G), int(rank), int(E), int(S), device, bool(emulate)
+        self.cap = self.n_cap = 0
+        self.err = torch.zeros(1, dtype=torch.int32, device=device)
+        self.barrier = barrier
+        if not self.emulate and barrier is None:
+            from .sharded import PeerBarrier
+            self.barrier = PeerBarrier(device)
+        self._ws = {}
+
+    def _grow(self, cap, n):
+        if cap <= self.cap and n <= self.n_cap:
+            return
+        cap, n = max(cap, self.cap, 1), max(n, self.n_cap, 1)
+        dev, S = self.device, self.S
+        sizes = (cap * S, 4 + cap, n * S)
+        if self.emulate:
+            bufs = [[torch.zeros(k, dtype=dt, device=dev) for k, dt in zip(sizes, (torch.float32, torch.int32, torch.float32))]
+                    for _ in range(self.G)]
+            self._bufs = bufs
+            self.ptrs = [[b[k].data_ptr() for b in bufs] for k in range(3)]
+        else:
+            import torch.distributed as dist
+            import torch.distributed._symmetric_memory as symm_mem
+            torch.cuda.synchronize(dev)
+            dist.barrier()                                   # no peer still reads the buffers being replaced
+            mine = [symm_mem.empty(k, dtype=dt, device=dev) for k, dt in zip(sizes, (torch.float32, torch.int32, torch.float32))]
+            hs = [symm_mem.rendezvous(b, dist.group.WORLD.group_name) for b in mine]
+            for b in mine:
+                b.zero_()
+            self._bufs, self._handles = mine, hs
+            self.ptrs = [list(h.buffer_ptrs) for h in hs]
+            torch.cuda.synchronize(dev)
+            dist.barrier()
+        self.c_all = torch.empty(n * S, dtype=torch.float32, device=dev)
+        self.ids_all = torch.empty(n, dtype=torch.int32, device=dev)
+        self.cap, self.n_cap = cap, n
+
+    def _struct(self, r, counts):
+        g = N.brk_twotower_global()
+        off = 0
+        for p in range(self.G):
+            g.cand[p], g.ids[p], g.slot[p] = self.ptrs[0][p], self.ptrs[1][p], self.ptrs[2][p]
+            g.offset[p], g.count[p] = off, counts[p]
+            off += counts[p]
+        g.cap, g.n_cap = self.cap, self.n_cap
+        g.c_all, g.ids_all, g.err = self.c_all.data_ptr(), self.ids_all.data_ptr(), self.err.data_ptr()
+        g.world, g.rank = self.G, r
+        return g
+
+    def _workspace(self, r, b, n):
+        have = self._ws.get(r)
+        if have is None or have[0] < b or have[1] < n:
+            dev, E, S = self.device, self.E, self.S
+            f = lambda k: torch.empty(max(k, 1), dtype=torch.float32, device=dev)
+            bufs = dict(eu=f(b * E), ei=f(b * E), deu=f(b * E), dei=f(b * E), q=f(b * S), dq=f(b * S), dc=f(b * S),
+                        scores=f(b * n), acc=torch.zeros(1, dtype=torch.float64, device=dev))
+            have = self._ws[r] = (b, n, bufs)
+        b_ = have[2]
+        return N.brk_twotower_workspace(b_["eu"].data_ptr(), b_["ei"].data_ptr(), b_["q"].data_ptr(), None, b_["dq"].data_ptr(),
+                                        b_["dc"].data_ptr(), b_["scores"].data_ptr(), None, b_["acc"].data_ptr(),
+                                        b_["deu"].data_ptr(), b_["dei"].data_ptr())
+
+    def step(self, user, item, shards, parts, counts, tensor_cores, loss_out):
+        """Forward and backward of one step (no optimizer).  parts: {rank: (u, i)} int32 slices of the ranks this process
+        drives (every rank under emulation, else this one); counts: the G slice sizes of the global batch, the same on
+        every rank.  shards(r): the brk_twotower_shards of rank r, or None for mirrored tables.  loss_out receives the
+        sum of the driven ranks' losses."""
+        counts = [int(c) for c in counts]
+        if len(counts) != self.G or min(counts) < 0:
+            raise ValueError(f"global negatives: split {counts} is not {self.G} slice sizes")
+        for r, (u, _) in parts.items():
+            if u.numel() != counts[r]:
+                raise ValueError(f"global negatives: rank {r} passes {u.numel()} rows, the split says {counts[r]}")
+        n = sum(counts)
+        self._grow(max(counts), n)
+        lib, ctx, st = N.lib(), N.ctx(self.device), N.stream_ptr()
+        mode = 0x100 if tensor_cores else 0
+        losses = loss_out if len(parts) == 1 else torch.zeros(len(parts), dtype=torch.float32, device=self.device)
+        calls = [(r, self._struct(r, counts), self._workspace(r, counts[r], n), shards(r), u, i, losses[k:k + 1])
+                 for k, (r, (u, i)) in enumerate(parts.items())]
+        for phase in (0, 1, 2):
+            for r, g, ws, sh, u, i, lo in calls:
+                N.check(lib.brk_twotower_step_global(ctx, phase, C.byref(user), C.byref(item), C.byref(sh) if sh is not None else None,
+                                                     C.byref(g), N.ptr(u), N.ptr(i), mode, C.byref(ws), N.ptr(lo), st),
+                        "brk_twotower_step_global")
+            if phase < 2 and self.barrier is not None:
+                self.barrier()                               # every rank's phase is complete before any rank reads it
+        if len(parts) != 1:
+            torch.sum(losses, 0, keepdim=True, out=loss_out)
+        return loss_out
+
+    def check(self):
+        if self.barrier is not None:
+            self.barrier.check()
+        err = int(self.err.item())
+        if err:
+            self.err.zero_()
+            raise RuntimeError(f"global negatives: rank {err - 1}'s published slice differs from the split this rank was "
+                               "given (the ranks passed different splits, or a rank skipped a step)")
+
+
 class TwoTowerModel:
     def __init__(self, embedDim, nbrItem, nbrUser, userKey, itemKey, usersId, itemsId, eval_batch_size=8000,
-                 loss=None, rdZero=False, resKey=None, semb=100, seed=42, device=None, tensor_cores=False):
+                 loss=None, rdZero=False, resKey=None, semb=100, seed=42, device=None, tensor_cores=False,
+                 global_negatives=False):
         self.device = torch.device(device or f"cuda:{torch.cuda.current_device()}")
         self.embedDim, self.nbrItem, self.nbrUser = embedDim, nbrItem, nbrUser
         self.userKey, self.itemKey, self.resKey = userKey, itemKey, resKey
         self.eval_batch_size, self.rdZero, self.semb = eval_batch_size, rdZero, semb
         # tensor_cores: Dense / in-batch products on tcgen05 with TF32 operands (csrc/gemm_tc.cu); fp32 FMA otherwise
         self.tensor_cores = bool(tensor_cores)
+        # global_negatives: under torch.distributed every rank's queries take the candidates of the whole global batch as
+        # negatives (GlobalNegatives) instead of its own slice's (the per-replica loss, MirroredStrategy's default)
+        if global_negatives and rdZero:
+            raise ValueError("global_negatives needs the in-batch softmax: rdZero has no in-batch negatives")
+        self.global_negatives = bool(global_negatives)
         self.userTowerIn = StringLookup(usersId)
         self.itemTowerIn = StringLookup(itemsId)
         rng = np.random.Generator(np.random.Philox(key=seed))
@@ -117,6 +235,8 @@ class TwoTowerModel:
             self.grad_arena, self._reducer = D.gradient_arena(sum(sizes), self.device)
             for t, v in zip(tabs, torch.split(self.grad_arena[:sum(sizes)], sizes)):
                 t.g = v.view(t.rows, t.d)
+        self._global = GlobalNegatives(D.world_size(), D.rank(), embedDim, semb, self.device, emulate=False) \
+            if self.global_negatives and D.world_size() > 1 else None
         self.bruteForceLayer = None
         self._candidates = None
         self.optimizer = None
@@ -197,12 +317,13 @@ class TwoTowerModel:
             return None
         return torch.as_tensor(np.asarray(info[self.resKey], dtype=np.float32)).to(self.device)
 
-    def train_step(self, info):
+    def train_step(self, info, split=None):
         """One fused forward/backward + Adagrad step; returns {"loss": device scalar} (twoTower.py:89-102).
         Under torch.distributed the replicas' SUM-reduced gradients are summed by one all-reduce per
-        tower (MirroredStrategy sums per-replica gradients of a SUM-reduced loss)."""
+        tower (MirroredStrategy sums per-replica gradients of a SUM-reduced loss).  With global_negatives, `info` is
+        this rank's slice of the global batch and `split` the slice sizes of all ranks (default: equal slices)."""
         u, i = self._ids(info)
-        return {"loss": self._train_ids(u, i, self._labels(info))}
+        return {"loss": self._train_ids(u, i, self._labels(info), split=split)}
 
     def _train_step_native(self, u, i, labels, loss_out=None):
         """Step + Keras Adagrad in one library call (brk_twotower_train_step): ONE cooperative launch when the in-batch
@@ -219,12 +340,17 @@ class TwoTowerModel:
                                                 N.stream_ptr()), "brk_twotower_train_step")
         return loss_out
 
-    def _train_ids(self, u, i, labels, loss_out=None):
+    def _train_ids(self, u, i, labels, loss_out=None, split=None):
         if self.optimizer is None:
             self.compile()
         if D.world_size() == 1 and u.numel() > 0 and isinstance(self.optimizer, H.Adagrad):
             return self._train_step_native(u, i, labels, loss_out)
-        if u.numel() > 0:
+        if self._global is not None:                         # every rank calls, an empty slice included
+            loss = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=self.device)
+            self._global.step(self.userTower.c_struct(), self.itemTower.c_struct(), lambda r: None,
+                              {D.rank(): (u, i)}, split if split is not None else [u.numel()] * D.world_size(),
+                              self.tensor_cores, loss)
+        elif u.numel() > 0:
             loss = self._step(u, i, labels, True, loss_out)
         else:                                                # this rank's slice of a small global batch is empty
             loss = loss_out if loss_out is not None else torch.zeros(1, dtype=torch.float32, device=self.device)
@@ -254,13 +380,16 @@ class TwoTowerModel:
         staged = [(self._ids(info), self._labels(info)) for info in batches]
         if D.world_size() > 1:
             # mirrored data parallelism: a batch of the dataset is the GLOBAL batch (MultiWorkerMirroredStrategy auto-shards
-            # it); this rank trains its slice, with its slice's items as in-batch negatives (the per-replica loss), and the
-            # SUM-reduced gradients are summed over the ranks (peer all-reduce in _train_ids)
+            # it); this rank trains its slice, with its slice's items as in-batch negatives (the per-replica loss) or, with
+            # global_negatives, the items of the whole global batch, and the SUM-reduced gradients are summed over the
+            # ranks (peer all-reduce in _train_ids)
             def mine(t):
                 if t is None:
                     return None
                 lo, hi = D.local_slice(t.numel())
                 return t[lo:hi].contiguous()
+            G = D.world_size()
+            splits = [[(lambda s: s[1] - s[0])(D.local_slice(u.numel(), r, G)) for r in range(G)] for (u, _), _ in staged]
             staged = [((mine(u), mine(i)), mine(lab)) for (u, i), lab in staged]
             D.barrier()
         sizes = [u.numel() for (u, _), _ in staged]
@@ -284,11 +413,13 @@ class TwoTowerModel:
                 rest = range(len(staged))
             for k in rest:
                 (u, i), lab = staged[k]
-                self._train_ids(u, i, lab, losses[k:k + 1])
+                self._train_ids(u, i, lab, losses[k:k + 1], split=splits[k] if D.world_size() > 1 else None)
             # one host sync per epoch: Keras reports the running mean of the per-batch losses
             self.history["loss"].append(float(losses.double().sum().item()) / max(len(staged), 1))
             if self._reducer is not None:
                 self._reducer.check()                        # a peer all-reduce that timed out aborted its step: raise here
+            if self._global is not None:
+                self._global.check()
             if verbose:
                 print(f"epoch {e + 1}: loss {self.history['loss'][-1]:.6f}")
         return self

@@ -437,6 +437,49 @@ int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, const brk_tow
                               void* stream);
 int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const brk_shards* sh, const int32_t* ids, int64_t n,
                               float* emb_out, float* out, void* stream);
+/* Two-tower training with GLOBAL in-batch negatives (csrc/twotower_global.cu): every rank's queries are scored against
+ * the candidates of the whole global batch of n rows.  Rank p holds rows [offset[p], offset[p] + count[p]) (the
+ * offsets tile [0, n); slices may be empty).  For rank r's row i (global row o = offset[r] + i) the logits are
+ * q_i . c_j over all n candidates, the label column is o, and a candidate j != o whose id equals the row's positive id
+ * gets finfo(float32).min/100 added (accidental hits masked across slices); loss_out = the SUM of -log softmax over
+ * this rank's rows.  dq stays local; dc_j sums (P - Y)_ij q_i over the queries of every rank: each rank writes its
+ * partial for all n candidates into its slot buffer, and the owner of row j adds the world partials in rank order
+ * (reproducible run to run).  Then the backward chain of brk_twotower_step / brk_twotower_step_sharded: Dense
+ * gradients added into user / item dense.g, row gradients scattered into emb.g (sh == NULL, mirrored tables; touched
+ * bits set) or sent as REDs into the owners' shards (sh != NULL).  No optimizer runs.
+ * The step is three calls on `stream`, each one phase; every rank calls every phase, an empty slice included:
+ *   phase 0: towers; this rank's candidate vectors go to cand[rank], its header {count, S} and ids to ids[rank].
+ *   -- cross-GPU barrier (brk_peer_barrier) --
+ *   phase 1: gathers the world candidate blocks into c_all [n, S] / ids_all [n] (16-byte peer loads; a header that
+ *            disagrees with count[p] or S sets *err = 1 + p), scores = Q C_all^T [count[rank], n] in ws->scores,
+ *            masked row softmax, loss, dq = (P - Y) C_all, and this rank's partial (P - Y)^T Q [n, S] in slot[rank].
+ *   -- cross-GPU barrier --
+ *   phase 2: dc = the rows [offset[rank], offset[rank] + count[rank]) of every slot, summed in rank order; Dense and
+ *            row gradients of both towers.
+ * Ordering: the phase-0 barrier of the next step comes after every rank's phase 2 in stream order, so no rank
+ * overwrites its candidate block or slot buffer while a peer may still read them; the barriers after the step are
+ * those of brk_twotower_step_sharded (row-sharded tables) or the Dense all-reduce (mirrored tables).
+ * Pointers: cand / ids / slot are every rank's symmetric (peer-mapped) buffers -- cand [cap, S], ids [4 + cap] int32,
+ * slot [n_cap, S] -- or G local buffers when one process drives every rank; c_all, ids_all and err are local.
+ * Workspace as brk_twotower_step with B = count[rank], except ws->scores [B, n] and ws->c unused.  mode: 0, or 0x100
+ * for the tensor-core products; rdZero (mode & 0xFF != 0) has no in-batch negatives and is rejected.  BRK_E_ARG for
+ * world outside 1..BRK_MAX_PEERS, rank outside [0, world), offsets that do not tile [0, n), a count above cap or n above
+ * n_cap, user and item S that differ, S not a multiple of 4, and null pointers a non-empty slice needs. */
+typedef struct brk_twotower_global {
+  float*   cand[BRK_MAX_PEERS];
+  int32_t* ids[BRK_MAX_PEERS];
+  float*   slot[BRK_MAX_PEERS];
+  int64_t  offset[BRK_MAX_PEERS], count[BRK_MAX_PEERS];
+  int64_t  cap, n_cap;
+  float*   c_all;
+  int32_t* ids_all;
+  int32_t* err;
+  int32_t  world, rank;
+} brk_twotower_global;
+int brk_twotower_step_global(brk_ctx* ctx, int32_t phase, const brk_tower* user, const brk_tower* item,
+                             const brk_twotower_shards* sh, const brk_twotower_global* g, const int32_t* u,
+                             const int32_t* i, int32_t mode, const brk_twotower_workspace* ws, float* loss_out,
+                             void* stream);
 
 /* ---- K7/K8: full-catalog scoring + top-K ------------------------------------------------------
  * Stands in for tfrs.layers.factorized_top_k.BruteForce(k).index(candidates) + call(queries)
