@@ -67,6 +67,11 @@ class brk_twotower_workspace(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("eu", "ei", "q", "c", "dq", "dc", "scores", "ones", "acc", "deu", "dei")]
 
 
+class brk_tt_retrieval(C.Structure):
+    _fields_ = [("cand_prob", C.c_void_p), ("row_weight", C.c_void_p), ("last", C.c_void_p), ("gap", C.c_void_p),
+                ("step", C.c_void_p), ("rows", C.c_int64), ("inv_temperature", C.c_float), ("alpha", C.c_float)]
+
+
 class brk_twotower_shards(C.Structure):
     _fields_ = [("user", brk_shards), ("item", brk_shards)]
 
@@ -138,6 +143,11 @@ SIGNATURES = {
                                     C.POINTER(brk_twotower_workspace), _P, _P]),
     "brk_twotower_train_step": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), _P, _P, _P, _P, _I64, _I32,
                                           C.POINTER(brk_twotower_workspace), _F32, _F32, _I64, _P, _P]),
+    "brk_twotower_step_retrieval": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), _P, _P, _P, _P, _I64, _I32,
+                                              _I32, C.POINTER(brk_twotower_workspace), _P, _P, C.POINTER(brk_tt_retrieval)]),
+    "brk_twotower_train_step_retrieval": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), _P, _P, _P, _P, _I64, _I32,
+                                                    C.POINTER(brk_twotower_workspace), _F32, _F32, _I64, _P, _P,
+                                                    C.POINTER(brk_tt_retrieval)]),
     "brk_twotower_step_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards), _P,
                                             _P, _P, _P, _I64, _I32, C.POINTER(brk_twotower_workspace), _P, _P]),
     "brk_tower_forward_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_shards), _P, _I64, _P, _P, _P]),

@@ -31,6 +31,9 @@ struct brk_ctx {
   // one-launch two-tower step (csrc/twotower_fused.cu): per-tile softmax partials
   float*        tt_part;
   size_t        tt_part_floats;
+  // multi-kernel two-tower step with retrieval options (csrc/twotower.cu): the log-probability term of every column
+  float*        tt_logq;
+  size_t        tt_logq_floats;
   // grid-barrier words of the cooperative step kernels (layout at brk_grid_barrier): bar[BRK_BAR_*], each on its own
   // 128-byte line of one allocation (bar[0]).  Launches of one family on one context are stream-ordered: a launch reads
   // the base (and tag) that its predecessor wrote back.

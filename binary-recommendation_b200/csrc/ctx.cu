@@ -77,6 +77,7 @@ extern "C" int brk_destroy(brk_ctx* c) {
   if (c->neumf_part) cudaFree(c->neumf_part);
   if (c->neumf_gen) cudaFree(c->neumf_gen);
   if (c->tt_part) cudaFree(c->tt_part);
+  if (c->tt_logq) cudaFree(c->tt_logq);
   if (c->bar[0]) cudaFree(c->bar[0]);
   for (int j = 0; j < BRK_FORK_STREAMS; ++j)
     if (c->fork_stream[j]) { cudaStreamDestroy(c->fork_stream[j]); cudaEventDestroy(c->ev_fork[j]); cudaEventDestroy(c->ev_join[j]); }

@@ -13,6 +13,7 @@
 // bytes: 2 rows gathered + 2 row gradients per interaction (8E B each way) + 12 B^2 for the scores.
 #include "common.cuh"
 #include <math_constants.h>
+#include <cmath>
 
 namespace {
 
@@ -115,7 +116,7 @@ __global__ void __launch_bounds__(128) colsum_kernel(const float* __restrict__ X
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
                             float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
-                            const brk_twotower_shards* sh);                                                       // twotower_fused.cu
+                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt);                           // twotower_fused.cu
 int brk_gemm_tf32_impl(brk_ctx* ctx, const float* A, const float* B, float* C, const float* bias, int M, int N, int K, int lda,
                        int ldb, int ldc, int trans_a, int trans_b, float alpha, int accumulate, bool allow_split,
                        cudaStream_t st);
@@ -133,10 +134,14 @@ int gemm(brk_ctx* ctx, cudaStream_t st, int tcore, const float* A, const float* 
 
 // One CTA per row of the [B,B] score matrix: accidental-hit masking, log-sum-exp, loss, and in place
 // P = softmax - I (the gradient of the SUM-reduced cross-entropy w.r.t. the logits).
+// RT (brk_twotower_step_retrieval): logits s * inv_tau - logq[j] (logq null: no correction), the row's loss and gradient
+// weighted by w[row] (null: 1), P = w (softmax - I) * inv_tau.
 constexpr float kMinFloatOver100 = -3.4028234663852886e36f;     // np.finfo(np.float32).min / 100
+struct SoftmaxOptions { float inv_tau; const float* logq; const float* w; };
+template <bool RT = false>
 __global__ void __launch_bounds__(256)
 inbatch_softmax_kernel(float* __restrict__ S, const int32_t* __restrict__ cand_ids, int B, int training,
-                       double* __restrict__ loss_acc) {
+                       double* __restrict__ loss_acc, SoftmaxOptions o = {}) {
   __shared__ float redf[32];
   __shared__ double redd[32];
   const int row = blockIdx.x, t = threadIdx.x;
@@ -145,7 +150,14 @@ inbatch_softmax_kernel(float* __restrict__ S, const int32_t* __restrict__ cand_i
   float mx = -CUDART_INF_F;
   for (int j = t; j < B; j += 256) {
     float v = s[j];
-    if (cand_ids && j != row && __ldg(cand_ids + j) == pos_id) { v += kMinFloatOver100; s[j] = v; }
+    if constexpr (RT) {
+      v *= o.inv_tau;
+      if (o.logq) v -= __ldg(o.logq + j);
+      if (cand_ids && j != row && __ldg(cand_ids + j) == pos_id) v += kMinFloatOver100;
+      s[j] = v;
+    } else {
+      if (cand_ids && j != row && __ldg(cand_ids + j) == pos_id) { v += kMinFloatOver100; s[j] = v; }
+    }
     mx = fmaxf(mx, v);
   }
   for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
@@ -161,12 +173,45 @@ inbatch_softmax_kernel(float* __restrict__ S, const int32_t* __restrict__ cand_i
   if (t == 0) {
     const float lse = mx + logf(float(sum));
     lse_sm = lse;
-    atomicAdd(loss_acc, double(lse - s[row]));            // -log softmax_row[row]
+    if constexpr (RT) atomicAdd(loss_acc, double(o.w ? __ldg(o.w + row) : 1.f) * double(lse - s[row]));
+    else atomicAdd(loss_acc, double(lse - s[row]));       // -log softmax_row[row]
   }
   __syncthreads();
   if (!training) return;
   const float lse = lse_sm;
-  for (int j = t; j < B; j += 256) s[j] = expf(s[j] - lse) - (j == row ? 1.f : 0.f);
+  if constexpr (RT) {
+    const float wt = (o.w ? __ldg(o.w + row) : 1.f) * o.inv_tau;
+    for (int j = t; j < B; j += 256) s[j] = (expf(s[j] - lse) - (j == row ? 1.f : 0.f)) * wt;
+  } else {
+    for (int j = t; j < B; j += 256) s[j] = expf(s[j] - lse) - (j == row ? 1.f : 0.f);
+  }
+}
+
+// The log-probability term of every column for inbatch_softmax_kernel<true>: logq[j] = log(clip(p_j, 1e-6, 1)), p_j =
+// cand_prob[j] or the streaming frequency estimate of item row ids[j].  With the estimator and training, first the
+// update of Yi et al.'s Algorithm 2 at t = *step + 1: the thread whose exchange of last[y] returned another step is the
+// sole updater of y, so duplicates update once; then *step = t.  One CTA: the update must be complete before any
+// column reads gap, and a batch is a few thousand ids.
+__global__ void __launch_bounds__(1024)
+tt_logq_kernel(const int32_t* __restrict__ ids, int B, const float* __restrict__ cand_prob, long long* last, float* gap,
+               long long* step, float alpha, int training, float* __restrict__ logq) {
+  const int t = threadIdx.x;
+  if (last && training) {
+    const long long ts = *step + 1;
+    for (int j = t; j < B; j += 1024) {
+      const int32_t y = __ldg(ids + j);
+      const long long prev = (long long)atomicExch(reinterpret_cast<unsigned long long*>(last + y), (unsigned long long)ts);
+      if (prev != ts) gap[y] = __fadd_rn(__fmul_rn(__fsub_rn(1.f, alpha), gap[y]), __fmul_rn(alpha, __ll2float_rn(ts - prev)));
+    }
+    __syncthreads();
+    if (t == 0) *step = ts;
+  }
+  for (int j = t; j < B; j += 1024) {
+    float p = 1.f;
+    if (cand_prob) p = __ldg(cand_prob + j);
+    else { const float gp = gap[__ldg(ids + j)]; if (gp >= 1.f) p = __frcp_rn(gp); }
+    logq[j] = logf(fminf(fmaxf(p, 1e-6f), 1.f));
+  }
 }
 
 // rdZero mode: pred = sigmoid(<q_b, c_b>), mean BCE against labels; dq = g c, dc = g q, g = (p - y)/B.
@@ -229,9 +274,11 @@ extern "C" int brk_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t
 
 // The step after argument checks (brk_twotower_step, brk_twotower_step_sharded).  sh != nullptr: the embedding rows are
 // gathered from and their gradients scattered into the row-sharded tables sh instead of user->emb / item->emb.
+// rt != nullptr (unsharded, softmax mode only): the retrieval options, brk_twotower_step_retrieval.
 static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
                          const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
-                         int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out, void* stream) {
+                         int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out, void* stream,
+                         const brk_tt_retrieval* rt = nullptr) {
   // mode bit 8 (0x100): Dense / in-batch products on the tensor cores (TF32 operands, gemm_tc.cu)
   const int tcore = (mode & 0x100) ? 1 : 0;
   mode &= 0xFF;
@@ -242,7 +289,7 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   if (mode == 0 && tcore) {                         // the whole step as one cooperative launch when the batch fits on chip
     int handled = 0;
     if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, training, ws, loss_out, st, &handled, 0, 0.f, 0.f,
-                                      sh))) return rc;
+                                      sh, rt))) return rc;
     if (handled) return 0;
   }
   // The user chain and the item chain are independent until the score product and again after the loss gradient, and
@@ -258,6 +305,22 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   cudaStream_t fk = ctx->fork_stream[0];
   float* dz[2] = {ws->dq, ws->dc};
   // towers: q = Eu[u] Wu + bu, c = Ei[i] Wi + bi
+  SoftmaxOptions so = {};
+  if (rt) {                                           // the column terms are ready before the score product is
+    so.inv_tau = rt->inv_temperature; so.w = rt->row_weight;
+    if (rt->cand_prob || rt->last) {
+      if (ctx->tt_logq_floats < size_t(B)) {
+        if (ctx->tt_logq) BRK_CUDA(cudaFree(ctx->tt_logq));
+        ctx->tt_logq = nullptr; ctx->tt_logq_floats = 0;
+        BRK_CUDA(cudaMalloc(&ctx->tt_logq, size_t(B) * sizeof(float)));
+        ctx->tt_logq_floats = size_t(B);
+      }
+      tt_logq_kernel<<<1, 1024, 0, st>>>(i, B, rt->cand_prob, reinterpret_cast<long long*>(rt->last), rt->gap,
+                                          reinterpret_cast<long long*>(rt->step), rt->alpha, training, ctx->tt_logq);
+      BRK_LAUNCH_CHECK();
+      so.logq = ctx->tt_logq;
+    }
+  }
   BRK_FORK(ctx, st, 0);
   if (training && mode == 0) BRK_CUDA(cudaMemsetAsync(dz[1], 0, size_t(B) * S * sizeof(float), fk));   // RED targets of
   if ((rc = tower_forward(ctx, item, i, batch, ws->ei, ws->c, tcore, fk, tsh[1]))) return rc;            // the split-K
@@ -267,7 +330,8 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   if (mode == 0) {
     // scores = q c^T; softmax CE (SUM) with accidental-hit removal; in place P = softmax - I
     if ((rc = gemm(ctx, st, tcore, ws->q, ws->c, ws->scores, nullptr, B, B, S, S, S, B, 0, 1, 1.f, 0, false))) return rc;
-    inbatch_softmax_kernel<<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc);
+    if (rt) inbatch_softmax_kernel<true><<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc, so);
+    else inbatch_softmax_kernel<<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc);
     BRK_LAUNCH_CHECK();
   } else {
     rowdot_bce_kernel<<<(B * 32 + 255) / 256, 256, 0, st>>>(ws->q, ws->c, labels, B, S, training, ws->dq, ws->dc, ws->acc);
@@ -319,10 +383,25 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   return 0;
 }
 
-extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+static int check_retrieval(const brk_tower* item, int32_t mode, const brk_tt_retrieval* rt, const char* fn) {
+  BRK_REQUIRE(std::isfinite(rt->inv_temperature) && rt->inv_temperature > 0.f, BRK_E_ARG,
+              "%s: 1 / temperature = %g is not finite and > 0", fn, double(rt->inv_temperature));
+  BRK_REQUIRE((mode & 0xFF) == 0, BRK_E_ARG, "%s: the retrieval options need the in-batch softmax (rdZero mode has no "
+              "in-batch negatives)", fn);
+  if (rt->last) {
+    BRK_REQUIRE(!rt->cand_prob, BRK_E_ARG, "%s: candidate probabilities and the streaming estimator are exclusive", fn);
+    BRK_REQUIRE(rt->gap && rt->step, BRK_E_ARG, "%s: the streaming estimator needs gap and a step counter", fn);
+    BRK_REQUIRE(rt->rows >= item->emb.rows, BRK_E_ARG, "%s: estimator arrays of %lld rows, the item table has %lld", fn,
+                (long long)rt->rows, (long long)item->emb.rows);
+    BRK_REQUIRE(rt->alpha > 0.f && rt->alpha <= 1.f, BRK_E_ARG, "%s: estimator alpha = %g outside (0, 1]", fn, double(rt->alpha));
+  }
+  return 0;
+}
+
+static int twotower_step_checked(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
                                  const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                                  int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
-                                 void* stream) {
+                                 void* stream, const brk_tt_retrieval* rt) {
   BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_step: null argument");
   BRK_REQUIRE(user->S == item->S && batch > 0 && batch < (1 << 30), BRK_E_ARG, "brk_twotower_step: S %d vs %d, batch %lld",
               user->S, item->S, (long long)batch);
@@ -331,7 +410,25 @@ extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_
               "brk_twotower_step: workspace missing");
   BRK_REQUIRE(!training || (user->emb.g && item->emb.g && user->dense.g && item->dense.g && ws->deu && ws->dei), BRK_E_ARG,
               "brk_twotower_step: gradient accumulators / deu, dei workspace missing");
-  return twotower_step(ctx, user, item, nullptr, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream);
+  if (rt) {
+    int rc;
+    if ((rc = check_retrieval(item, mode, rt, "brk_twotower_step_retrieval"))) return rc;
+  }
+  return twotower_step(ctx, user, item, nullptr, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream, rt);
+}
+
+extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                 const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                 int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
+                                 void* stream) {
+  return twotower_step_checked(ctx, user, item, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream, nullptr);
+}
+
+extern "C" int brk_twotower_step_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                           const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                           int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
+                                           void* stream, const brk_tt_retrieval* rt) {
+  return twotower_step_checked(ctx, user, item, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream, rt);
 }
 
 static int check_shards(const brk_shards* s, int32_t E, const char* which, const char* fn = "brk_twotower_step_sharded") {
@@ -396,21 +493,23 @@ int brk_tt_check_shards(const brk_shards* s, int32_t E, const char* which, const
 // on the tensor cores whose batch fits on chip run as ONE launch (twotower_fused.cu: the optimizer is the last phase of the
 // same cooperative kernel and only visits the rows the batch touched); everything else is brk_twotower_step followed by
 // the dense or row-sparse Adagrad pass of optim.cu (row-sparse for tables above rows_threshold_bytes that carry a bitmask).
-extern "C" int brk_twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
-                                       const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
-                                       int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
-                                       int64_t rows_threshold_bytes, float* loss_out, void* stream) {
+static int twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                               const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                               int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
+                               int64_t rows_threshold_bytes, float* loss_out, void* stream, const brk_tt_retrieval* rt) {
   BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_train_step: null argument");
   cudaStream_t st = (cudaStream_t)stream;
   int rc;
+  if (rt && (rc = check_retrieval(item, mode, rt, "brk_twotower_train_step_retrieval"))) return rc;
   if ((mode & 0xFF) == 0 && (mode & 0x100) && user->S == item->S && batch > 0 && batch < (1 << 30) && ws->q && ws->c && ws->dq &&
       ws->dc && ws->acc && user->emb.g && item->emb.g && user->dense.g && item->dense.g) {
     int handled = 0;
-    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps, nullptr)))
+    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps, nullptr,
+                                      rt)))
       return rc;
     if (handled) return 0;
   }
-  if ((rc = brk_twotower_step(ctx, user, item, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream))) return rc;
+  if ((rc = twotower_step_checked(ctx, user, item, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream, rt))) return rc;
   brk_table dense_pass[4], rows_pass[2];
   int nd = 0, nr = 0;
   const brk_tower* tw[2] = {user, item};
@@ -423,4 +522,21 @@ extern "C" int brk_twotower_train_step(brk_ctx* ctx, const brk_tower* user, cons
   if ((rc = brk_adagrad_dense(ctx, dense_pass, nd, lr, eps, stream))) return rc;
   if (nr && (rc = brk_adagrad_rows(ctx, rows_pass, nr, lr, eps, stream))) return rc;
   return 0;
+}
+
+extern "C" int brk_twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                       const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                       int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
+                                       int64_t rows_threshold_bytes, float* loss_out, void* stream) {
+  return twotower_train_step(ctx, user, item, u, i, cand_ids, labels, batch, mode, ws, lr, eps, rows_threshold_bytes, loss_out,
+                             stream, nullptr);
+}
+
+extern "C" int brk_twotower_train_step_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                                 const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                                 int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
+                                                 int64_t rows_threshold_bytes, float* loss_out, void* stream,
+                                                 const brk_tt_retrieval* rt) {
+  return twotower_train_step(ctx, user, item, u, i, cand_ids, labels, batch, mode, ws, lr, eps, rows_threshold_bytes, loss_out,
+                             stream, rt);
 }

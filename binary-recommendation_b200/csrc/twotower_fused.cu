@@ -26,6 +26,12 @@
 // The grid barrier (brk_grid_barrier, common.cuh) keeps its base in device memory (bar[2]), so the launch can be captured
 // into a CUDA graph and replayed (TwoTowerModel.fit does).
 //
+// fused_step<false, true> is the step with TFRS Retrieval's options (brk_twotower_step_retrieval): temperature, candidate
+// sampling probabilities (caller-supplied or the streaming frequency estimate), sample weights.  Phase F's item-tower CTAs
+// update the estimator for their rows; phase S turns each column's probability into a log2-domain term in shared memory
+// (after the F -> S barrier, so a column sees the update of its id whichever CTA made it), folds 1/tau into the
+// read-out FFMA and w/tau into the P scale, and weighs the diagonal loss.
+//
 // fused_step<true> is the same step on row-sharded tables (brk_twotower_step_sharded): row r of a table lives on rank
 // r % G at local row r / G.  The ids are split into (owner, local row) once, where they are staged in shared memory; the
 // gathers of phases F and G read the owner's shard (NVLink peer memory across GPUs) and phase G's row-gradient REDs and
@@ -73,6 +79,13 @@ struct ShardedParams : Params {
   brk_shards su, si;
 };
 template <bool SH> using ParamsT = typename std::conditional<SH, ShardedParams, Params>::type;
+// fused_step<false, true>: the retrieval options (brk_tt_retrieval) behind the same block
+struct RetrievalParams : Params {
+  const float* cand_prob; const float* row_weight;                   // [B] or null
+  long long* last; float* gap; long long* step;                      // streaming estimator (last == null: off)
+  float inv_tau, alpha;
+};
+template <bool SH, bool RT> using KParamsT = typename std::conditional<RT, RetrievalParams, ParamsT<SH>>::type;
 
 __device__ __forceinline__ void adagrad4(float4* w, float4* a, float4* g, float lr, float eps) {
   float4 w4 = *w, a4 = *a;
@@ -174,8 +187,8 @@ __device__ __forceinline__ void stage_ids(const ParamsT<SH>& P, int k, int r0, i
   }
 }
 
-template <bool SH>
-__global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
+template <bool SH, bool RT = false>
+__global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* buf0 = sm; uint8_t* buf1 = sm + TILE; uint8_t* buf2 = sm + 2 * TILE;
@@ -185,6 +198,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
   __shared__ int32_t own_s[SH ? TS : 1];                                // SH: owner rank of the row in ids_s
   __shared__ __align__(16) int32_t cand_c[TS];
   __shared__ float pm[2][TS], ps[2][TS], diag_s[TS], lse_s[TS];
+  __shared__ __align__(16) float lq_s[RT ? TS : 1];                    // RT: log2 of the column's clipped probability
   __shared__ double red[32];
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int T = P.T, B = P.B, S = P.S;
@@ -199,6 +213,10 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
   uint32_t phase = 0;
   unsigned int bar_target = *reinterpret_cast<volatile unsigned int*>(P.bar + 2);
   auto wait_mma = [&]() { tc::mbar_wait(tc::smem_u32(&mbar), phase); phase ^= 1u; tc::fence_after_sync(); };
+  long long tstep = 0;                                                  // RT: this training step's estimator time
+  if constexpr (RT) {
+    if (P.last && P.training) tstep = *reinterpret_cast<volatile long long*>(P.step) + 1;   // written back after barrier 1
+  }
 
   // ---------------- phase F: the two towers ----------------
   if (P.training) {                                                     // RED targets of phase S
@@ -210,6 +228,14 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
     const int k = b / T, r0 = (b % T) * TS, valid = min(TS, B - r0), E = P.E[k];
     const brk_table& tab = k == 0 ? P.eu : P.ei;
     stage_ids<SH>(P, k, r0, valid, ids_s, own_s);
+    if constexpr (RT) {                                                 // Yi et al. Algorithm 2: the thread whose exchange
+      if (k == 1 && P.last && P.training && t < valid) {                // saw another step is the sole updater of y
+        const int32_t y = ids_s[t];
+        const long long prev = (long long)atomicExch(reinterpret_cast<unsigned long long*>(P.last + y), (unsigned long long)tstep);
+        if (prev != tstep)
+          P.gap[y] = __fadd_rn(__fmul_rn(__fsub_rn(1.f, P.alpha), P.gap[y]), __fmul_rn(P.alpha, __ll2float_rn(tstep - prev)));
+      }
+    }
     load_tile<1>(buf1, P.W[k], S, 0, E, S);                             // W [K = E][N = S]: MN-major B operand
     __syncthreads();
     gather_tile<0, SH>(buf0, tab.w, P, k, E, ids_s, own_s, valid);   // e [M = samples][K = E]: K-major A operand
@@ -237,6 +263,9 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
   stamp(P, 1);
   brk_grid_barrier(P.bar, bar_target);
   stamp(P, 2);
+  if constexpr (RT) {
+    if (P.last && P.training && b == 0 && t == 0) *P.step = tstep;      // every CTA read the counter before the barrier
+  }
 
   // ---------------- phase S: one score tile per CTA ----------------
   const bool tile_cta = b < T * T;
@@ -253,6 +282,17 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
     if (t < TS) {
       cand_r[t] = (P.cand && ti * TS + t < B) ? __ldg(P.cand + ti * TS + t) : -1;
       cand_c[t] = (P.cand && tj * TS + t < B) ? __ldg(P.cand + tj * TS + t) : -2;
+      if constexpr (RT) {                                               // the estimator's gap is read after the F -> S barrier
+        const int j = tj * TS + t;
+        float l2 = 0.f;
+        if (j < B && (P.cand_prob || P.last)) {
+          float p = 1.f;
+          if (P.cand_prob) p = __ldg(P.cand_prob + j);
+          else { const float gp = __ldcg(P.gap + __ldg(P.ids[1] + j)); if (gp >= 1.f) p = __frcp_rn(gp); }
+          l2 = __log2f(fminf(fmaxf(p, 1e-6f), 1.f));
+        }
+        lq_s[t] = l2;
+      }
     }
     TTF_OPERANDS_READY();
     stamp(P, 8);
@@ -275,9 +315,13 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
     for (int k = 0; k < 64; k += 4) {
       const int4 cc = *reinterpret_cast<const int4*>(&cand_c[h * 64 + k]);
       const int32_t c4v[4] = {cc.x, cc.y, cc.z, cc.w};
+      float l4[4] = {0.f, 0.f, 0.f, 0.f};
+      if constexpr (RT) { const float4 lv = *reinterpret_cast<const float4*>(&lq_s[h * 64 + k]); l4[0] = lv.x; l4[1] = lv.y; l4[2] = lv.z; l4[3] = lv.w; }
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
-        float v = pv[k + q] * kLog2e;
+        float v;
+        if constexpr (RT) v = fmaf(pv[k + q], kLog2e * P.inv_tau, -l4[q]);     // s / tau - log p, log2 domain
+        else v = pv[k + q] * kLog2e;
         if (check && c4v[q] == my_id && k + q != diag_k) v += kMinFloatOver100;
         if (k + q >= ncol) v = -CUDART_INF_F;
         if (k + q == diag_k) diag_s[r] = v;
@@ -323,18 +367,23 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
     __syncthreads();
     stamp(P, 11);
     const float lse2 = lse_s[r];
+    float wrow = 1.f;                                                   // RT: the row's sample weight
+    if constexpr (RT) { if (P.row_weight && ig < B) wrow = __ldg(P.row_weight + ig); }
     if (ti == tj) {                                                     // loss = sum over rows of lse - S[row][row]
-      const double mine = (h == 0 && ig < B) ? double((lse2 - diag_s[r]) * kLn2) : 0.0;
+      double mine = (h == 0 && ig < B) ? double((lse2 - diag_s[r]) * kLn2) : 0.0;
+      if constexpr (RT) mine *= double(wrow);
       const double tot = block_sum_double(mine, red);
       if (t == 0) atomicAdd(P.acc, tot);
     }
     if (P.training) {
-      const float scale = (ig < B && mloc != -CUDART_INF_F) ? ex2(mloc - lse2) : 0.f;
+      float scale = (ig < B && mloc != -CUDART_INF_F) ? ex2(mloc - lse2) : 0.f;
+      float one = 1.f;                                                  // RT: d loss / d logit = w (P - I) / tau
+      if constexpr (RT) { one = wrow * P.inv_tau; scale *= one; }
 #pragma unroll
       for (int k = 0; k < 64; ++k) pv[k] *= scale;
       if (ig < B && diag_k >= 0 && diag_k < 64) {
 #pragma unroll
-        for (int k = 0; k < 64; ++k) if (k == diag_k) pv[k] -= 1.f;
+        for (int k = 0; k < 64; ++k) if (k == diag_k) pv[k] -= one;
       }
       // dq_i += P_ij c_j : A = P [M = i][K = j] K-major, B = c_j [K = j][N = S] MN-major
 #pragma unroll
@@ -531,7 +580,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const ParamsT<SH> P) {
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
                             float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
-                            const brk_twotower_shards* sh) {
+                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt) {
   using namespace ttf;
   *handled = 0;
   const int S = user->S, B = int(batch), T = (B + TS - 1) / TS;
@@ -553,12 +602,14 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
       return 0;
   if (!brk_aligned16(ws->q) || !brk_aligned16(ws->c) || (training && (!brk_aligned16(ws->dq) || !brk_aligned16(ws->dc)))) return 0;
   const size_t smem = 3 * size_t(TILE) + 1024;
-  const void* kern = sh ? (const void*)fused_step<true> : (const void*)fused_step<false>;
+  if (sh && rt) return 0;                                          // not instantiated: the options are unsharded only
+  const int kv = sh ? 1 : (rt ? 2 : 0);
+  const void* kern = sh ? (const void*)fused_step<true> : (rt ? (const void*)fused_step<false, true> : (const void*)fused_step<false>);
   // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of each instantiation,
   // queried once
   BRK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  static int per_sm[2] = {-1, -1};
-  int& occ = per_sm[sh ? 1 : 0];
+  static int per_sm[3] = {-1, -1, -1};
+  int& occ = per_sm[kv];
   if (occ < 0) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
   if (grid > occ * ctx->sm_count) return 0;
   const size_t part_floats = size_t(T) * TS * T * 2;
@@ -590,7 +641,15 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
     P.dn[0] = user->dense; P.dn[1] = item->dense;
   }
   if (sh) { P.su = sh->user; P.si = sh->item; }
-  void* args[] = {sh ? (void*)&P : (void*)static_cast<Params*>(&P)};
+  RetrievalParams R;
+  memset(&R, 0, sizeof(R));
+  if (rt) {
+    static_cast<Params&>(R) = static_cast<const Params&>(P);
+    R.cand_prob = rt->cand_prob; R.row_weight = rt->row_weight;
+    R.last = reinterpret_cast<long long*>(rt->last); R.gap = rt->gap; R.step = reinterpret_cast<long long*>(rt->step);
+    R.inv_tau = rt->inv_temperature; R.alpha = rt->alpha;
+  }
+  void* args[] = {sh ? (void*)&P : (rt ? (void*)&R : (void*)static_cast<Params*>(&P))};
   BRK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(NT), args, smem, st));
   *handled = 1;
   return 0;

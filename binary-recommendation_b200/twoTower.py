@@ -15,6 +15,7 @@ Differences from the reference, stated once:
     table (csrc/pipeline.cu) for ids with an exact 64-bit key, by a host dictionary for longer strings.
 """
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -206,7 +207,7 @@ class GlobalNegatives:
 class TwoTowerModel:
     def __init__(self, embedDim, nbrItem, nbrUser, userKey, itemKey, usersId, itemsId, eval_batch_size=8000,
                  loss=None, rdZero=False, resKey=None, semb=100, seed=42, device=None, tensor_cores=False,
-                 global_negatives=False):
+                 global_negatives=False, temperature=None, candidateProbKey=None, weightKey=None, streamingFrequency=None):
         self.device = torch.device(device or f"cuda:{torch.cuda.current_device()}")
         self.embedDim, self.nbrItem, self.nbrUser = embedDim, nbrItem, nbrUser
         self.userKey, self.itemKey, self.resKey = userKey, itemKey, resKey
@@ -218,6 +219,11 @@ class TwoTowerModel:
         if global_negatives and rdZero:
             raise ValueError("global_negatives needs the in-batch softmax: rdZero has no in-batch negatives")
         self.global_negatives = bool(global_negatives)
+        # tfrs.tasks.Retrieval(temperature=...) called with candidate_sampling_probability / sample_weight
+        # (brk_twotower_step_retrieval): candidateProbKey / weightKey name columns of the batch info, as resKey does;
+        # streamingFrequency=alpha (True: 0.01) estimates the candidate probabilities on the device instead (Yi et al.,
+        # RecSys 2019, Algorithm 2), with one slot per item-table row owned by the model
+        self._configure_retrieval(temperature, candidateProbKey, weightKey, streamingFrequency, nbrItem + 2)
         self.userTowerIn = StringLookup(usersId)
         self.itemTowerIn = StringLookup(itemsId)
         rng = np.random.Generator(np.random.Philox(key=seed))
@@ -243,6 +249,68 @@ class TwoTowerModel:
         self.computeLoss = self.computeLossRdZero if rdZero else self.computeLossTfrs
         self._ws_batch = 0
         self.history = {"loss": []}
+
+    def _configure_retrieval(self, temperature, candidateProbKey, weightKey, streamingFrequency, item_rows):
+        self.temperature, self.candidateProbKey, self.weightKey = temperature, candidateProbKey, weightKey
+        if streamingFrequency is False:
+            streamingFrequency = None
+        self.streamingFrequency = streamingFrequency
+        self._retrieval = any(x is not None for x in (temperature, candidateProbKey, weightKey, streamingFrequency))
+        self._freq = None
+        if not self._retrieval:
+            return
+        if self.rdZero:
+            raise ValueError("temperature / candidateProbKey / weightKey / streamingFrequency need the in-batch softmax: "
+                             "rdZero has no in-batch negatives")
+        if self.global_negatives:
+            raise ValueError("temperature / candidateProbKey / weightKey / streamingFrequency are not offered with "
+                             "global_negatives: the probabilities would have to be published with the peers' candidate blocks")
+        if temperature is not None and not (math.isfinite(float(temperature)) and float(temperature) > 0):
+            raise ValueError(f"temperature must be finite and > 0, got {temperature}")
+        if temperature is not None and not math.isfinite(1.0 / float(temperature)):
+            raise ValueError(f"temperature {temperature} is too small: 1 / temperature is not finite")
+        if streamingFrequency is not None:
+            if candidateProbKey is not None:
+                raise ValueError("candidateProbKey and streamingFrequency both give the candidate probabilities: pass one")
+            if D.world_size() > 1:
+                raise ValueError("streamingFrequency is single-process only: the estimator state is not shared across ranks")
+            alpha = 0.01 if streamingFrequency is True else float(streamingFrequency)
+            if not 0.0 < alpha <= 1.0:
+                raise ValueError(f"streamingFrequency (the estimator's alpha) must be in (0, 1], got {streamingFrequency}")
+            self._alpha = alpha
+            dev = self.device
+            self._freq = dict(last=torch.zeros(item_rows, dtype=torch.int64, device=dev),
+                              gap=torch.zeros(item_rows, dtype=torch.float32, device=dev),
+                              step=torch.zeros(1, dtype=torch.int64, device=dev))
+
+    def _extras(self, info):
+        """(candidate probabilities, sample weights) of a batch as float32 device tensors (None where not configured)."""
+        n = len(info[self.itemKey])
+        out = []
+        for key in (self.candidateProbKey, self.weightKey):
+            if key is None:
+                out.append(None)
+                continue
+            v = torch.as_tensor(np.asarray(info[key], dtype=np.float32)).to(self.device)
+            if v.numel() != n:
+                raise ValueError(f"column {key!r} has {v.numel()} entries, the batch {n}")
+            out.append(v)
+        return tuple(out)
+
+    def _rt(self, extras):
+        """brk_tt_retrieval of one call, or None when the model has no retrieval options (the option-free kernels)."""
+        if not self._retrieval:
+            return None
+        prob, weight = extras if extras is not None else (None, None)
+        rt = N.brk_tt_retrieval()
+        rt.cand_prob = prob.data_ptr() if prob is not None else None
+        rt.row_weight = weight.data_ptr() if weight is not None else None
+        rt.inv_temperature = 1.0 / float(self.temperature) if self.temperature is not None else 1.0
+        if self._freq is not None:
+            f = self._freq
+            rt.last, rt.gap, rt.step, rt.rows = f["last"].data_ptr(), f["gap"].data_ptr(), f["step"].data_ptr(), f["gap"].numel()
+            rt.alpha = self._alpha
+        return rt
 
     # ---- Keras-like surface -----------------------------------------------------------------------
     def compile(self, optimizer="Adagrad", loss=None, learningRate=0.1):
@@ -273,11 +341,18 @@ class TwoTowerModel:
         dev = self.device
         return self.userTowerIn.lookup_device(info[self.userKey], dev), self.itemTowerIn.lookup_device(info[self.itemKey], dev)
 
-    def _step(self, u, i, labels, training, loss_out=None):
+    def _step(self, u, i, labels, training, loss_out=None, extras=None):
         B = u.numel()
         loss_out = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=self.device)
         ws = self._workspace(B)
         ut, it = self.userTower.c_struct(), self.itemTower.c_struct()
+        rt = self._rt(extras)
+        if rt is not None:
+            N.check(N.lib().brk_twotower_step_retrieval(N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), N.ptr(i),
+                                                        None, B, 0x100 if self.tensor_cores else 0, 1 if training else 0,
+                                                        C.byref(ws), N.ptr(loss_out), N.stream_ptr(), C.byref(rt)),
+                    "brk_twotower_step_retrieval")
+            return loss_out
         N.check(N.lib().brk_twotower_step(N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), N.ptr(i),
                                           N.ptr(labels) if labels is not None else None, B,
                                           (1 if self.rdZero else 0) | (0x100 if self.tensor_cores else 0),
@@ -300,13 +375,23 @@ class TwoTowerModel:
         return out
 
     def computeLossTfrs(self, usersCaracteristics, itemCaracteristics, info):
-        """In-batch softmax loss of already computed tower outputs (twoTower.py:82-83), forward only."""
+        """In-batch softmax loss of already computed tower outputs (twoTower.py:82-83), forward only.  With the retrieval
+        options, in the order of tfrs Retrieval.call: scores / temperature, minus log(clip(p, 1e-6, 1)) of each column,
+        accidental hits masked, loss weighted per row; the estimator's probabilities are read, not updated."""
         scores = usersCaracteristics @ itemCaracteristics.T
         ids = torch.from_numpy(self.itemTowerIn(info[self.itemKey])).to(self.device)
         B = scores.shape[0]
+        prob, weight = self._extras(info) if self._retrieval else (None, None)
+        if self.temperature is not None:
+            scores = scores / float(self.temperature)
+        if self._freq is not None:
+            gap = self._freq["gap"][ids.long()]
+            prob = torch.where(gap >= 1.0, 1.0 / gap, torch.ones_like(gap))
+        if prob is not None:
+            scores = scores - torch.log(torch.clamp(prob, 1e-6, 1.0))[None, :]
         dup = (ids[:, None] == ids[None, :]).float() - torch.eye(B, device=self.device)
         scores = scores + dup * (float(np.finfo(np.float32).min) / 100.0)
-        return torch.nn.functional.cross_entropy(scores, torch.arange(B, device=self.device), reduction="sum")
+        return torch.nn.functional.cross_entropy(scores, torch.arange(B, device=self.device), weight=weight, reduction="sum")
 
     def computeLossRdZero(self, usersCaracteristics, itemCaracteristics, info):
         y = torch.as_tensor(np.asarray(info[self.resKey], dtype=np.float32)).to(self.device)
@@ -323,9 +408,9 @@ class TwoTowerModel:
         tower (MirroredStrategy sums per-replica gradients of a SUM-reduced loss).  With global_negatives, `info` is
         this rank's slice of the global batch and `split` the slice sizes of all ranks (default: equal slices)."""
         u, i = self._ids(info)
-        return {"loss": self._train_ids(u, i, self._labels(info), split=split)}
+        return {"loss": self._train_ids(u, i, self._labels(info), split=split, extras=self._extras(info))}
 
-    def _train_step_native(self, u, i, labels, loss_out=None):
+    def _train_step_native(self, u, i, labels, loss_out=None, extras=None):
         """Step + Keras Adagrad in one library call (brk_twotower_train_step): ONE cooperative launch when the in-batch
         softmax step runs on the tensor cores and the batch fits on chip, the step + optimizer kernels otherwise."""
         B = u.numel()
@@ -333,6 +418,13 @@ class TwoTowerModel:
         ws = self._workspace(B)
         ut, it = self.userTower.c_struct(), self.itemTower.c_struct()
         opt = self.optimizer
+        rt = self._rt(extras)
+        if rt is not None:
+            N.check(N.lib().brk_twotower_train_step_retrieval(
+                N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), N.ptr(i), None, B,
+                0x100 if self.tensor_cores else 0, C.byref(ws), float(opt.lr), float(opt.eps), int(opt.rows_threshold_bytes),
+                N.ptr(loss_out), N.stream_ptr(), C.byref(rt)), "brk_twotower_train_step_retrieval")
+            return loss_out
         N.check(N.lib().brk_twotower_train_step(N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), N.ptr(i),
                                                 N.ptr(labels) if labels is not None else None, B,
                                                 (1 if self.rdZero else 0) | (0x100 if self.tensor_cores else 0), C.byref(ws),
@@ -340,18 +432,18 @@ class TwoTowerModel:
                                                 N.stream_ptr()), "brk_twotower_train_step")
         return loss_out
 
-    def _train_ids(self, u, i, labels, loss_out=None, split=None):
+    def _train_ids(self, u, i, labels, loss_out=None, split=None, extras=None):
         if self.optimizer is None:
             self.compile()
         if D.world_size() == 1 and u.numel() > 0 and isinstance(self.optimizer, H.Adagrad):
-            return self._train_step_native(u, i, labels, loss_out)
+            return self._train_step_native(u, i, labels, loss_out, extras)
         if self._global is not None:                         # every rank calls, an empty slice included
             loss = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=self.device)
             self._global.step(self.userTower.c_struct(), self.itemTower.c_struct(), lambda r: None,
                               {D.rank(): (u, i)}, split if split is not None else [u.numel()] * D.world_size(),
                               self.tensor_cores, loss)
         elif u.numel() > 0:
-            loss = self._step(u, i, labels, True, loss_out)
+            loss = self._step(u, i, labels, True, loss_out, extras)
         else:                                                # this rank's slice of a small global batch is empty
             loss = loss_out if loss_out is not None else torch.zeros(1, dtype=torch.float32, device=self.device)
             loss.zero_()
@@ -367,7 +459,7 @@ class TwoTowerModel:
 
     def test_step(self, info):
         u, i = self._ids(info)
-        return {"loss": self._step(u, i, self._labels(info), False)}
+        return {"loss": self._step(u, i, self._labels(info), False, extras=self._extras(info))}
 
     def fit(self, dataset, epochs=1, verbose=0, graph=True):
         """dataset: iterable of info dicts (batches), replayed every epoch like a cached tf.data set.
@@ -377,7 +469,7 @@ class TwoTowerModel:
         batches = list(dataset)
         # string -> index lookups and H2D of the ids once per fit, not once per step and epoch (the reference caches
         # its batched dataset too: trainSetCached, twoTower.py:197-198)
-        staged = [(self._ids(info), self._labels(info)) for info in batches]
+        staged = [(self._ids(info), self._labels(info), self._extras(info)) for info in batches]
         if D.world_size() > 1:
             # mirrored data parallelism: a batch of the dataset is the GLOBAL batch (MultiWorkerMirroredStrategy auto-shards
             # it); this rank trains its slice, with its slice's items as in-batch negatives (the per-replica loss) or, with
@@ -389,10 +481,10 @@ class TwoTowerModel:
                 lo, hi = D.local_slice(t.numel())
                 return t[lo:hi].contiguous()
             G = D.world_size()
-            splits = [[(lambda s: s[1] - s[0])(D.local_slice(u.numel(), r, G)) for r in range(G)] for (u, _), _ in staged]
-            staged = [((mine(u), mine(i)), mine(lab)) for (u, i), lab in staged]
+            splits = [[(lambda s: s[1] - s[0])(D.local_slice(u.numel(), r, G)) for r in range(G)] for (u, _), _, _ in staged]
+            staged = [((mine(u), mine(i)), mine(lab), tuple(mine(x) for x in ex)) for (u, i), lab, ex in staged]
             D.barrier()
-        sizes = [u.numel() for (u, _), _ in staged]
+        sizes = [u.numel() for (u, _), _, _ in staged]
         n_full = 0
         while n_full < len(sizes) and sizes[n_full] == sizes[0]:
             n_full += 1
@@ -403,8 +495,8 @@ class TwoTowerModel:
             if use_graph:
                 # batch 0 runs eagerly (first-use initialisation of the library happens outside the capture), the other
                 # full batches replay the graph, a shorter last batch runs eagerly again: same order, same arithmetic
-                (u, i), lab = staged[0]
-                self._train_ids(u, i, lab, losses[0:1])
+                (u, i), lab, ex = staged[0]
+                self._train_ids(u, i, lab, losses[0:1], extras=ex)
                 if replay is None:
                     replay = self._capture_fit_graph(staged[:n_full])
                 replay(losses, 1, n_full)
@@ -412,8 +504,8 @@ class TwoTowerModel:
             else:
                 rest = range(len(staged))
             for k in rest:
-                (u, i), lab = staged[k]
-                self._train_ids(u, i, lab, losses[k:k + 1], split=splits[k] if D.world_size() > 1 else None)
+                (u, i), lab, ex = staged[k]
+                self._train_ids(u, i, lab, losses[k:k + 1], split=splits[k] if D.world_size() > 1 else None, extras=ex)
             # one host sync per epoch: Keras reports the running mean of the per-batch losses
             self.history["loss"].append(float(losses.double().sum().item()) / max(len(staged), 1))
             if self._reducer is not None:
@@ -428,11 +520,15 @@ class TwoTowerModel:
         """Captures `copy batch [pos] into the static id buffers -> fused step -> Adagrad -> store the loss at [pos] ->
         pos += 1` once; returns replay(losses, first, last) that runs batches first..last-1 of `full`."""
         dev = self.device
-        all_u = torch.stack([u for (u, _), _ in full]); all_i = torch.stack([i for (_, i), _ in full])
-        all_lab = torch.stack([lab for _, lab in full]) if full[0][1] is not None else None
+        all_u = torch.stack([u for (u, _), _, _ in full]); all_i = torch.stack([i for (_, i), _, _ in full])
+        all_lab = torch.stack([lab for _, lab, _ in full]) if full[0][1] is not None else None
+        # the retrieval columns (candidate probabilities, sample weights) are staged like the ids; the estimator's step
+        # counter lives on the device, so every replay is the next step
+        all_ex = [torch.stack([ex[k] for _, _, ex in full]) if full[0][2][k] is not None else None for k in range(2)]
         B = all_u.shape[1]
         cur_u, cur_i = torch.empty_like(all_u[0]), torch.empty_like(all_i[0])
         cur_lab = torch.empty_like(all_lab[0]) if all_lab is not None else None
+        cur_ex = tuple(torch.empty_like(a[0]) if a is not None else None for a in all_ex)
         cur_loss = torch.zeros(1, dtype=torch.float32, device=dev)
         pos = torch.zeros(1, dtype=torch.int64, device=dev)
         sink = torch.zeros(len(full), dtype=torch.float32, device=dev)
@@ -443,7 +539,10 @@ class TwoTowerModel:
             cur_u.copy_(all_u.index_select(0, pos)[0]); cur_i.copy_(all_i.index_select(0, pos)[0])
             if cur_lab is not None:
                 cur_lab.copy_(all_lab.index_select(0, pos)[0])
-            self._train_ids(cur_u, cur_i, cur_lab, cur_loss)
+            for a, c in zip(all_ex, cur_ex):
+                if c is not None:
+                    c.copy_(a.index_select(0, pos)[0])
+            self._train_ids(cur_u, cur_i, cur_lab, cur_loss, extras=cur_ex)
             sink.index_copy_(0, pos, cur_loss)
             pos.add_(1)
 
@@ -452,7 +551,7 @@ class TwoTowerModel:
             for _ in range(first, last):
                 g.replay()
             losses[first:last].copy_(sink[first:last])
-        self._fit_graph_keepalive = (g, all_u, all_i, all_lab, cur_u, cur_i, cur_lab, cur_loss, pos, sink)
+        self._fit_graph_keepalive = (g, all_u, all_i, all_lab, all_ex, cur_u, cur_i, cur_lab, cur_ex, cur_loss, pos, sink)
         return replay
 
     # ---- retrieval --------------------------------------------------------------------------------------

@@ -417,6 +417,40 @@ int brk_twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_tower
                             const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                             int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
                             int64_t rows_threshold_bytes, float* loss_out, void* stream);
+/* Sampling-bias-corrected in-batch softmax (tfrs.tasks.Retrieval(temperature) called with candidate_sampling_probability
+ * and sample_weight; Yi et al., RecSys 2019).  For query row b and in-batch candidate column j, in TFRS's order:
+ *   s_bj = (q_b . c_j) * inv_temperature;  s_bj -= log(clip(p_j, 1e-6, 1)) (every column, the label column included);
+ *   accidental hits masked as in brk_twotower_step;  loss = sum_b w_b (logsumexp_j s_bj - s_bb);
+ *   gradient of the logits w_b (softmax_bj - [b == j]) * inv_temperature.
+ * p_j: cand_prob[j] (caller-supplied, [batch]), or the streaming frequency estimate of candidate row i[j] (Yi et al.,
+ * Algorithm 2, one exact slot per item-table row instead of a hash): state last[rows] (int64, initially 0), gap[rows]
+ * (fp32, initially 0) and a device step counter *step (initially 0).  A training step sets t = *step + 1 and, once per
+ * distinct item row y of the batch, gap[y] = (1 - alpha) gap[y] + alpha (t - last[y]) (each product and the sum rounded
+ * to fp32), last[y] = t; it then stores t in *step and uses p_y = 1 / gap[y] (1 where gap[y] < 1).  training == 0 uses
+ * the state as it is and changes nothing.  Neither cand_prob nor last: no correction.  row_weight NULL: w = 1.
+ *   brk_twotower_step_retrieval / brk_twotower_train_step_retrieval: brk_twotower_step / brk_twotower_train_step with
+ *     these options; rt == NULL is exactly the call without them.  BRK_E_ARG for inv_temperature not finite or <= 0,
+ *     cand_prob together with the estimator, alpha outside (0, 1], gap or step NULL with last given, rows below the item
+ *     table's rows, and rdZero mode. */
+typedef struct brk_tt_retrieval {
+  const float* cand_prob;     /* [batch] or NULL */
+  const float* row_weight;    /* [batch] or NULL */
+  int64_t*     last;          /* [rows] or NULL (no estimator) */
+  float*       gap;           /* [rows] */
+  int64_t*     step;          /* device counter of training steps */
+  int64_t      rows;
+  float        inv_temperature;
+  float        alpha;
+} brk_tt_retrieval;
+int brk_twotower_step_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
+                                void* stream, const brk_tt_retrieval* rt);
+int brk_twotower_train_step_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                      const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
+                                      int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
+                                      int64_t rows_threshold_bytes, float* loss_out, void* stream,
+                                      const brk_tt_retrieval* rt);
 /* Two-tower training on row-sharded embedding tables (sharded.ShardedTwoTowerNet): row r of a table lives on
  * rank r % world at local row r / world (brk_shards above); the Dense blocks are mirrored.
  *   brk_twotower_step_sharded: brk_twotower_step with training = 1 on THIS rank's slice of the global batch (its
