@@ -76,6 +76,16 @@ class brk_twotower_shards(C.Structure):
     _fields_ = [("user", brk_shards), ("item", brk_shards)]
 
 
+class brk_tt_estimator_sharded(C.Structure):
+    _fields_ = [("last", C.c_void_p * BRK_MAX_PEERS), ("gap", C.c_void_p * BRK_MAX_PEERS), ("rows", C.c_int64),
+                ("world", C.c_int32), ("rank", C.c_int32)]
+
+
+class brk_tt_retrieval_sharded(C.Structure):
+    _fields_ = [("cand_prob", C.c_void_p), ("row_weight", C.c_void_p), ("est", C.POINTER(brk_tt_estimator_sharded)),
+                ("inv_temperature", C.c_float)]
+
+
 class brk_twotower_global(C.Structure):
     _fields_ = [("cand", C.c_void_p * BRK_MAX_PEERS), ("ids", C.c_void_p * BRK_MAX_PEERS),
                 ("slot", C.c_void_p * BRK_MAX_PEERS), ("offset", C.c_int64 * BRK_MAX_PEERS),
@@ -151,6 +161,11 @@ SIGNATURES = {
     "brk_twotower_step_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards), _P,
                                             _P, _P, _P, _I64, _I32, C.POINTER(brk_twotower_workspace), _P, _P]),
     "brk_tower_forward_sharded": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_shards), _P, _I64, _P, _P, _P]),
+    "brk_tt_estimator_update_sharded": (C.c_int, [_P, C.POINTER(brk_tt_estimator_sharded), _P, _I64, _F32, _P, _P]),
+    "brk_twotower_step_sharded_retrieval": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower),
+                                                      C.POINTER(brk_twotower_shards), _P, _P, _P, _P, _I64, _I32,
+                                                      C.POINTER(brk_twotower_workspace), _P, _P,
+                                                      C.POINTER(brk_tt_retrieval_sharded)]),
     "brk_twotower_step_global": (C.c_int, [_P, _I32, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards),
                                            C.POINTER(brk_twotower_global), _P, _P, _I32, C.POINTER(brk_twotower_workspace), _P,
                                            _P]),

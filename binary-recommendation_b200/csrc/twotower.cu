@@ -116,7 +116,8 @@ __global__ void __launch_bounds__(128) colsum_kernel(const float* __restrict__ X
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
                             float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
-                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt);                           // twotower_fused.cu
+                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt,
+                            const brk_tt_retrieval_sharded* srt);                                                 // twotower_fused.cu
 int brk_gemm_tf32_impl(brk_ctx* ctx, const float* A, const float* B, float* C, const float* bias, int M, int N, int K, int lda,
                        int ldb, int ldc, int trans_a, int trans_b, float alpha, int accumulate, bool allow_split,
                        cudaStream_t st);
@@ -214,6 +215,64 @@ tt_logq_kernel(const int32_t* __restrict__ ids, int B, const float* __restrict__
   }
 }
 
+// Every rank's shard of the sharded estimator (brk_tt_estimator_sharded) as a kernel argument: row y at [y % world][y / world]
+struct EstimatorShards {
+  long long* last[BRK_MAX_PEERS];
+  float* gap[BRK_MAX_PEERS];
+  int world;
+};
+
+// The estimator's update on row-sharded state (brk_tt_estimator_update_sharded), one thread per id of this rank's slice.
+// Every CTA reads t = *step + 1 first; the last CTA to take a ticket -- every other CTA has read the counter by then --
+// writes t back and resets the ticket, so graph replays advance the counter too.  The exchange is system-scope: ranks on
+// other GPUs exchange the same last[y] in the same step, and the one thread that sees another step is y's sole updater.
+// gap is read past L1: its last writer may have been another GPU.
+__global__ void __launch_bounds__(256)
+tt_estimator_update_sharded_kernel(const int32_t* __restrict__ ids, int n, EstimatorShards e, float alpha, long long* step,
+                                   unsigned int* ticket) {
+  __shared__ long long ts_s;
+  if (threadIdx.x == 0) ts_s = *reinterpret_cast<volatile long long*>(step) + 1;
+  __syncthreads();
+  const long long ts = ts_s;
+  const int j = blockIdx.x * 256 + threadIdx.x;
+  if (j < n) {
+    const int32_t y = __ldg(ids + j);
+    const int o = y % e.world;
+    const int64_t l = y / e.world;
+    const long long prev = (long long)atomicExch_system(reinterpret_cast<unsigned long long*>(e.last[o] + l), (unsigned long long)ts);
+    if (prev != ts) {
+      float* g = e.gap[o] + l;
+      *g = __fadd_rn(__fmul_rn(__fsub_rn(1.f, alpha), __ldcg(g)), __fmul_rn(alpha, __ll2float_rn(ts - prev)));
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(ticket, 1u) == gridDim.x - 1) {
+      *step = ts;
+      *ticket = 0u;
+      __threadfence();
+    }
+  }
+}
+
+// The column terms of inbatch_softmax_kernel<true> on row-sharded state (brk_twotower_step_sharded_retrieval): logq[j] =
+// log(clip(p_j, 1e-6, 1)), p_j = cand_prob[j] or 1 / gap of item row ids[j] at its owner.  Reads only.
+__global__ void __launch_bounds__(256)
+tt_logq_sharded_kernel(const int32_t* __restrict__ ids, int B, const float* __restrict__ cand_prob, EstimatorShards e,
+                       float* __restrict__ logq) {
+  const int j = blockIdx.x * 256 + threadIdx.x;
+  if (j >= B) return;
+  float p = 1.f;
+  if (cand_prob) p = __ldg(cand_prob + j);
+  else {
+    const int32_t y = __ldg(ids + j);
+    const float gp = __ldcg(e.gap[y % e.world] + y / e.world);
+    if (gp >= 1.f) p = __frcp_rn(gp);
+  }
+  logq[j] = logf(fminf(fmaxf(p, 1e-6f), 1.f));
+}
+
 // rdZero mode: pred = sigmoid(<q_b, c_b>), mean BCE against labels; dq = g c, dc = g q, g = (p - y)/B.
 __global__ void __launch_bounds__(256)
 rowdot_bce_kernel(const float* __restrict__ q, const float* __restrict__ c, const float* __restrict__ y, int B, int S,
@@ -274,11 +333,12 @@ extern "C" int brk_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t
 
 // The step after argument checks (brk_twotower_step, brk_twotower_step_sharded).  sh != nullptr: the embedding rows are
 // gathered from and their gradients scattered into the row-sharded tables sh instead of user->emb / item->emb.
-// rt != nullptr (unsharded, softmax mode only): the retrieval options, brk_twotower_step_retrieval.
+// rt != nullptr (unsharded, softmax mode only): the retrieval options, brk_twotower_step_retrieval; srt != nullptr
+// (sharded, softmax mode only): brk_twotower_step_sharded_retrieval.
 static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
                          const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                          int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out, void* stream,
-                         const brk_tt_retrieval* rt = nullptr) {
+                         const brk_tt_retrieval* rt = nullptr, const brk_tt_retrieval_sharded* srt = nullptr) {
   // mode bit 8 (0x100): Dense / in-batch products on the tensor cores (TF32 operands, gemm_tc.cu)
   const int tcore = (mode & 0x100) ? 1 : 0;
   mode &= 0xFF;
@@ -289,7 +349,7 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   if (mode == 0 && tcore) {                         // the whole step as one cooperative launch when the batch fits on chip
     int handled = 0;
     if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, training, ws, loss_out, st, &handled, 0, 0.f, 0.f,
-                                      sh, rt))) return rc;
+                                      sh, rt, srt))) return rc;
     if (handled) return 0;
   }
   // The user chain and the item chain are independent until the score product and again after the loss gradient, and
@@ -306,17 +366,27 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   float* dz[2] = {ws->dq, ws->dc};
   // towers: q = Eu[u] Wu + bu, c = Ei[i] Wi + bi
   SoftmaxOptions so = {};
-  if (rt) {                                           // the column terms are ready before the score product is
-    so.inv_tau = rt->inv_temperature; so.w = rt->row_weight;
-    if (rt->cand_prob || rt->last) {
+  if (rt || srt) {                                    // the column terms are ready before the score product is
+    so.inv_tau = rt ? rt->inv_temperature : srt->inv_temperature; so.w = rt ? rt->row_weight : srt->row_weight;
+    if (rt ? (rt->cand_prob || rt->last) : (srt->cand_prob || srt->est)) {
       if (ctx->tt_logq_floats < size_t(B)) {
         if (ctx->tt_logq) BRK_CUDA(cudaFree(ctx->tt_logq));
         ctx->tt_logq = nullptr; ctx->tt_logq_floats = 0;
         BRK_CUDA(cudaMalloc(&ctx->tt_logq, size_t(B) * sizeof(float)));
         ctx->tt_logq_floats = size_t(B);
       }
-      tt_logq_kernel<<<1, 1024, 0, st>>>(i, B, rt->cand_prob, reinterpret_cast<long long*>(rt->last), rt->gap,
-                                          reinterpret_cast<long long*>(rt->step), rt->alpha, training, ctx->tt_logq);
+      if (rt) {
+        tt_logq_kernel<<<1, 1024, 0, st>>>(i, B, rt->cand_prob, reinterpret_cast<long long*>(rt->last), rt->gap,
+                                            reinterpret_cast<long long*>(rt->step), rt->alpha, training, ctx->tt_logq);
+      } else {
+        EstimatorShards e = {};
+        e.world = 1;
+        if (srt->est) {
+          e.world = srt->est->world;
+          for (int p = 0; p < e.world; ++p) e.gap[p] = srt->est->gap[p];
+        }
+        tt_logq_sharded_kernel<<<(B + 255) / 256, 256, 0, st>>>(i, B, srt->cand_prob, e, ctx->tt_logq);
+      }
       BRK_LAUNCH_CHECK();
       so.logq = ctx->tt_logq;
     }
@@ -330,7 +400,7 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   if (mode == 0) {
     // scores = q c^T; softmax CE (SUM) with accidental-hit removal; in place P = softmax - I
     if ((rc = gemm(ctx, st, tcore, ws->q, ws->c, ws->scores, nullptr, B, B, S, S, S, B, 0, 1, 1.f, 0, false))) return rc;
-    if (rt) inbatch_softmax_kernel<true><<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc, so);
+    if (rt || srt) inbatch_softmax_kernel<true><<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc, so);
     else inbatch_softmax_kernel<<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc);
     BRK_LAUNCH_CHECK();
   } else {
@@ -441,10 +511,19 @@ static int check_shards(const brk_shards* s, int32_t E, const char* which, const
   return 0;
 }
 
-extern "C" int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
-                                         const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels,
-                                         int64_t batch, int32_t mode, const brk_twotower_workspace* ws, float* loss_out,
-                                         void* stream) {
+static int check_estimator(const brk_tt_estimator_sharded* e, const char* fn) {
+  BRK_REQUIRE(e->world >= 1 && e->world <= BRK_MAX_PEERS, BRK_E_ARG, "%s: estimator world=%d (1..%d)", fn, e->world,
+              BRK_MAX_PEERS);
+  BRK_REQUIRE(e->rank >= 0 && e->rank < e->world, BRK_E_ARG, "%s: estimator rank=%d world=%d", fn, e->rank, e->world);
+  BRK_REQUIRE(e->rows >= 1, BRK_E_ARG, "%s: estimator shards of %lld rows", fn, (long long)e->rows);
+  return 0;
+}
+
+static int twotower_step_sharded_checked(brk_ctx* ctx, const brk_tower* user, const brk_tower* item,
+                                         const brk_twotower_shards* sh, const int32_t* u, const int32_t* i,
+                                         const int32_t* cand_ids, const float* labels, int64_t batch, int32_t mode,
+                                         const brk_twotower_workspace* ws, float* loss_out, void* stream,
+                                         const brk_tt_retrieval_sharded* srt) {
   BRK_REQUIRE(ctx && user && item && ws, BRK_E_ARG, "brk_twotower_step_sharded: null argument");
   BRK_REQUIRE(sh, BRK_E_ARG, "brk_twotower_step_sharded: null shards");
   int rc;
@@ -461,7 +540,59 @@ extern "C" int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, co
               ((mode & 0xFF) != 0 || ws->scores), BRK_E_ARG, "brk_twotower_step_sharded: workspace missing");
   BRK_REQUIRE(user->dense.w && item->dense.w && user->dense.g && item->dense.g, BRK_E_ARG,
               "brk_twotower_step_sharded: Dense blocks or their gradients missing");
-  return twotower_step(ctx, user, item, sh, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream);
+  return twotower_step(ctx, user, item, sh, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream, nullptr, srt);
+}
+
+extern "C" int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
+                                         const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels,
+                                         int64_t batch, int32_t mode, const brk_twotower_workspace* ws, float* loss_out,
+                                         void* stream) {
+  return twotower_step_sharded_checked(ctx, user, item, sh, u, i, cand_ids, labels, batch, mode, ws, loss_out, stream, nullptr);
+}
+
+extern "C" int brk_twotower_step_sharded_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item,
+                                                   const brk_twotower_shards* sh, const int32_t* u, const int32_t* i,
+                                                   const int32_t* cand_ids, const float* labels, int64_t batch, int32_t mode,
+                                                   const brk_twotower_workspace* ws, float* loss_out, void* stream,
+                                                   const brk_tt_retrieval_sharded* rt) {
+  static const char* fn = "brk_twotower_step_sharded_retrieval";
+  if (rt) {
+    BRK_REQUIRE(std::isfinite(rt->inv_temperature) && rt->inv_temperature > 0.f, BRK_E_ARG,
+                "%s: 1 / temperature = %g is not finite and > 0", fn, double(rt->inv_temperature));
+    BRK_REQUIRE((mode & 0xFF) == 0, BRK_E_ARG, "%s: the retrieval options need the in-batch softmax (rdZero mode has no "
+                "in-batch negatives)", fn);
+    if (const brk_tt_estimator_sharded* e = rt->est) {
+      BRK_REQUIRE(!rt->cand_prob, BRK_E_ARG, "%s: candidate probabilities and the streaming estimator are exclusive", fn);
+      int rc;
+      if ((rc = check_estimator(e, fn))) return rc;
+      BRK_REQUIRE(sh && e->world == sh->item.world && e->rank == sh->item.rank, BRK_E_ARG,
+                  "%s: estimator of world %d rank %d, item shards of another world or rank", fn, e->world, e->rank);
+      for (int p = 0; p < e->world; ++p)
+        BRK_REQUIRE(e->gap[p], BRK_E_ARG, "%s: estimator shard %d has a null gap", fn, p);
+    }
+  }
+  return twotower_step_sharded_checked(ctx, user, item, sh, u, i, cand_ids, labels, batch, mode, ws, loss_out, stream, rt);
+}
+
+extern "C" int brk_tt_estimator_update_sharded(brk_ctx* ctx, const brk_tt_estimator_sharded* est, const int32_t* ids,
+                                               int64_t n, float alpha, int64_t* step, void* stream) {
+  static const char* fn = "brk_tt_estimator_update_sharded";
+  BRK_REQUIRE(ctx && est && step, BRK_E_ARG, "%s: null argument", fn);
+  BRK_REQUIRE(n >= 0 && n < (1 << 30) && (n == 0 || ids), BRK_E_ARG, "%s: n = %lld, ids %p", fn, (long long)n, (const void*)ids);
+  BRK_REQUIRE(alpha > 0.f && alpha <= 1.f, BRK_E_ARG, "%s: estimator alpha = %g outside (0, 1]", fn, double(alpha));
+  int rc;
+  if ((rc = check_estimator(est, fn))) return rc;
+  EstimatorShards e = {};
+  e.world = est->world;
+  for (int p = 0; p < e.world; ++p) {
+    BRK_REQUIRE(est->last[p] && est->gap[p], BRK_E_ARG, "%s: estimator shard %d has a null last / gap", fn, p);
+    e.last[p] = reinterpret_cast<long long*>(est->last[p]); e.gap[p] = est->gap[p];
+  }
+  const int grid = n > 0 ? int((n + 255) / 256) : 1;          // an empty slice still advances the counter
+  tt_estimator_update_sharded_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(ids, int(n), e, alpha,
+                                                                              reinterpret_cast<long long*>(step), ctx->tickets + 7);
+  BRK_LAUNCH_CHECK();
+  return 0;
 }
 
 extern "C" int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const brk_shards* sh, const int32_t* ids, int64_t n,
@@ -505,7 +636,7 @@ static int twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_to
       ws->dc && ws->acc && user->emb.g && item->emb.g && user->dense.g && item->dense.g) {
     int handled = 0;
     if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps, nullptr,
-                                      rt)))
+                                      rt, nullptr)))
       return rc;
     if (handled) return 0;
   }

@@ -37,6 +37,11 @@
 // gathers of phases F and G read the owner's shard (NVLink peer memory across GPUs) and phase G's row-gradient REDs and
 // touched bits go to the owner's accumulator and bitmask.  Phase O does not run: an owner's accumulator is complete only
 // after a cross-GPU barrier and the Dense gradients only after their all-reduce, so the launch ends after phase G.
+//
+// fused_step<true, true> is the row-sharded step with the options (brk_twotower_step_sharded_retrieval).  The estimator's
+// state is sharded like the item table and only read here: its update is brk_tt_estimator_update_sharded, a launch of its
+// own that every rank runs before a cross-GPU barrier.  Phase S reads the gap of column j's item row y at its owner,
+// gap[y % G][y / G], with an L2-only load (the row may have been updated through NVLink by another GPU).
 #include "common.cuh"
 #include "tc.cuh"
 #include "tc_tiles.cuh"
@@ -85,7 +90,22 @@ struct RetrievalParams : Params {
   long long* last; float* gap; long long* step;                      // streaming estimator (last == null: off)
   float inv_tau, alpha;
 };
-template <bool SH, bool RT> using KParamsT = typename std::conditional<RT, RetrievalParams, ParamsT<SH>>::type;
+// fused_step<true, true>: the options behind the sharded block; gap[p] is rank p's shard of the estimator's gap
+struct ShardedRetrievalParams : ShardedParams {
+  const float* cand_prob; const float* row_weight;                   // [B] or null
+  const float* gap[BRK_MAX_PEERS];                                   // gap[0] == null: no estimator
+  float inv_tau;
+};
+template <bool SH, bool RT> using KParamsT =
+    typename std::conditional<RT, typename std::conditional<SH, ShardedRetrievalParams, RetrievalParams>::type, ParamsT<SH>>::type;
+// the estimator's gap of item row y as phase S reads it (after the F -> S barrier, past L1)
+__device__ __forceinline__ bool has_estimator(const RetrievalParams& P) { return P.last != nullptr; }
+__device__ __forceinline__ bool has_estimator(const ShardedRetrievalParams& P) { return P.gap[0] != nullptr; }
+__device__ __forceinline__ float estimator_gap(const RetrievalParams& P, int32_t y) { return __ldcg(P.gap + y); }
+__device__ __forceinline__ float estimator_gap(const ShardedRetrievalParams& P, int32_t y) {
+  const int G = P.si.world;
+  return __ldcg(P.gap[y % G] + y / G);
+}
 
 __device__ __forceinline__ void adagrad4(float4* w, float4* a, float4* g, float lr, float eps) {
   float4 w4 = *w, a4 = *a;
@@ -214,7 +234,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   unsigned int bar_target = *reinterpret_cast<volatile unsigned int*>(P.bar + 2);
   auto wait_mma = [&]() { tc::mbar_wait(tc::smem_u32(&mbar), phase); phase ^= 1u; tc::fence_after_sync(); };
   long long tstep = 0;                                                  // RT: this training step's estimator time
-  if constexpr (RT) {
+  if constexpr (RT && !SH) {
     if (P.last && P.training) tstep = *reinterpret_cast<volatile long long*>(P.step) + 1;   // written back after barrier 1
   }
 
@@ -228,7 +248,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
     const int k = b / T, r0 = (b % T) * TS, valid = min(TS, B - r0), E = P.E[k];
     const brk_table& tab = k == 0 ? P.eu : P.ei;
     stage_ids<SH>(P, k, r0, valid, ids_s, own_s);
-    if constexpr (RT) {                                                 // Yi et al. Algorithm 2: the thread whose exchange
+    if constexpr (RT && !SH) {                                          // Yi et al. Algorithm 2: the thread whose exchange
       if (k == 1 && P.last && P.training && t < valid) {                // saw another step is the sole updater of y
         const int32_t y = ids_s[t];
         const long long prev = (long long)atomicExch(reinterpret_cast<unsigned long long*>(P.last + y), (unsigned long long)tstep);
@@ -263,7 +283,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   stamp(P, 1);
   brk_grid_barrier(P.bar, bar_target);
   stamp(P, 2);
-  if constexpr (RT) {
+  if constexpr (RT && !SH) {
     if (P.last && P.training && b == 0 && t == 0) *P.step = tstep;      // every CTA read the counter before the barrier
   }
 
@@ -285,10 +305,10 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
       if constexpr (RT) {                                               // the estimator's gap is read after the F -> S barrier
         const int j = tj * TS + t;
         float l2 = 0.f;
-        if (j < B && (P.cand_prob || P.last)) {
+        if (j < B && (P.cand_prob || has_estimator(P))) {
           float p = 1.f;
           if (P.cand_prob) p = __ldg(P.cand_prob + j);
-          else { const float gp = __ldcg(P.gap + __ldg(P.ids[1] + j)); if (gp >= 1.f) p = __frcp_rn(gp); }
+          else { const float gp = estimator_gap(P, __ldg(P.ids[1] + j)); if (gp >= 1.f) p = __frcp_rn(gp); }
           l2 = __log2f(fminf(fmaxf(p, 1e-6f), 1.f));
         }
         lq_s[t] = l2;
@@ -576,11 +596,11 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
 
 // Internal entry (twotower.cu): *handled = 0 when the shape is not this kernel's (the caller then takes the multi-kernel step).
 // sh != nullptr: the tables are row-sharded (brk_twotower_step_sharded, training only, do_opt = 0); the embedding
-// tables of user / item are then not read.
+// tables of user / item are then not read.  rt: the options on unsharded tables, srt: on sharded ones (null: none).
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
                             float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
-                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt) {
+                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt, const brk_tt_retrieval_sharded* srt) {
   using namespace ttf;
   *handled = 0;
   const int S = user->S, B = int(batch), T = (B + TS - 1) / TS;
@@ -602,13 +622,14 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
       return 0;
   if (!brk_aligned16(ws->q) || !brk_aligned16(ws->c) || (training && (!brk_aligned16(ws->dq) || !brk_aligned16(ws->dc)))) return 0;
   const size_t smem = 3 * size_t(TILE) + 1024;
-  if (sh && rt) return 0;                                          // not instantiated: the options are unsharded only
-  const int kv = sh ? 1 : (rt ? 2 : 0);
-  const void* kern = sh ? (const void*)fused_step<true> : (rt ? (const void*)fused_step<false, true> : (const void*)fused_step<false>);
+  if (sh && rt) return 0;                                          // unsharded options on sharded tables: not a caller's call
+  const int kv = sh ? (srt ? 3 : 1) : (rt ? 2 : 0);
+  const void* kern = sh ? (srt ? (const void*)fused_step<true, true> : (const void*)fused_step<true>)
+                        : (rt ? (const void*)fused_step<false, true> : (const void*)fused_step<false>);
   // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of each instantiation,
   // queried once
   BRK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  static int per_sm[3] = {-1, -1, -1};
+  static int per_sm[4] = {-1, -1, -1, -1};
   int& occ = per_sm[kv];
   if (occ < 0) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
   if (grid > occ * ctx->sm_count) return 0;
@@ -649,7 +670,15 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
     R.last = reinterpret_cast<long long*>(rt->last); R.gap = rt->gap; R.step = reinterpret_cast<long long*>(rt->step);
     R.inv_tau = rt->inv_temperature; R.alpha = rt->alpha;
   }
-  void* args[] = {sh ? (void*)&P : (rt ? (void*)&R : (void*)static_cast<Params*>(&P))};
+  ShardedRetrievalParams SR;
+  memset(&SR, 0, sizeof(SR));
+  if (sh && srt) {
+    static_cast<ShardedParams&>(SR) = P;
+    SR.cand_prob = srt->cand_prob; SR.row_weight = srt->row_weight; SR.inv_tau = srt->inv_temperature;
+    if (srt->est)
+      for (int p = 0; p < srt->est->world; ++p) SR.gap[p] = srt->est->gap[p];
+  }
+  void* args[] = {sh ? (srt ? (void*)&SR : (void*)&P) : (rt ? (void*)&R : (void*)static_cast<Params*>(&P))};
   BRK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(NT), args, smem, st));
   *handled = 1;
   return 0;

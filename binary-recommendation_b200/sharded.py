@@ -34,7 +34,7 @@ from . import _native as N
 from . import distributed as D
 from . import hotpath as H
 from .NeuMFModel import NeuMFTopKIndex, NeuMFTopKIndexFP32
-from .twoTower import GlobalNegatives, Tower, TwoTowerModel
+from .twoTower import GlobalNegatives, Tower, TwoTowerModel, check_retrieval_options
 
 
 def shard_rows(rows, G):
@@ -42,10 +42,11 @@ def shard_rows(rows, G):
     return (rows + G - 1) // G
 
 
-def save_sharded_model(dirpath, tables, replicated, G, rank, emulate, meta=None):
+def save_sharded_model(dirpath, tables, replicated, G, rank, emulate, meta=None, extra=None):
     """Checkpoint of a row-sharded model (checkpoint.py; SURVEY.md section 8 row f3): every rank writes its shards of
     the weights and optimizer slots, rank 0 the replicated tensors and -- after a barrier -- the manifest.
-    tables: {name: ShardedTable}."""
+    tables: {name: ShardedTable}; extra: {name: (shard(r) -> rank r's [local_rows, d] tensor, global rows)}, other
+    row-sharded state."""
     from . import checkpoint as CK
     ranks = list(range(G - 1, -1, -1)) if emulate else [rank]          # emulation: rank 0 (the manifest) goes last
     barrier = None
@@ -61,13 +62,16 @@ def save_sharded_model(dirpath, tables, replicated, G, rank, emulate, meta=None)
                 shd[name + "_m"] = (tab.m, t.rows)
             if tab.v is not None:
                 shd[name + "_v"] = (tab.v, t.rows)
+        for name, (shard, rows) in (extra or {}).items():
+            shd[name] = (shard(r), rows)
         CK.save_checkpoint(dirpath, replicated=replicated if r == 0 else None, sharded=shd, rank=r, world=G,
                            meta=meta, barrier=barrier)
     return dirpath
 
 
-def load_sharded_model(dirpath, tables, G, rank, emulate):
-    """Restores the shards this process owns -- whatever world size wrote the checkpoint.  Returns (replicated, meta)."""
+def load_sharded_model(dirpath, tables, G, rank, emulate, extra=None):
+    """Restores the shards this process owns -- whatever world size wrote the checkpoint.  Returns (replicated, meta).
+    extra: {name: shard(r) -> rank r's tensor}, restored where the checkpoint has the entry and zeroed where not."""
     from . import checkpoint as CK
     rep, meta = {}, {}
     for r in (range(G) if emulate else [rank]):
@@ -79,6 +83,11 @@ def load_sharded_model(dirpath, tables, G, rank, emulate):
                 tab.m.copy_(torch.from_numpy(shd[name + "_m"]))
             if tab.v is not None and name + "_v" in shd:
                 tab.v.copy_(torch.from_numpy(shd[name + "_v"]))
+        for name, shard in (extra or {}).items():
+            if name in shd:
+                shard(r).copy_(torch.from_numpy(shd[name]))
+            else:
+                shard(r).zero_()
     if not emulate and G > 1:
         torch.cuda.synchronize()
         dist.barrier()                                   # nobody gathers peer rows before every owner has loaded
@@ -487,6 +496,63 @@ class ShardedBPRNet:
         return meta
 
 
+class ShardedEstimator:
+    """The streaming frequency estimator of Yi et al. (brk_tt_retrieval's, one slot per item-table row) with its state
+    sharded like the item table: last (int64) and gap (fp32) of row y live on rank y % G at local row y // G, in
+    symmetric memory on real ranks and as G local arrays under emulation (as ShardedTable).  `step` is this process's
+    training-step counter, equal on every rank."""
+
+    def __init__(self, rows, G, rank, device, alpha, symmetric, emulate):
+        self.rows, self.G, self.rank, self.device, self.alpha = int(rows), int(G), int(rank), device, float(alpha)
+        self.local_rows = shard_rows(rows, G)
+        self.emulate = emulate
+        self.last, self.gap, self._keep = {}, {}, []
+        ptr_l, ptr_g = [0] * G, [0] * G
+        for r in (range(G) if emulate else [rank]):
+            if symmetric and not emulate:
+                import torch.distributed._symmetric_memory as symm_mem
+                group = dist.group.WORLD.group_name
+                last = symm_mem.empty(self.local_rows, dtype=torch.int64, device=device)
+                gap = symm_mem.empty(self.local_rows, dtype=torch.float32, device=device)
+                hs = [symm_mem.rendezvous(x, group) for x in (last, gap)]
+                self._keep.append(hs)
+                ptr_l, ptr_g = (list(h.buffer_ptrs) for h in hs)
+            else:
+                last = torch.empty(self.local_rows, dtype=torch.int64, device=device)
+                gap = torch.empty(self.local_rows, dtype=torch.float32, device=device)
+                ptr_l[r], ptr_g[r] = last.data_ptr(), gap.data_ptr()
+            last.zero_(); gap.zero_()
+            self.last[r], self.gap[r] = last, gap
+        self.step = torch.zeros(1, dtype=torch.int64, device=device)
+        self.c = N.brk_tt_estimator_sharded()
+        for p in range(G):
+            self.c.last[p], self.c.gap[p] = ptr_l[p], ptr_g[p]
+        self.c.rows, self.c.world, self.c.rank = self.local_rows, G, self.rank
+
+    def update(self, ids):
+        """The training-step update for this rank's slice `ids` (int32 item rows; may be empty)."""
+        N.check(N.lib().brk_tt_estimator_update_sharded(N.ctx(self.device), C.byref(self.c), N.ptr(ids) if ids.numel() else None,
+                                                         ids.numel(), self.alpha, N.ptr(self.step), N.stream_ptr()),
+                "brk_tt_estimator_update_sharded")
+
+    def state(self):
+        """(last [rows] int64, gap [rows] float32, step) of the whole table on the host; collective on real ranks."""
+        if self.emulate or self.G == 1:
+            parts = [(self.last[r].cpu().numpy(), self.gap[r].cpu().numpy()) for r in range(self.G)]
+        else:
+            gathered = []
+            for mine in (self.last[self.rank], self.gap[self.rank]):
+                ts = [torch.empty_like(mine) for _ in range(self.G)]
+                dist.all_gather(ts, mine)
+                gathered.append([t.cpu().numpy() for t in ts])
+            parts = list(zip(*gathered))
+        last, gap = np.zeros(self.rows, np.int64), np.zeros(self.rows, np.float32)
+        for r, (lr, gr) in enumerate(parts):
+            n = len(range(r, self.rows, self.G))
+            last[r::self.G], gap[r::self.G] = lr[:n], gr[:n]
+        return last, gap, int(self.step.item())
+
+
 class ShardedTwoTowerNet:
     """Two-tower retrieval model (twoTower.TwoTowerModel: Embedding -> linear Dense(semb) per tower, in-batch softmax or
     rdZero BCE, Keras Adagrad) with row-sharded embedding tables, for catalogs too large to mirror on every GPU.
@@ -509,14 +575,27 @@ class ShardedTwoTowerNet:
     With global_negatives=True, `emulate=G` splits each batch with local_slice over the G emulated ranks and runs the
     three phases of brk_twotower_step_global rank by rank; with one rank (G = 1) the flag changes nothing.
 
+    tfrs Retrieval's sampling-bias correction (brk_twotower_step_sharded_retrieval), per replica as the softmax above:
+    temperature=tau, per-call candidate sampling probabilities `cand_prob` and sample weights `weights` ([b] float32 device
+    tensors of this rank's slice; under emulation of the whole batch), or streamingFrequency=alpha (True: 0.01): the
+    streaming frequency estimator (ShardedEstimator) updated on the GLOBAL batch -- every rank updates the rows of its
+    slice, a cross-GPU barrier, then every replica's step reads p_y = 1 / gap[y] at the owner -- so its state equals the
+    single-process estimator's on the global batch bit for bit.  Not offered with rdZero or global_negatives.
+
     Ids arrive as int32 table rows (already looked up).  full_init: {"user", "item": full tables [rows, E];
     "user_dense", "item_dense": flat Dense blocks as Tower.init_dense lays them out}; without it the tables are
     U(-0.05, 0.05) and the Dense blocks Glorot-uniform from Philox(seed + 77)."""
 
     def __init__(self, numUser, numItem, embedDim, semb, learning_rate=0.1, rdZero=False, tensor_cores=True, seed=42,
-                 device=None, emulate=0, full_init=None, global_negatives=False):
+                 device=None, emulate=0, full_init=None, global_negatives=False, temperature=None, streamingFrequency=None):
         if global_negatives and rdZero:
             raise ValueError("global_negatives needs the in-batch softmax: rdZero has no in-batch negatives")
+        if streamingFrequency is False:
+            streamingFrequency = None
+        self.temperature, self.streamingFrequency = temperature, streamingFrequency
+        self._retrieval = temperature is not None or streamingFrequency is not None
+        alpha = check_retrieval_options(rdZero, global_negatives, temperature, streamingFrequency, False) \
+            if self._retrieval else None
         self.device = torch.device(device or f"cuda:{torch.cuda.current_device()}")
         self.emulate = int(emulate)
         self.G, self.rank = (self.emulate, 0) if self.emulate else (D.world_size(), D.rank())
@@ -528,6 +607,9 @@ class ShardedTwoTowerNet:
         dev, E, S = self.device, self.embedDim, self.semb
         symmetric = not self.emulate and self.G > 1
         fi = full_init or {}
+        # before the peer barrier below: its set-up barrier fences the zeroed estimator shards too
+        self._est = ShardedEstimator(self.numItem + 2, self.G, self.rank, dev, alpha, symmetric, bool(self.emulate)) \
+            if alpha is not None else None
         mk = lambda name, rows, k: ShardedTable(rows, E, self.G, self.rank, dev, full_init=fi.get(name), init_seed=seed * 16 + k,
                                                 symmetric=symmetric, emulate=bool(self.emulate), slots=1,
                                                 slot_init=H.Adagrad.INITIAL_ACCUMULATOR)
@@ -562,23 +644,60 @@ class ShardedTwoTowerNet:
     def _shards(self):
         return N.brk_twotower_shards(self.user.c_shards(), self.item.c_shards())
 
-    def train_on_batch(self, u, i, labels=None, loss_out=None, split=None):
+    def train_on_batch(self, u, i, labels=None, loss_out=None, split=None, cand_prob=None, weights=None):
         """One step on this rank's slice (u, i: int32 table rows; labels: rdZero targets).  Every rank must call it, an
         empty slice included.  Returns the slice's loss as a device scalar.  With global_negatives on real ranks, `split`
         lists the slice sizes of all G ranks (default: every slice has this one's size); under emulation u, i are the
-        global batch and the loss is the sum over the emulated ranks."""
-        loss_out = self.forward_backward(u, i, labels, loss_out, split)
+        global batch and the loss is the sum over the emulated ranks.  cand_prob / weights: the slice's candidate
+        sampling probabilities and sample weights (see the class docstring)."""
+        loss_out = self.forward_backward(u, i, labels, loss_out, split, cand_prob, weights)
         self.apply_gradients()
         return loss_out
 
-    def forward_backward(self, u, i, labels=None, loss_out=None, split=None):
+    def _rt(self, B, cand_prob, weights):
+        """brk_tt_retrieval_sharded of one step, or None without any option (the option-free step)."""
+        if not self._retrieval and cand_prob is None and weights is None:
+            return None
+        check_retrieval_options(self.rdZero, self.global_negatives, None, self.streamingFrequency, cand_prob is not None)
+        cols = []
+        for name, v in (("cand_prob", cand_prob), ("weights", weights)):
+            if v is not None and v.numel() != B:
+                raise ValueError(f"{name} has {v.numel()} entries, the slice {B}")
+            cols.append(H._f32(v, name) if v is not None else None)
+        rt = N.brk_tt_retrieval_sharded()
+        rt.cand_prob, rt.row_weight = (N.ptr(v).value if v is not None and B > 0 else None for v in cols)
+        rt._cols = cols                                     # alive as long as the struct
+        rt.inv_temperature = 1.0 / float(self.temperature) if self.temperature is not None else 1.0
+        if self._est is not None:
+            rt.est = C.pointer(self._est.c)
+        return rt
+
+    def forward_backward(self, u, i, labels=None, loss_out=None, split=None, cand_prob=None, weights=None):
         """The step without the optimizer: row gradients in the owners' accumulators (touched bits set there), Dense
-        gradients in this rank's Dense blocks."""
+        gradients in this rank's Dense blocks.  With the estimator, every rank's update of the global batch, then a
+        cross-GPU barrier, comes first."""
         B = u.numel()
         dev = self.device
         loss_out = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=dev)
         lib, ctx, st = N.lib(), N.ctx(dev), N.stream_ptr()
-        if self._global is not None:
+        rt = self._rt(B, cand_prob, weights)
+        if rt is not None:
+            u, i = H._i32(u, "u"), H._i32(i, "i")
+            if self._est is not None:
+                self._est.update(i)
+                if self.barrier is not None:
+                    self.barrier()                          # every rank's update has landed before any step reads gap
+            if B > 0:
+                ws = self._workspace(B)
+                ut, it = self._towers()
+                sh = self._shards()
+                N.check(lib.brk_twotower_step_sharded_retrieval(ctx, C.byref(ut), C.byref(it), C.byref(sh), N.ptr(u), N.ptr(i),
+                                                                N.ptr(i), None, B, 0x100 if self.tensor_cores else 0,
+                                                                C.byref(ws), N.ptr(loss_out), st, C.byref(rt)),
+                        "brk_twotower_step_sharded_retrieval")
+            else:
+                loss_out.zero_()
+        elif self._global is not None:
             u, i = H._i32(u, "u"), H._i32(i, "i")
             if self.emulate:
                 bounds = {r: D.local_slice(B, r, self.G) for r in range(self.G)}
@@ -629,8 +748,14 @@ class ShardedTwoTowerNet:
         D.all_reduce_sum_(self.grad_arena, self._reducer)
         N.check(lib.brk_adagrad_dense(ctx, H._pack(self.dense), 2, opt.lr, opt.eps, st), "brk_adagrad_dense")
 
+    def estimator_state(self):
+        """(last [rows] int64, gap [rows] float32, step) of the streaming frequency estimator on the host (None without
+        it); collective on real ranks, like ShardedTable.full_weights."""
+        return self._est.state() if self._est is not None else None
+
     def check(self):
-        """Raises when a cross-GPU barrier or the Dense all-reduce timed out (call at epoch ends, not per step)."""
+        """Raises when a cross-GPU barrier (the estimator's included: it shares the model's flag block) or the Dense
+        all-reduce timed out (call at epoch ends, not per step)."""
         if self.barrier is not None:
             self.barrier.check()
         if self._reducer is not None:
@@ -661,19 +786,36 @@ class ShardedTwoTowerNet:
         return ShardedDotTopKIndex(self, itemsId, k, self._tower_forward, self.semb, self.item.rows)
 
     # ---- checkpoint: shards of the tables and their accumulators, replicated Dense blocks and theirs ------------
+    # With the estimator also its state: last / gap as row-sharded [rows, 1] entries (re-sharded across world sizes
+    # like the tables) and the step counter replicated.
+    def _estimator_shards(self):
+        e = self._est
+        if e is None:
+            return {}
+        return {"estimator_last": lambda r: e.last[r].view(-1, 1), "estimator_gap": lambda r: e.gap[r].view(-1, 1)}
+
     def save_checkpoint(self, dirpath):
         rep = {}
         for name, t in zip(("user_dense", "item_dense"), self.dense):
             rep[name], rep[name + "_m"] = t.w.view(-1), t.m.view(-1)
+        if self._est is not None:
+            rep["estimator_step"] = self._est.step
+        extra = {name: (shard, self._est.rows) for name, shard in self._estimator_shards().items()}
         return save_sharded_model(dirpath, {"user": self.user, "item": self.item}, rep, self.G, self.rank, self.emulate,
                                   meta={"model": "ShardedTwoTowerNet", "E": self.embedDim, "S": self.semb,
-                                        "numUser": self.numUser, "numItem": self.numItem})
+                                        "numUser": self.numUser, "numItem": self.numItem}, extra=extra)
 
     def load_checkpoint(self, dirpath):
-        rep, meta = load_sharded_model(dirpath, {"user": self.user, "item": self.item}, self.G, self.rank, self.emulate)
+        """Restores what save_checkpoint wrote, whatever world size wrote it.  A model with the estimator that loads a
+        checkpoint without its state (one saved without streamingFrequency) starts the estimator from zero: every row
+        unseen and the step counter at 0."""
+        rep, meta = load_sharded_model(dirpath, {"user": self.user, "item": self.item}, self.G, self.rank, self.emulate,
+                                       extra=self._estimator_shards())
         for name, t in zip(("user_dense", "item_dense"), self.dense):
             t.w.view(-1).copy_(torch.from_numpy(rep[name]))
             t.m.view(-1).copy_(torch.from_numpy(rep[name + "_m"]))
+        if self._est is not None:
+            self._est.step.fill_(int(rep["estimator_step"][0]) if "estimator_step" in rep else 0)
         return meta
 
 

@@ -204,6 +204,31 @@ class GlobalNegatives:
                                "given (the ranks passed different splits, or a rank skipped a step)")
 
 
+def check_retrieval_options(rdZero, global_negatives, temperature, streamingFrequency, candidate_probs):
+    """The checks of tfrs Retrieval's options that TwoTowerModel and sharded.ShardedTwoTowerNet share (ValueError).
+    candidate_probs: the caller also supplies candidate probabilities.  Returns the estimator's alpha (streamingFrequency
+    True: 0.01), or None without the estimator."""
+    if rdZero:
+        raise ValueError("temperature / candidateProbKey / weightKey / streamingFrequency need the in-batch softmax: "
+                         "rdZero has no in-batch negatives")
+    if global_negatives:
+        raise ValueError("temperature / candidateProbKey / weightKey / streamingFrequency are not offered with "
+                         "global_negatives: the probabilities would have to be published with the peers' candidate blocks")
+    if temperature is not None and not (math.isfinite(float(temperature)) and float(temperature) > 0):
+        raise ValueError(f"temperature must be finite and > 0, got {temperature}")
+    if temperature is not None and not math.isfinite(1.0 / float(temperature)):
+        raise ValueError(f"temperature {temperature} is too small: 1 / temperature is not finite")
+    if streamingFrequency is None or streamingFrequency is False:
+        return None
+    if candidate_probs:
+        raise ValueError("candidate probabilities (candidateProbKey, cand_prob) and streamingFrequency both give p: "
+                         "pass one")
+    alpha = 0.01 if streamingFrequency is True else float(streamingFrequency)
+    if not 0.0 < alpha <= 1.0:
+        raise ValueError(f"streamingFrequency (the estimator's alpha) must be in (0, 1], got {streamingFrequency}")
+    return alpha
+
+
 class TwoTowerModel:
     def __init__(self, embedDim, nbrItem, nbrUser, userKey, itemKey, usersId, itemsId, eval_batch_size=8000,
                  loss=None, rdZero=False, resKey=None, semb=100, seed=42, device=None, tensor_cores=False,
@@ -259,24 +284,11 @@ class TwoTowerModel:
         self._freq = None
         if not self._retrieval:
             return
-        if self.rdZero:
-            raise ValueError("temperature / candidateProbKey / weightKey / streamingFrequency need the in-batch softmax: "
-                             "rdZero has no in-batch negatives")
-        if self.global_negatives:
-            raise ValueError("temperature / candidateProbKey / weightKey / streamingFrequency are not offered with "
-                             "global_negatives: the probabilities would have to be published with the peers' candidate blocks")
-        if temperature is not None and not (math.isfinite(float(temperature)) and float(temperature) > 0):
-            raise ValueError(f"temperature must be finite and > 0, got {temperature}")
-        if temperature is not None and not math.isfinite(1.0 / float(temperature)):
-            raise ValueError(f"temperature {temperature} is too small: 1 / temperature is not finite")
-        if streamingFrequency is not None:
-            if candidateProbKey is not None:
-                raise ValueError("candidateProbKey and streamingFrequency both give the candidate probabilities: pass one")
+        alpha = check_retrieval_options(self.rdZero, self.global_negatives, temperature, streamingFrequency,
+                                        candidateProbKey is not None)
+        if alpha is not None:
             if D.world_size() > 1:
                 raise ValueError("streamingFrequency is single-process only: the estimator state is not shared across ranks")
-            alpha = 0.01 if streamingFrequency is True else float(streamingFrequency)
-            if not 0.0 < alpha <= 1.0:
-                raise ValueError(f"streamingFrequency (the estimator's alpha) must be in (0, 1], got {streamingFrequency}")
             self._alpha = alpha
             dev = self.device
             self._freq = dict(last=torch.zeros(item_rows, dtype=torch.int64, device=dev),

@@ -471,6 +471,49 @@ int brk_twotower_step_sharded(brk_ctx* ctx, const brk_tower* user, const brk_tow
                               void* stream);
 int brk_tower_forward_sharded(brk_ctx* ctx, const brk_tower* t, const brk_shards* sh, const int32_t* ids, int64_t n,
                               float* emb_out, float* out, void* stream);
+/* Sampling-bias-corrected softmax on row-sharded tables (sharded.ShardedTwoTowerNet(temperature=, streamingFrequency=)):
+ * brk_tt_retrieval's semantics on each rank's slice, with the streaming estimator's state sharded like the item table.
+ * last / gap of item row y live on rank y % world at local row y / world (rows per shard each, every rank's shard
+ * pointer given: NVLink peer mappings, or local buffers when one process drives every rank); step is this rank's counter.
+ *   brk_tt_estimator_update_sharded: the training-step update of the estimator for this rank's slice ids[0..n) of the
+ *     global batch.  t = *step + 1; for every distinct row y of the GLOBAL batch exactly one thread on any GPU -- the one
+ *     whose system-scope exchange of last[y] returned another step -- sets gap[y] = (1 - alpha) gap[y] + alpha (t -
+ *     last[y]) (products and sum rounded to fp32); then *step = t.  So after every rank's update the state equals the
+ *     single-process estimator run on the global batch, bit for bit.  n == 0 still advances the counter.  A grid-wide
+ *     launch that waits on no other GPU; its launches on one context are stream-ordered (the context's last-block ticket
+ *     writes the counter back).  BRK_E_ARG for null est / step / ids (n > 0), n < 0, alpha outside (0, 1], world outside
+ *     1..BRK_MAX_PEERS, rank outside [0, world), rows < 1, and a null last / gap shard.
+ *   brk_twotower_step_sharded_retrieval: brk_twotower_step_sharded with the options of brk_tt_retrieval on this rank's
+ *     slice: logits (q_b . c_j) * inv_temperature - log(clip(p_j, 1e-6, 1)), accidental hits masked, loss = sum_b w_b
+ *     (logsumexp_j s_bj - s_bb), logit gradient w_b (softmax_bj - [b == j]) * inv_temperature.  p_j: cand_prob[j]
+ *     ([batch], caller-supplied), or with est != NULL 1 / gap of column j's item row read from its owner (1 where gap < 1);
+ *     the estimator's state is only read.  row_weight NULL: w = 1.  rt == NULL is exactly brk_twotower_step_sharded.
+ *     BRK_E_ARG as brk_twotower_step_sharded, and for inv_temperature not finite or <= 0, cand_prob together with est,
+ *     rdZero mode, and an est whose world or rank differ from the shards', with rows < 1 or a null gap shard.
+ * Ordering of one training step with the estimator: every rank (an empty slice included) calls
+ * brk_tt_estimator_update_sharded, then passes brk_peer_barrier, then calls brk_twotower_step_sharded_retrieval; after it
+ * the barriers of brk_twotower_step_sharded.  The next step's update comes after those barriers, so no rank updates the
+ * state while another still reads it.  When one process drives every rank (or world == 1) the updates and the step are
+ * ordered by the stream and no barrier is needed. */
+typedef struct brk_tt_estimator_sharded {
+  int64_t* last[BRK_MAX_PEERS];
+  float*   gap[BRK_MAX_PEERS];
+  int64_t  rows;              /* rows per shard */
+  int32_t  world, rank;
+} brk_tt_estimator_sharded;
+typedef struct brk_tt_retrieval_sharded {
+  const float* cand_prob;     /* [batch] or NULL */
+  const float* row_weight;    /* [batch] or NULL */
+  const brk_tt_estimator_sharded* est;   /* NULL: no estimator */
+  float        inv_temperature;
+} brk_tt_retrieval_sharded;
+int brk_tt_estimator_update_sharded(brk_ctx* ctx, const brk_tt_estimator_sharded* est, const int32_t* ids, int64_t n,
+                                    float alpha, int64_t* step, void* stream);
+int brk_twotower_step_sharded_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item,
+                                        const brk_twotower_shards* sh, const int32_t* u, const int32_t* i,
+                                        const int32_t* cand_ids, const float* labels, int64_t batch, int32_t mode,
+                                        const brk_twotower_workspace* ws, float* loss_out, void* stream,
+                                        const brk_tt_retrieval_sharded* rt);
 /* Two-tower training with GLOBAL in-batch negatives (csrc/twotower_global.cu): every rank's queries are scored against
  * the candidates of the whole global batch of n rows.  Rank p holds rows [offset[p], offset[p] + count[p]) (the
  * offsets tile [0, n); slices may be empty).  For rank r's row i (global row o = offset[r] + i) the logits are
