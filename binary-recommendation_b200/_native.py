@@ -86,6 +86,11 @@ class brk_tt_retrieval_sharded(C.Structure):
                 ("inv_temperature", C.c_float)]
 
 
+class brk_tt_sampled(C.Structure):
+    _fields_ = [("ids", C.c_void_p), ("step", C.c_void_p), ("count", C.c_int64), ("lo", C.c_int64), ("hi", C.c_int64),
+                ("rows", C.c_int64), ("seed", C.c_uint32), ("replica", C.c_uint32)]
+
+
 class brk_twotower_global(C.Structure):
     _fields_ = [("cand", C.c_void_p * BRK_MAX_PEERS), ("ids", C.c_void_p * BRK_MAX_PEERS),
                 ("slot", C.c_void_p * BRK_MAX_PEERS), ("offset", C.c_int64 * BRK_MAX_PEERS),
@@ -166,6 +171,16 @@ SIGNATURES = {
                                                       C.POINTER(brk_twotower_shards), _P, _P, _P, _P, _I64, _I32,
                                                       C.POINTER(brk_twotower_workspace), _P, _P,
                                                       C.POINTER(brk_tt_retrieval_sharded)]),
+    "brk_twotower_step_sampled": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), _P, _P, _I64, _I32,
+                                            C.POINTER(brk_twotower_workspace), _P, _P, C.POINTER(brk_tt_sampled),
+                                            C.POINTER(brk_tt_retrieval)]),
+    "brk_twotower_train_step_sampled": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower), _P, _P, _I64, _I32,
+                                                  C.POINTER(brk_twotower_workspace), _F32, _F32, _I64, _P, _P,
+                                                  C.POINTER(brk_tt_sampled), C.POINTER(brk_tt_retrieval)]),
+    "brk_twotower_step_sharded_sampled": (C.c_int, [_P, C.POINTER(brk_tower), C.POINTER(brk_tower),
+                                                    C.POINTER(brk_twotower_shards), _P, _P, _I64, _I32,
+                                                    C.POINTER(brk_twotower_workspace), _P, _P, C.POINTER(brk_tt_sampled),
+                                                    C.POINTER(brk_tt_retrieval_sharded)]),
     "brk_twotower_step_global": (C.c_int, [_P, _I32, C.POINTER(brk_tower), C.POINTER(brk_tower), C.POINTER(brk_twotower_shards),
                                            C.POINTER(brk_twotower_global), _P, _P, _I32, C.POINTER(brk_twotower_workspace), _P,
                                            _P]),

@@ -210,6 +210,7 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1
 // [0, n] such that t == n or a[t] - t > r (a = the user's sorted positive list).  One binary search, no
 // rejection loop, so the slowest sample of a batch costs the same as every other one.
 constexpr uint32_t kBrkTagBpr = 0xB9u;
+constexpr uint32_t kBrkTagTwoTowerNeg = 0x7Eu;     // two-tower sampled negatives (brk_tt_sampled)
 __device__ __forceinline__ int32_t brk_sample_bpr_negative(uint64_t idx, int64_t u, uint32_t seed, uint32_t epoch,
                                                            uint32_t num_items, const int64_t* __restrict__ indptr,
                                                            const int32_t* __restrict__ items) {

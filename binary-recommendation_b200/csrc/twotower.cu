@@ -117,7 +117,7 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
                             float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
                             const brk_twotower_shards* sh, const brk_tt_retrieval* rt,
-                            const brk_tt_retrieval_sharded* srt);                                                 // twotower_fused.cu
+                            const brk_tt_retrieval_sharded* srt, const brk_tt_sampled* smp);                      // twotower_fused.cu
 int brk_gemm_tf32_impl(brk_ctx* ctx, const float* A, const float* B, float* C, const float* bias, int M, int N, int K, int lda,
                        int ldb, int ldc, int trans_a, int trans_b, float alpha, int accumulate, bool allow_split,
                        cudaStream_t st);
@@ -273,6 +273,62 @@ tt_logq_sharded_kernel(const int32_t* __restrict__ ids, int B, const float* __re
   logq[j] = logf(fminf(fmaxf(p, 1e-6f), 1.f));
 }
 
+// The draws of brk_tt_sampled at t = *step + 1: ids[k] = lo + mulshift(philox((k, t, t >> 32, tag), (seed, replica)).x,
+// range).  One CTA: every thread has read the counter before thread 0 writes t back, so graph replays draw the next step.
+__global__ void __launch_bounds__(1024)
+tt_sample_negatives_kernel(int32_t* __restrict__ ids, int M, int32_t lo, uint32_t range, uint32_t seed, uint32_t replica,
+                           long long* step) {
+  __shared__ long long ts_s;
+  if (threadIdx.x == 0) ts_s = *step + 1;
+  __syncthreads();
+  const unsigned long long ts = (unsigned long long)ts_s;
+  for (int k = threadIdx.x; k < M; k += 1024) {
+    const uint4 w = philox4x32_10(make_uint4(uint32_t(k), uint32_t(ts), uint32_t(ts >> 32), kBrkTagTwoTowerNeg), seed, replica);
+    ids[k] = lo + int32_t(__umulhi(w.x, range));
+  }
+  if (threadIdx.x == 0) *step = (long long)ts;
+}
+
+// One CTA per query row of the [B, n] scores of the sampled-negatives step (n = B + M): columns j < B are the batch's
+// candidates (item rows ids[j]), columns B + k the draws smp[k].  Logits s * inv_tau, a column j != row whose item row
+// equals the row's positive masked, loss w_row (lse - s_row,row), in place P = w_row (softmax - Y) * inv_tau.
+__global__ void __launch_bounds__(256)
+sampled_softmax_kernel(float* __restrict__ Sc, const int32_t* __restrict__ ids, const int32_t* __restrict__ smp, int B, int n,
+                       double* __restrict__ loss_acc, float inv_tau, const float* __restrict__ w) {
+  __shared__ float redf[32];
+  __shared__ double redd[32];
+  __shared__ float lse_sm;
+  const int row = blockIdx.x, t = threadIdx.x;
+  float* s = Sc + int64_t(row) * n;
+  const int32_t pos_id = __ldg(ids + row);
+  float mx = -CUDART_INF_F;
+  for (int j = t; j < n; j += 256) {
+    float v = s[j] * inv_tau;
+    const int32_t id = j < B ? __ldg(ids + j) : __ldg(smp + (j - B));
+    if (j != row && id == pos_id) v += kMinFloatOver100;
+    s[j] = v;
+    mx = fmaxf(mx, v);
+  }
+  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if ((t & 31) == 0) redf[t >> 5] = mx;
+  __syncthreads();
+  mx = redf[0];
+#pragma unroll
+  for (int k = 1; k < 8; ++k) mx = fmaxf(mx, redf[k]);
+  double sum = 0.0;
+  for (int j = t; j < n; j += 256) sum += double(expf(s[j] - mx));
+  sum = block_sum_double(sum, redd);
+  const float wr = w ? __ldg(w + row) : 1.f;
+  if (t == 0) {
+    const float lse = mx + logf(float(sum));
+    lse_sm = lse;
+    atomicAdd(loss_acc, double(wr) * double(lse - s[row]));
+  }
+  __syncthreads();
+  const float lse = lse_sm, wt = wr * inv_tau;
+  for (int j = t; j < n; j += 256) s[j] = (expf(s[j] - lse) - (j == row ? 1.f : 0.f)) * wt;
+}
+
 // rdZero mode: pred = sigmoid(<q_b, c_b>), mean BCE against labels; dq = g c, dc = g q, g = (p - y)/B.
 __global__ void __launch_bounds__(256)
 rowdot_bce_kernel(const float* __restrict__ q, const float* __restrict__ c, const float* __restrict__ y, int B, int S,
@@ -313,15 +369,23 @@ extern "C" int brk_sgemm(brk_ctx* ctx, const float* A, const float* B, float* C,
                true);
 }
 
-// sh != nullptr: the rows come from the row-sharded table sh instead of t->emb
+// sh != nullptr: the rows come from the row-sharded table sh instead of t->emb.  extra [m]: rows gathered after ids[0..n)
+// (the sampled negatives), the tower then runs over all n + m rows.
 static int tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t* ids, int64_t n, float* emb_out, float* out,
-                         int tcore, void* stream, const brk_shards* sh = nullptr) {
+                         int tcore, void* stream, const brk_shards* sh = nullptr, const int32_t* extra = nullptr,
+                         int64_t m = 0) {
   int rc = sh ? brk_gather_rows_sharded(ctx, sh, t->E, ids, n, emb_out, stream)
               : brk_gather_rows(ctx, t->emb.w, t->emb.rows, t->E, ids, n, emb_out, stream);
   if (rc) return rc;
+  if (m > 0) {
+    float* dst = emb_out + n * t->E;
+    rc = sh ? brk_gather_rows_sharded(ctx, sh, t->E, extra, m, dst, stream)
+            : brk_gather_rows(ctx, t->emb.w, t->emb.rows, t->E, extra, m, dst, stream);
+    if (rc) return rc;
+  }
   const float* W = t->dense.w;                       // [E, S] Keras kernel, then bias [S]
-  return gemm(ctx, (cudaStream_t)stream, tcore, emb_out, W, out, W + int64_t(t->E) * t->S, int(n), t->S, t->E, t->E, t->S,
-              t->S, 0, 0, 1.f, 0, false);
+  return gemm(ctx, (cudaStream_t)stream, tcore, emb_out, W, out, W + int64_t(t->E) * t->S, int(n + m), t->S, t->E, t->E,
+              t->S, t->S, 0, 0, 1.f, 0, false);
 }
 
 extern "C" int brk_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t* ids, int64_t n, float* emb_out,
@@ -335,21 +399,34 @@ extern "C" int brk_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t
 // gathered from and their gradients scattered into the row-sharded tables sh instead of user->emb / item->emb.
 // rt != nullptr (unsharded, softmax mode only): the retrieval options, brk_twotower_step_retrieval; srt != nullptr
 // (sharded, softmax mode only): brk_twotower_step_sharded_retrieval.
+static int launch_sampler(const brk_tt_sampled* smp, cudaStream_t st) {
+  tt_sample_negatives_kernel<<<1, 1024, 0, st>>>(smp->ids, int(smp->count), int32_t(smp->lo), uint32_t(smp->hi - smp->lo),
+                                                 smp->seed, smp->replica, reinterpret_cast<long long*>(smp->step));
+  BRK_LAUNCH_CHECK();
+  return 0;
+}
+
+// smp != nullptr (softmax mode, training, no probabilities or estimator in rt / srt): sampled negatives -- the draws are
+// made first, the item side of every buffer and product has n = B + M rows, the scores are [B, n].
+// drawn: the caller has launched the sampler already (the train step, after its one-launch attempt).
 static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const brk_twotower_shards* sh,
                          const int32_t* u, const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                          int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out, void* stream,
-                         const brk_tt_retrieval* rt = nullptr, const brk_tt_retrieval_sharded* srt = nullptr) {
+                         const brk_tt_retrieval* rt = nullptr, const brk_tt_retrieval_sharded* srt = nullptr,
+                         const brk_tt_sampled* smp = nullptr, bool drawn = false) {
   // mode bit 8 (0x100): Dense / in-batch products on the tensor cores (TF32 operands, gemm_tc.cu)
   const int tcore = (mode & 0x100) ? 1 : 0;
   mode &= 0xFF;
   cudaStream_t st = (cudaStream_t)stream;
   const int B = int(batch), S = user->S, Eu = user->E, Ei = item->E;
+  const int M = smp ? int(smp->count) : 0, n = B + M;
   const brk_shards* tsh[2] = {sh ? &sh->user : nullptr, sh ? &sh->item : nullptr};
   int rc;
+  if (smp && !drawn && (rc = launch_sampler(smp, st))) return rc;
   if (mode == 0 && tcore) {                         // the whole step as one cooperative launch when the batch fits on chip
     int handled = 0;
     if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, training, ws, loss_out, st, &handled, 0, 0.f, 0.f,
-                                      sh, rt, srt))) return rc;
+                                      sh, rt, srt, smp))) return rc;
     if (handled) return 0;
   }
   // The user chain and the item chain are independent until the score product and again after the loss gradient, and
@@ -392,16 +469,24 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
     }
   }
   BRK_FORK(ctx, st, 0);
-  if (training && mode == 0) BRK_CUDA(cudaMemsetAsync(dz[1], 0, size_t(B) * S * sizeof(float), fk));   // RED targets of
-  if ((rc = tower_forward(ctx, item, i, batch, ws->ei, ws->c, tcore, fk, tsh[1]))) return rc;            // the split-K
+  if (training && mode == 0) BRK_CUDA(cudaMemsetAsync(dz[1], 0, size_t(n) * S * sizeof(float), fk));   // RED targets of
+  if ((rc = tower_forward(ctx, item, i, batch, ws->ei, ws->c, tcore, fk, tsh[1], smp ? smp->ids : nullptr, M)))
+    return rc;                                                                                           // the split-K
   if (training && mode == 0) BRK_CUDA(cudaMemsetAsync(dz[0], 0, size_t(B) * S * sizeof(float), st));   // products below
   if ((rc = tower_forward(ctx, user, u, batch, ws->eu, ws->q, tcore, stream, tsh[0]))) return rc;
   BRK_JOIN(ctx, st, 0);
   if (mode == 0) {
-    // scores = q c^T; softmax CE (SUM) with accidental-hit removal; in place P = softmax - I
-    if ((rc = gemm(ctx, st, tcore, ws->q, ws->c, ws->scores, nullptr, B, B, S, S, S, B, 0, 1, 1.f, 0, false))) return rc;
-    if (rt || srt) inbatch_softmax_kernel<true><<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc, so);
-    else inbatch_softmax_kernel<<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc);
+    // scores = q c^T [B, n]; softmax CE (SUM) with accidental-hit removal; in place P = softmax - I
+    if ((rc = gemm(ctx, st, tcore, ws->q, ws->c, ws->scores, nullptr, B, n, S, S, S, n, 0, 1, 1.f, 0, false))) return rc;
+    if (smp) {
+      const float* w = rt ? rt->row_weight : (srt ? srt->row_weight : nullptr);
+      const float inv_tau = rt ? rt->inv_temperature : (srt ? srt->inv_temperature : 1.f);
+      sampled_softmax_kernel<<<B, 256, 0, st>>>(ws->scores, i, smp->ids, B, n, ws->acc, inv_tau, w);
+    } else if (rt || srt) {
+      inbatch_softmax_kernel<true><<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc, so);
+    } else {
+      inbatch_softmax_kernel<<<B, 256, 0, st>>>(ws->scores, cand_ids, B, training, ws->acc);
+    }
     BRK_LAUNCH_CHECK();
   } else {
     rowdot_bce_kernel<<<(B * 32 + 255) / 256, 256, 0, st>>>(ws->q, ws->c, labels, B, S, training, ws->dq, ws->dc, ws->acc);
@@ -424,17 +509,20 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
   const float* other[2] = {ws->c, ws->q};
   const int32_t* ids[2] = {u, i};
   const int E[2] = {Eu, Ei};
+  const int rows[2] = {B, n};                      // the item side has the sampled rows after the batch's
   for (int k = 0; k < 2; ++k) {
     cudaStream_t sk = k == 0 ? st : fk;
     cudaStream_t sd = wide ? ctx->fork_stream[1 + k] : sk;
-    if (mode == 0) {
-      if ((rc = gemm(ctx, sk, tcore, ws->scores, other[k], dz[k], nullptr, B, S, B, B, S, S, k, 0, 1.f, 1, true))) return rc;
+    const int R = rows[k];
+    if (mode == 0) {   // k = 0: dq = P c [B, S] (K = n); k = 1: dc = P^T q [n, S] (K = B); P is [B, n], ld n
+      if ((rc = gemm(ctx, sk, tcore, ws->scores, other[k], dz[k], nullptr, R, S, rows[1 - k], n, S, S, k, 0, 1.f, 1, true)))
+        return rc;
     }
     if (wide) BRK_FORK(ctx, sk, 1 + k);
     float* gW = tw[k]->dense.g;
     float* gb = gW + int64_t(E[k]) * S;
-    if ((rc = gemm(ctx, sd, tcore, e[k], dz[k], gW, nullptr, E[k], S, B, E[k], S, S, 1, 0, 1.f, 1, true))) return rc;
-    colsum_kernel<<<dim3((S + 127) / 128, (B + 63) / 64), 128, 0, sd>>>(dz[k], B, S, S, gb);
+    if ((rc = gemm(ctx, sd, tcore, e[k], dz[k], gW, nullptr, E[k], S, R, E[k], S, S, 1, 0, 1.f, 1, true))) return rc;
+    colsum_kernel<<<dim3((S + 127) / 128, (R + 63) / 64), 128, 0, sd>>>(dz[k], R, S, S, gb);
     BRK_LAUNCH_CHECK();
     if (k == 0) {                                  // the loss scalar rides on the user tower's side stream
       finish_loss_kernel<<<1, 1, 0, sd>>>(ws->acc, loss_out);
@@ -442,11 +530,16 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
     }
     // de = dz W^T: W stored [E,S] = "B stored [N,K]" with N = E, K = S  (tb = 1); its own buffer: the dW product
     // beside it is still reading the gathered rows e
-    if ((rc = gemm(ctx, sk, tcore, dz[k], tw[k]->dense.w, de[k], nullptr, B, E[k], S, S, S, E[k], 0, 1, 1.f, 0, false))) return rc;
-    rc = tsh[k] ? brk_scatter_add_rows_sharded(ctx, tsh[k], E[k], ids[k], batch, de[k], (void*)sk)
-                : brk_scatter_add_rows(ctx, tw[k]->emb.g, tw[k]->emb.rows, E[k], ids[k], batch, de[k], tw[k]->emb.touched, 0,
-                                       (void*)sk);
-    if (rc) return rc;
+    if ((rc = gemm(ctx, sk, tcore, dz[k], tw[k]->dense.w, de[k], nullptr, R, E[k], S, S, S, E[k], 0, 1, 1.f, 0, false))) return rc;
+    for (int part = 0; part < (k == 1 && smp ? 2 : 1); ++part) {   // the batch's rows, then the sampled rows
+      const int32_t* pid = part ? smp->ids : ids[k];
+      const int64_t cnt = part ? M : batch;
+      const float* val = de[k] + (part ? int64_t(B) * E[k] : 0);
+      rc = tsh[k] ? brk_scatter_add_rows_sharded(ctx, tsh[k], E[k], pid, cnt, val, (void*)sk)
+                  : brk_scatter_add_rows(ctx, tw[k]->emb.g, tw[k]->emb.rows, E[k], pid, cnt, val, tw[k]->emb.touched, 0,
+                                         (void*)sk);
+      if (rc) return rc;
+    }
     if (wide) BRK_JOIN(ctx, sk, 1 + k);
   }
   BRK_JOIN(ctx, st, 0);
@@ -468,10 +561,52 @@ static int check_retrieval(const brk_tower* item, int32_t mode, const brk_tt_ret
   return 0;
 }
 
+// The checks that every sampled-negatives entry point shares (brk_tt_sampled).  item_rows < 0: the sharded step, which
+// only has smp->rows.  cand_prob / has_est: what rt carries beside temperature and weights.
+static int check_sampled(const brk_tt_sampled* smp, int32_t mode, int64_t batch, int64_t item_rows, const float* cand_prob,
+                         bool has_est, float inv_temperature, const char* fn) {
+  BRK_REQUIRE(smp, BRK_E_ARG, "%s: null sampled-negatives argument", fn);
+  BRK_REQUIRE(smp->count >= 1 && smp->count < (1 << 30), BRK_E_ARG, "%s: sampled count M = %lld (at least 1)", fn,
+              (long long)smp->count);
+  BRK_REQUIRE(smp->ids && smp->step, BRK_E_ARG, "%s: sampled negatives need an ids buffer [M] and a step counter", fn);
+  BRK_REQUIRE(item_rows < 0 || smp->rows == item_rows, BRK_E_ARG, "%s: sampled rows = %lld, the item table has %lld", fn,
+              (long long)smp->rows, (long long)item_rows);
+  BRK_REQUIRE(smp->lo >= 0 && smp->lo < smp->hi && smp->hi <= smp->rows && smp->rows < (int64_t(1) << 31), BRK_E_ARG,
+              "%s: sampled range [%lld, %lld) is empty or outside the item table's %lld rows", fn, (long long)smp->lo,
+              (long long)smp->hi, (long long)smp->rows);
+  BRK_REQUIRE((mode & 0xFF) == 0, BRK_E_ARG, "%s: sampled negatives need the in-batch softmax (rdZero mode has no "
+              "candidates)", fn);
+  BRK_REQUIRE(!cand_prob && !has_est, BRK_E_ARG, "%s: candidate probabilities and the streaming estimator are not offered "
+              "with sampled negatives (the logQ correction of a mixed pool needs both routes' probabilities)", fn);
+  BRK_REQUIRE(std::isfinite(inv_temperature) && inv_temperature > 0.f, BRK_E_ARG,
+              "%s: 1 / temperature = %g is not finite and > 0", fn, double(inv_temperature));
+  BRK_REQUIRE(batch >= 0 && batch < (1 << 30) && batch * (batch + smp->count) < (int64_t(1) << 31), BRK_E_ARG,
+              "%s: score matrix [%lld, %lld] has 2^31 or more entries", fn, (long long)batch,
+              (long long)(batch + smp->count));
+  return 0;
+}
+
+// batch == 0 with sampled negatives: the draws still advance the counter, the loss is 0
+static int sampled_empty_step(const brk_tt_sampled* smp, float* loss_out, cudaStream_t st) {
+  int rc;
+  if ((rc = launch_sampler(smp, st))) return rc;
+  if (loss_out) BRK_CUDA(cudaMemsetAsync(loss_out, 0, sizeof(float), st));
+  return 0;
+}
+
 static int twotower_step_checked(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
                                  const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                                  int32_t mode, int32_t training, const brk_twotower_workspace* ws, float* loss_out,
-                                 void* stream, const brk_tt_retrieval* rt) {
+                                 void* stream, const brk_tt_retrieval* rt, const brk_tt_sampled* smp = nullptr,
+                                 bool drawn = false) {
+  if (smp) {
+    static const char* fn = "brk_twotower_step_sampled";
+    BRK_REQUIRE(ctx && user && item && ws, BRK_E_ARG, "%s: null argument", fn);
+    int rc;
+    if ((rc = check_sampled(smp, mode, batch, item->emb.rows, rt ? rt->cand_prob : nullptr, rt && rt->last,
+                            rt ? rt->inv_temperature : 1.f, fn))) return rc;
+    if (batch == 0) return sampled_empty_step(smp, loss_out, (cudaStream_t)stream);
+  }
   BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_step: null argument");
   BRK_REQUIRE(user->S == item->S && batch > 0 && batch < (1 << 30), BRK_E_ARG, "brk_twotower_step: S %d vs %d, batch %lld",
               user->S, item->S, (long long)batch);
@@ -484,7 +619,15 @@ static int twotower_step_checked(brk_ctx* ctx, const brk_tower* user, const brk_
     int rc;
     if ((rc = check_retrieval(item, mode, rt, "brk_twotower_step_retrieval"))) return rc;
   }
-  return twotower_step(ctx, user, item, nullptr, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream, rt);
+  return twotower_step(ctx, user, item, nullptr, u, i, cand_ids, labels, batch, mode, training, ws, loss_out, stream, rt,
+                       nullptr, smp, drawn);
+}
+
+extern "C" int brk_twotower_step_sampled(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                         const int32_t* i, int64_t batch, int32_t mode, const brk_twotower_workspace* ws,
+                                         float* loss_out, void* stream, const brk_tt_sampled* smp, const brk_tt_retrieval* rt) {
+  BRK_REQUIRE(smp, BRK_E_ARG, "brk_twotower_step_sampled: null sampled-negatives argument");
+  return twotower_step_checked(ctx, user, item, u, i, i, nullptr, batch, mode, 1, ws, loss_out, stream, rt, smp);
 }
 
 extern "C" int brk_twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
@@ -574,6 +717,29 @@ extern "C" int brk_twotower_step_sharded_retrieval(brk_ctx* ctx, const brk_tower
   return twotower_step_sharded_checked(ctx, user, item, sh, u, i, cand_ids, labels, batch, mode, ws, loss_out, stream, rt);
 }
 
+extern "C" int brk_twotower_step_sharded_sampled(brk_ctx* ctx, const brk_tower* user, const brk_tower* item,
+                                                 const brk_twotower_shards* sh, const int32_t* u, const int32_t* i,
+                                                 int64_t batch, int32_t mode, const brk_twotower_workspace* ws, float* loss_out,
+                                                 void* stream, const brk_tt_sampled* smp, const brk_tt_retrieval_sharded* rt) {
+  static const char* fn = "brk_twotower_step_sharded_sampled";
+  int rc;
+  if ((rc = check_sampled(smp, mode, batch, -1, rt ? rt->cand_prob : nullptr, rt && rt->est, rt ? rt->inv_temperature : 1.f,
+                          fn))) return rc;
+  BRK_REQUIRE(ctx && user && item && ws && sh, BRK_E_ARG, "%s: null argument", fn);
+  if ((rc = check_shards(&sh->user, user->E, "user", fn))) return rc;
+  if ((rc = check_shards(&sh->item, item->E, "item", fn))) return rc;
+  if (batch == 0) return sampled_empty_step(smp, loss_out, (cudaStream_t)stream);
+  BRK_REQUIRE(u && i, BRK_E_ARG, "%s: null ids", fn);
+  BRK_REQUIRE(sh->user.world == sh->item.world && sh->user.rank == sh->item.rank, BRK_E_ARG,
+              "%s: user / item shards of different worlds or ranks", fn);
+  BRK_REQUIRE(user->S == item->S, BRK_E_ARG, "%s: S %d vs %d", fn, user->S, item->S);
+  BRK_REQUIRE(ws->eu && ws->ei && ws->q && ws->c && ws->dq && ws->dc && ws->acc && ws->deu && ws->dei && ws->scores, BRK_E_ARG,
+              "%s: workspace missing", fn);
+  BRK_REQUIRE(user->dense.w && item->dense.w && user->dense.g && item->dense.g, BRK_E_ARG,
+              "%s: Dense blocks or their gradients missing", fn);
+  return twotower_step(ctx, user, item, sh, u, i, i, nullptr, batch, mode, 1, ws, loss_out, stream, nullptr, rt, smp);
+}
+
 extern "C" int brk_tt_estimator_update_sharded(brk_ctx* ctx, const brk_tt_estimator_sharded* est, const int32_t* ids,
                                                int64_t n, float alpha, int64_t* step, void* stream) {
   static const char* fn = "brk_tt_estimator_update_sharded";
@@ -627,20 +793,42 @@ int brk_tt_check_shards(const brk_shards* s, int32_t E, const char* which, const
 static int twotower_train_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
                                const int32_t* i, const int32_t* cand_ids, const float* labels, int64_t batch,
                                int32_t mode, const brk_twotower_workspace* ws, float lr, float eps,
-                               int64_t rows_threshold_bytes, float* loss_out, void* stream, const brk_tt_retrieval* rt) {
-  BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_train_step: null argument");
-  cudaStream_t st = (cudaStream_t)stream;
+                               int64_t rows_threshold_bytes, float* loss_out, void* stream, const brk_tt_retrieval* rt,
+                               const brk_tt_sampled* smp = nullptr) {
   int rc;
-  if (rt && (rc = check_retrieval(item, mode, rt, "brk_twotower_train_step_retrieval"))) return rc;
-  if ((mode & 0xFF) == 0 && (mode & 0x100) && user->S == item->S && batch > 0 && batch < (1 << 30) && ws->q && ws->c && ws->dq &&
-      ws->dc && ws->acc && user->emb.g && item->emb.g && user->dense.g && item->dense.g) {
-    int handled = 0;
-    if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps, nullptr,
-                                      rt, nullptr)))
+  if (smp) {          // the draws, then the one launch with Adagrad when it fits, else the multi-kernel step
+    static const char* fn = "brk_twotower_train_step_sampled";
+    BRK_REQUIRE(ctx && user && item && ws, BRK_E_ARG, "%s: null argument", fn);
+    if ((rc = check_sampled(smp, mode, batch, item->emb.rows, rt ? rt->cand_prob : nullptr, rt && rt->last,
+                            rt ? rt->inv_temperature : 1.f, fn))) return rc;
+    if (batch == 0) return sampled_empty_step(smp, loss_out, (cudaStream_t)stream);
+    BRK_REQUIRE(u && i, BRK_E_ARG, "%s: null ids", fn);
+    if ((rc = launch_sampler(smp, (cudaStream_t)stream))) return rc;
+    if ((mode & 0x100) && user->S == item->S && ws->q && ws->c && ws->dq && ws->dc && ws->acc && user->emb.g && item->emb.g &&
+        user->dense.g && item->dense.g) {
+      int handled = 0;
+      if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, i, batch, 1, ws, loss_out, (cudaStream_t)stream, &handled, 1, lr,
+                                        eps, nullptr, rt, nullptr, smp)))
+        return rc;
+      if (handled) return 0;
+    }
+    if ((rc = twotower_step_checked(ctx, user, item, u, i, i, labels, batch, mode, 1, ws, loss_out, stream, rt, smp, true)))
       return rc;
-    if (handled) return 0;
+  } else {
+    BRK_REQUIRE(ctx && user && item && u && i && ws, BRK_E_ARG, "brk_twotower_train_step: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (rt && (rc = check_retrieval(item, mode, rt, "brk_twotower_train_step_retrieval"))) return rc;
+    if ((mode & 0xFF) == 0 && (mode & 0x100) && user->S == item->S && batch > 0 && batch < (1 << 30) && ws->q && ws->c &&
+        ws->dq && ws->dc && ws->acc && user->emb.g && item->emb.g && user->dense.g && item->dense.g) {
+      int handled = 0;
+      if ((rc = brk_twotower_step_fused(ctx, user, item, u, i, cand_ids, batch, 1, ws, loss_out, st, &handled, 1, lr, eps,
+                                        nullptr, rt, nullptr, nullptr)))
+        return rc;
+      if (handled) return 0;
+    }
+    if ((rc = twotower_step_checked(ctx, user, item, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream, rt)))
+      return rc;
   }
-  if ((rc = twotower_step_checked(ctx, user, item, u, i, cand_ids, labels, batch, mode, 1, ws, loss_out, stream, rt))) return rc;
   brk_table dense_pass[4], rows_pass[2];
   int nd = 0, nr = 0;
   const brk_tower* tw[2] = {user, item};
@@ -670,4 +858,13 @@ extern "C" int brk_twotower_train_step_retrieval(brk_ctx* ctx, const brk_tower* 
                                                  const brk_tt_retrieval* rt) {
   return twotower_train_step(ctx, user, item, u, i, cand_ids, labels, batch, mode, ws, lr, eps, rows_threshold_bytes, loss_out,
                              stream, rt);
+}
+
+extern "C" int brk_twotower_train_step_sampled(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                               const int32_t* i, int64_t batch, int32_t mode, const brk_twotower_workspace* ws,
+                                               float lr, float eps, int64_t rows_threshold_bytes, float* loss_out, void* stream,
+                                               const brk_tt_sampled* smp, const brk_tt_retrieval* rt) {
+  BRK_REQUIRE(smp, BRK_E_ARG, "brk_twotower_train_step_sampled: null sampled-negatives argument");
+  return twotower_train_step(ctx, user, item, u, i, i, nullptr, batch, mode, ws, lr, eps, rows_threshold_bytes, loss_out,
+                             stream, rt, smp);
 }

@@ -38,6 +38,13 @@
 // touched bits go to the owner's accumulator and bitmask.  Phase O does not run: an owner's accumulator is complete only
 // after a cross-GPU barrier and the Dense gradients only after their all-reduce, so the launch ends after phase G.
 //
+// fused_step<false, true, true> / fused_step<true, true, true> are the two steps with sampled negatives (brk_tt_sampled,
+// drawn by tt_sample_negatives_kernel ahead of the launch): the item side has n = B + M rows (the batch's, then the draws)
+// in Tc = ceil(n / 128) row blocks.  Phase F runs T + Tc row blocks, phase S T * Tc score tiles (the identity of P only in
+// tiles with j < T -- the diagonal tiles -- and columns >= n dropped), phase G 2 (T + Tc) tower blocks, and phase O also
+// walks the sampled rows.  Temperature and weights go where fused_step<false, true> puts them; no probabilities.  The
+// launch needs max(T * Tc, 2 (T + Tc)) <= SM count.
+//
 // fused_step<true, true> is the row-sharded step with the options (brk_twotower_step_sharded_retrieval).  The estimator's
 // state is sharded like the item table and only read here: its update is brk_tt_estimator_update_sharded, a launch of its
 // own that every rank runs before a cross-GPU barrier.  Phase S reads the gap of column j's item row y at its owner,
@@ -96,8 +103,13 @@ struct ShardedRetrievalParams : ShardedParams {
   const float* gap[BRK_MAX_PEERS];                                   // gap[0] == null: no estimator
   float inv_tau;
 };
-template <bool SH, bool RT> using KParamsT =
-    typename std::conditional<RT, typename std::conditional<SH, ShardedRetrievalParams, RetrievalParams>::type, ParamsT<SH>>::type;
+// fused_step<SH, true, true>: sampled negatives (brk_tt_sampled) behind the options block (no probabilities, no estimator):
+// the item side has n = B + M rows, item row x is ids[1][x] for x < B and smp[x - B] after, Tc = ceil(n / 128)
+struct SampledParams : RetrievalParams { const int32_t* smp; int M, n, Tc; };
+struct ShardedSampledParams : ShardedRetrievalParams { const int32_t* smp; int M, n, Tc; };
+template <bool SH, bool RT, bool SM = false> using KParamsT = typename std::conditional<SM,
+    typename std::conditional<SH, ShardedSampledParams, SampledParams>::type,
+    typename std::conditional<RT, typename std::conditional<SH, ShardedRetrievalParams, RetrievalParams>::type, ParamsT<SH>>::type>::type;
 // the estimator's gap of item row y as phase S reads it (after the F -> S barrier, past L1)
 __device__ __forceinline__ bool has_estimator(const RetrievalParams& P) { return P.last != nullptr; }
 __device__ __forceinline__ bool has_estimator(const ShardedRetrievalParams& P) { return P.gap[0] != nullptr; }
@@ -207,8 +219,20 @@ __device__ __forceinline__ void stage_ids(const ParamsT<SH>& P, int k, int r0, i
   }
 }
 
-template <bool SH, bool RT = false>
-__global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
+// ids_s[t] <- item row r0 + t of the sampled step's n = B + M item rows (the batch's, then the draws)
+template <bool SH, class PT>
+__device__ __forceinline__ void stage_item_ids(const PT& P, int r0, int valid, int32_t* ids_s, int32_t* own_s) {
+  const int t = threadIdx.x;
+  if (t < TS) {
+    const int x = r0 + t;
+    const int32_t id = t < valid ? (x < P.B ? __ldg(P.ids[1] + x) : __ldg(P.smp + (x - P.B))) : 0;
+    if constexpr (SH) { ids_s[t] = id / P.su.world; own_s[t] = id % P.su.world; }
+    else ids_s[t] = id;
+  }
+}
+
+template <bool SH, bool RT = false, bool SM = false>
+__global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT, SM> P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* buf0 = sm; uint8_t* buf1 = sm + TILE; uint8_t* buf2 = sm + 2 * TILE;
@@ -222,6 +246,8 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   __shared__ double red[32];
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int T = P.T, B = P.B, S = P.S;
+  int n = B, Tc = T;                                                    // item-side rows and row blocks
+  if constexpr (SM) { n = P.n; Tc = P.Tc; }
   const int b = blockIdx.x;
   stamp(P, 0);
   if (t == 0) { tc::mbar_init(tc::smem_u32(&mbar), 1); tc::fence_barrier_init(); }
@@ -241,13 +267,24 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   // ---------------- phase F: the two towers ----------------
   if (P.training) {                                                     // RED targets of phase S
     const int64_t n4 = int64_t(B) * S / 4;
-    for (int k = 0; k < 2; ++k)
-      for (int64_t x = int64_t(b) * NT + t; x < n4; x += int64_t(gridDim.x) * NT) reinterpret_cast<float4*>(P.dz[k])[x] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if constexpr (SM) {
+      for (int k = 0; k < 2; ++k) {
+        const int64_t nk4 = int64_t(k ? n : B) * S / 4;
+        for (int64_t x = int64_t(b) * NT + t; x < nk4; x += int64_t(gridDim.x) * NT) reinterpret_cast<float4*>(P.dz[k])[x] = make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    } else {
+      for (int k = 0; k < 2; ++k)
+        for (int64_t x = int64_t(b) * NT + t; x < n4; x += int64_t(gridDim.x) * NT) reinterpret_cast<float4*>(P.dz[k])[x] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
   }
-  if (b < 2 * T) {
-    const int k = b / T, r0 = (b % T) * TS, valid = min(TS, B - r0), E = P.E[k];
+  if (b < (SM ? T + Tc : 2 * T)) {
+    int k, r0, valid;
+    if constexpr (SM) { k = b < T ? 0 : 1; r0 = (b - k * T) * TS; valid = min(TS, (k ? n : B) - r0); }
+    else { k = b / T; r0 = (b % T) * TS; valid = min(TS, B - r0); }
+    const int E = P.E[k];
     const brk_table& tab = k == 0 ? P.eu : P.ei;
-    stage_ids<SH>(P, k, r0, valid, ids_s, own_s);
+    if constexpr (SM) { if (k == 1) stage_item_ids<SH>(P, r0, valid, ids_s, own_s); else stage_ids<SH>(P, k, r0, valid, ids_s, own_s); }
+    else stage_ids<SH>(P, k, r0, valid, ids_s, own_s);
     if constexpr (RT && !SH) {                                          // Yi et al. Algorithm 2: the thread whose exchange
       if (k == 1 && P.last && P.training && t < valid) {                // saw another step is the sole updater of y
         const int32_t y = ids_s[t];
@@ -288,8 +325,8 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   }
 
   // ---------------- phase S: one score tile per CTA ----------------
-  const bool tile_cta = b < T * T;
-  const int ti = b / T, tj = b % T;
+  const bool tile_cta = b < T * Tc;
+  const int ti = b / Tc, tj = b % Tc;
   const int r = (warp & 3) * 32 + lane, h = warp >> 2;                  // this thread's tile row and column half
   const int ig = ti * TS + r;
   float pv[64];                                                         // S_ij, then P_ij: row r, columns [h * 64, h * 64 + 64)
@@ -297,11 +334,12 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   const int diag_k = (ti == tj) ? r - h * 64 : -1;                      // this thread's diagonal column, if it has one
   if (tile_cta) {
     load_tile<0>(buf0, P.z[0], S, ti * TS, B, S);                       // q_i [M][K = S]
-    load_tile<0>(buf1, P.z[1], S, tj * TS, B, S);                       // c_j [N][K = S]
+    load_tile<0>(buf1, P.z[1], S, tj * TS, n, S);                       // c_j [N][K = S]
     cp_async_commit();
     if (t < TS) {
       cand_r[t] = (P.cand && ti * TS + t < B) ? __ldg(P.cand + ti * TS + t) : -1;
       cand_c[t] = (P.cand && tj * TS + t < B) ? __ldg(P.cand + tj * TS + t) : -2;
+      if constexpr (SM) { const int j = tj * TS + t; if (P.cand && j >= B && j < n) cand_c[t] = __ldg(P.smp + (j - B)); }
       if constexpr (RT) {                                               // the estimator's gap is read after the F -> S barrier
         const int j = tj * TS + t;
         float l2 = 0.f;
@@ -328,7 +366,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
     // per score: P_k = e_k * 2^(m - lse).
     tmem_load64(tmem, warp, h * 64, pv);
     const int32_t my_id = cand_r[r];
-    const int ncol = B - tj * TS - h * 64;                              // valid columns of this half (<= 0: none)
+    const int ncol = n - tj * TS - h * 64;                              // valid columns of this half (<= 0: none)
     const bool check = P.cand != nullptr;
     float m4[4] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
 #pragma unroll
@@ -360,10 +398,10 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
     if (h == 0) {
       const float m0 = pm[0][r], m1 = pm[1][r], M = fmaxf(m0, m1);
       const float Ms = M == -CUDART_INF_F ? 0.f : M;
-      P.part[int64_t(ig) * T + tj] = make_float2(M, ps[0][r] * ex2(m0 - Ms) + ps[1][r] * ex2(m1 - Ms));
+      P.part[int64_t(ig) * Tc + tj] = make_float2(M, ps[0][r] * ex2(m0 - Ms) + ps[1][r] * ex2(m1 - Ms));
     }
     if (P.training) {                                                   // the gradient products' B operands travel while the grid
-      load_tile<1>(buf0, P.z[1], S, tj * TS, B, S);                     // waits at the barrier: c_j [K = j][N = S]
+      load_tile<1>(buf0, P.z[1], S, tj * TS, n, S);                     // waits at the barrier: c_j [K = j][N = S]
       load_tile<1>(buf1, P.z[0], S, ti * TS, B, S);                     // q_i [K = i][N = S]
       cp_async_commit();
     }
@@ -372,7 +410,16 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
   brk_grid_barrier(P.bar, bar_target);
   stamp(P, 4);
   if (tile_cta) {
-    if (h == 0) {                                                       // log-sum-exp of the row over its T tiles (log2 domain)
+    if (SM && h == 0) {                                                 // Tc may exceed 12: two passes over the partials
+      float M = -CUDART_INF_F;
+      for (int k = 0; k < Tc; ++k) M = fmaxf(M, __ldcg(&P.part[int64_t(ig) * Tc + k]).x);
+      float sum = 0.f;
+      for (int k = 0; k < Tc; ++k) {
+        const float2 pk = __ldcg(&P.part[int64_t(ig) * Tc + k]);
+        if (pk.x != -CUDART_INF_F) sum += pk.y * ex2(pk.x - M);
+      }
+      lse_s[r] = M + __log2f(sum);
+    } else if (h == 0) {                                                // log-sum-exp of the row over its T tiles (log2 domain)
       float2 pp[12];                                                    // T <= 12 (T^2 <= SM count): one round trip for all of them
 #pragma unroll
       for (int k = 0; k < 12; ++k) pp[k] = k < T ? __ldcg(&P.part[int64_t(ig) * T + k]) : make_float2(-CUDART_INF_F, 0.f);
@@ -442,18 +489,22 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
       __syncthreads();
       for (int idx = t; idx < TS * 32; idx += NT) {
         const int rr = idx >> 5, c4 = idx & 31;
-        if (tj * TS + rr < B && c4 * 4 < S) red_add_f4(P.dz[1] + int64_t(tj * TS + rr) * S + c4 * 4, staging_ld(buf0, rr, c4));
+        if (tj * TS + rr < n && c4 * 4 < S) red_add_f4(P.dz[1] + int64_t(tj * TS + rr) * S + c4 * 4, staging_ld(buf0, rr, c4));
       }
       tc::fence_before_sync();
     }
   }
   // phase G's operands that do not depend on the barrier travel across it: the Dense kernel (rows job) or the embedding rows,
   // gathered again straight into the MN-major view (weights job)
-  const bool g_cta = P.training && b < 4 * T;
-  const int gk = b / (2 * T), g_r0 = ((b % (2 * T)) >> 1) * TS, g_valid = min(TS, B - g_r0), g_job = b & 1;
+  const bool g_cta = P.training && b < (SM ? 2 * (T + Tc) : 4 * T);
+  int gk, g_r0, g_valid;
+  if constexpr (SM) { gk = b < 2 * T ? 0 : 1; g_r0 = ((b - gk * 2 * T) >> 1) * TS; g_valid = min(TS, (gk ? n : B) - g_r0); }
+  else { gk = b / (2 * T); g_r0 = ((b % (2 * T)) >> 1) * TS; g_valid = min(TS, B - g_r0); }
+  const int g_job = b & 1;
   if (g_cta) {
     __syncthreads();                                                    // staging and operand tiles of the phase above are done with
-    stage_ids<SH>(P, gk, g_r0, g_valid, ids_s, own_s);
+    if constexpr (SM) { if (gk == 1) stage_item_ids<SH>(P, g_r0, g_valid, ids_s, own_s); else stage_ids<SH>(P, gk, g_r0, g_valid, ids_s, own_s); }
+    else stage_ids<SH>(P, gk, g_r0, g_valid, ids_s, own_s);
     if (g_job == 0) {
       load_tile<0>(buf1, P.W[gk], S, 0, P.E[gk], S);
     } else {
@@ -477,7 +528,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
     const brk_table& tab = k == 0 ? P.eu : P.ei;
     if (job == 0) {
       // de = dz W^T : A = dz [M = samples][K = S] K-major, B = W [N = E][K = S] K-major -> REDs into the rows' accumulators
-      load_tile<0>(buf0, P.dz[k], S, r0, B, S);
+      load_tile<0>(buf0, P.dz[k], S, r0, SM && k ? n : B, S);
       cp_async_commit();
       TTF_OPERANDS_READY();
       if (t == 0) {
@@ -504,7 +555,7 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
       }
     } else {
       // dW += e^T dz : A = e [K = samples][M = E] MN-major (gathered again, straight into that view), B = dz [K][N = S] MN-major
-      load_tile<1>(buf1, P.dz[k], S, r0, B, S);
+      load_tile<1>(buf1, P.dz[k], S, r0, SM && k ? n : B, S);
       cp_async_commit();
       TTF_OPERANDS_READY();
       if (t == 0) {
@@ -536,15 +587,17 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
     // the warp walks its run, two rows' loads in flight, E/4 lanes per row
     {
       const int nwarps = int(gridDim.x) * (NT / 32), gw = b * (NT / 32) + warp;
-      const int per = (2 * B + nwarps - 1) / nwarps;                    // <= 32: 2B <= 8 * 32 * max(T^2, 4T)
+      const int npairs = SM ? B + n : 2 * B;                            // SM: the sampled rows after the batch's
+      const int per = (npairs + nwarps - 1) / nwarps;                   // <= 32: 2B <= 8 * 32 * max(T^2, 4T)
       const int x = gw * per + lane;
-      const bool mine = lane < per && x < 2 * B;
+      const bool mine = lane < per && x < npairs;
       const int k = x >= B ? 1 : 0;
       int64_t row = 0;
       uint32_t own = 0u;
       if (mine) {
         const brk_table& tab = k == 0 ? P.eu : P.ei;
-        row = __ldg(P.ids[k] + (x - k * B));
+        if constexpr (SM) row = x < 2 * B ? __ldg(P.ids[k] + (x - k * B)) : __ldg(P.smp + (x - 2 * B));
+        else row = __ldg(P.ids[k] + (x - k * B));
         const uint32_t bit = 1u << (row & 31);
         own = atomicAnd(tab.touched + (row >> 5), ~bit) & bit;
       }
@@ -600,11 +653,14 @@ __global__ void __launch_bounds__(NT, 1) fused_step(const KParamsT<SH, RT> P) {
 int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u, const int32_t* i,
                             const int32_t* cand_ids, int64_t batch, int32_t training, const brk_twotower_workspace* ws,
                             float* loss_out, cudaStream_t st, int* handled, int do_opt, float lr, float eps,
-                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt, const brk_tt_retrieval_sharded* srt) {
+                            const brk_twotower_shards* sh, const brk_tt_retrieval* rt, const brk_tt_retrieval_sharded* srt,
+                            const brk_tt_sampled* smp) {
   using namespace ttf;
   *handled = 0;
   const int S = user->S, B = int(batch), T = (B + TS - 1) / TS;
-  const int need = T * T > 4 * T ? T * T : 4 * T;
+  // sampled negatives: the item side has n = B + M rows in Tc row blocks; T * Tc score tiles, 2 (T + Tc) tower blocks
+  const int n = smp ? B + int(smp->count) : B, Tc = (n + TS - 1) / TS;
+  const int need = smp ? (T * Tc > 2 * (T + Tc) ? T * Tc : 2 * (T + Tc)) : (T * T > 4 * T ? T * T : 4 * T);
   const int grid = need > ctx->sm_count ? need : ctx->sm_count;   // the CTAs without a tile share the zeroing and the optimizer phase
   if (getenv("BRK_TT_NO_FUSED")) return 0;
   if (S > 128 || user->E > 128 || item->E > 128 || (S & 3) || (user->E & 3) || (item->E & 3) || need > ctx->sm_count || T > 12) return 0;
@@ -623,17 +679,19 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
   if (!brk_aligned16(ws->q) || !brk_aligned16(ws->c) || (training && (!brk_aligned16(ws->dq) || !brk_aligned16(ws->dc)))) return 0;
   const size_t smem = 3 * size_t(TILE) + 1024;
   if (sh && rt) return 0;                                          // unsharded options on sharded tables: not a caller's call
-  const int kv = sh ? (srt ? 3 : 1) : (rt ? 2 : 0);
-  const void* kern = sh ? (srt ? (const void*)fused_step<true, true> : (const void*)fused_step<true>)
+  if (smp && !training) return 0;
+  const int kv = smp ? (sh ? 5 : 4) : (sh ? (srt ? 3 : 1) : (rt ? 2 : 0));
+  const void* kern = smp ? (sh ? (const void*)fused_step<true, true, true> : (const void*)fused_step<false, true, true>)
+                   : sh ? (srt ? (const void*)fused_step<true, true> : (const void*)fused_step<true>)
                         : (rt ? (const void*)fused_step<false, true> : (const void*)fused_step<false>);
   // the shared-memory opt-in is per device: set it for the current one; occupancy is a property of each instantiation,
   // queried once
   BRK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  static int per_sm[4] = {-1, -1, -1, -1};
+  static int per_sm[6] = {-1, -1, -1, -1, -1, -1};
   int& occ = per_sm[kv];
   if (occ < 0) BRK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
   if (grid > occ * ctx->sm_count) return 0;
-  const size_t part_floats = size_t(T) * TS * T * 2;
+  const size_t part_floats = size_t(T) * TS * Tc * 2;
   if (ctx->tt_part_floats < part_floats) {
     if (ctx->tt_part) BRK_CUDA(cudaFree(ctx->tt_part));
     ctx->tt_part = nullptr; ctx->tt_part_floats = 0;
@@ -678,7 +736,24 @@ int brk_twotower_step_fused(brk_ctx* ctx, const brk_tower* user, const brk_tower
     if (srt->est)
       for (int p = 0; p < srt->est->world; ++p) SR.gap[p] = srt->est->gap[p];
   }
-  void* args[] = {sh ? (srt ? (void*)&SR : (void*)&P) : (rt ? (void*)&R : (void*)static_cast<Params*>(&P))};
+  // sampled negatives: the options block with no probabilities or estimator (rejected by the callers), then the draws
+  SampledParams SM_;
+  ShardedSampledParams SSM;
+  memset(&SM_, 0, sizeof(SM_));
+  memset(&SSM, 0, sizeof(SSM));
+  if (smp) {
+    if (sh) {
+      static_cast<ShardedParams&>(SSM) = P;
+      SSM.row_weight = srt ? srt->row_weight : nullptr; SSM.inv_tau = srt ? srt->inv_temperature : 1.f;
+      SSM.smp = smp->ids; SSM.M = int(smp->count); SSM.n = n; SSM.Tc = Tc;
+    } else {
+      static_cast<Params&>(SM_) = static_cast<const Params&>(P);
+      SM_.row_weight = rt ? rt->row_weight : nullptr; SM_.inv_tau = rt ? rt->inv_temperature : 1.f;
+      SM_.smp = smp->ids; SM_.M = int(smp->count); SM_.n = n; SM_.Tc = Tc;
+    }
+  }
+  void* args[] = {smp ? (sh ? (void*)&SSM : (void*)&SM_)
+                      : sh ? (srt ? (void*)&SR : (void*)&P) : (rt ? (void*)&R : (void*)static_cast<Params*>(&P))};
   BRK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(NT), args, smem, st));
   *handled = 1;
   return 0;

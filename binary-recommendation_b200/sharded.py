@@ -34,7 +34,8 @@ from . import _native as N
 from . import distributed as D
 from . import hotpath as H
 from .NeuMFModel import NeuMFTopKIndex, NeuMFTopKIndexFP32
-from .twoTower import GlobalNegatives, Tower, TwoTowerModel, check_retrieval_options
+from .twoTower import (GlobalNegatives, SampledNegatives, Tower, TwoTowerModel, check_retrieval_options,
+                       check_sampled_options)
 
 
 def shard_rows(rows, G):
@@ -582,12 +583,21 @@ class ShardedTwoTowerNet:
     slice, a cross-GPU barrier, then every replica's step reads p_y = 1 / gap[y] at the owner -- so its state equals the
     single-process estimator's on the global batch bit for bit.  Not offered with rdZero or global_negatives.
 
+    sampledNegatives=M (brk_twotower_step_sharded_sampled): every training step draws M item rows uniformly from
+    [2, numItem + 2) and adds them as candidate columns of every row of the replica's slice, with temperature and weights
+    as above.  Each replica draws its own rows (Philox keyed by (seed, rank); rank 0 under emulation and at G = 1, so
+    `emulate=G` gives TwoTowerModel(sampledNegatives=M)'s result); the sampled rows are gathered from and their gradients
+    sent to their owners like the batch's.  The sampler's step counter is checkpointed as a replicated entry.  Not
+    offered with rdZero, global_negatives, cand_prob or streamingFrequency.
+
     Ids arrive as int32 table rows (already looked up).  full_init: {"user", "item": full tables [rows, E];
     "user_dense", "item_dense": flat Dense blocks as Tower.init_dense lays them out}; without it the tables are
     U(-0.05, 0.05) and the Dense blocks Glorot-uniform from Philox(seed + 77)."""
 
     def __init__(self, numUser, numItem, embedDim, semb, learning_rate=0.1, rdZero=False, tensor_cores=True, seed=42,
-                 device=None, emulate=0, full_init=None, global_negatives=False, temperature=None, streamingFrequency=None):
+                 device=None, emulate=0, full_init=None, global_negatives=False, temperature=None, streamingFrequency=None,
+                 sampledNegatives=None):
+        self.sampledNegatives = check_sampled_options(sampledNegatives, rdZero, global_negatives, streamingFrequency, False)
         if global_negatives and rdZero:
             raise ValueError("global_negatives needs the in-batch softmax: rdZero has no in-batch negatives")
         if streamingFrequency is False:
@@ -634,6 +644,8 @@ class ShardedTwoTowerNet:
             self.barrier = PeerBarrier(dev)
         self._global = GlobalNegatives(self.G, self.rank, E, S, dev, emulate=bool(self.emulate), barrier=self.barrier) \
             if self.global_negatives and self.G > 1 else None
+        self._smp = SampledNegatives(self.sampledNegatives, self.numItem + 2, seed, self.rank, dev) \
+            if self.sampledNegatives else None
         self._ws_batch = 0
 
     _workspace = TwoTowerModel._workspace               # the mirrored model's step buffers (same attribute names)
@@ -658,6 +670,8 @@ class ShardedTwoTowerNet:
         """brk_tt_retrieval_sharded of one step, or None without any option (the option-free step)."""
         if not self._retrieval and cand_prob is None and weights is None:
             return None
+        check_sampled_options(self.sampledNegatives or None, self.rdZero, self.global_negatives, self.streamingFrequency,
+                              cand_prob is not None)
         check_retrieval_options(self.rdZero, self.global_negatives, None, self.streamingFrequency, cand_prob is not None)
         cols = []
         for name, v in (("cand_prob", cand_prob), ("weights", weights)):
@@ -681,7 +695,17 @@ class ShardedTwoTowerNet:
         loss_out = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=dev)
         lib, ctx, st = N.lib(), N.ctx(dev), N.stream_ptr()
         rt = self._rt(B, cand_prob, weights)
-        if rt is not None:
+        if self._smp is not None:                           # every rank draws, an empty slice included
+            u, i = H._i32(u, "u"), H._i32(i, "i")
+            ws = self._workspace(max(B, 1))
+            ut, it = self._towers()
+            sh = self._shards()
+            smp = self._smp.c_struct()
+            N.check(lib.brk_twotower_step_sharded_sampled(ctx, C.byref(ut), C.byref(it), C.byref(sh), N.ptr(u), N.ptr(i), B,
+                                                          0x100 if self.tensor_cores else 0, C.byref(ws), N.ptr(loss_out), st,
+                                                          C.byref(smp), C.byref(rt) if rt is not None else None),
+                    "brk_twotower_step_sharded_sampled")
+        elif rt is not None:
             u, i = H._i32(u, "u"), H._i32(i, "i")
             if self._est is not None:
                 self._est.update(i)
@@ -787,7 +811,7 @@ class ShardedTwoTowerNet:
 
     # ---- checkpoint: shards of the tables and their accumulators, replicated Dense blocks and theirs ------------
     # With the estimator also its state: last / gap as row-sharded [rows, 1] entries (re-sharded across world sizes
-    # like the tables) and the step counter replicated.
+    # like the tables) and the step counter replicated.  With sampled negatives the sampler's step counter, replicated.
     def _estimator_shards(self):
         e = self._est
         if e is None:
@@ -800,6 +824,8 @@ class ShardedTwoTowerNet:
             rep[name], rep[name + "_m"] = t.w.view(-1), t.m.view(-1)
         if self._est is not None:
             rep["estimator_step"] = self._est.step
+        if self._smp is not None:
+            rep["sampler_step"] = self._smp.step
         extra = {name: (shard, self._est.rows) for name, shard in self._estimator_shards().items()}
         return save_sharded_model(dirpath, {"user": self.user, "item": self.item}, rep, self.G, self.rank, self.emulate,
                                   meta={"model": "ShardedTwoTowerNet", "E": self.embedDim, "S": self.semb,
@@ -816,6 +842,8 @@ class ShardedTwoTowerNet:
             t.m.view(-1).copy_(torch.from_numpy(rep[name + "_m"]))
         if self._est is not None:
             self._est.step.fill_(int(rep["estimator_step"][0]) if "estimator_step" in rep else 0)
+        if self._smp is not None:                           # a checkpoint saved without sampled negatives: counter 0
+            self._smp.step.fill_(int(rep["sampler_step"][0]) if "sampler_step" in rep else 0)
         return meta
 
 

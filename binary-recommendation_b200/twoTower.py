@@ -229,10 +229,55 @@ def check_retrieval_options(rdZero, global_negatives, temperature, streamingFreq
     return alpha
 
 
+def check_sampled_options(sampledNegatives, rdZero, global_negatives, streamingFrequency, candidate_probs):
+    """The checks of sampled negatives that TwoTowerModel and sharded.ShardedTwoTowerNet share (ValueError).  Returns M,
+    the number of rows drawn per step (0: none).  candidate_probs: the caller also supplies candidate probabilities."""
+    if sampledNegatives is None or sampledNegatives is False:
+        return 0
+    if isinstance(sampledNegatives, bool) or int(sampledNegatives) != sampledNegatives or int(sampledNegatives) < 1:
+        raise ValueError(f"sampledNegatives must be an integer >= 1 (rows drawn per step), got {sampledNegatives!r}")
+    if rdZero:
+        raise ValueError("sampledNegatives needs the in-batch softmax: rdZero has no candidate columns")
+    if global_negatives:
+        raise ValueError("sampledNegatives is not offered with global_negatives: the draws would have to be published "
+                         "with the peers' candidate blocks")
+    if streamingFrequency is not None and streamingFrequency is not False:
+        raise ValueError("sampledNegatives is not offered with streamingFrequency: the logQ correction of a mixed pool needs "
+                         "each sampled column's probability under both routes")
+    if candidate_probs:
+        raise ValueError("sampledNegatives is not offered with candidate probabilities (candidateProbKey, cand_prob): the "
+                         "logQ correction of a mixed pool needs each sampled column's probability under both routes")
+    return int(sampledNegatives)
+
+
+class SampledNegatives:
+    """The sampler state of a model with sampledNegatives=M (brk_tt_sampled): the draws of the last training step (ids,
+    int32 [M]) and the device counter of training steps (step, int64 [1]).  Rows are drawn from [2, item_rows): never
+    StringLookup's mask row 0 or OOV row 1."""
+
+    def __init__(self, M, item_rows, seed, replica, device):
+        self.M, self.item_rows, self.seed, self.replica = int(M), int(item_rows), int(seed) & 0xFFFFFFFF, int(replica)
+        self.ids = torch.zeros(self.M, dtype=torch.int32, device=device)
+        self.step = torch.zeros(1, dtype=torch.int64, device=device)
+
+    def c_struct(self):
+        s = N.brk_tt_sampled()
+        s.ids, s.step, s.count = self.ids.data_ptr(), self.step.data_ptr(), self.M
+        s.lo, s.hi, s.rows = 2, self.item_rows, self.item_rows
+        s.seed, s.replica = self.seed, self.replica
+        return s
+
+
 class TwoTowerModel:
     def __init__(self, embedDim, nbrItem, nbrUser, userKey, itemKey, usersId, itemsId, eval_batch_size=8000,
                  loss=None, rdZero=False, resKey=None, semb=100, seed=42, device=None, tensor_cores=False,
-                 global_negatives=False, temperature=None, candidateProbKey=None, weightKey=None, streamingFrequency=None):
+                 global_negatives=False, temperature=None, candidateProbKey=None, weightKey=None, streamingFrequency=None,
+                 sampledNegatives=None):
+        # sampledNegatives=M: mixed negative sampling (Yang et al., WWW 2020) -- every training step draws M item rows
+        # uniformly from the catalog on the device and adds them as candidate columns shared by every row
+        # (brk_twotower_train_step_sampled); evaluation stays the in-batch loss
+        self.sampledNegatives = check_sampled_options(sampledNegatives, rdZero, global_negatives, streamingFrequency,
+                                                      candidateProbKey is not None)
         self.device = torch.device(device or f"cuda:{torch.cuda.current_device()}")
         self.embedDim, self.nbrItem, self.nbrUser = embedDim, nbrItem, nbrUser
         self.userKey, self.itemKey, self.resKey = userKey, itemKey, resKey
@@ -249,6 +294,8 @@ class TwoTowerModel:
         # streamingFrequency=alpha (True: 0.01) estimates the candidate probabilities on the device instead (Yi et al.,
         # RecSys 2019, Algorithm 2), with one slot per item-table row owned by the model
         self._configure_retrieval(temperature, candidateProbKey, weightKey, streamingFrequency, nbrItem + 2)
+        self._smp = SampledNegatives(self.sampledNegatives, nbrItem + 2, seed, D.rank(), self.device) \
+            if self.sampledNegatives else None
         self.userTowerIn = StringLookup(usersId)
         self.itemTowerIn = StringLookup(itemsId)
         rng = np.random.Generator(np.random.Philox(key=seed))
@@ -339,9 +386,10 @@ class TwoTowerModel:
         if B > self._ws_batch:
             dev, S = self.device, self.semb
             f = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=dev)
-            self._bufs = dict(eu=f(B, self.embedDim), ei=f(B, self.embedDim), deu=f(B, self.embedDim),
-                              dei=f(B, self.embedDim), q=f(B, S), c=f(B, S), dq=f(B, S),
-                              dc=f(B, S), scores=f(B, B) if not self.rdZero else None,
+            n = B + self.sampledNegatives                      # item-side rows: the batch's, then the sampled ones
+            self._bufs = dict(eu=f(B, self.embedDim), ei=f(n, self.embedDim), deu=f(B, self.embedDim),
+                              dei=f(n, self.embedDim), q=f(B, S), c=f(n, S), dq=f(B, S),
+                              dc=f(n, S), scores=f(B, n) if not self.rdZero else None,
                               ones=torch.ones(B, dtype=torch.float32, device=dev),
                               acc=torch.zeros(1, dtype=torch.float64, device=dev))
             self._ws_batch = B
@@ -356,9 +404,16 @@ class TwoTowerModel:
     def _step(self, u, i, labels, training, loss_out=None, extras=None):
         B = u.numel()
         loss_out = loss_out if loss_out is not None else torch.empty(1, dtype=torch.float32, device=self.device)
-        ws = self._workspace(B)
+        ws = self._workspace(max(B, 1))
         ut, it = self.userTower.c_struct(), self.itemTower.c_struct()
         rt = self._rt(extras)
+        if training and self._smp is not None:               # evaluation draws nothing: the in-batch loss below
+            smp = self._smp.c_struct()
+            N.check(N.lib().brk_twotower_step_sampled(N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), B,
+                                                      0x100 if self.tensor_cores else 0, C.byref(ws), N.ptr(loss_out),
+                                                      N.stream_ptr(), C.byref(smp), C.byref(rt) if rt is not None else None),
+                    "brk_twotower_step_sampled")
+            return loss_out
         if rt is not None:
             N.check(N.lib().brk_twotower_step_retrieval(N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), N.ptr(i),
                                                         None, B, 0x100 if self.tensor_cores else 0, 1 if training else 0,
@@ -431,6 +486,13 @@ class TwoTowerModel:
         ut, it = self.userTower.c_struct(), self.itemTower.c_struct()
         opt = self.optimizer
         rt = self._rt(extras)
+        if self._smp is not None:
+            smp = self._smp.c_struct()
+            N.check(N.lib().brk_twotower_train_step_sampled(
+                N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), B, 0x100 if self.tensor_cores else 0,
+                C.byref(ws), float(opt.lr), float(opt.eps), int(opt.rows_threshold_bytes), N.ptr(loss_out), N.stream_ptr(),
+                C.byref(smp), C.byref(rt) if rt is not None else None), "brk_twotower_train_step_sampled")
+            return loss_out
         if rt is not None:
             N.check(N.lib().brk_twotower_train_step_retrieval(
                 N.ctx(self.device), C.byref(ut), C.byref(it), N.ptr(u), N.ptr(i), N.ptr(i), None, B,
@@ -454,7 +516,7 @@ class TwoTowerModel:
             self._global.step(self.userTower.c_struct(), self.itemTower.c_struct(), lambda r: None,
                               {D.rank(): (u, i)}, split if split is not None else [u.numel()] * D.world_size(),
                               self.tensor_cores, loss)
-        elif u.numel() > 0:
+        elif u.numel() > 0 or self._smp is not None:          # an empty slice still draws: the counters stay in step
             loss = self._step(u, i, labels, True, loss_out, extras)
         else:                                                # this rank's slice of a small global batch is empty
             loss = loss_out if loss_out is not None else torch.zeros(1, dtype=torch.float32, device=self.device)

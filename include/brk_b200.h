@@ -509,6 +509,49 @@ typedef struct brk_tt_retrieval_sharded {
 } brk_tt_retrieval_sharded;
 int brk_tt_estimator_update_sharded(brk_ctx* ctx, const brk_tt_estimator_sharded* est, const int32_t* ids, int64_t n,
                                     float alpha, int64_t* step, void* stream);
+/* Mixed negative sampling (Yang et al., WWW 2020): each training step draws M item-table rows uniformly, with
+ * replacement, from [lo, hi) and adds them as candidate columns shared by every query row (TFRS Retrieval called with
+ * more candidates than queries).  The models draw from [2, numItem + 2): StringLookup's mask row 0 and OOV row 1 never.
+ *   Draw k (0 <= k < M) of step t for replica r: lo + ((w.x * (hi - lo)) >> 32) with w = Philox4x32-10 of counter
+ *     (k, uint32(t), uint32(t >> 32), 0x7E) and key (seed, r) (oracle/twotower_sampled.py).  t = *step + 1; the call
+ *     writes t back to *step on the device, so CUDA-graph replays draw fresh rows.  The draws go to ids[0..M).
+ *   Scores: c_all = item tower of concat(i, ids) (n = batch + M rows); logits Q c_all^T [batch, n] times inv_temperature;
+ *     the label of row b is column b; column j != b gets finfo(float32).min/100 added where its item row equals i[b]
+ *     (a sampled copy of the row's own positive is masked too); loss = sum_b w_b (logsumexp_j s_bj - s_bb) (SUM).
+ *   Gradients: dq = (P - Y) c_all, dc = (P - Y)^T Q over all n rows; the Dense gradient of the item tower covers the
+ *     sampled rows, and a sampled row gets its embedding gradient and touched bit like a batch row.
+ *   brk_twotower_step_sampled / brk_twotower_train_step_sampled: brk_twotower_step (training = 1) /
+ *     brk_twotower_train_step with sampled negatives; rt (optional) gives inv_temperature and row_weight only.
+ *   brk_twotower_step_sharded_sampled: brk_twotower_step_sharded with sampled negatives on this rank's slice (rows
+ *     gathered from and row gradients sent to their owners); rt (optional) gives inv_temperature and row_weight only.
+ *     Each replica passes its own counter and replica number (its rank), so each replica draws its own rows.
+ * With mode bit 0x100, widths <= 128 and max(T Tc, 2 (T + Tc)) <= SM count (T = ceil(batch / 128), Tc =
+ * ceil((batch + M) / 128)) the step (and for the train step Adagrad) is ONE cooperative launch (csrc/twotower_fused.cu),
+ * else the multi-kernel step; same results up to summation order and TF32 rounding.  Workspace as brk_twotower_step
+ * except the item side: ei / dei [batch + M, Ei], c / dc [batch + M, S], scores [batch, batch + M].  batch == 0 draws (the counter advances), writes 0 to
+ * loss_out and does nothing else.  Evaluation draws nothing: use brk_twotower_step(_retrieval) with training = 0.
+ * BRK_E_ARG as the calls they extend, and for: count < 1; [lo, hi) empty, lo < 0 or hi above rows (for the unsharded
+ * calls rows must also equal the item table's rows); a null step or ids; cand_prob, an estimator (last / est) or a
+ * non-finite or non-positive inv_temperature in rt; rdZero mode; batch * (batch + M) >= 2^31. */
+typedef struct brk_tt_sampled {
+  int32_t* ids;               /* [count] output: this step's draws */
+  int64_t* step;              /* device counter of training steps (initially 0) */
+  int64_t  count;             /* M >= 1 */
+  int64_t  lo, hi;            /* drawn from item-table rows [lo, hi) */
+  int64_t  rows;              /* rows of the (global) item table */
+  uint32_t seed, replica;
+} brk_tt_sampled;
+int brk_twotower_step_sampled(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                              const int32_t* i, int64_t batch, int32_t mode, const brk_twotower_workspace* ws,
+                              float* loss_out, void* stream, const brk_tt_sampled* smp, const brk_tt_retrieval* rt);
+int brk_twotower_train_step_sampled(brk_ctx* ctx, const brk_tower* user, const brk_tower* item, const int32_t* u,
+                                    const int32_t* i, int64_t batch, int32_t mode, const brk_twotower_workspace* ws,
+                                    float lr, float eps, int64_t rows_threshold_bytes, float* loss_out, void* stream,
+                                    const brk_tt_sampled* smp, const brk_tt_retrieval* rt);
+int brk_twotower_step_sharded_sampled(brk_ctx* ctx, const brk_tower* user, const brk_tower* item,
+                                      const brk_twotower_shards* sh, const int32_t* u, const int32_t* i, int64_t batch,
+                                      int32_t mode, const brk_twotower_workspace* ws, float* loss_out, void* stream,
+                                      const brk_tt_sampled* smp, const brk_tt_retrieval_sharded* rt);
 int brk_twotower_step_sharded_retrieval(brk_ctx* ctx, const brk_tower* user, const brk_tower* item,
                                         const brk_twotower_shards* sh, const int32_t* u, const int32_t* i,
                                         const int32_t* cand_ids, const float* labels, int64_t batch, int32_t mode,
