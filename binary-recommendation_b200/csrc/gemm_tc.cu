@@ -38,7 +38,7 @@ struct Params {
   unsigned long long* trace;   // optional [8] globaltimer stamps of CTA 0 (brk_gemm_tf32_trace), else null
 };
 __device__ __forceinline__ void stamp(const Params& P, int k) {
-  if (P.trace && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 0) {
+  if (P.trace && blockIdx.x == 0 && blockIdx.z == 0 && threadIdx.x == 0) {
     unsigned long long t;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
     P.trace[k] = t;
@@ -89,7 +89,8 @@ __global__ void __launch_bounds__(NT) gemm_tf32_kernel(const Params P) {
   __shared__ uint32_t tmem_slot;
   constexpr int TCOLS = BN < 32 ? 32 : BN;
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  const int m0 = blockIdx.y * BM, n0 = blockIdx.x * BN;
+  const unsigned col_tiles = unsigned(P.N + BN - 1) / BN;      // grid x = row tile * col_tiles + column tile
+  const int m0 = int(blockIdx.x / col_tiles) * BM, n0 = int(blockIdx.x % col_tiles) * BN;
   const int kbeg = blockIdx.z * P.k_per_split;
   const int kend = min(P.K, kbeg + P.k_per_split);
   const int m_end = P.M, n_end = P.N;
@@ -210,7 +211,8 @@ int launch(brk_ctx* ctx, const Params& P, int splits, cudaStream_t st) {
   const size_t smem = (pipe > stagec ? pipe : stagec) + 1024;
   // the shared-memory opt-in is per device: set it for the current one on every call
   BRK_CUDA(cudaFuncSetAttribute(gemm_tf32_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  dim3 grid((P.N + BN - 1) / BN, (P.M + BM - 1) / BM, splits);
+  // row and column tiles both on x: gridDim.y would cap M at 65535 row tiles
+  dim3 grid(unsigned((P.N + BN - 1) / BN) * unsigned((P.M + BM - 1) / BM), 1, splits);
   gemm_tf32_kernel<BN, A_MN, B_MN><<<grid, NT, smem, st>>>(P);
   BRK_LAUNCH_CHECK();
   (void)ctx;
@@ -270,6 +272,9 @@ extern "C" int brk_gemm_tf32(brk_ctx* ctx, const float* A, const float* B, float
                              int32_t accumulate, void* stream) {
   BRK_REQUIRE(ctx && A && B && C, BRK_E_ARG, "brk_gemm_tf32: null argument");
   BRK_REQUIRE(M > 0 && N > 0 && K > 0, BRK_E_ARG, "brk_gemm_tf32: M=%d N=%d K=%d", M, N, K);
+  BRK_REQUIRE(lda >= (trans_a ? M : K) && ldb >= (trans_b ? K : N) && ldc >= N, BRK_E_ARG,
+              "brk_gemm_tf32: lda=%d ldb=%d ldc=%d below the stored row length (M=%d N=%d K=%d trans_a=%d trans_b=%d)", lda,
+              ldb, ldc, M, N, K, trans_a, trans_b);
   return brk_gemm_tf32_impl(ctx, A, B, C, bias, M, N, K, lda, ldb, ldc, trans_a, trans_b, alpha, accumulate, true,
                             (cudaStream_t)stream);
 }
@@ -281,6 +286,9 @@ extern "C" int brk_gemm_tf32_trace(brk_ctx* ctx, const float* A, const float* B,
                                    int32_t trans_b, float alpha, int32_t accumulate, uint64_t* trace, void* stream) {
   BRK_REQUIRE(ctx && A && B && C && trace, BRK_E_ARG, "brk_gemm_tf32_trace: null argument");
   BRK_REQUIRE(M > 0 && N > 0 && K > 0, BRK_E_ARG, "brk_gemm_tf32_trace: M=%d N=%d K=%d", M, N, K);
+  BRK_REQUIRE(lda >= (trans_a ? M : K) && ldb >= (trans_b ? K : N) && ldc >= N, BRK_E_ARG,
+              "brk_gemm_tf32_trace: lda=%d ldb=%d ldc=%d below the stored row length (M=%d N=%d K=%d trans_a=%d trans_b=%d)", lda,
+              ldb, ldc, M, N, K, trans_a, trans_b);
   return gemm_tf32_run(ctx, A, B, C, bias, M, N, K, lda, ldb, ldc, trans_a, trans_b, alpha, accumulate, true,
                        (cudaStream_t)stream, reinterpret_cast<unsigned long long*>(trace));
 }

@@ -23,6 +23,7 @@ constexpr int TM = 64, TN = 64, TK = 16, kGemmThreads = 256;
 //   ta == 0: A is [M,K] row-major (lda = K-stride);  ta == 1: A is stored [K,M] (A^T used)
 //   tb == 0: B is [K,N] row-major;                    tb == 1: B is stored [N,K]
 //   accumulate != 0: C += (RED.ADD when split-K > 1, plain += otherwise); bias added by split 0 only
+//   grid: x = row tile * column tiles + column tile (gridDim.y would cap M at 65535 row tiles), z = K split
 __global__ void __launch_bounds__(kGemmThreads)
 sgemm_kernel(const float* __restrict__ A, const float* __restrict__ Bm, float* __restrict__ C,
              const float* __restrict__ bias, int M, int N, int K, int lda, int ldb, int ldc, int ta, int tb,
@@ -30,7 +31,8 @@ sgemm_kernel(const float* __restrict__ A, const float* __restrict__ Bm, float* _
   __shared__ __align__(16) float As[TK][TM + 4];
   __shared__ __align__(16) float Bs[TK][TN + 4];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;       // 16 x 16 threads, 4x4 outputs each
-  const int m0 = blockIdx.y * TM, n0 = blockIdx.x * TN;
+  const unsigned col_tiles = unsigned(N + TN - 1) / TN;
+  const int m0 = int(blockIdx.x / col_tiles) * TM, n0 = int(blockIdx.x % col_tiles) * TN;
   const int kbeg = blockIdx.z * k_per_split, kend = min(K, kbeg + k_per_split);
   float acc[4][4] = {};
   for (int k0 = kbeg; k0 < kend; k0 += TK) {
@@ -96,20 +98,29 @@ int sgemm(brk_ctx* ctx, cudaStream_t st, const float* A, const float* B, float* 
   }
   int kps = ((K + splits - 1) / splits + TK - 1) / TK * TK;
   splits = (K + kps - 1) / kps;
-  sgemm_kernel<<<dim3(gx, gy, splits), kGemmThreads, 0, st>>>(A, B, C, bias, M, N, K, lda, ldb, ldc, ta, tb, alpha,
-                                                              accumulate, kps);
+  sgemm_kernel<<<dim3(unsigned(gx) * unsigned(gy), 1, splits), kGemmThreads, 0, st>>>(A, B, C, bias, M, N, K, lda, ldb, ldc,
+                                                                                      ta, tb, alpha, accumulate, kps);
   BRK_LAUNCH_CHECK();
   return 0;
 }
 
-// out[n] += sum_m X[m][n]: bias gradients (ones^T dz) without a degenerate M = 1 product
+// out[n] += sum_m X[m][n]: bias gradients (ones^T dz) without a degenerate M = 1 product.  A block sums the 64-row chunks
+// blockIdx.y, blockIdx.y + gridDim.y, ... and adds its sum once; gridDim.y is capped at 65535, below which a block has
+// one chunk.
 __global__ void __launch_bounds__(128) colsum_kernel(const float* __restrict__ X, int M, int N, int ld, float* __restrict__ out) {
   const int n = blockIdx.x * 128 + threadIdx.x;
-  const int m0 = blockIdx.y * 64, m1 = min(M, m0 + 64);
   if (n >= N) return;
   float s = 0.f;
-  for (int m = m0; m < m1; ++m) s += __ldg(X + int64_t(m) * ld + n);
+  for (int64_t m0 = int64_t(blockIdx.y) * 64; m0 < M; m0 += int64_t(gridDim.y) * 64)
+    for (int m = int(m0), m1 = int(min(int64_t(M), m0 + 64)); m < m1; ++m) s += __ldg(X + int64_t(m) * ld + n);
   atomicAdd(out + n, s);
+}
+
+int colsum(cudaStream_t st, const float* X, int M, int N, float* out) {
+  const int chunks = (M + 63) / 64;
+  colsum_kernel<<<dim3((N + 127) / 128, chunks < 65535 ? chunks : 65535), 128, 0, st>>>(X, M, N, N, out);
+  BRK_LAUNCH_CHECK();
+  return 0;
 }
 
 }  // namespace
@@ -365,6 +376,9 @@ extern "C" int brk_sgemm(brk_ctx* ctx, const float* A, const float* B, float* C,
                          float alpha, int32_t accumulate, void* stream) {
   BRK_REQUIRE(ctx && A && B && C, BRK_E_ARG, "brk_sgemm: null argument");
   BRK_REQUIRE(M > 0 && N > 0 && K > 0, BRK_E_ARG, "brk_sgemm: M=%d N=%d K=%d", M, N, K);
+  BRK_REQUIRE(lda >= (trans_a ? M : K) && ldb >= (trans_b ? K : N) && ldc >= N, BRK_E_ARG,
+              "brk_sgemm: lda=%d ldb=%d ldc=%d below the stored row length (M=%d N=%d K=%d trans_a=%d trans_b=%d)", lda, ldb,
+              ldc, M, N, K, trans_a, trans_b);
   return sgemm(ctx, (cudaStream_t)stream, A, B, C, bias, M, N, K, lda, ldb, ldc, trans_a, trans_b, alpha, accumulate,
                true);
 }
@@ -522,8 +536,7 @@ static int twotower_step(brk_ctx* ctx, const brk_tower* user, const brk_tower* i
     float* gW = tw[k]->dense.g;
     float* gb = gW + int64_t(E[k]) * S;
     if ((rc = gemm(ctx, sd, tcore, e[k], dz[k], gW, nullptr, E[k], S, R, E[k], S, S, 1, 0, 1.f, 1, true))) return rc;
-    colsum_kernel<<<dim3((S + 127) / 128, (R + 63) / 64), 128, 0, sd>>>(dz[k], R, S, S, gb);
-    BRK_LAUNCH_CHECK();
+    if ((rc = colsum(sd, dz[k], R, S, gb))) return rc;
     if (k == 0) {                                  // the loss scalar rides on the user tower's side stream
       finish_loss_kernel<<<1, 1, 0, sd>>>(ws->acc, loss_out);
       BRK_LAUNCH_CHECK();
@@ -777,11 +790,7 @@ int brk_tt_tower_forward(brk_ctx* ctx, const brk_tower* t, const int32_t* ids, i
                          cudaStream_t st, const brk_shards* sh) {
   return tower_forward(ctx, t, ids, n, emb_out, out, tcore, st, sh);
 }
-int brk_tt_colsum(cudaStream_t st, const float* X, int M, int N, float* out) {
-  colsum_kernel<<<dim3((N + 127) / 128, (M + 63) / 64), 128, 0, st>>>(X, M, N, N, out);
-  BRK_LAUNCH_CHECK();
-  return 0;
-}
+int brk_tt_colsum(cudaStream_t st, const float* X, int M, int N, float* out) { return colsum(st, X, M, N, out); }
 int brk_tt_check_shards(const brk_shards* s, int32_t E, const char* which, const char* fn) {
   return check_shards(s, E, which, fn);
 }

@@ -375,8 +375,14 @@ int brk_bpr_train_steps_dp(brk_ctx* ctx, const brk_table* user, const brk_table*
  * Inside the call the item-tower chain and the two Dense-gradient chains run on streams owned by the context,
  * forked from and joined back into `stream` (under stream capture they become branches of the graph).
  *   brk_sgemm : C (+)= alpha opA(A) opB(B) (+ bias); trans_a: A stored [K,M]; trans_b: B stored [N,K]; fp32 FMA.
+ *     lda >= (trans_a ? M : K), ldb >= (trans_b ? K : N) and ldc >= N, else BRK_E_ARG before any launch; only
+ *     C[0:M, 0:N] is written, for any M and N up to 2^31 - 1.  accumulate = 0 never splits K: row r of C is the same
+ *     bits whatever M is and whichever other rows share the call (the item-range top-K indexes are bit-equal to the
+ *     whole-catalog index only so).  accumulate != 0 may split K over CTAs that add into C with REDs, the bias once.
  *   brk_gemm_tf32 : the same product on tcgen05 with TF32 operands and fp32 accumulation in TMEM (gemm_tc.cu);
- *     needs 16-byte aligned operands with leading dimensions that are multiples of 4 (else BRK_E_ALIGN).
+ *     needs 16-byte aligned operands with leading dimensions that are multiples of 4 (else BRK_E_ALIGN).  The same
+ *     leading-dimension minimums and the same row guarantee: the tile width it picks from M, N and the SM count does
+ *     not change a row's bits (tests/test_gpu_dense_products.py).
  *   brk_twotower_step mode bit 0x100 routes every Dense / in-batch product through brk_gemm_tf32 (falling back to
  *     the fp32 product where the alignment rule fails); results then agree with the fp32 path to TF32 rounding. */
 typedef struct brk_tower {
